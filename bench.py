@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA engine
     python bench.py --impl reference [--gpus N] [--steps K] ...     # the reference itself on the host CPU cores
+    python bench.py ... --dump-outputs DIR                           # also save the headline leg's results as .npy
 
 One "step" = one pass of the hot path over one batch of synthetic input: ONE rollout call that advances every vehicle
 of the ensemble by 1000 RK4 steps (configs[1]; 100 for configs[2], whose snapshots are written every 10 steps).  The
@@ -242,6 +243,15 @@ def measured_peaks():
     return {"hbm_gbs": 6650.0}, "fallback (B200_PROFILING.md)"
 
 
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Writes the headline leg's final results as <path>/<name>.npy in float64 (rank 0's shard: 65,536 vehicles,
+    xT [N,12] and the allocation-projected lag [N,18], 15.7 MB).  x0 and the command stream are seeded, so two builds
+    run with the same arguments can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.double().cpu().numpy())
+
+
 def timed(torch, dist, world, dev, fn, warmup, steps, windows):
     """W untimed calls, then K timed ones between CUDA events on the launching stream, barrier + synchronize on both
     sides, max over ranks."""
@@ -296,6 +306,7 @@ def run_rollout_legs(torch, dist, B, cfg, steps, warmup, rank, local, world, win
                                      xT_out=x, lag_out=lag, traj_out=traj[k % 2] if stride else None, lag_repr="projected"),
                warmup, steps, windows)
     out["streamed"] = dict(ms_total=ms, ms_per_step=ms / steps, finite=bool(torch.isfinite(x).all().item()))
+    out["outputs"] = {"xT": x, "lag": lag}     # what the last timed call returned (it writes in place)
     # --- generated in the kernel: every step of every launch is a distinct step of the stream
     x, lag = fresh()
     gst = torch.zeros((n, 8), device=eng.device, dtype=eng.tdtype)
@@ -625,12 +636,14 @@ def main_ours(args):
     fp32_peak, _ = B.fma_peak("f32", local, 8192)
 
     leg2 = run_rollout_legs(torch, dist, B, CFG2, args.steps, args.warmup, rank, local, world, windows, default_api=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, leg2["outputs"])
     e2e = run_e2e_legs(torch, dist, B, CFG2, leg2, min(args.steps, args.e2e_steps), args.warmup, world, windows)
-    for k in ("U", "x0", "eng", "gen"):
+    for k in ("U", "x0", "eng", "gen", "outputs"):
         leg2.pop(k)
     torch.cuda.empty_cache()
     leg3 = run_rollout_legs(torch, dist, B, CFG3, args.steps, args.warmup, rank, local, world, windows)
-    for k in ("U", "x0", "eng", "gen"):
+    for k in ("U", "x0", "eng", "gen", "outputs"):
         leg3.pop(k)
     torch.cuda.empty_cache()
     rmse = run_rmse_leg(torch, dist, B, local, rank, world, windows, fp64_peak) if not args.no_rmse else None
@@ -763,7 +776,11 @@ if __name__ == "__main__":
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-rmse", action="store_true")
     ap.add_argument("--no-compare", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the final state and lag of the headline leg's last timed step to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs saves the CUDA engine's results; the reference arm has none to save")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":
         main_reference(a)

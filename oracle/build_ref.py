@@ -25,8 +25,9 @@ FILES = ["fossen/__init__.py", "fossen/BlueROV2.py", "fossen/BlueROV2_thrust.py"
 
 def build() -> bool:
     if not os.path.isdir(REF):
+        # no copy of the reference here: nothing to build, which is not an error (the live-reference tests skip)
         print(f"[build_ref] {REF} not present: keeping whatever oracle/_ref holds")
-        return os.path.isdir(OUT)
+        return True
     shutil.rmtree(OUT, ignore_errors=True)
     for rel in FILES:
         src = os.path.join(REF, rel)

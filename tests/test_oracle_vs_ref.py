@@ -1,7 +1,7 @@
 """The CPU oracles against the UNMODIFIED reference executed live from oracle/_ref/ (byte-compiled by
-oracle/build_ref.py from /root/reference; present in the build container and on the GPU box, skipped elsewhere):
-fresh seeded inputs every run of the suite would be pointless, so the seeds are fixed — what this adds to the frozen
-golden files is that the comparison runs against the reference ITSELF wherever the suite runs."""
+oracle/build_ref.py from a copy of the reference project, which the repository does not contain; skipped where
+oracle/_ref is not built): fresh seeded inputs every run of the suite would be pointless, so the seeds are fixed — what
+this adds to the frozen golden files is that the comparison runs against the reference ITSELF wherever it is built."""
 import numpy as np
 import pytest
 
@@ -10,7 +10,7 @@ from oracle import fossen_np as O
 from oracle import ref_loader as RL
 from conftest import normwise
 
-pytestmark = [pytest.mark.skipif(not RL.available(), reason="oracle/_ref not built (needs /root/reference once)"),
+pytestmark = [pytest.mark.skipif(not RL.available(), reason="oracle/_ref not built (oracle/build_ref.py needs a copy of the reference project)"),
               pytest.mark.filterwarnings("ignore")]
 DT = 0.02
 
