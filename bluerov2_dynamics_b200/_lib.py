@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("BROV_LIB") or os.path.join(_HERE, "libbrov.so")  # BROV_LIB: a tuning variant
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 THRUSTER8_LAG3, WRENCH_EULER12, WRENCH_QUAT13 = 0, 1, 2
 DI_EULER12_U8, DI_EULER12_U6, DI_QUAT13_U6 = 3, 4, 5
 F64, F32 = 0, 1
@@ -57,6 +57,17 @@ class SeDesc(C.Structure):
                 ("workspace_bytes", C.c_size_t), ("lag_carry", C.c_int32), ("time_slices", C.c_int32),
                 ("window0", C.c_longlong), ("row0", C.c_longlong), ("health_dev", C.c_void_p),
                 ("singular_eps", C.c_double)]
+
+
+class SeSweepDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("rows", C.c_longlong),
+                ("n_windows", C.c_longlong), ("dt", C.c_double), ("X_dev", C.c_void_p), ("U_dev", C.c_void_p),
+                ("lag0_dev", C.c_void_p), ("n_horizons", C.c_int32), ("horizons", C.c_int32 * MAX_H),
+                ("lag_carry", C.c_int32), ("window0", C.c_longlong), ("row0", C.c_longlong),
+                ("n_candidates", C.c_longlong), ("kp_soa_dev", C.c_void_p), ("any_current", C.c_int32),
+                ("reserved", C.c_int32), ("se_out_dev", C.c_void_p), ("count_out", C.POINTER(C.c_longlong)),
+                ("health_dev", C.c_void_p), ("singular_eps", C.c_double), ("workspace_dev", C.c_void_p),
+                ("workspace_bytes", C.c_size_t)]
 
 
 class RolloutHostDesc(C.Structure):
@@ -116,6 +127,8 @@ _PROTOS = {
     "brov_se_workspace_bytes": (C.c_size_t, [C.c_longlong]),
     "brov_multistep_se": (C.c_int, [C.c_void_p, C.POINTER(SeDesc), C.c_void_p]),
     "brov_se_carry_steps": (C.c_int, [C.c_void_p, C.c_double, C.c_int, C.POINTER(C.c_longlong)]),
+    "brov_se_sweep_workspace_bytes": (C.c_size_t, [C.c_longlong, C.c_longlong, C.c_int]),
+    "brov_multistep_se_sweep": (C.c_int, [C.c_void_p, C.POINTER(SeSweepDesc), C.c_void_p]),
     "brov_reduced9_rhs": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "brov_koopman_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_void_p)]),
     "brov_koopman_destroy": (None, [C.c_void_p]),

@@ -911,6 +911,30 @@ extern "C" size_t brov_se_workspace_bytes(long long n_windows) {
            se_align((size_t)n_windows * 18 * sizeof(double)) + 2 * se_align((size_t)n_windows * 4);
 }
 
+// Windows per thread of a carried-lag pass: the replay (m lag-only steps, each about a fifth of a full step: 152 of 838
+// FP64 operations) is paid once per wpt windows of H steps each; more windows per thread mean fewer threads — pick the
+// count that minimises rounds x work per thread (any count up to 64, not only powers of two: with 1M windows of
+// H = 100, wpt = 7 fills 3.77 -> 4 rounds, wpt = 4 fills 6.6 -> 7)
+static int carry_wpt(const brov_engine* e, long long n_windows, long long H, long long m) {
+    const double slots = 2.0 * e->num_sms * ROLLOUT_BLOCK * (e->dtype == BROV_F32 ? 2.0 : 1.0);
+    double best = 1e300;
+    int wpt = 1;
+    for (int w = 1; w <= 64; ++w) {
+        const double threads = std::ceil((double)n_windows / w);
+        const double cost = std::ceil(threads / slots) * ((double)w * (double)H + 0.2 * (double)m);
+        if (cost < best * 0.98) { best = cost; wpt = w; }
+    }
+    return wpt;
+}
+// the replay of window0's history reads input rows back to window (window0 * H - m) / H: they must be local
+static int check_carry_rows(long long window0, long long row0, long long H, long long m) {
+    const long long first_hist = window0 * H - m;
+    const long long need_row = first_hist > 0 ? first_hist / H : 0;
+    if (row0 > need_row)
+        return fail(BROV_EINVAL, "lag_carry: the shard must start at row %lld or earlier (row0 = %lld): window %lld replays %lld steps of history", need_row, row0, window0, m);
+    return BROV_OK;
+}
+
 template <typename T>
 static int se_impl(brov_engine* e, const brov_se_desc* d, cudaStream_t st) {
     SeArgs<T> a;
@@ -925,26 +949,8 @@ static int se_impl(brov_engine* e, const brov_se_desc* d, cudaStream_t st) {
         long long m = 0;
         if ((rc = carry_depth(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &m))) return rc;
         a.carry_steps = (int)m;
-        // windows per thread: the replay (m lag-only steps, each about a fifth of a full step: 152 of 838 FP64
-        // operations) is paid once per wpt windows of H steps each; more windows per thread mean fewer threads —
-        // pick the count that minimises rounds x work per thread (any count up to 64, not only powers of two: with
-        // 1M windows of H = 100, wpt = 7 fills 3.77 -> 4 rounds, wpt = 4 fills 6.6 -> 7)
-        {
-            const long long H = d->horizons[0];
-            const double slots = 2.0 * e->num_sms * ROLLOUT_BLOCK * (e->dtype == BROV_F32 ? 2.0 : 1.0);
-            double best = 1e300;
-            for (int w = 1; w <= 64; ++w) {
-                const double threads = std::ceil((double)d->n_windows / w);
-                const double cost = std::ceil(threads / slots) * ((double)w * (double)H + 0.2 * (double)m);
-                if (cost < best * 0.98) { best = cost; a.wpt = w; }
-            }
-        }
-        // the replay of window0's history reads input rows back to window (window0 * H - m) / H: they must be local
-        const long long H = d->horizons[0];
-        const long long first_hist = d->window0 * H - m;
-        const long long need_row = first_hist > 0 ? first_hist / H : 0;
-        if (d->row0 > need_row)
-            return fail(BROV_EINVAL, "lag_carry: the shard must start at row %lld or earlier (row0 = %lld): window %lld replays %lld steps of history", need_row, d->row0, d->window0, m);
+        a.wpt = carry_wpt(e, d->n_windows, d->horizons[0], m);
+        if ((rc = check_carry_rows(d->window0, d->row0, d->horizons[0], m))) return rc;
     }
     a.health.counters = (unsigned long long*)d->health_dev;
     a.health.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
@@ -981,12 +987,9 @@ static int se_impl(brov_engine* e, const brov_se_desc* d, cudaStream_t st) {
     return BROV_OK;
 }
 
-extern "C" int brov_multistep_se(brov_engine_t* e, const brov_se_desc* d, void* stream) {
-    if (!e) return fail(BROV_EINVAL, "NULL engine");
-    if (!d || d->struct_size != sizeof(brov_se_desc)) return fail(BROV_EINVAL, "brov_se_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+// argument checks of the sliding-window geometry shared by brov_multistep_se and brov_multistep_se_sweep
+template <class D> static int check_se_geometry(const D* d) {
     if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
-    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "the evaluator does not support the first-order wrench lag");
-    if (e->pv) return fail(BROV_EUNSUPPORTED, "the evaluator scores one vehicle; clear the per-vehicle table first");
     if (d->n_horizons < 1 || d->n_horizons > MAX_H) return fail(BROV_EINVAL, "n_horizons must be 1..%d", MAX_H);
     if (d->lag_carry && (d->n_horizons != 1 || d->lag0_dev)) return fail(BROV_EINVAL, "lag_carry scores one horizon per call and excludes lag0");
     if (d->window0 < 0 || d->row0 < 0 || d->row0 > d->window0) return fail(BROV_EINVAL, "window0 / row0 out of range");
@@ -998,8 +1001,10 @@ extern "C" int brov_multistep_se(brov_engine_t* e, const brov_se_desc* d, void* 
     if (d->n_windows + (d->window0 - d->row0) > d->rows)
         return fail(BROV_EINVAL, "n_windows = %lld starting at local row %lld exceed the %lld rows of the series", d->n_windows, d->window0 - d->row0, d->rows);
     if (!(d->dt > 0.0)) return fail(BROV_EINVAL, "dt must be > 0");
-    if (!d->se_out_dev) return fail(BROV_EINVAL, "se_out is NULL");
-    CUDA_TRY(cudaSetDevice(e->device));
+    return BROV_OK;
+}
+// count_out (host, may be NULL): the number of windows that reach each horizon
+template <class D> static void se_counts(const D* d) {
     for (int h = 0; h < MAX_H; ++h) {
         long long cnt = 0;
         if (h < d->n_horizons) {
@@ -1009,6 +1014,19 @@ extern "C" int brov_multistep_se(brov_engine_t* e, const brov_se_desc* d, void* 
         }
         if (d->count_out) d->count_out[h] = cnt;
     }
+}
+
+extern "C" int brov_multistep_se(brov_engine_t* e, const brov_se_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_se_desc)) return fail(BROV_EINVAL, "brov_se_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "the evaluator does not support the first-order wrench lag");
+    if (e->pv) return fail(BROV_EUNSUPPORTED, "the evaluator scores one vehicle; clear the per-vehicle table first");
+    int rc = check_se_geometry(d);
+    if (rc) return rc;
+    if (!d->se_out_dev) return fail(BROV_EINVAL, "se_out is NULL");
+    CUDA_TRY(cudaSetDevice(e->device));
+    se_counts(d);
     if (d->n_windows == 0 || d->rows < 2) {
         CUDA_TRY(cudaMemsetAsync(d->se_out_dev, 0, MAX_H * sizeof(double), (cudaStream_t)stream));
         if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), (cudaStream_t)stream));
@@ -1018,6 +1036,86 @@ extern "C" int brov_multistep_se(brov_engine_t* e, const brov_se_desc* d, void* 
     if (d->time_slices < 0 || d->time_slices > SE_MAX_QUANTA) return fail(BROV_EINVAL, "time_slices must be 0 (automatic) .. %d", SE_MAX_QUANTA);
     if (!d->workspace_dev || d->workspace_bytes < brov_se_workspace_bytes(d->n_windows)) return fail(BROV_EINVAL, "workspace too small: need %zu bytes", brov_se_workspace_bytes(d->n_windows));
     return e->dtype == BROV_F32 ? se_impl<float>(e, d, (cudaStream_t)stream) : se_impl<double>(e, d, (cudaStream_t)stream);
+}
+
+// sweep workspace: per-candidate partial sums [P][window blocks][MAX_H], then (carry mode) the lag each window inherits
+// [n_windows][18] (sized for fp64 whatever the engine's scalar type)
+static size_t sweep_partial_bytes(long long n_candidates, long long n_windows) {
+    return se_align((size_t)n_candidates * (size_t)((n_windows + ROLLOUT_BLOCK - 1) / ROLLOUT_BLOCK) * MAX_H * sizeof(double));
+}
+extern "C" size_t brov_se_sweep_workspace_bytes(long long n_candidates, long long n_windows, int lag_carry) {
+    if (n_candidates < 0) n_candidates = 0;
+    if (n_windows < 0) n_windows = 0;
+    return sweep_partial_bytes(n_candidates, n_windows) + (lag_carry ? se_align((size_t)n_windows * 18 * sizeof(double)) : 0);
+}
+
+template <typename T>
+static int se_sweep_impl(brov_engine* e, const brov_se_sweep_desc* d, cudaStream_t st) {
+    SweepArgs<T> a;
+    memset(&a, 0, sizeof(a));
+    const int nsub = d->integrator == BROV_RK4 ? 4 : 1;
+    int rc = make_consts<T>(e, d->dt, nsub, &a.c);
+    if (rc) return rc;
+    a.c.has_current = d->any_current ? 1 : 0;   // the candidates' currents, not the engine's
+    a.X = (const T*)d->X_dev; a.U = (const T*)d->U_dev;
+    a.kp = (const T*)d->kp_soa_dev;
+    a.partial = (double*)d->workspace_dev;
+    a.health = (unsigned long long*)d->health_dev;
+    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    a.off = d->window0 - d->row0;
+    a.rows = (int)d->rows; a.nwin = (int)d->n_windows; a.nH = d->n_horizons;
+    for (int h = 0; h < MAX_H; ++h) a.H[h] = h < d->n_horizons ? d->horizons[h] : 0x7fffffff;
+    a.P = (int)d->n_candidates;
+    a.nwb = se_blocks<T>(a.nwin);
+    a.lag0 = (const T*)d->lag0_dev;
+    a.lag0_w = 0;
+    if (d->lag_carry && e->model == BROV_THRUSTER8_LAG3) {
+        long long m = 0;
+        if ((rc = carry_depth(e, d->dt, nsub, &m))) return rc;
+        if ((rc = check_carry_rows(d->window0, d->row0, d->horizons[0], m))) return rc;
+        CarryLagArgs<T> c;
+        memset(&c, 0, sizeof(c));
+        c.c = a.c;
+        c.U = a.U;
+        c.lag_out = (T*)((unsigned char*)d->workspace_dev + sweep_partial_bytes(d->n_candidates, d->n_windows));
+        c.win0 = d->window0; c.row0 = d->row0;
+        c.rows = a.rows; c.nwin = a.nwin; c.H = d->horizons[0]; c.carry_steps = (int)m;
+        c.wpt = carry_wpt(e, d->n_windows, d->horizons[0], m);
+        CUDA_TRY(launch_se_carry_lag<T>(c, st));
+        a.lag0 = c.lag_out;
+        a.lag0_w = 1;
+    }
+    if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, (size_t)d->n_candidates * 2 * sizeof(unsigned long long), st));
+    CUDA_TRY(launch_se_sweep<T>(e->model, d->integrator, a, d->se_out_dev, st));
+    return BROV_OK;
+}
+
+extern "C" int brov_multistep_se_sweep(brov_engine_t* e, const brov_se_sweep_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_se_sweep_desc)) return fail(BROV_EINVAL, "brov_se_sweep_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "the sweep serves the Fossen models; double-integrator engines have no coefficient table");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "the evaluator does not support the first-order wrench lag");
+    int rc = check_se_geometry(d);
+    if (rc) return rc;
+    if (d->n_candidates < 0) return fail(BROV_EINVAL, "n_candidates = %lld", d->n_candidates);
+    const long long nwb = (d->n_windows + ROLLOUT_BLOCK - 1) / ROLLOUT_BLOCK;
+    if (d->n_candidates * nwb > 0x7fffffffLL)
+        return fail(BROV_EINVAL, "%lld candidates x %lld window blocks exceed 2^31 - 1 blocks: split the candidates over several calls", d->n_candidates, nwb);
+    se_counts(d);
+    if (d->n_candidates == 0) return BROV_OK;
+    if (!d->se_out_dev) return fail(BROV_EINVAL, "se_out is NULL");
+    CUDA_TRY(cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d->n_windows == 0 || d->rows < 2) {
+        CUDA_TRY(cudaMemsetAsync(d->se_out_dev, 0, (size_t)d->n_candidates * MAX_H * sizeof(double), st));
+        if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, (size_t)d->n_candidates * 2 * sizeof(unsigned long long), st));
+        return BROV_OK;
+    }
+    if (!d->X_dev || !d->U_dev) return fail(BROV_EINVAL, "X and U must not be NULL");
+    if (!d->kp_soa_dev) return fail(BROV_EINVAL, "kp_soa is NULL");
+    const size_t need = brov_se_sweep_workspace_bytes(d->n_candidates, d->n_windows, d->lag_carry && e->model == BROV_THRUSTER8_LAG3);
+    if (!d->workspace_dev || d->workspace_bytes < need) return fail(BROV_EINVAL, "workspace too small: need %zu bytes", need);
+    return e->dtype == BROV_F32 ? se_sweep_impl<float>(e, d, st) : se_sweep_impl<double>(e, d, st);
 }
 
 // fossen/parameters.py:3-33

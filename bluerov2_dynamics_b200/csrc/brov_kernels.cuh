@@ -835,6 +835,211 @@ static __global__ void __launch_bounds__(256) se_finish_kernel(const double* __r
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// candidate sweep: the endpoint squared error of P coefficient sets against ONE recorded series in one launch
+// (calibration, sensitivity studies, scoring a Monte-Carlo cloud of vehicles).  A block is one item (candidate c,
+// window block wb of ROLLOUT_BLOCK consecutive windows); its body is se_kernel's reset mode with one window per
+// thread, so a candidate's sums equal those of brov_multistep_se(time_slices = 1) with that candidate's coefficients.
+// ---------------------------------------------------------------------------------------------------------------
+template <typename T> struct SweepArgs {
+    Consts<T> c;        // engine constants (allocation, lag discretisation, dt, has_current); c.kp is not read
+    const T* X;         // [rows][NX]
+    const T* U;         // [rows][NU]
+    const T* kp;        // [KP_COUNT][P] candidate coefficient table
+    const T* lag0;      // per-window initial lag or nullptr (zeros): [nwin][24] (projected on load) or [nwin][18]
+    int lag0_w;         // lag0 holds allocation-projected states [nwin][18] (carry mode: se_carry_lag_kernel's output)
+    double* partial;    // [P][nwb][MAX_H]
+    unsigned long long* health;   // [P][2] (non-finite, near-singular windows) or nullptr; zeroed before the launch
+    double eps;
+    long long off;      // local row of window 0 (window0 - row0)
+    int rows, nwin, nH;
+    int H[MAX_H];       // ascending
+    int P, nwb;         // candidates, window blocks
+};
+
+// Item order: window-block-major (item = wb * P + c): the blocks resident at one time read the same few X / U rows,
+// which L2 serves to all candidates.  Candidate-major (item = c * nwb + wb, BROV_SWEEP_CAND_MAJOR=1) measured the same
+// on B200 within run-to-run noise (profiles/sweep_timing*.json: the build timed second was 2 % faster on the 1M-row
+// series whichever order it had).
+#ifndef BROV_SWEEP_CAND_MAJOR
+#define BROV_SWEEP_CAND_MAJOR 0
+#endif
+// Candidate coefficients: staged once per block into shared memory and read as broadcasts (ParamsShared, pitch 1), so
+// the kernel holds no per-thread table.  fp32 copies in registers (ParamsRegs, as the fp32 Monte-Carlo rollout does;
+// BROV_SWEEP_KP_REGS=1) measured the same within noise and take a larger stack frame (96 against 72 bytes).
+#ifndef BROV_SWEEP_KP_REGS
+#define BROV_SWEEP_KP_REGS 0
+#endif
+
+template <typename T, int MODEL, int INTEG>
+__global__ void __launch_bounds__(ROLLOUT_BLOCK) __maxnreg__(MaxReg<T>::N)
+se_sweep_kernel(const __grid_constant__ SweepArgs<T> a) {
+    constexpr int BLOCK = ROLLOUT_BLOCK;
+    constexpr int NX = ModelDim<MODEL>::NX;
+    constexpr int NU = ModelDim<MODEL>::NU;
+    using LR = LagRegs<T, MODEL, false>;
+    constexpr int NL = LR::N;
+    __shared__ double red[BLOCK / 32][MAX_H];
+    __shared__ T kps[KP_COUNT];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int hmax = a.H[a.nH - 1];
+    const int item = blockIdx.x;
+    const int cand = BROV_SWEEP_CAND_MAJOR ? item / a.nwb : item % a.P;
+    const int wb = BROV_SWEEP_CAND_MAJOR ? item - cand * a.nwb : item / a.P;
+    if (tid < KP_COUNT) kps[tid] = __ldg(a.kp + (long long)tid * a.P + cand);
+    __syncthreads();
+    constexpr bool KPR = BROV_SWEEP_KP_REGS && sizeof(T) == 4;
+    typename std::conditional<KPR, ParamsRegs<T>, ParamsShared<T>>::type p;
+    if constexpr (KPR) {
+#pragma unroll
+        for (int j = 0; j < KP_COUNT; ++j) p.v[j] = kps[j];
+    } else {
+        p.base = kps;
+        p.pitch = 1;
+    }
+    const long long k = (long long)wb * BLOCK + tid;
+    const bool uvec = ((reinterpret_cast<uintptr_t>(a.U) & 15) == 0) && (sizeof(T) * NU % 16 == 0);
+    double se[MAX_H];
+#pragma unroll
+    for (int h = 0; h < MAX_H; ++h) se[h] = 0.0;
+    int n_bad = 0, n_sing = 0;
+    if (k < a.nwin) {
+        const long long kr = k + a.off;
+        T x[NX], lag[NL];
+#pragma unroll
+        for (int j = 0; j < NX; ++j) x[j] = __ldg(a.X + kr * NX + j);
+        load_lag<T, MODEL, false>(a.c, a.lag0, a.lag0_w != 0, k, lag);
+        // window k may run j steps while row k + j exists
+        const long long room = (long long)a.rows - 1 - kr;
+        const int nsteps = (int)(room < hmax ? (room < 0 ? 0 : room) : hmax);
+        float mc = 1.0f;
+        bool bad = false;
+        T u[NU], un[NU];
+        if (nsteps > 0) load_u<T, NU, false>(a.U + kr * NU, uvec, u);
+        for (int j = 0; j < nsteps; ++j) {
+            const T* nxt = a.U + (kr + (j + 1 < nsteps ? j + 1 : j)) * NU;
+            auto pf = [&]() { load_u<T, NU, false>(nxt, uvec, un); };
+            LateSide<decltype(pf)> late{pf, 1};
+            T acth;
+            integrate_step<T, MODEL, INTEG, false, decltype(p)>(a.c, p, x, lag, u, acth, late);
+#pragma unroll
+            for (int q = 0; q < NU; ++q) u[q] = un[q];
+            mc = fminf(mc, (float)acth);
+#pragma unroll
+            for (int h = 0; h < MAX_H; ++h) {
+                if (h < a.nH && j + 1 == a.H[h]) {
+                    const T* tgt = a.X + (kr + j + 1) * NX;
+                    double s = 0.0;
+#pragma unroll
+                    for (int q = 0; q < NX; ++q) {
+                        double e = (double)x[q] - (double)__ldg(tgt + q);
+                        s += e * e;
+                    }
+                    se[h] += s;
+                    bad |= !(s <= 1.7976931348623157e308);
+                }
+            }
+        }
+        n_bad = bad ? 1 : 0;
+        n_sing = ((double)mc < a.eps) ? 1 : 0;
+    }
+    if (a.health) {
+        const int tb = __reduce_add_sync(0xffffffffu, n_bad), ts = __reduce_add_sync(0xffffffffu, n_sing);
+        if (lane == 0) {
+            if (tb) atomicAdd(a.health + 2 * cand + 0, (unsigned long long)tb);
+            if (ts) atomicAdd(a.health + 2 * cand + 1, (unsigned long long)ts);
+        }
+    }
+#pragma unroll
+    for (int h = 0; h < MAX_H; ++h) {
+        double v = se[h];
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
+        if (lane == 0) red[warp][h] = v;
+    }
+    __syncthreads();
+    if (tid < MAX_H) {
+        double v = 0.0;
+#pragma unroll
+        for (int w = 0; w < BLOCK / 32; ++w) v += red[w][tid];
+        a.partial[((long long)cand * a.nwb + wb) * MAX_H + tid] = v;
+    }
+}
+
+// one block per candidate, each the fixed-order sum of se_finish_kernel over that candidate's nwb partials
+static __global__ void __launch_bounds__(256) se_sweep_finish_kernel(const double* __restrict__ partial, int nwb,
+                                                                     double* __restrict__ se_out) {
+    __shared__ double sh[256];
+    partial += (long long)blockIdx.x * nwb * MAX_H;
+    se_out += (long long)blockIdx.x * MAX_H;
+    for (int h = 0; h < MAX_H; ++h) {
+        double v = 0.0;
+        for (int b = threadIdx.x; b < nwb; b += 256) v += partial[(long long)b * MAX_H + h];
+        sh[threadIdx.x] = v;
+        __syncthreads();
+        for (int s = 128; s > 0; s >>= 1) {
+            if (threadIdx.x < s) sh[threadIdx.x] += sh[threadIdx.x + s];
+            __syncthreads();
+        }
+        if (threadIdx.x == 0) se_out[h] = sh[0];
+        __syncthreads();
+    }
+}
+
+// Carried lag of the sweep (thruster model, one horizon H): the allocation-projected lag state [nwin][18] that window k
+// inherits from windows 0..k-1 of the reference's single model object.  It depends on the inputs, dt, the integrator
+// and the allocation only — never on the 36 coefficients — so one pass serves every candidate.  Same replay and
+// window-to-window hand-over as se_kernel's carried-lag mode, with the dynamics left out: lag-only steps.
+template <typename T> struct CarryLagArgs {
+    Consts<T> c;
+    const T* U;         // [rows][8]
+    T* lag_out;         // [nwin][18]
+    long long win0, row0;
+    int rows, nwin, H, carry_steps, wpt;
+};
+
+template <typename T>
+__global__ void __launch_bounds__(RHS_BLOCK) se_carry_lag_kernel(const __grid_constant__ CarryLagArgs<T> a) {
+    const long long gk = ((long long)blockIdx.x * RHS_BLOCK + threadIdx.x) * a.wpt;
+    const bool uvec = (reinterpret_cast<uintptr_t>(a.U) & 15) == 0;
+    const long long H0 = a.H;
+    T lag[18];
+    for (int c = 0; c < a.wpt; ++c) {
+        const long long k = gk + c;
+        if (k >= a.nwin) break;
+        const long long kr = k + (a.win0 - a.row0);
+        T u[8], F[8], TF[6];
+        if (c == 0) {
+#pragma unroll
+            for (int j = 0; j < 18; ++j) lag[j] = T(0);
+            // history of the shared model object: windows w = 0..kg-1, each feeding U[w..w+H-1]; replay its tail
+            const long long total = (a.win0 + k) * H0;
+            const long long m = total < a.carry_steps ? total : a.carry_steps;
+            for (long long s = total - m; s < total; ++s) {
+                const long long w = s / H0;
+                const long long row = w + (s - w * H0) - a.row0;
+                load_u<T, 8, false>(a.U + row * 8, uvec, u);
+#pragma unroll
+                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<T>(u[i]);
+                allocate_wrench<T>(a.c, F, TF);
+                lag_advance<T, true>(a.c, lag, TF);
+            }
+        }   // c > 0: the lag the previous window ended with IS the state the shared object hands to this one
+#pragma unroll
+        for (int j = 0; j < 18; ++j) a.lag_out[k * 18 + j] = lag[j];
+        // window k: the lag advances once per step it runs (as in integrate_step)
+        const long long room = (long long)a.rows - 1 - kr;
+        const int nsteps = (int)(room < H0 ? (room < 0 ? 0 : room) : H0);
+        for (int j = 0; j < nsteps; ++j) {
+            load_u<T, 8, false>(a.U + (kr + j) * 8, uvec, u);
+#pragma unroll
+            for (int i = 0; i < 8; ++i) F[i] = thrust_poly<T>(a.c, u[i]);
+            allocate_wrench<T>(a.c, F, TF);
+            lag_advance<T, true>(a.c, lag, TF);
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------------
 // reduced 9-state model RHS (bluerov_compute): 13 scalars in, 9 out per row; rows staged through shared memory so
 // that every global access is a full-line coalesced (vector) transaction
 // ---------------------------------------------------------------------------------------------------------------
@@ -934,6 +1139,9 @@ cudaError_t launch_rhs(int model, bool lag1, const RhsArgs<T>& a, cudaStream_t s
 template <typename T>
 cudaError_t launch_se(int model, int integ, const SeArgs<T>& a, double* se_out, cudaStream_t st);
 template <typename T> int se_blocks(long long nwin);
+template <typename T>
+cudaError_t launch_se_sweep(int model, int integ, const SweepArgs<T>& a, double* se_out, cudaStream_t st);
+template <typename T> cudaError_t launch_se_carry_lag(const CarryLagArgs<T>& a, cudaStream_t st);
 template <typename T>
 cudaError_t launch_reduced9(const Red9Consts<T>& c, const T* X, const T* U, T* O, long long B, cudaStream_t st);
 template <typename T>

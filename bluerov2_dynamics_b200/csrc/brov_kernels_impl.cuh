@@ -181,6 +181,36 @@ cudaError_t launch_se(int model, int integ, const SeArgs<T>& a, double* se_out, 
     return cudaGetLastError();
 }
 
+// the sweep serves the three Fossen models (the double integrator has no coefficient table to sweep)
+template <typename T, int MODEL>
+static cudaError_t se_sweep_go(int integ, const SweepArgs<T>& a, cudaStream_t st) {
+    const unsigned grid = (unsigned)((long long)a.P * a.nwb);
+    if (integ == INTEG_RK4) se_sweep_kernel<T, MODEL, INTEG_RK4><<<grid, ROLLOUT_BLOCK, 0, st>>>(a);
+    else se_sweep_kernel<T, MODEL, INTEG_EULER><<<grid, ROLLOUT_BLOCK, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+template <typename T>
+cudaError_t launch_se_sweep(int model, int integ, const SweepArgs<T>& a, double* se_out, cudaStream_t st) {
+    if (a.P <= 0 || a.nwb <= 0) return cudaSuccess;
+    cudaError_t e = cudaErrorInvalidValue;
+    switch (model) {
+        case MODEL_THRUSTER8: e = se_sweep_go<T, MODEL_THRUSTER8>(integ, a, st); break;
+        case MODEL_WRENCH12: e = se_sweep_go<T, MODEL_WRENCH12>(integ, a, st); break;
+        case MODEL_QUAT13: e = se_sweep_go<T, MODEL_QUAT13>(integ, a, st); break;
+    }
+    if (e != cudaSuccess) return e;
+    se_sweep_finish_kernel<<<a.P, 256, 0, st>>>(a.partial, a.nwb, se_out);
+    return cudaGetLastError();
+}
+
+template <typename T> cudaError_t launch_se_carry_lag(const CarryLagArgs<T>& a, cudaStream_t st) {
+    if (a.nwin <= 0) return cudaSuccess;
+    const long long threads = (a.nwin + a.wpt - 1) / a.wpt;
+    se_carry_lag_kernel<T><<<(unsigned)((threads + RHS_BLOCK - 1) / RHS_BLOCK), RHS_BLOCK, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
 template <typename T>
 cudaError_t launch_reduced9(const Red9Consts<T>& c, const T* X, const T* U, T* O, long long B, cudaStream_t st) {
     if (B <= 0) return cudaSuccess;
@@ -218,6 +248,8 @@ cudaError_t launch_thruster_series(const ThrusterSeriesArgs<T>& a, cudaStream_t 
     template cudaError_t launch_rhs<T>(int, bool, const RhsArgs<T>&, cudaStream_t);                                \
     template cudaError_t launch_se<T>(int, int, const SeArgs<T>&, double*, cudaStream_t);                          \
     template int se_blocks<T>(long long);                                                                          \
+    template cudaError_t launch_se_sweep<T>(int, int, const SweepArgs<T>&, double*, cudaStream_t);                 \
+    template cudaError_t launch_se_carry_lag<T>(const CarryLagArgs<T>&, cudaStream_t);                             \
     template cudaError_t launch_reduced9<T>(const Red9Consts<T>&, const T*, const T*, T*, long long, cudaStream_t); \
     template cudaError_t launch_fma_peak<T>(int, int, T*, cudaStream_t);                                           \
     template cudaError_t launch_thruster_wrench<T>(const ThrusterArgs<T>&, cudaStream_t);                          \

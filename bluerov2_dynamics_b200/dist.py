@@ -1,8 +1,9 @@
 """Multi-GPU plumbing: one process per GPU, `torch.distributed` (NCCL on B200s, gloo in CPU tests).
 
-The path shards without any data-path exchange: vehicles of a rollout and windows of the RMSE evaluator are
-independent, so each rank takes a contiguous index range.  The only collective is the sum of the per-rank squared
-error vectors and health counters (6 doubles) of the evaluator."""
+The path shards without any data-path exchange: vehicles of a rollout, windows of the RMSE evaluator and candidates
+of an evaluator sweep are independent, so each rank takes a contiguous index range.  The only collective is the sum of
+the per-rank squared error vectors and health counters (6 doubles) of the evaluator, or of the [P, 4] table of a
+sweep."""
 from __future__ import annotations
 
 import os
@@ -194,6 +195,22 @@ def allreduce_sum_(t: torch.Tensor) -> torch.Tensor:
 
 def global_counts(T: int, horizons: Sequence[int]) -> list[int]:
     return [max(T - int(h), 0) for h in horizons]
+
+
+def sharded_sweep(local_fn: Callable[[int, int], torch.Tensor], P: int, rank: int, world: int,
+                  width: int = 4) -> torch.Tensor:
+    """Candidate sweep on `world` GPUs: candidates [lo, hi) of `rank` (shard_range) are scored on the whole series by
+    local_fn(lo, hi) -> [hi - lo, width] squared-error sums (on the GPU: Engine.multistep_se_sweep on the rank's rows of
+    the table; in CPU tests a stand-in) and written into the rank's slice of a zero [P, width] float64 tensor; one
+    all-reduce assembles the table.  Exact: every entry is one rank's value plus zeros.  width = BROV_MAX_H."""
+    lo, hi = shard_range(int(P), rank, world)
+    part = local_fn(lo, hi) if hi > lo else None
+    dev = part.device if part is not None else (torch.device("cuda", torch.cuda.current_device())
+                                                if dist.is_initialized() and dist.get_backend() == "nccl" else torch.device("cpu"))
+    out = torch.zeros((int(P), width), dtype=torch.float64, device=dev)
+    if part is not None:
+        out[lo:hi] = part.to(torch.float64)
+    return allreduce_sum_(out)
 
 
 def sharded_multistep_rmse(local_se: Callable[[np.ndarray, np.ndarray, Sequence[int], int], torch.Tensor],

@@ -24,6 +24,7 @@ _NX13 = ("quat13", "diq13_u6")
 _NU8 = ("thruster8", "di12_u8")
 DTYPES = {"f64": (L.F64, torch.float64, np.float64), "f32": (L.F32, torch.float32, np.float32)}
 INTEGRATORS = {"rk4": L.RK4, "euler": L.EULER}
+SWEEP_WORKSPACE_CAP = 256 << 20   # bytes of sweep workspace per launch (Engine.multistep_se_sweep splits P to fit)
 
 
 def default_physical(rho: float = 1000.0) -> np.ndarray:
@@ -41,6 +42,18 @@ def derive_params(phys: np.ndarray) -> np.ndarray:
     for i in range(flat.shape[0]):
         L.check(L.lib.brov_derive_params(L.dptr(flat[i]), L.dptr(out[i])))
     return out.reshape(phys.shape[:-1] + (L.NKP,))
+
+
+def with_minv(phys: np.ndarray) -> np.ndarray:
+    """Copy of physical vector(s) [..., NPHYS] whose diag(Minv) entries are rebuilt from m, the inertias and the added
+    masses, as the reference's __init__ computes them: 1/(m - X_udot), ..., 1/(Iz - N_rdot).  The kernels use the Minv
+    they are given (the reference freezes it at construction, SURVEY trap T5), so a candidate table that perturbs the
+    masses must pass through this to describe the vehicle it means."""
+    ph = np.array(phys, dtype=np.float64)
+    m = ph[..., L.PH_M:L.PH_M + 1]
+    ph[..., L.PH_MINV:L.PH_MINV + 3] = 1.0 / (m - ph[..., L.PH_ADDED:L.PH_ADDED + 3])
+    ph[..., L.PH_MINV + 3:L.PH_MINV + 6] = 1.0 / (ph[..., L.PH_I:L.PH_I + 3] - ph[..., L.PH_ADDED + 3:L.PH_ADDED + 6])
+    return ph
 
 
 def default_allocation():
@@ -524,6 +537,102 @@ class Engine:
             for j, h in enumerate(part):
                 out[h] = float(np.sqrt(se[j] / (cnt[j] * self.nx))) if cnt[j] > 0 else float("nan")
         return out[hs[0]] if single else [out[h] for h in hs]
+
+    def multistep_se_sweep(self, X, U, horizons: Sequence[int], phys_table: np.ndarray, dt: float = 0.02,
+                           integrator: str = "rk4", lag_mode: str = "reset", lag0=None,
+                           health_out: Optional[torch.Tensor] = None, workspace: Optional[torch.Tensor] = None,
+                           singular_eps: float = 0.0, workspace_cap: int = SWEEP_WORKSPACE_CAP):
+        """`multistep_se` for P candidate vehicles against one recorded series (brov_multistep_se_sweep).
+        phys_table [P, NPHYS]: one physical vector per candidate (derived row by row as set_vehicle_physical does; see
+        with_minv for tables that perturb the masses).  The engine's own coefficients are not used; allocation and lag
+        discretisation are the engine's.  Returns (se [P, MAX_H] float64 device tensor, counts list): row c equals
+        `set_physical(phys_table[c])` + `multistep_se(..., time_slices=1)`.
+        lag_mode="carry" (thruster model, one horizon): the carried lag each window starts from is computed once for all
+        candidates.  lag0 [n_windows, 24] (reset mode) is shared by every candidate.  health_out: int64 [P, 2] device
+        tensor receiving, per candidate, the windows with a non-finite endpoint error / that came within singular_eps of
+        theta = +-pi/2.  The candidates are split over several launches so that the workspace stays within
+        workspace_cap bytes (a workspace passed in must hold one launch: brov_se_sweep_workspace_bytes)."""
+        X = self.tensor(X)
+        U = self.tensor(U)
+        self._check_rows(X, self.nx, "X")
+        self._check_rows(U, self.nu, "U")
+        rows = X.shape[0]
+        if U.shape[0] != rows:
+            raise ValueError("X and U must have the same number of rows")
+        hs = [int(h) for h in horizons]
+        if not 1 <= len(hs) <= L.MAX_H or any(h < 1 for h in hs) or sorted(set(hs)) != hs:
+            raise ValueError(f"horizons must be 1..{L.MAX_H} strictly ascending positive integers")
+        if lag_mode not in ("reset", "carry"):
+            raise ValueError("lag_mode must be 'reset' or 'carry'")
+        carry = lag_mode == "carry" and self.model == "thruster8"
+        ph = np.asarray(phys_table, dtype=np.float64)
+        if ph.ndim != 2 or ph.shape[1] != L.NPHYS:
+            raise ValueError(f"phys_table must have shape [P, {L.NPHYS}]")
+        P = ph.shape[0]
+        kp = derive_params(ph)                                                   # [P, NKP]
+        # one flag for the whole table: a split sweep runs the same kernel build in every launch
+        any_current = int(bool(np.any(ph[:, L.PH_CURRENT:L.PH_CURRENT + 3] != 0.0)))
+        nwin = max(rows - hs[0], 0)
+        per_launch = P
+        while per_launch > 1 and L.lib.brov_se_sweep_workspace_bytes(per_launch, nwin, int(carry)) > workspace_cap:
+            per_launch = (per_launch + 1) // 2
+        nbytes = L.lib.brov_se_sweep_workspace_bytes(max(per_launch, 1), nwin, int(carry))
+        if workspace is not None:
+            if workspace.dtype != torch.uint8 or workspace.device != self.device or workspace.numel() < nbytes:
+                raise ValueError(f"workspace must be a uint8 tensor of at least {nbytes} bytes on {self.device}")
+            ws = workspace
+        else:
+            ws = torch.empty(nbytes, dtype=torch.uint8, device=self.device)
+        if health_out is not None and (health_out.dtype != torch.int64 or health_out.device != self.device
+                                       or not health_out.is_contiguous() or health_out.numel() != 2 * P):
+            raise ValueError(f"health_out must be a contiguous int64 tensor with {2 * P} elements on {self.device}")
+        lag_t = self.tensor(lag0).reshape(nwin, 24) if (lag0 is not None and self.model == "thruster8") else None
+        se = torch.zeros((P, L.MAX_H), dtype=torch.float64, device=self.device)
+        counts = (C.c_longlong * L.MAX_H)()
+        d = L.SeSweepDesc()
+        d.struct_size = C.sizeof(L.SeSweepDesc)
+        d.integrator = INTEGRATORS[integrator]
+        d.rows, d.n_windows, d.dt = rows, nwin, float(dt)
+        d.X_dev, d.U_dev = X.data_ptr(), U.data_ptr()
+        d.lag0_dev = lag_t.data_ptr() if lag_t is not None else None
+        d.n_horizons = len(hs)
+        for i, h in enumerate(hs):
+            d.horizons[i] = h
+        d.lag_carry = int(carry)
+        d.any_current = any_current
+        d.count_out = counts
+        d.singular_eps = float(singular_eps)
+        d.workspace_dev, d.workspace_bytes = ws.data_ptr(), ws.numel()
+        with torch.cuda.device(self.device):
+            for lo in range(0, max(P, 1), max(per_launch, 1)):
+                hi = min(P, lo + per_launch)
+                soa = torch.from_numpy(np.ascontiguousarray(kp[lo:hi].T)).to(self.device, self.tdtype).contiguous()
+                d.n_candidates = hi - lo
+                d.kp_soa_dev = soa.data_ptr() if hi > lo else None
+                d.se_out_dev = se[lo:hi].data_ptr() if hi > lo else None
+                d.health_dev = health_out.reshape(P, 2)[lo:hi].data_ptr() if (health_out is not None and hi > lo) else None
+                L.check(L.lib.brov_multistep_se_sweep(self._h, C.byref(d), self._stream()))
+        return se, [int(counts[i]) for i in range(len(hs))]
+
+    def multistep_rmse_sweep(self, X, U, horizons, phys_table: np.ndarray, dt: float = 0.02, integrator: str = "rk4",
+                             lag_mode: str = "reset", lag0=None) -> np.ndarray:
+        """RMSE per candidate and horizon, numpy [P, len(horizons)] (`multistep_rmse` for every row of phys_table;
+        NaN where no window fits).  lag_mode="carry" (thruster model) runs one pass per horizon."""
+        single = np.isscalar(horizons)
+        hs = [int(horizons)] if single else [int(h) for h in horizons]
+        order = sorted(set(hs))
+        P = np.shape(phys_table)[0]
+        out = {}
+        group = 1 if (lag_mode == "carry" and self.model == "thruster8") else L.MAX_H
+        X = self.tensor(X)
+        U = self.tensor(U)
+        for i in range(0, len(order), group):
+            part = order[i:i + group]
+            se, cnt = self.multistep_se_sweep(X, U, part, phys_table, dt, integrator, lag_mode=lag_mode, lag0=lag0)
+            se = se.cpu().numpy()
+            for j, h in enumerate(part):
+                out[h] = np.sqrt(se[:, j] / (cnt[j] * self.nx)) if cnt[j] > 0 else np.full(P, np.nan)
+        return np.stack([out[h] for h in hs], axis=1) if P else np.zeros((0, len(hs)))
 
     # ------------------------------------------------------------------ host-buffer API (end-to-end path)
     def rollout_host(self, x0: np.ndarray, U: Optional[np.ndarray] = None, dt: float = 0.02, integrator: str = "rk4",

@@ -62,6 +62,18 @@ def multistep_rmse_endpoint_physics(X_test: np.ndarray, U_test: np.ndarray, H, d
     return eng.multistep_rmse(X_test, U_test, H, dt=dt, integrator=integrator, lag_mode=lag_mode)
 
 
+def multistep_rmse_endpoint_physics_sweep(X_test: np.ndarray, U_test: np.ndarray, H, dt: float, phys_table: np.ndarray,
+                                          model: str = None, lag_mode: str = "carry", dtype: str = "f64",
+                                          integrator: str = "rk4", engine: Engine = None) -> np.ndarray:
+    """`multistep_rmse_endpoint_physics` for P candidate vehicles at once: phys_table [P, NPHYS] holds one physical
+    vector per candidate (engine.with_minv rebuilds diag(Minv) after the masses are perturbed).  Returns the RMSE as a
+    numpy array [P] for a scalar H, [P, len(H)] for a list; NaN where T <= H.  Same lag modes as the single-vehicle
+    function (carry: the thruster lag leaks from window to window; the carried state is shared by all candidates)."""
+    eng = _engine_for(X_test, model, dtype, engine)
+    out = eng.multistep_rmse_sweep(X_test, U_test, H, phys_table, dt=dt, integrator=integrator, lag_mode=lag_mode)
+    return out[:, 0] if np.isscalar(H) else out
+
+
 def one_step_rmse_physics(X_test: np.ndarray, U_test: np.ndarray, dt: float, model: str = None, dtype: str = "f64",
                           engine: Engine = None, lag_mode: str = "carry") -> float:
     """Teacher-forced one-step Euler prediction RMSE, rmse(X[1:], X[:-1] + dt f(X[:-1], U[:-1])); with

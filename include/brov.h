@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define BROV_ABI_VERSION 7
+#define BROV_ABI_VERSION 8
 
 enum { BROV_THRUSTER8_LAG3 = 0, BROV_WRENCH_EULER12 = 1, BROV_WRENCH_QUAT13 = 2,
        /* double-integrator comparison model of the reference's evaluation tables (kinematics + a learned linear map
@@ -289,6 +289,50 @@ typedef struct brov_se_desc {
 int brov_se_carry_steps(brov_engine_t* e, double dt, int integrator, long long* steps_out);
 size_t brov_se_workspace_bytes(long long n_windows);
 int brov_multistep_se(brov_engine_t* e, const brov_se_desc* d, void* stream);
+
+/* Candidate sweep of the evaluator: the squared-error sums of brov_multistep_se for n_candidates coefficient sets
+ * against ONE recorded series, in one launch — calibration of the uncertain hydrodynamic coefficients against a tank
+ * recording, sensitivity studies, scoring a Monte-Carlo cloud of vehicles.  Fossen models only (thruster8, wrench12,
+ * quat13); the first-order wrench lag is not supported.
+ * kp_soa_dev: [BROV_NKP][n_candidates], engine scalar type, the layout of brov_set_vehicle_params (candidate c is
+ * column c); any_current: non-zero if some candidate has a non-zero ocean current.  The table travels in the
+ * descriptor: the engine's shared coefficients and its per-vehicle table are neither used nor changed.  Allocation and
+ * lag discretisation come from the engine.
+ * se_out_dev [n_candidates][BROV_MAX_H] (double, dev): row c is what brov_multistep_se(time_slices = 1) returns with
+ * candidate c's coefficients (the same per-window arithmetic and summation order); count_out (host, may be NULL) is the
+ * same for every candidate.  health_dev [n_candidates][2] (unsigned long long, dev) or NULL: per candidate, the windows
+ * with a non-finite endpoint error / that came within singular_eps of theta = +-pi/2 (zeroed by the call).
+ * Geometry fields (integrator ... lag_carry, window0, row0) as in brov_se_desc.  lag_carry: the lag state each window
+ * inherits does not depend on the coefficients, so one pre-pass computes it for all candidates.  workspace_dev: at least
+ * brov_se_sweep_workspace_bytes(n_candidates, n_windows, lag_carry) bytes.  n_candidates * ceil(n_windows / 128) must
+ * stay below 2^31 (split larger sweeps into several calls). */
+typedef struct brov_se_sweep_desc {
+    uint32_t struct_size;
+    int32_t integrator;
+    long long rows;
+    long long n_windows;
+    double dt;
+    const void* X_dev;
+    const void* U_dev;
+    const void* lag0_dev;           /* [n_windows][24] or NULL, shared by all candidates (reset mode) */
+    int32_t n_horizons;
+    int32_t horizons[BROV_MAX_H];
+    int32_t lag_carry;
+    long long window0;
+    long long row0;
+    long long n_candidates;
+    const void* kp_soa_dev;         /* [BROV_NKP][n_candidates] */
+    int32_t any_current;
+    int32_t reserved;
+    double* se_out_dev;             /* [n_candidates][BROV_MAX_H] */
+    long long* count_out;           /* host [BROV_MAX_H] or NULL */
+    void* health_dev;               /* [n_candidates][2] or NULL */
+    double singular_eps;            /* 0 = 1e-3 */
+    void* workspace_dev;
+    size_t workspace_bytes;
+} brov_se_sweep_desc;
+size_t brov_se_sweep_workspace_bytes(long long n_candidates, long long n_windows, int lag_carry);
+int brov_multistep_se_sweep(brov_engine_t* e, const brov_se_sweep_desc* d, void* stream);
 
 /* Reduced 9-state RHS — `bluerov_compute(t, x_, u_)` (fossen/bluerov_torch.py:20-67, constants fossen/parameters.py).
  * x [B][9], u [B][4], out [B][9]. */
