@@ -70,6 +70,17 @@ class SeSweepDesc(C.Structure):
                 ("workspace_bytes", C.c_size_t)]
 
 
+class SeGradDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("rows", C.c_longlong),
+                ("n_windows", C.c_longlong), ("dt", C.c_double), ("X_dev", C.c_void_p), ("U_dev", C.c_void_p),
+                ("lag0_dev", C.c_void_p), ("n_horizons", C.c_int32), ("horizons", C.c_int32 * MAX_H),
+                ("lag_carry", C.c_int32), ("window0", C.c_longlong), ("row0", C.c_longlong),
+                ("kp_dev", C.c_void_p), ("any_current", C.c_int32), ("n_dirs", C.c_int32), ("dirs_dev", C.c_void_p),
+                ("se_out_dev", C.c_void_p), ("grad_out_dev", C.c_void_p), ("gn_out_dev", C.c_void_p),
+                ("count_out", C.POINTER(C.c_longlong)), ("health_dev", C.c_void_p), ("singular_eps", C.c_double),
+                ("workspace_dev", C.c_void_p), ("workspace_bytes", C.c_size_t)]
+
+
 class RolloutHostDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
                 ("dt", C.c_double), ("x0_host", C.c_void_p), ("xT_host", C.c_void_p), ("u_host", C.c_void_p),
@@ -129,6 +140,8 @@ _PROTOS = {
     "brov_se_carry_steps": (C.c_int, [C.c_void_p, C.c_double, C.c_int, C.POINTER(C.c_longlong)]),
     "brov_se_sweep_workspace_bytes": (C.c_size_t, [C.c_longlong, C.c_longlong, C.c_int]),
     "brov_multistep_se_sweep": (C.c_int, [C.c_void_p, C.POINTER(SeSweepDesc), C.c_void_p]),
+    "brov_se_grad_workspace_bytes": (C.c_size_t, [C.c_longlong, C.c_int, C.c_int]),
+    "brov_multistep_se_grad": (C.c_int, [C.c_void_p, C.POINTER(SeGradDesc), C.c_void_p]),
     "brov_reduced9_rhs": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "brov_koopman_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_void_p)]),
     "brov_koopman_destroy": (None, [C.c_void_p]),

@@ -18,7 +18,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 OUT = os.path.join(PKG, "libbrov.so")
 BUILD = os.path.join(PKG, "build")
-SOURCES = ["brov_api.cu", "brov_kernels_f32.cu", "brov_kernels_f64.cu", "brov_koopman.cu", "brov_pinc.cu"]
+SOURCES = ["brov_api.cu", "brov_kernels_f32.cu", "brov_kernels_f64.cu", "brov_koopman.cu", "brov_pinc.cu", "brov_grad.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 

@@ -13,6 +13,7 @@
 #include "../../include/brov.h"
 #include "brov_internal.cuh"
 #include "brov_kernels.cuh"
+#include "brov_grad.cuh"
 
 using namespace brov;
 
@@ -1116,6 +1117,89 @@ extern "C" int brov_multistep_se_sweep(brov_engine_t* e, const brov_se_sweep_des
     const size_t need = brov_se_sweep_workspace_bytes(d->n_candidates, d->n_windows, d->lag_carry && e->model == BROV_THRUSTER8_LAG3);
     if (!d->workspace_dev || d->workspace_bytes < need) return fail(BROV_EINVAL, "workspace too small: need %zu bytes", need);
     return e->dtype == BROV_F32 ? se_sweep_impl<float>(e, d, st) : se_sweep_impl<double>(e, d, st);
+}
+
+// gradient workspace: per-block partials [GRAD_MAX_GRID][MAX_H][1 + p + p(p+1)/2], then (carry mode) the lag each
+// window inherits [n_windows][18]
+static size_t grad_partial_bytes(int n_dirs) {
+    const size_t ne = 1 + (size_t)n_dirs + (size_t)n_dirs * (n_dirs + 1) / 2;
+    return se_align((size_t)GRAD_MAX_GRID * MAX_H * ne * sizeof(double));
+}
+extern "C" size_t brov_se_grad_workspace_bytes(long long n_windows, int n_dirs, int lag_carry) {
+    if (n_windows < 0) n_windows = 0;
+    if (n_dirs < 1 || n_dirs > KP_COUNT) return 0;
+    return grad_partial_bytes(n_dirs) + (lag_carry ? se_align((size_t)n_windows * 18 * sizeof(double)) : 0);
+}
+
+static int se_grad_impl(brov_engine* e, const brov_se_grad_desc* d, cudaStream_t st) {
+    GradArgs a;
+    memset(&a, 0, sizeof(a));
+    const int nsub = d->integrator == BROV_RK4 ? 4 : 1;
+    int rc = make_consts<double>(e, d->dt, nsub, &a.c);
+    if (rc) return rc;
+    a.c.has_current = d->any_current ? 1 : 0;   // the point's and the directions' currents, not the engine's
+    a.X = (const double*)d->X_dev; a.U = (const double*)d->U_dev;
+    a.kp = d->kp_dev; a.dirs = d->dirs_dev;
+    a.partial = (double*)d->workspace_dev;
+    a.health = (unsigned long long*)d->health_dev;
+    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    a.off = d->window0 - d->row0;
+    a.rows = (int)d->rows; a.nwin = (int)d->n_windows; a.nH = d->n_horizons;
+    for (int h = 0; h < MAX_H; ++h) a.H[h] = h < d->n_horizons ? d->horizons[h] : 0x7fffffff;
+    a.p = d->n_dirs;
+    a.W = GRAD_BLOCK / a.p;
+    a.ntiles = (int)((d->n_windows + a.W - 1) / a.W);
+    a.ne = 1 + a.p + a.p * (a.p + 1) / 2;
+    a.lag0 = (const double*)d->lag0_dev;
+    a.lag0_w = 0;
+    if (d->lag_carry && e->model == BROV_THRUSTER8_LAG3) {
+        // the inherited lag does not depend on the coefficients: the sweep's pre-pass serves every direction
+        long long m = 0;
+        if ((rc = carry_depth(e, d->dt, nsub, &m))) return rc;
+        if ((rc = check_carry_rows(d->window0, d->row0, d->horizons[0], m))) return rc;
+        CarryLagArgs<double> c;
+        memset(&c, 0, sizeof(c));
+        c.c = a.c;
+        c.U = a.U;
+        c.lag_out = (double*)((unsigned char*)d->workspace_dev + grad_partial_bytes(d->n_dirs));
+        c.win0 = d->window0; c.row0 = d->row0;
+        c.rows = a.rows; c.nwin = a.nwin; c.H = d->horizons[0]; c.carry_steps = (int)m;
+        c.wpt = carry_wpt(e, d->n_windows, d->horizons[0], m);
+        CUDA_TRY(launch_se_carry_lag<double>(c, st));
+        a.lag0 = c.lag_out;
+        a.lag0_w = 1;
+    }
+    if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+    CUDA_TRY(launch_se_grad(e->model, d->integrator, a, e->num_sms, d->se_out_dev, d->grad_out_dev, d->gn_out_dev, st));
+    return BROV_OK;
+}
+
+extern "C" int brov_multistep_se_grad(brov_engine_t* e, const brov_se_grad_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_se_grad_desc)) return fail(BROV_EINVAL, "brov_se_grad_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "the gradient serves the Fossen models; double-integrator engines have no coefficient table");
+    if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the gradient is computed in fp64: create the engine with BROV_F64");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "the evaluator does not support the first-order wrench lag");
+    int rc = check_se_geometry(d);
+    if (rc) return rc;
+    if (d->n_dirs < 1 || d->n_dirs > KP_COUNT) return fail(BROV_EINVAL, "n_dirs = %d must be 1..%d", d->n_dirs, KP_COUNT);
+    if (!d->se_out_dev || !d->grad_out_dev || !d->gn_out_dev) return fail(BROV_EINVAL, "se_out, grad_out and gn_out must not be NULL");
+    se_counts(d);
+    CUDA_TRY(cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d->n_windows == 0 || d->rows < 2) {
+        const size_t p = (size_t)d->n_dirs;
+        CUDA_TRY(cudaMemsetAsync(d->se_out_dev, 0, MAX_H * sizeof(double), st));
+        CUDA_TRY(cudaMemsetAsync(d->grad_out_dev, 0, MAX_H * p * sizeof(double), st));
+        CUDA_TRY(cudaMemsetAsync(d->gn_out_dev, 0, MAX_H * p * p * sizeof(double), st));
+        if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+        return BROV_OK;
+    }
+    if (!d->X_dev || !d->U_dev) return fail(BROV_EINVAL, "X and U must not be NULL");
+    if (!d->kp_dev || !d->dirs_dev) return fail(BROV_EINVAL, "kp and dirs must not be NULL");
+    const size_t need = brov_se_grad_workspace_bytes(d->n_windows, d->n_dirs, d->lag_carry && e->model == BROV_THRUSTER8_LAG3);
+    if (!d->workspace_dev || d->workspace_bytes < need) return fail(BROV_EINVAL, "workspace too small: need %zu bytes", need);
+    return se_grad_impl(e, d, st);
 }
 
 // fossen/parameters.py:3-33

@@ -802,4 +802,126 @@ __device__ __forceinline__ void integrate_step(const Consts<T>& c, const P& p, T
     if constexpr (ModelDim<MODEL>::QUAT) quat_renorm<T>(x + 3);
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// forward-mode sensitivities: a dual number (value, tangent), both fp64.  nu_dot, rhs_euler12, rhs_quat13 and
+// quat_renorm instantiated with it carry the derivative of the state along one direction of the coefficient vector
+// (brov_grad.cu).  The derivative is that of the function the code computes, branch taken: d|x| = sign(x) dx with
+// sign(0) = 0, the clamped cos(theta) and the quaternion fallback are constants.  Comparisons look at the value.
+// ---------------------------------------------------------------------------------------------------------------
+struct Dual {
+    double v, d;
+    Dual() = default;
+    __device__ __forceinline__ Dual(double x) : v(x), d(0.0) {}
+    __device__ __forceinline__ Dual(double x, double dx) : v(x), d(dx) {}
+};
+__device__ __forceinline__ Dual operator+(Dual a, Dual b) { return Dual(a.v + b.v, a.d + b.d); }
+__device__ __forceinline__ Dual operator-(Dual a, Dual b) { return Dual(a.v - b.v, a.d - b.d); }
+__device__ __forceinline__ Dual operator-(Dual a) { return Dual(-a.v, -a.d); }
+__device__ __forceinline__ Dual operator*(Dual a, Dual b) { return Dual(a.v * b.v, fma(a.v, b.d, a.d * b.v)); }
+__device__ __forceinline__ Dual operator*(double a, Dual b) { return Dual(a * b.v, a * b.d); }
+__device__ __forceinline__ Dual operator*(Dual a, double b) { return Dual(a.v * b, a.d * b); }
+__device__ __forceinline__ Dual& operator+=(Dual& a, Dual b) { a = a + b; return a; }
+__device__ __forceinline__ Dual& operator-=(Dual& a, Dual b) { a = a - b; return a; }
+__device__ __forceinline__ Dual& operator*=(Dual& a, Dual b) { a = a * b; return a; }
+__device__ __forceinline__ bool operator<(Dual a, Dual b) { return a.v < b.v; }
+__device__ __forceinline__ bool operator>(Dual a, Dual b) { return a.v > b.v; }
+__device__ __forceinline__ bool operator==(Dual a, Dual b) { return a.v == b.v; }
+__device__ __forceinline__ Dual abs_(Dual a) {
+    const double s = a.v > 0.0 ? 1.0 : (a.v < 0.0 ? -1.0 : 0.0);
+    return Dual(fabs(a.v), s * a.d);
+}
+__device__ __forceinline__ Dual sqrt_(Dual a) {
+    const double r = sqrt(a.v);
+    return Dual(r, 0.5 * a.d * rcp_nr(r));
+}
+__device__ __forceinline__ Dual rcp_nr(Dual a) {
+    const double r = rcp_nr(a.v);
+    return Dual(r, -a.d * r * r);
+}
+__device__ __forceinline__ void sincos_(Dual a, Dual* s, Dual* c, const double* K = kSinCos64) {
+    double sv, cv;
+    sincos_(a.v, &sv, &cv, K);
+    *s = Dual(sv, cv * a.d);
+    *c = Dual(cv, -sv * a.d);
+}
+
+// kernel coefficients of a dual evaluation: the point kp (shared by the block) with the tangent dk of this thread's
+// direction
+struct ParamsDual {
+    const double* kp;
+    const double* dk;
+    __device__ __forceinline__ Dual operator[](int i) const { return Dual(kp[i], dk[i]); }
+};
+
+// integrate_step with the state carried as dual numbers.  The thruster map, the T200 polynomial and the lag do not
+// depend on the coefficients: they stay plain double and the body wrench enters the dual right-hand side as a
+// constant.  Every stage evaluates its sines and cosines in full (no stage-rotation shortcut), so the values agree
+// with integrate_step to rounding, not bit for bit.
+template <int MODEL, int INTEG, class P>
+__device__ __forceinline__ void integrate_step_dual(const Consts<double>& c, const P& p, Dual* __restrict__ x,
+                                                    double* __restrict__ lag, const double* __restrict__ u,
+                                                    double& abs_cth) {
+    constexpr int NX = ModelDim<MODEL>::NX;
+    constexpr bool EULER_ANGLES = !ModelDim<MODEL>::QUAT;
+    const bool cur = c.has_current != 0;
+    const double dt = c.dt;
+    double Fu[6];
+    if constexpr (MODEL == MODEL_THRUSTER8) {
+        double F[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, u[i]);
+        allocate_wrench<double>(c, F, Fu);
+    } else {
+#pragma unroll
+        for (int i = 0; i < 6; ++i) Fu[i] = u[i];
+    }
+    auto rhs = [&](int s, const Dual* xs, Dual* out) {
+        Dual tau[6];
+        if constexpr (MODEL == MODEL_THRUSTER8) {
+            double t[6];
+            thruster_tau<double, true>(c, s, lag, Fu, t);
+#pragma unroll
+            for (int r = 0; r < 6; ++r) tau[r] = Dual(t[r]);
+        } else {
+#pragma unroll
+            for (int r = 0; r < 6; ++r) tau[r] = Dual(Fu[r]);
+        }
+        if constexpr (EULER_ANGLES) {
+            Trig<Dual> tr;
+            trig_full<Dual>(xs + 3, tr);
+            if (s == 0) abs_cth = fabs(tr.cth.v);
+            rhs_euler12<Dual>(xs, tr, tau, p, cur, out);
+        } else {
+            rhs_quat13<Dual>(xs, tau, p, cur, out);
+        }
+    };
+    if constexpr (!EULER_ANGLES) abs_cth = 1.0;
+    Dual k[NX];
+    if constexpr (INTEG == INTEG_EULER) {
+        rhs(0, x, k);
+#pragma unroll
+        for (int i = 0; i < NX; ++i) x[i] += dt * k[i];
+    } else {
+        Dual acc[NX], xs[NX];
+        const double hdt = 0.5 * dt;
+        rhs(0, x, k);
+#pragma unroll
+        for (int s = 1; s <= 3; ++s) {
+            const double w = (s == 1) ? 1.0 : 2.0;
+            const double h = (s == 3) ? dt : hdt;
+#pragma unroll
+            for (int i = 0; i < NX; ++i) {
+                if (s == 1) acc[i] = k[i]; else acc[i] += w * k[i];
+                xs[i] = x[i] + h * k[i];
+            }
+            rhs(s, xs, k);
+        }
+        const double dt6 = dt * (1.0 / 6.0);
+#pragma unroll
+        for (int i = 0; i < NX; ++i) x[i] += dt6 * (acc[i] + k[i]);
+    }
+    if constexpr (MODEL == MODEL_THRUSTER8) lag_advance<double, true>(c, lag, Fu);
+    if constexpr (ModelDim<MODEL>::QUAT) quat_renorm<Dual>(x + 3);
+}
+
 }  // namespace brov

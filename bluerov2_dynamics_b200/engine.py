@@ -56,6 +56,109 @@ def with_minv(phys: np.ndarray) -> np.ndarray:
     return ph
 
 
+# kernel coefficient vector layout (include/brov.h, csrc/brov_device.cuh KP_*)
+KP_MINV, KP_A, KP_DA, KP_DB, KP_DL, KP_DQ, KP_WMB, KP_XBB, KP_CUR = 0, 6, 9, 12, 15, 21, 27, 28, 31
+
+# names of the physical vector's entries: the reference's attribute names (fossen/BlueROV2.py:81-150); the ocean
+# current is `current_speed` split into its NED components, diag(Minv) is named after the velocity it scales
+_AXES = ("u", "v", "w", "p", "q", "r")
+PHYS_NAMES = (["m", "W", "B", "xb", "yb", "zb", "Ix", "Iy", "Iz"]
+              + ["Xu_dot", "Yv_dot", "Zw_dot", "Kp_dot", "Mq_dot", "Nr_dot"]
+              + ["Xu", "Yv", "Zw", "Kp", "Mq", "Nr"]
+              + ["Xu_abs", "Yv_abs", "Zw_abs", "Kp_abs", "Mq_abs", "Nr_abs"]
+              + [f"Minv_{a}" for a in _AXES]
+              + ["current_n", "current_e", "current_d", "T_lag1"])
+PARAM_GROUPS = {"added": list(range(L.PH_ADDED, L.PH_ADDED + 6)), "lin": list(range(L.PH_LIN, L.PH_LIN + 6)),
+                "quad": list(range(L.PH_QUAD, L.PH_QUAD + 6)),
+                "current": list(range(L.PH_CURRENT, L.PH_CURRENT + 3))}
+
+
+def parameter_indices(params) -> list:
+    """Physical-vector indices of a parameter selection: PH_* indices, attribute names (PHYS_NAMES) or the groups
+    "added", "lin", "quad", "current", in any mix.  The first-order wrench lag (T_lag1) is not a parameter."""
+    if isinstance(params, (str, int, np.integer)):
+        params = [params]
+    idx = []
+    for q in params:
+        if isinstance(q, (int, np.integer)):
+            if not 0 <= int(q) < L.NPHYS:
+                raise ValueError(f"parameter index {q} out of range")
+            idx.append(int(q))
+        elif q in PARAM_GROUPS:
+            idx.extend(PARAM_GROUPS[q])
+        elif q in PHYS_NAMES:
+            idx.append(PHYS_NAMES.index(q))
+        else:
+            raise ValueError(f"unknown parameter {q!r}: use a PH_* index, one of {PHYS_NAMES[:-1]} or a group "
+                             f"{list(PARAM_GROUPS)}")
+    if L.PH_TLAG1 in idx:
+        raise ValueError("T_lag1 (the first-order wrench lag) is not supported as a parameter")
+    if len(set(idx)) != len(idx):
+        raise ValueError("a parameter is selected twice")
+    if not 1 <= len(idx) <= L.NKP:
+        raise ValueError(f"select 1..{L.NKP} parameters")
+    return idx
+
+
+def coefficient_directions(phys: np.ndarray, params, rebuild_minv: bool = True) -> np.ndarray:
+    """Analytic Jacobian [p, NKP] of the kernel coefficients in the selected physical parameters at `phys`: row j is
+    d derive_params(with_minv(phys)) / d phys[params[j]] (without with_minv if rebuild_minv is False).
+    With rebuild_minv, diag(Minv) follows m, the inertias and the added masses as the reference's __init__ computes it,
+    and the Minv entries cannot be parameters; without it they are parameters of their own (the reference freezes
+    Minv at construction, SURVEY trap T5)."""
+    ph = np.asarray(phys, dtype=np.float64).reshape(L.NPHYS)
+    idx = parameter_indices(params)
+    if rebuild_minv and any(L.PH_MINV <= i < L.PH_MINV + 6 for i in idx):
+        raise ValueError("Minv entries follow the masses with rebuild_minv=True: select them with rebuild_minv=False")
+    add = ph[L.PH_ADDED:L.PH_ADDED + 6]
+    a = ph[L.PH_M] - add[:3]                       # m - X_udot, ...
+    b = ph[L.PH_I:L.PH_I + 3] - add[3:]            # Ix - K_pdot, ...
+    D = np.zeros((len(idx), L.NKP))
+    for r, i in enumerate(idx):
+        row, da, db = D[r], np.zeros(3), np.zeros(3)
+        if i == L.PH_M:
+            da[:] = 1.0
+        elif i == L.PH_W:
+            row[KP_WMB] = 1.0
+        elif i == L.PH_B:
+            row[KP_WMB] = -1.0
+            row[KP_XBB:KP_XBB + 3] = ph[L.PH_XB:L.PH_XB + 3]
+        elif L.PH_XB <= i < L.PH_XB + 3:
+            row[KP_XBB + i - L.PH_XB] = ph[L.PH_B]
+        elif L.PH_I <= i < L.PH_I + 3:
+            db[i - L.PH_I] = 1.0
+        elif L.PH_ADDED <= i < L.PH_ADDED + 3:
+            da[i - L.PH_ADDED] = -1.0
+        elif L.PH_ADDED + 3 <= i < L.PH_ADDED + 6:
+            db[i - L.PH_ADDED - 3] = -1.0
+        elif L.PH_LIN <= i < L.PH_LIN + 6:
+            row[KP_DL + i - L.PH_LIN] = -1.0
+        elif L.PH_QUAD <= i < L.PH_QUAD + 6:
+            row[KP_DQ + i - L.PH_QUAD] = -1.0
+        elif L.PH_MINV <= i < L.PH_MINV + 6:
+            row[KP_MINV + i - L.PH_MINV] = 1.0
+        else:                                      # ocean current
+            row[KP_CUR + i - L.PH_CURRENT] = 1.0
+        row[KP_A:KP_A + 3] += da
+        row[KP_DA:KP_DA + 3] += [da[2] - da[1], da[0] - da[2], da[1] - da[0]]
+        row[KP_DB:KP_DB + 3] += [db[2] - db[1], db[0] - db[2], db[1] - db[0]]
+        if rebuild_minv:
+            row[KP_MINV:KP_MINV + 3] -= da / a ** 2
+            row[KP_MINV + 3:KP_MINV + 6] -= db / b ** 2
+    return D
+
+
+@dataclass
+class GradResult:
+    """Endpoint error and its exact derivatives in the selected parameters (Engine.multistep_se_grad)."""
+    se: torch.Tensor                 # [nH] float64: sum over windows of |r_w|^2 per horizon
+    grad: torch.Tensor               # [nH, p]: d se / d theta
+    gn: torch.Tensor                 # [nH, p, p]: Gauss-Newton matrix sum_w J_w^T J_w (exactly symmetric)
+    counts: list                     # windows per horizon
+    names: list                      # parameter names (PHYS_NAMES)
+    index: list                      # their physical-vector indices
+
+
 def default_allocation():
     """(alloc [6,8], r [8,3], dir [8,3]) from the reference's thruster geometry formula."""
     a, r, d = np.zeros((6, 8)), np.zeros((8, 3)), np.zeros((8, 3))
@@ -633,6 +736,91 @@ class Engine:
             for j, h in enumerate(part):
                 out[h] = np.sqrt(se[:, j] / (cnt[j] * self.nx)) if cnt[j] > 0 else np.full(P, np.nan)
         return np.stack([out[h] for h in hs], axis=1) if P else np.zeros((0, len(hs)))
+
+    def multistep_se_grad(self, X, U, horizons: Sequence[int], phys: np.ndarray, params, dt: float = 0.02,
+                          integrator: str = "rk4", lag_mode: str = "reset", lag0=None, rebuild_minv: bool = True,
+                          health_out: Optional[torch.Tensor] = None, singular_eps: float = 0.0,
+                          n_windows: Optional[int] = None, window0: int = 0, row0: int = 0) -> GradResult:
+        """`multistep_se` of the vehicle `phys` together with its exact gradient and Gauss-Newton matrix in the
+        selected physical parameters (brov_multistep_se_grad; forward-mode sensitivities through every integrator
+        step).  params: PH_* indices, attribute names or groups (see parameter_indices); the coefficient directions
+        come from coefficient_directions(phys, params, rebuild_minv), the point is derive_params(with_minv(phys)) (or
+        of phys itself without rebuild_minv).  The engine's own coefficients are not used.  fp64 engines only.
+        lag_mode="carry" (thruster model) makes one call per horizon, as multistep_rmse does.  health_out: int64 [2]
+        device tensor (accumulated over the calls of a carried-lag evaluation).  window0 / row0 / n_windows: a shard
+        of a longer series, as in multistep_se."""
+        X = self.tensor(X)
+        U = self.tensor(U)
+        self._check_rows(X, self.nx, "X")
+        self._check_rows(U, self.nu, "U")
+        rows = X.shape[0]
+        if U.shape[0] != rows:
+            raise ValueError("X and U must have the same number of rows")
+        hs = [int(h) for h in horizons]
+        if not 1 <= len(hs) <= L.MAX_H or any(h < 1 for h in hs) or sorted(set(hs)) != hs:
+            raise ValueError(f"horizons must be 1..{L.MAX_H} strictly ascending positive integers")
+        if lag_mode not in ("reset", "carry"):
+            raise ValueError("lag_mode must be 'reset' or 'carry'")
+        carry = lag_mode == "carry" and self.model == "thruster8"
+        off = int(window0) - int(row0)
+        if off and not carry:
+            raise ValueError("window0 != row0 needs lag_mode='carry'")
+        ph = np.asarray(phys, dtype=np.float64).reshape(L.NPHYS)
+        idx = parameter_indices(params)
+        dirs = coefficient_directions(ph, idx, rebuild_minv)
+        kp = derive_params(with_minv(ph) if rebuild_minv else ph)
+        p = len(idx)
+        any_current = int(bool(np.any(kp[KP_CUR:KP_CUR + 3] != 0.0) or np.any(dirs[:, KP_CUR:KP_CUR + 3] != 0.0)))
+        kp_t = torch.as_tensor(kp, dtype=torch.float64, device=self.device)
+        dirs_t = torch.as_tensor(np.ascontiguousarray(dirs), dtype=torch.float64, device=self.device)
+        if health_out is not None:
+            if health_out.dtype != torch.int64 or health_out.device != self.device or health_out.numel() != 2:
+                raise ValueError("health_out must be an int64 tensor with 2 elements on the engine's device")
+        groups = [[h] for h in hs] if carry else [hs]
+        se = torch.zeros((len(hs),), dtype=torch.float64, device=self.device)
+        grad = torch.zeros((len(hs), p), dtype=torch.float64, device=self.device)
+        gn = torch.zeros((len(hs), p, p), dtype=torch.float64, device=self.device)
+        counts = []
+        hc = health_out
+        if health_out is not None and carry:      # one count over the per-horizon calls
+            health_out.zero_()
+            hc = torch.zeros(2, dtype=torch.int64, device=self.device)
+        for g in groups:
+            nwin = max(rows - off - g[0], 0) if n_windows is None else int(n_windows)
+            nbytes = L.lib.brov_se_grad_workspace_bytes(nwin, p, int(carry))
+            ws = torch.empty(max(nbytes, 1), dtype=torch.uint8, device=self.device)
+            se_o = torch.zeros(L.MAX_H, dtype=torch.float64, device=self.device)
+            gr_o = torch.zeros((L.MAX_H, p), dtype=torch.float64, device=self.device)
+            gn_o = torch.zeros((L.MAX_H, p, p), dtype=torch.float64, device=self.device)
+            cnt = (C.c_longlong * L.MAX_H)()
+            d = L.SeGradDesc()
+            d.struct_size = C.sizeof(L.SeGradDesc)
+            d.integrator = INTEGRATORS[integrator]
+            d.rows, d.n_windows, d.dt = rows, nwin, float(dt)
+            d.X_dev, d.U_dev = X.data_ptr(), U.data_ptr()
+            lag_t = self.tensor(lag0).reshape(nwin, 24) if (lag0 is not None and self.model == "thruster8") else None
+            d.lag0_dev = lag_t.data_ptr() if lag_t is not None else None
+            d.n_horizons = len(g)
+            for i, h in enumerate(g):
+                d.horizons[i] = h
+            d.lag_carry = int(carry)
+            d.window0, d.row0 = (int(window0), int(row0)) if carry else (0, 0)
+            d.kp_dev, d.any_current, d.n_dirs, d.dirs_dev = kp_t.data_ptr(), any_current, p, dirs_t.data_ptr()
+            d.se_out_dev, d.grad_out_dev, d.gn_out_dev = se_o.data_ptr(), gr_o.data_ptr(), gn_o.data_ptr()
+            d.count_out = cnt
+            d.health_dev = hc.data_ptr() if hc is not None else None
+            d.singular_eps = float(singular_eps)
+            d.workspace_dev, d.workspace_bytes = ws.data_ptr(), nbytes
+            with torch.cuda.device(self.device):
+                L.check(L.lib.brov_multistep_se_grad(self._h, C.byref(d), self._stream()))
+            if carry and health_out is not None:
+                health_out += hc
+            at = hs.index(g[0])
+            se[at:at + len(g)] = se_o[:len(g)]
+            grad[at:at + len(g)] = gr_o[:len(g)]
+            gn[at:at + len(g)] = gn_o[:len(g)]
+            counts += [int(cnt[i]) for i in range(len(g))]
+        return GradResult(se=se, grad=grad, gn=gn, counts=counts, names=[PHYS_NAMES[i] for i in idx], index=idx)
 
     # ------------------------------------------------------------------ host-buffer API (end-to-end path)
     def rollout_host(self, x0: np.ndarray, U: Optional[np.ndarray] = None, dt: float = 0.02, integrator: str = "rk4",

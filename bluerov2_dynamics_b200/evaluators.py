@@ -8,10 +8,12 @@ Euler everywhere else); here it is the `integrator` argument.  One kernel launch
 steps (rollout) or the double loop over windows and steps (evaluators)."""
 from __future__ import annotations
 
+from dataclasses import dataclass, field
+
 import numpy as np
 import torch
 
-from .engine import Engine
+from .engine import PHYS_NAMES, Engine, parameter_indices, with_minv
 from .fossen.BlueROV2 import BlueROV2 as _Thruster
 
 
@@ -72,6 +74,126 @@ def multistep_rmse_endpoint_physics_sweep(X_test: np.ndarray, U_test: np.ndarray
     eng = _engine_for(X_test, model, dtype, engine)
     out = eng.multistep_rmse_sweep(X_test, U_test, H, phys_table, dt=dt, integrator=integrator, lag_mode=lag_mode)
     return out[:, 0] if np.isscalar(H) else out
+
+
+@dataclass
+class CalibrationResult:
+    phys: np.ndarray                 # fitted physical vector [NPHYS] (diag(Minv) rebuilt when rebuild_minv)
+    names: list                      # fitted parameters
+    theta: np.ndarray                # their fitted values [p]
+    rmse: dict                       # horizon -> endpoint RMSE of the fitted vehicle
+    gn: np.ndarray                   # final Gauss-Newton matrix of the objective in the parameters [p, p]
+    cost: float                      # final objective
+    cost0: float                     # objective at phys0
+    iterations: int
+    converged: bool
+    history: list = field(default_factory=list)   # per iteration: cost, lam, step_norm, accepted
+
+
+def calibrate_physical(X: np.ndarray, U: np.ndarray, dt: float, phys0: np.ndarray, params, horizons=(1, 10, 100),
+                       weights=None, model: str = None, integrator: str = "rk4", lag_mode: str = "carry",
+                       bounds=None, max_iter: int = 50, tol: float = 1e-10, engine: Engine = None,
+                       rebuild_minv: bool = True, lambdas=(0.1, 1.0, 10.0)) -> CalibrationResult:
+    """Levenberg-Marquardt fit of physical parameters to a recorded series by the reference's endpoint error:
+    minimises  sum_h w_h se_h / (count_h NX)  (the squared endpoint RMSE per horizon, weighted; w_h = 1 by default)
+    over the selected parameters (PH_* indices, attribute names or groups, see engine.parameter_indices), starting
+    from phys0.  Works in relative units theta_j / theta0_j (1 where theta0_j = 0) so that masses, damping terms and
+    currents are on one scale.  Every iteration makes one Engine.multistep_se_grad call (cost, exact gradient, Gauss-
+    Newton matrix) and scores the trial steps of all damping values `lambdas` x lam in one multistep_se_sweep call;
+    the best trial that lowers the cost is taken, otherwise lam grows tenfold.  bounds: (lo, hi) arrays [p] in
+    physical units, enforced by projection.  Stops when the relative cost decrease or the relative step falls below
+    tol, or after max_iter iterations.  fp64 engines only.  Raises FloatingPointError where the error or its derivatives
+    are not finite (windows through the Euler-angle singularity theta = +-pi/2)."""
+    eng = _engine_for(X, model, "f64", engine)
+    if eng.dtype != "f64":
+        raise ValueError("calibrate_physical needs an fp64 engine")
+    hs = sorted(int(h) for h in horizons)
+    w = np.ones(len(hs)) if weights is None else np.asarray(weights, float).reshape(len(hs))
+    idx = parameter_indices(params)
+    ph = np.array(phys0, dtype=np.float64).reshape(-1)
+    if rebuild_minv:
+        ph = with_minv(ph)
+    th0 = ph[idx].copy()
+    scale = np.where(th0 != 0.0, np.abs(th0), 1.0)
+    lo = hi = None
+    if bounds is not None:
+        lo, hi = (np.asarray(b, float).reshape(len(idx)) for b in bounds)
+    carry = lag_mode == "carry" and eng.model == "thruster8"
+    Xt, Ut = eng.tensor(X), eng.tensor(U)
+
+    def vehicle(theta):
+        q = ph.copy()
+        q[idx] = theta
+        return with_minv(q) if rebuild_minv else q
+
+    def project(theta):
+        return theta if lo is None else np.clip(theta, lo, hi)
+
+    def trial_costs(table):
+        tot = np.zeros(table.shape[0])
+        for part in ([[h] for h in hs] if carry else [hs]):
+            se, cnt = eng.multistep_se_sweep(Xt, Ut, part, table, dt=dt, integrator=integrator, lag_mode=lag_mode)
+            se = se.cpu().numpy()
+            for j, h in enumerate(part):
+                if cnt[j] > 0:
+                    tot += w[hs.index(h)] * se[:, j] / (cnt[j] * eng.nx)
+        return np.where(np.isfinite(tot), tot, np.inf)
+
+    health = torch.zeros(2, dtype=torch.int64, device=eng.device)
+
+    def evaluate(theta):
+        r = eng.multistep_se_grad(Xt, Ut, hs, vehicle(theta), idx, dt=dt, integrator=integrator, lag_mode=lag_mode,
+                                  rebuild_minv=rebuild_minv, health_out=health)
+        se, g, G = r.se.cpu().numpy(), r.grad.cpu().numpy(), r.gn.cpu().numpy()
+        c = np.array([w[i] / (r.counts[i] * eng.nx) if r.counts[i] > 0 else 0.0 for i in range(len(hs))])
+        cost, g, G = float(c @ se), c @ g, 2.0 * np.einsum("h,hij->ij", c, G)
+        if not (np.isfinite(cost) and np.all(np.isfinite(g)) and np.all(np.isfinite(G))):
+            n_bad, n_sing = (int(v) for v in health.tolist())
+            raise FloatingPointError(
+                f"the endpoint error or its derivatives are not finite at this vehicle ({n_bad} windows with a "
+                f"non-finite error, {n_sing} within 1e-3 of theta = +-pi/2, where the Euler-angle kinematics and their "
+                "sensitivities blow up): use a series that stays away from the singularity, or the quaternion model")
+        return cost, g, G
+
+    theta = project(th0.copy())
+    cost, g, G = evaluate(theta)
+    cost0, lam, history, converged, it = cost, 1e-3, [], False, 0
+    for it in range(1, max_iter + 1):
+        gz, Gz = g * scale, G * np.outer(scale, scale)           # relative units z = theta / scale
+        dG = np.maximum(np.diag(Gz), 1e-12 * max(np.max(np.diag(Gz)), 1e-300))
+        lams = [lam * f for f in lambdas]
+        steps = []
+        for lm in lams:
+            dz = np.linalg.solve(Gz + lm * np.diag(dG), -gz)
+            steps.append(project(theta + dz * scale))
+        costs = trial_costs(np.stack([vehicle(t) for t in steps]))
+        b = int(np.argmin(costs))
+        accepted = bool(costs[b] < cost)
+        step_norm = float(np.linalg.norm((steps[b] - theta) / scale))
+        history.append(dict(cost=float(costs[b] if accepted else cost), lam=float(lams[b]), step_norm=step_norm,
+                            accepted=accepted))
+        if not accepted:
+            lam *= 10.0
+            if lam > 1e12 or step_norm <= tol:
+                converged = True
+                break
+            continue
+        decrease = (cost - costs[b]) / max(cost, 1e-300)
+        theta = steps[b]
+        lam = max(lams[b] / 10.0, 1e-12)
+        cost, g, G = evaluate(theta)
+        if decrease <= tol or step_norm <= tol:
+            converged = True
+            break
+    fitted = vehicle(theta)
+    rmse = {}
+    for part in ([[h] for h in hs] if carry else [hs]):
+        se, cnt = eng.multistep_se_sweep(Xt, Ut, part, fitted[None], dt=dt, integrator=integrator, lag_mode=lag_mode)
+        se = se.cpu().numpy()[0]
+        for j, h in enumerate(part):
+            rmse[h] = float(np.sqrt(se[j] / (cnt[j] * eng.nx))) if cnt[j] > 0 else float("nan")
+    return CalibrationResult(phys=fitted, names=[PHYS_NAMES[i] for i in idx], theta=theta.copy(), rmse=rmse, gn=G,
+                             cost=cost, cost0=cost0, iterations=it, converged=converged, history=history)
 
 
 def one_step_rmse_physics(X_test: np.ndarray, U_test: np.ndarray, dt: float, model: str = None, dtype: str = "f64",

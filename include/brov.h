@@ -334,6 +334,55 @@ typedef struct brov_se_sweep_desc {
 size_t brov_se_sweep_workspace_bytes(long long n_candidates, long long n_windows, int lag_carry);
 int brov_multistep_se_sweep(brov_engine_t* e, const brov_se_sweep_desc* d, void* stream);
 
+/* Exact derivatives of the evaluator's squared-error sums in the coefficients — what a least-squares calibration of the
+ * hydrodynamic coefficients against a recorded series needs.  With r_w the endpoint residual of window w at horizon
+ * H_h and J_w = d x_end / d theta its sensitivity (forward mode, propagated through the integrator steps):
+ *     se_out_dev[h]          = sum_w |r_w|^2                 (brov_multistep_se's sum, to rounding)
+ *     grad_out_dev[h][j]     = sum_w 2 r_w . J_w[:, j]       (d se_h / d theta_j)
+ *     gn_out_dev[h][i][j]    = sum_w J_w[:, i] . J_w[:, j]   (Gauss-Newton matrix; exactly symmetric)
+ * theta is a point of n_dirs parameters given through the coefficient vector it maps to: kp_dev [BROV_NKP] (double,
+ * dev) is the point, row j of dirs_dev [n_dirs][BROV_NKP] (double, dev) is d kp / d theta_j — any directions, so the
+ * call knows nothing about physical parameters (bluerov2_dynamics_b200.engine.coefficient_directions builds them from
+ * the physical vector).  The engine's own coefficients are neither used nor changed; allocation and lag
+ * discretisation come from the engine.  any_current: non-zero if kp has an ocean current or some direction moves it.
+ * The derivative is that of the computed function, branch taken: d|x| = sign(x) dx, the clamped cos(theta) and the
+ * quaternion fallback have zero derivative.  The thruster map and its lag do not depend on the coefficients.
+ * fp64 engines, Fossen models (thruster8, wrench12, quat13), RK4 / Euler; f32 engines, double-integrator engines and
+ * the first-order wrench lag return BROV_EUNSUPPORTED; 1 <= n_dirs <= BROV_NKP.  Geometry fields (integrator ...
+ * lag_carry, window0, row0), count_out and the health counters (unsigned long long[2], dev, zeroed by the call) as in
+ * brov_se_desc.  The sums are added in a fixed order: bit-reproducible run to run.  workspace_dev: at least
+ * brov_se_grad_workspace_bytes(n_windows, n_dirs, lag_carry) bytes; it does not grow with n_windows except for the
+ * carried lag ([n_windows][18]). */
+typedef struct brov_se_grad_desc {
+    uint32_t struct_size;
+    int32_t integrator;
+    long long rows;
+    long long n_windows;
+    double dt;
+    const void* X_dev;
+    const void* U_dev;
+    const void* lag0_dev;           /* [n_windows][24] or NULL (reset mode) */
+    int32_t n_horizons;
+    int32_t horizons[BROV_MAX_H];
+    int32_t lag_carry;
+    long long window0;
+    long long row0;
+    const double* kp_dev;           /* [BROV_NKP] */
+    int32_t any_current;
+    int32_t n_dirs;
+    const double* dirs_dev;         /* [n_dirs][BROV_NKP] */
+    double* se_out_dev;             /* [BROV_MAX_H] */
+    double* grad_out_dev;           /* [BROV_MAX_H][n_dirs] */
+    double* gn_out_dev;             /* [BROV_MAX_H][n_dirs][n_dirs] */
+    long long* count_out;           /* host [BROV_MAX_H] or NULL */
+    void* health_dev;               /* [2] or NULL */
+    double singular_eps;            /* 0 = 1e-3 */
+    void* workspace_dev;
+    size_t workspace_bytes;
+} brov_se_grad_desc;
+size_t brov_se_grad_workspace_bytes(long long n_windows, int n_dirs, int lag_carry);
+int brov_multistep_se_grad(brov_engine_t* e, const brov_se_grad_desc* d, void* stream);
+
 /* Reduced 9-state RHS — `bluerov_compute(t, x_, u_)` (fossen/bluerov_torch.py:20-67, constants fossen/parameters.py).
  * x [B][9], u [B][4], out [B][9]. */
 int brov_reduced9_rhs(int dtype, const void* x_dev, const void* u_dev, void* out_dev, long long B, void* stream);
