@@ -81,6 +81,13 @@ class SeGradDesc(C.Structure):
                 ("workspace_dev", C.c_void_p), ("workspace_bytes", C.c_size_t)]
 
 
+class LinearizeDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
+                ("dt", C.c_double), ("z0_dev", C.c_void_p), ("u_dev", C.c_void_p), ("u_stride_t", C.c_longlong),
+                ("u_stride_n", C.c_longlong), ("z_out_dev", C.c_void_p), ("z_traj_dev", C.c_void_p),
+                ("jac_dev", C.c_void_p), ("health_dev", C.c_void_p), ("singular_eps", C.c_double)]
+
+
 class RolloutHostDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
                 ("dt", C.c_double), ("x0_host", C.c_void_p), ("xT_host", C.c_void_p), ("u_host", C.c_void_p),
@@ -142,6 +149,7 @@ _PROTOS = {
     "brov_multistep_se_sweep": (C.c_int, [C.c_void_p, C.POINTER(SeSweepDesc), C.c_void_p]),
     "brov_se_grad_workspace_bytes": (C.c_size_t, [C.c_longlong, C.c_int, C.c_int]),
     "brov_multistep_se_grad": (C.c_int, [C.c_void_p, C.POINTER(SeGradDesc), C.c_void_p]),
+    "brov_linearize": (C.c_int, [C.c_void_p, C.POINTER(LinearizeDesc), C.c_void_p]),
     "brov_reduced9_rhs": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "brov_koopman_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_void_p)]),
     "brov_koopman_destroy": (None, [C.c_void_p]),

@@ -14,6 +14,7 @@
 #include "brov_internal.cuh"
 #include "brov_kernels.cuh"
 #include "brov_grad.cuh"
+#include "brov_lin.cuh"
 
 using namespace brov;
 
@@ -1200,6 +1201,42 @@ extern "C" int brov_multistep_se_grad(brov_engine_t* e, const brov_se_grad_desc*
     const size_t need = brov_se_grad_workspace_bytes(d->n_windows, d->n_dirs, d->lag_carry && e->model == BROV_THRUSTER8_LAG3);
     if (!d->workspace_dev || d->workspace_bytes < need) return fail(BROV_EINVAL, "workspace too small: need %zu bytes", need);
     return se_grad_impl(e, d, st);
+}
+
+extern "C" int brov_linearize(brov_engine_t* e, const brov_linearize_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_linearize_desc)) return fail(BROV_EINVAL, "brov_linearize_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "linearize serves the Fossen models, not double-integrator engines");
+    if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the Jacobians are computed in fp64: create the engine with BROV_F64");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "linearize does not support the first-order wrench lag");
+    if (e->pv) return fail(BROV_EUNSUPPORTED, "linearize uses the shared coefficients: clear the per-vehicle table first");
+    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
+    if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
+    if (d->steps < 1 || d->steps > (1LL << 30)) return fail(BROV_EINVAL, "steps = %lld must be 1 .. 2^30", d->steps);
+    if (!(d->dt > 0.0) || !std::isfinite(d->dt)) return fail(BROV_EINVAL, "dt must be a positive finite number");
+    if (!d->jac_dev) return fail(BROV_EINVAL, "jac is NULL");
+    if (!d->z0_dev || !d->u_dev) return fail(BROV_EINVAL, "z0 and u must not be NULL");
+    if (d->u_stride_t < 0 || d->u_stride_n < 0) return fail(BROV_EINVAL, "negative input stride");
+    if (d->n == 0) return BROV_OK;
+    LinArgs a;
+    memset(&a, 0, sizeof(a));
+    int rc = make_consts<double>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c);
+    if (rc) return rc;
+    a.z0 = (const double*)d->z0_dev;
+    a.U = (const double*)d->u_dev;
+    a.ust = d->u_stride_t; a.usn = d->u_stride_n;
+    a.z_out = (double*)d->z_out_dev;
+    a.z_traj = (double*)d->z_traj_dev;
+    a.jac = (double*)d->jac_dev;
+    a.health = (unsigned long long*)d->health_dev;
+    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    a.n = d->n;
+    a.steps = (int)d->steps;
+    CUDA_TRY(cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+    CUDA_TRY(launch_linearize(e->model, d->integrator, a, st));
+    return BROV_OK;
 }
 
 // fossen/parameters.py:3-33

@@ -1,0 +1,234 @@
+// brov_lin.cu — exact Jacobians of the discrete step, A_k = dPhi/dz (z_k, u_k) and B_k = dPhi/du (z_k, u_k), along
+// batched trajectories.
+//
+//   linearize_kernel   one thread per (vehicle, column j of J = [A | B]).  At every step the thread seeds the tangent of
+//                      its column (x.d = e_j for a state column; the body wrench's tangent for a lag or input column),
+//                      takes one dual step from the primal (z_k, u_k), writes column j of J_k and continues with the
+//                      primal z_{k+1}.  The primal is recomputed by every thread of a vehicle (identical arithmetic,
+//                      identical bits), as se_grad_kernel does per direction, so no thread waits on another inside a
+//                      step.  A block stages the J_k of its V vehicles in shared memory and writes it out contiguously.
+//
+// The thruster map and the lag stay outside the dual arithmetic: within a step the lag is a fixed linear filter of the
+// held input, so the wrench's tangent at sub-step s is a per-thread constant and the lag rows of J are closed form.
+// The coefficients carry no tangent: the right-hand side reads them as plain doubles (ParamsConst).
+#include "brov_lin.cuh"
+
+namespace brov {
+
+// a tangent-free operand: no zero tangent to add (ptxas cannot fold x + 0.0)
+__device__ __forceinline__ Dual operator+(Dual a, double b) { return Dual(a.v + b, a.d); }
+__device__ __forceinline__ Dual operator-(Dual a, double b) { return Dual(a.v - b, a.d); }
+
+// dF/dV of the T200 curve F(V) = V p(V^2): 9 a z^4 + 7 b z^3 + 5 c z^2 + 3 d z + e with z = V^2
+__device__ __forceinline__ double thrust_poly_d(const Consts<double>& c, double V) {
+    const double z = V * V;
+    double p = 9.0 * c.poly[0] * z + 7.0 * c.poly[1];
+    p = p * z + 5.0 * c.poly[2];
+    p = p * z + 3.0 * c.poly[3];
+    return p * z + c.poly[4];
+}
+
+// One integrator step with the state as dual numbers.  The body wrench of sub-step s has the value of Fw (thruster: the
+// allocated static thrust, turned into the lagged wrench here; wrench models: the input) and the tangent g_s * tvec,
+// g_s = lagG[s][lagk] for a lag column and lagH[s] otherwise (thruster), 1 (wrench models).  Same stage structure as
+// integrate_step_dual, every stage with full sines and cosines; the lag is not advanced here.
+template <int MODEL, int INTEG>
+__device__ __forceinline__ void integrate_step_lin(const Consts<double>& c, Dual* __restrict__ x,
+                                                   const double* __restrict__ lag, const double* __restrict__ Fw,
+                                                   const double* __restrict__ tvec, int lagk, double& abs_cth) {
+    constexpr int NX = ModelDim<MODEL>::NX;
+    constexpr bool EULER_ANGLES = !ModelDim<MODEL>::QUAT;
+    const ParamsConst<double> p{c.kp};
+    const bool cur = c.has_current != 0;
+    const double dt = c.dt;
+    auto rhs = [&](int s, const Dual* xs, Dual* out) {
+        Dual tau[6];
+        if constexpr (MODEL == MODEL_THRUSTER8) {
+            double t[6];
+            thruster_tau<double, true>(c, s, lag, Fw, t);
+            // lag column (c, k): lagG[s][k] in row c; input column i: lagH[s] alloc[:, i] F'(u_i); state column: 0
+            const double g = lagk == 0 ? c.lagG[s][0] : lagk == 1 ? c.lagG[s][1] : lagk == 2 ? c.lagG[s][2] : c.lagH[s];
+#pragma unroll
+            for (int r = 0; r < 6; ++r) tau[r] = Dual(t[r], g * tvec[r]);
+        } else {
+#pragma unroll
+            for (int r = 0; r < 6; ++r) tau[r] = Dual(Fw[r], tvec[r]);
+        }
+        if constexpr (EULER_ANGLES) {
+            Trig<Dual> tr;
+            trig_full<Dual>(xs + 3, tr);
+            if (s == 0) abs_cth = fabs(tr.cth.v);
+            rhs_euler12<Dual>(xs, tr, tau, p, cur, out);
+        } else {
+            rhs_quat13<Dual>(xs, tau, p, cur, out);
+        }
+    };
+    if constexpr (!EULER_ANGLES) abs_cth = 1.0;
+    Dual k[NX];
+    if constexpr (INTEG == INTEG_EULER) {
+        rhs(0, x, k);
+#pragma unroll
+        for (int i = 0; i < NX; ++i) x[i] += dt * k[i];
+    } else {
+        Dual acc[NX], xs[NX];
+        const double hdt = 0.5 * dt;
+        rhs(0, x, k);
+#pragma unroll
+        for (int s = 1; s <= 3; ++s) {
+            const double w = (s == 1) ? 1.0 : 2.0;
+            const double h = (s == 3) ? dt : hdt;
+#pragma unroll
+            for (int i = 0; i < NX; ++i) {
+                if (s == 1) acc[i] = k[i]; else acc[i] += w * k[i];
+                xs[i] = x[i] + h * k[i];
+            }
+            rhs(s, xs, k);
+        }
+        const double dt6 = dt * (1.0 / 6.0);
+#pragma unroll
+        for (int i = 0; i < NX; ++i) x[i] += dt6 * (acc[i] + k[i]);
+    }
+    if constexpr (ModelDim<MODEL>::QUAT) quat_renorm<Dual>(x + 3);
+}
+
+__device__ __forceinline__ bool finite_(double v) { return fabs(v) <= 1.7976931348623157e308; }
+
+template <int MODEL, int INTEG>
+__global__ void __launch_bounds__(LinDim<MODEL>::THREADS) linearize_kernel(const __grid_constant__ LinArgs a) {
+    using D = LinDim<MODEL>;
+    constexpr int NX = D::NX, NU = D::NU, NZ = D::NZ, NC = D::NC, V = D::V;
+    constexpr bool THR = MODEL == MODEL_THRUSTER8;
+    constexpr int NL = THR ? 18 : 1;
+    constexpr int TILE = V * NZ * NC;
+    __shared__ double tile[TILE];          // [V][NZ][NC]: J_k of the block's vehicles, as laid out in memory
+    __shared__ int flags[V];               // bit 0: non-finite result, bit 1: came near theta = +-pi/2
+    const int tid = threadIdx.x;
+    const int vl = tid / NC, j = tid - vl * NC;
+    const long long v0 = (long long)blockIdx.x * V;
+    const long long v = v0 + vl;
+    const bool act = v < a.n;
+    const int nv = (int)(a.n - v0 < V ? a.n - v0 : V);
+    if (tid < V) flags[tid] = 0;
+    double x[NX], lag[NL];
+#pragma unroll
+    for (int q = 0; q < NX; ++q) x[q] = act ? a.z0[v * NZ + q] : 0.0;
+#pragma unroll
+    for (int q = 0; q < NL; ++q) lag[q] = (THR && act) ? a.z0[v * NZ + NX + q] : 0.0;
+    // column kind: state j < NX, lag column (lc, lagk) for NX <= j < NZ, input column ui = j - NZ
+    const int ui = j - NZ;
+    const int lj = j - NX;
+    const int lc = (THR && lj >= 0 && ui < 0) ? lj / 3 : -1;
+    const int lagk = lc >= 0 ? lj - 3 * lc : -1;
+    bool bad = false, sing = false;
+    for (int k = 0; k < a.steps; ++k) {
+        if (act) {
+            const double* uk = a.U + (long long)k * a.ust + v * a.usn;
+            double u[NU];
+#pragma unroll
+            for (int q = 0; q < NU; ++q) u[q] = uk[q];
+            double Fw[6], tvec[6];
+            if constexpr (THR) {
+                double F[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(a.c, u[i]);
+                allocate_wrench<double>(a.c, F, Fw);
+                // input column: alloc[:, ui] F'(u_ui); lag column: e_lc; state column: 0
+                const double fp = ui >= 0 ? thrust_poly_d(a.c, uk[ui]) : 0.0;
+#pragma unroll
+                for (int r = 0; r < 6; ++r) tvec[r] = ui >= 0 ? a.c.alloc[r][ui] * fp : (r == lc ? 1.0 : 0.0);
+            } else {
+#pragma unroll
+                for (int r = 0; r < 6; ++r) { Fw[r] = u[r]; tvec[r] = r == ui ? 1.0 : 0.0; }
+            }
+            Dual xd[NX];
+#pragma unroll
+            for (int q = 0; q < NX; ++q) xd[q] = Dual(x[q], q == j ? 1.0 : 0.0);
+            double acth;
+            integrate_step_lin<MODEL, INTEG>(a.c, xd, lag, Fw, tvec, lagk, acth);
+            sing |= acth < a.eps;
+            double* col = tile + vl * NZ * NC + j;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) {
+                col[q * NC] = xd[q].d;
+                bad |= !finite_(xd[q].d);
+                x[q] = xd[q].v;
+            }
+            if constexpr (THR) {
+                // dZ'/dx = 0, dZ'/dZ = lagA per channel, dZ'/du_i = lagB (x) alloc[:, i] F'(u_i)
+#pragma unroll
+                for (int cc = 0; cc < 6; ++cc) {
+#pragma unroll
+                    for (int kk = 0; kk < 3; ++kk) {
+                        double jv = 0.0;
+                        if (ui >= 0) jv = a.c.lagB[kk] * tvec[cc];
+                        else if (cc == lc) jv = lagk == 0 ? a.c.lagA[kk][0] : lagk == 1 ? a.c.lagA[kk][1] : a.c.lagA[kk][2];
+                        col[(NX + 3 * cc + kk) * NC] = jv;
+                        bad |= !finite_(jv);
+                    }
+                }
+                lag_advance<double, true>(a.c, lag, Fw);
+            }
+            if (j == 0) {
+#pragma unroll
+                for (int q = 0; q < NX; ++q) bad |= !finite_(x[q]);
+#pragma unroll
+                for (int q = 0; q < NL; ++q) bad |= THR && !finite_(lag[q]);
+                if (a.z_traj) {
+                    double* zt = a.z_traj + ((long long)k * a.n + v) * NZ;
+#pragma unroll
+                    for (int q = 0; q < NX; ++q) zt[q] = x[q];
+                    if constexpr (THR) {
+#pragma unroll
+                        for (int q = 0; q < NL; ++q) zt[NX + q] = lag[q];
+                    }
+                }
+            }
+        }
+        __syncthreads();
+        double* out = a.jac + ((long long)k * a.n + v0) * (NZ * NC);
+        for (int e = tid; e < nv * NZ * NC; e += D::THREADS) out[e] = tile[e];
+        __syncthreads();
+    }
+    if (act && j == 0 && a.z_out) {
+#pragma unroll
+        for (int q = 0; q < NX; ++q) a.z_out[v * NZ + q] = x[q];
+        if constexpr (THR) {
+#pragma unroll
+            for (int q = 0; q < NL; ++q) a.z_out[v * NZ + NX + q] = lag[q];
+        }
+    }
+    if (a.health) {
+        if (act && (bad || sing)) atomicOr(&flags[vl], (bad ? 1 : 0) | (sing && j == 0 ? 2 : 0));
+        __syncthreads();
+        if (tid == 0) {
+            unsigned long long nb = 0, ns = 0;
+            for (int w = 0; w < nv; ++w) { nb += flags[w] & 1; ns += (flags[w] >> 1) & 1; }
+            if (nb) atomicAdd(a.health + 0, nb);
+            if (ns) atomicAdd(a.health + 1, ns);
+        }
+    }
+}
+
+template <int MODEL, int INTEG>
+static cudaError_t linearize_go(const LinArgs& a, cudaStream_t st) {
+    using D = LinDim<MODEL>;
+    const long long grid = (a.n + D::V - 1) / D::V;
+    linearize_kernel<MODEL, INTEG><<<(unsigned)grid, D::THREADS, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+template <int MODEL>
+static cudaError_t linearize_integ(int integ, const LinArgs& a, cudaStream_t st) {
+    return integ == INTEG_RK4 ? linearize_go<MODEL, INTEG_RK4>(a, st) : linearize_go<MODEL, INTEG_EULER>(a, st);
+}
+
+cudaError_t launch_linearize(int model, int integ, const LinArgs& a, cudaStream_t st) {
+    switch (model) {
+        case MODEL_THRUSTER8: return linearize_integ<MODEL_THRUSTER8>(integ, a, st);
+        case MODEL_WRENCH12: return linearize_integ<MODEL_WRENCH12>(integ, a, st);
+        case MODEL_QUAT13: return linearize_integ<MODEL_QUAT13>(integ, a, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+}  // namespace brov

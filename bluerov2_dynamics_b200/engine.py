@@ -159,6 +159,16 @@ class GradResult:
     index: list                      # their physical-vector indices
 
 
+@dataclass
+class LinearizeResult:
+    """Exact Jacobians of every step along N trajectories (Engine.linearize), in projected lag coordinates."""
+    A: torch.Tensor                  # [T, N, NZ, NZ] dz_{k+1} / dz_k   (view of one J [T, N, NZ, NZ+NU])
+    B: torch.Tensor                  # [T, N, NZ, NU] dz_{k+1} / du_k   (view of the same J)
+    z: torch.Tensor                  # [N, NZ] z after the last step
+    z_traj: Optional[torch.Tensor]   # [T, N, NZ] z after every step, or None
+    health: Optional[torch.Tensor]   # int64 [2]: vehicles with a non-finite result / near theta = +-pi/2, or None
+
+
 def default_allocation():
     """(alloc [6,8], r [8,3], dir [8,3]) from the reference's thruster geometry formula."""
     a, r, d = np.zeros((6, 8)), np.zeros((8, 3)), np.zeros((8, 3))
@@ -821,6 +831,98 @@ class Engine:
             gn[at:at + len(g)] = gn_o[:len(g)]
             counts += [int(cnt[i]) for i in range(len(g))]
         return GradResult(se=se, grad=grad, gn=gn, counts=counts, names=[PHYS_NAMES[i] for i in idx], index=idx)
+
+    @property
+    def nz(self) -> int:
+        """Length of the augmented state z that linearize differentiates: x, plus the projected lag [18] (thruster)."""
+        return self.nx + (18 if self.model == "thruster8" else 0)
+
+    def linearize(self, x0, U, dt: float = 0.02, integrator: str = "rk4", lag0=None, lag_repr: str = "thruster",
+                  u_layout: str = "auto", want_traj: bool = True, health: bool = False,
+                  jac_out: Optional[torch.Tensor] = None, singular_eps: float = 0.0) -> LinearizeResult:
+        """Exact Jacobians of the discrete step along N trajectories (brov_linearize): for every step k and vehicle i,
+        A[k, i] = dPhi/dz and B[k, i] = dPhi/du at (z_k, u_k), where z_{k+1} = Phi(z_k, u_k) is one integrator step.
+
+        z = [x | Z]: for the thruster model Z [18] is the allocation-projected lag Z[c][k] = sum_i alloc[c][i] L[i][k]
+        (project_lag), the only form in which the dynamics see the lag; the result is ALWAYS in these projected
+        coordinates (NZ = 30), and per-thruster Jacobians follow by the chain rule with Z = P L.  Wrench models: z = x.
+        lag0 (thruster model): per-thruster [N,24] with lag_repr="thruster" (projected here), or projected [N,18] with
+        lag_repr="projected"; None = zeros.
+
+        U is one of
+          [T,N,NU]  per-vehicle series, time-major   (u_layout "tnc"; the default for a 3-D U)
+          [N,NU]    one step with one input per vehicle (the default for a 2-D U; T = 1)
+          [T,NU]    one series shared by every vehicle (u_layout "shared")
+          (U [N,NU], T) one constant input per vehicle for T steps (u_layout "const")
+        The outputs keep the step axis also for T = 1.  A and B are views of one J [T, N, NZ, NZ+NU] (jac_out, if
+        given: a contiguous float64 tensor of that shape on the engine's device).  The derivative is that of the
+        computed function, branch taken (d|x| = sign(x) dx; the clamped cos(theta) and the quaternion fallback are
+        constants).  health=True returns int64 [2] counts of vehicles with a non-finite z or Jacobian entry and of
+        vehicles that came within singular_eps (0 = 1e-3) of theta = +-pi/2.  fp64 engines with shared coefficients."""
+        x0 = self.tensor(x0)
+        self._check_rows(x0, self.nx, "x0")
+        n = x0.shape[0]
+        if u_layout == "const":
+            Ut, steps = U
+            Ut = self.tensor(Ut)
+            self._check_rows(Ut, self.nu, "U")
+            if Ut.shape[0] != n:
+                raise ValueError(f"U must have shape [{n}, {self.nu}], got {tuple(Ut.shape)}")
+            steps, st, sn = int(steps), 0, self.nu
+        else:
+            Ut = self.tensor(U)
+            if u_layout == "auto":
+                u_layout = "tnc" if Ut.dim() == 3 else "step"
+            if u_layout == "tnc":
+                if Ut.dim() != 3 or Ut.shape[1] != n or Ut.shape[2] != self.nu:
+                    raise ValueError(f"U must have shape [T, {n}, {self.nu}], got {tuple(Ut.shape)}")
+                steps, st, sn = Ut.shape[0], n * self.nu, self.nu
+            elif u_layout == "step":
+                if Ut.dim() != 2 or Ut.shape[0] != n or Ut.shape[1] != self.nu:
+                    raise ValueError(f"U must have shape [{n}, {self.nu}], got {tuple(Ut.shape)}")
+                steps, st, sn = 1, 0, self.nu
+            elif u_layout == "shared":
+                self._check_rows(Ut, self.nu, "U")
+                steps, st, sn = Ut.shape[0], self.nu, 0
+            else:
+                raise ValueError("u_layout must be auto|tnc|shared|const")
+        if lag_repr not in ("thruster", "projected"):
+            raise ValueError("lag_repr must be 'thruster' or 'projected'")
+        nz, nc = self.nz, self.nz + self.nu
+        z0 = x0
+        if self.model == "thruster8":
+            if lag0 is None:
+                Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
+            elif lag_repr == "thruster":
+                Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
+            else:
+                Z0 = self.tensor(lag0).reshape(n, 18)
+            z0 = torch.cat([x0, Z0], dim=1).contiguous()
+        shape = (steps, n, nz, nc)
+        if jac_out is not None:
+            if (not isinstance(jac_out, torch.Tensor) or jac_out.device != self.device or jac_out.dtype != torch.float64
+                    or not jac_out.is_contiguous() or tuple(jac_out.shape) != shape):
+                raise ValueError(f"jac_out must be a contiguous float64 tensor of shape {shape} on {self.device}")
+            J = jac_out
+        else:
+            J = torch.empty(shape, device=self.device, dtype=self.tdtype)
+        z = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
+        zt = torch.empty((steps, n, nz), device=self.device, dtype=self.tdtype) if want_traj else None
+        hc = torch.zeros(2, device=self.device, dtype=torch.int64) if health else None
+        d = L.LinearizeDesc()
+        d.struct_size = C.sizeof(L.LinearizeDesc)
+        d.integrator = INTEGRATORS[integrator]
+        d.n, d.steps, d.dt = n, steps, float(dt)
+        d.z0_dev, d.u_dev = z0.data_ptr(), Ut.data_ptr()
+        d.u_stride_t, d.u_stride_n = st, sn
+        d.z_out_dev = z.data_ptr()
+        d.z_traj_dev = zt.data_ptr() if zt is not None else None
+        d.jac_dev = J.data_ptr()
+        d.health_dev = hc.data_ptr() if hc is not None else None
+        d.singular_eps = float(singular_eps)
+        with torch.cuda.device(self.device):
+            L.check(L.lib.brov_linearize(self._h, C.byref(d), self._stream()))
+        return LinearizeResult(A=J[..., :nz], B=J[..., nz:], z=z, z_traj=zt, health=hc)
 
     # ------------------------------------------------------------------ host-buffer API (end-to-end path)
     def rollout_host(self, x0: np.ndarray, U: Optional[np.ndarray] = None, dt: float = 0.02, integrator: str = "rk4",

@@ -383,6 +383,46 @@ typedef struct brov_se_grad_desc {
 size_t brov_se_grad_workspace_bytes(long long n_windows, int n_dirs, int lag_carry);
 int brov_multistep_se_grad(brov_engine_t* e, const brov_se_grad_desc* d, void* stream);
 
+/* Exact Jacobians of every integrator step along batched trajectories — what LQR / MPC about a trim point, iLQR about
+ * a nominal trajectory or an EKF needs.  With Phi the discrete step of the engine (integrator, dt),
+ *     z_{k+1} = Phi(z_k, u_k),   jac_dev[k][i] = J_k = [A_k | B_k] = [dPhi/dz | dPhi/du] (z_k, u_k)   for vehicle i.
+ * z is the full state the step depends on: z = [x (NX) | Z (18, thruster model only)], with Z[c][k] (c = 0..5, k = 0..2)
+ * the allocation-projected lag (BROV_LAG_PROJECTED, see brov_rollout_desc) in that [6][3] order.  NZ = 30 / 12 / 13 and
+ * NU = 8 / 6 / 6 for thruster8 / wrench12 / quat13; J has NC = NZ + NU columns, state columns first, then the inputs.
+ * Jacobians in per-thruster lag coordinates L [8][3] follow by the chain rule with Z = P L (P = alloc per lag
+ * component); they are rank-deficient there, since the dynamics see L only through Z.
+ * The derivative is that of the computed function, branch taken (as brov_multistep_se_grad): d|x| = sign(x) dx, the
+ * clamped cos(theta) and the quaternion fallback are constants.  Every stage evaluates full sines and cosines, so the
+ * primal z agrees with brov_rollout to rounding, not bit for bit.  The lag rows are closed form: dZ'/dx = 0,
+ * dZ'/dZ = lagA per channel, dZ'/du_i = lagB (x) alloc[:, i] F'(u_i) with F the T200 curve.
+ * The engine's shared coefficients (brov_set_params), allocation and lag discretisation for dt (brov_set_lag_discrete
+ * overrides apply) are used.  fp64 engines, Fossen models, RK4 / Euler; f32 engines, double-integrator engines, the
+ * first-order wrench lag and an engine with a per-vehicle coefficient table (clear it first) return
+ * BROV_EUNSUPPORTED.  steps >= 1; n = 0 is a no-op.
+ *   z0_dev [n][NZ]; u_dev with u_stride_t / u_stride_n as in brov_rollout_desc (per-vehicle, shared or constant);
+ *   z_out_dev [n][NZ] or NULL: z after the last step (may alias z0_dev);
+ *   z_traj_dev [steps][n][NZ] or NULL: z after every step;
+ *   jac_dev [steps][n][NZ][NC] (row-major, so A = J[..., :NZ] and B = J[..., NZ:]);
+ *   health_dev (unsigned long long[2] or NULL, zeroed by the call): vehicles with a non-finite z or Jacobian entry
+ *   in the call / that came within singular_eps (0 = 1e-3) of theta = +-pi/2 at the start of some step.
+ * All arrays double, dev. */
+typedef struct brov_linearize_desc {
+    uint32_t struct_size;       /* = sizeof(brov_linearize_desc) */
+    int32_t integrator;
+    long long n;
+    long long steps;
+    double dt;
+    const void* z0_dev;
+    const void* u_dev;
+    long long u_stride_t, u_stride_n;
+    void* z_out_dev;
+    void* z_traj_dev;
+    void* jac_dev;
+    void* health_dev;
+    double singular_eps;
+} brov_linearize_desc;
+int brov_linearize(brov_engine_t* e, const brov_linearize_desc* d, void* stream);
+
 /* Reduced 9-state RHS — `bluerov_compute(t, x_, u_)` (fossen/bluerov_torch.py:20-67, constants fossen/parameters.py).
  * x [B][9], u [B][4], out [B][9]. */
 int brov_reduced9_rhs(int dtype, const void* x_dev, const void* u_dev, void* out_dev, long long B, void* stream);

@@ -50,6 +50,10 @@ for dtype in ("f64", "f32"):
                 e.rollout(x0, gen=gen, steps=5, dt=dt, lag0=np.full((n, 24), 0.01))
                 e.rollout(x0, gen=gen, steps=70, dt=dt, lag0=np.full((n, 24), 0.01))
                 e.rollout(x0, np.tile(U, (4, 1, 1)), dt=dt, lag0=np.full((n, 24), 0.01))
+            if dtype == "f64":   # step Jacobians: ragged last block of the shared-memory J tile, both integrators
+                for integ in ("rk4", "euler"):
+                    rl = e.linearize(x0[:101], U[:5, :101], dt=dt, integrator=integ, health=True)
+                    assert torch.isfinite(rl.A).all() and int(rl.health[0]) == 0
         e.rhs(x0, U[0])
         e.step(x0, U[0], dt=dt, integrator="euler")
         if model != "thruster8":
