@@ -88,6 +88,18 @@ class LinearizeDesc(C.Structure):
                 ("jac_dev", C.c_void_p), ("health_dev", C.c_void_p), ("singular_eps", C.c_double)]
 
 
+class ClosedLoopDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
+                ("dt", C.c_double), ("z0_dev", C.c_void_p), ("z_out_dev", C.c_void_p), ("K_dev", C.c_void_p),
+                ("K_stride_t", C.c_longlong), ("K_stride_n", C.c_longlong), ("z_ref_dev", C.c_void_p),
+                ("z_ref_stride_t", C.c_longlong), ("z_ref_stride_n", C.c_longlong), ("u_ref_dev", C.c_void_p),
+                ("u_ref_stride_t", C.c_longlong), ("u_ref_stride_n", C.c_longlong), ("u_min", C.c_double * 8),
+                ("u_max", C.c_double * 8), ("q", C.c_double * 30), ("r", C.c_double * 8), ("traj_dev", C.c_void_p),
+                ("u_traj_dev", C.c_void_p), ("stride", C.c_longlong), ("cost_dev", C.c_void_p),
+                ("cost_accumulate", C.c_int32), ("reserved", C.c_int32), ("health_dev", C.c_void_p),
+                ("singular_eps", C.c_double)]
+
+
 class RolloutHostDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
                 ("dt", C.c_double), ("x0_host", C.c_void_p), ("xT_host", C.c_void_p), ("u_host", C.c_void_p),
@@ -150,6 +162,7 @@ _PROTOS = {
     "brov_se_grad_workspace_bytes": (C.c_size_t, [C.c_longlong, C.c_int, C.c_int]),
     "brov_multistep_se_grad": (C.c_int, [C.c_void_p, C.POINTER(SeGradDesc), C.c_void_p]),
     "brov_linearize": (C.c_int, [C.c_void_p, C.POINTER(LinearizeDesc), C.c_void_p]),
+    "brov_closed_loop": (C.c_int, [C.c_void_p, C.POINTER(ClosedLoopDesc), C.c_void_p]),
     "brov_reduced9_rhs": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "brov_koopman_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_void_p)]),
     "brov_koopman_destroy": (None, [C.c_void_p]),

@@ -15,6 +15,7 @@
 #include "brov_kernels.cuh"
 #include "brov_grad.cuh"
 #include "brov_lin.cuh"
+#include "brov_cl.cuh"
 
 using namespace brov;
 
@@ -1237,6 +1238,77 @@ extern "C" int brov_linearize(brov_engine_t* e, const brov_linearize_desc* d, vo
     if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
     CUDA_TRY(launch_linearize(e->model, d->integrator, a, st));
     return BROV_OK;
+}
+
+template <typename T>
+static int closed_loop_impl(brov_engine* e, const brov_closed_loop_desc* d, int nz, int nu, cudaStream_t st) {
+    ClArgs<T> a;
+    memset(&a, 0, sizeof(a));
+    int rc = make_consts<T>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c);
+    if (rc) return rc;
+    a.z0 = (const T*)d->z0_dev;
+    a.z_out = (T*)d->z_out_dev;
+    a.K = (const T*)d->K_dev; a.K_st = d->K_stride_t; a.K_sn = d->K_stride_n;
+    a.zr = (const T*)d->z_ref_dev; a.zr_st = d->z_ref_stride_t; a.zr_sn = d->z_ref_stride_n;
+    a.ur = (const T*)d->u_ref_dev; a.ur_st = d->u_ref_stride_t; a.ur_sn = d->u_ref_stride_n;
+    a.k_smem = (a.K_st == 0 && a.K_sn == 0) ? 1 : 0;
+    if (a.k_smem) a.K_st = 0;
+    a.pv = (const T*)e->pv;
+    a.traj = (T*)d->traj_dev;
+    a.u_traj = (T*)d->u_traj_dev;
+    a.cost = (T*)d->cost_dev;
+    a.cost_accumulate = d->cost_accumulate ? 1 : 0;
+    a.health = (unsigned long long*)d->health_dev;
+    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    for (int r = 0; r < 8; ++r) { a.u_min[r] = (T)d->u_min[r]; a.u_max[r] = (T)d->u_max[r]; a.r[r] = r < nu ? (T)d->r[r] : T(0); }
+    for (int j = 0; j < CL_MAX_NZ; ++j) a.q[j] = j < nz ? (T)d->q[j] : T(0);
+    a.n = d->n;
+    a.steps = (int)d->steps;
+    a.stride = (d->traj_dev || d->u_traj_dev) ? (int)d->stride : 0x7fffffff;
+    a.traj_vec = d->traj_dev && aligned(d->traj_dev, 16) && ((size_t)d->n * nz * sizeof(T)) % 16 == 0;
+    a.u_traj_vec = d->u_traj_dev && aligned(d->u_traj_dev, 16) && ((size_t)d->n * nu * sizeof(T)) % 16 == 0;
+    // Threads per block: 128 once that still gives every SM a block, else 64 or 32 — one thread per vehicle leaves
+    // most SMs idle at small n (4096 vehicles in 128-thread blocks occupy 32 of 148 SMs)
+    int block = 128;
+    while (block > 32 && (d->n + block - 1) / block < e->num_sms) block /= 2;
+    if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+    CUDA_TRY(launch_closed_loop<T>(e->model, d->integrator, block, a, st));
+    return BROV_OK;
+}
+
+extern "C" int brov_closed_loop(brov_engine_t* e, const brov_closed_loop_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_closed_loop_desc)) return fail(BROV_EINVAL, "brov_closed_loop_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "closed_loop serves the Fossen models, not double-integrator engines");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "closed_loop does not support the first-order wrench lag");
+    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
+    if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
+    if (d->steps < 0 || d->steps > (1LL << 30)) return fail(BROV_EINVAL, "steps = %lld must be 0 .. 2^30", d->steps);
+    if (!(d->dt > 0.0) || !std::isfinite(d->dt)) return fail(BROV_EINVAL, "dt must be a positive finite number");
+    if (d->K_stride_t < 0 || d->K_stride_n < 0 || d->z_ref_stride_t < 0 || d->z_ref_stride_n < 0 || d->u_ref_stride_t < 0 ||
+        d->u_ref_stride_n < 0)
+        return fail(BROV_EINVAL, "negative operand stride");
+    const bool thr = e->model == BROV_THRUSTER8_LAG3;
+    const int nz = model_nx(e->model) + (thr ? 18 : 0), nu = model_nu(e->model);
+    for (int r = 0; r < nu; ++r)
+        if (std::isnan(d->u_min[r]) || std::isnan(d->u_max[r]) || d->u_min[r] > d->u_max[r])
+            return fail(BROV_EINVAL, "input bounds of channel %d: u_min = %g, u_max = %g", r, d->u_min[r], d->u_max[r]);
+    if ((d->traj_dev || d->u_traj_dev) && d->stride < 1) return fail(BROV_EINVAL, "stride must be >= 1 with a trajectory buffer");
+    if (e->pv && e->pv_n != d->n) return fail(BROV_EINVAL, "vehicle table has %lld rows, call has n = %lld", e->pv_n, d->n);
+    if (d->n == 0) return BROV_OK;
+    if (!d->z0_dev || !d->z_out_dev) return fail(BROV_EINVAL, "z0 and z_out must not be NULL");
+    if (d->steps > 0 && (!d->K_dev || !d->z_ref_dev || !d->u_ref_dev)) return fail(BROV_EINVAL, "K, z_ref and u_ref must not be NULL");
+    CUDA_TRY(cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d->steps == 0) {
+        const size_t sz = scalar_size(e->dtype);
+        if (d->z_out_dev != d->z0_dev)
+            CUDA_TRY(cudaMemcpyAsync(d->z_out_dev, d->z0_dev, (size_t)d->n * nz * sz, cudaMemcpyDeviceToDevice, st));
+        if (d->cost_dev && !d->cost_accumulate) CUDA_TRY(cudaMemsetAsync(d->cost_dev, 0, (size_t)d->n * sz, st));
+        if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+        return BROV_OK;
+    }
+    return e->dtype == BROV_F32 ? closed_loop_impl<float>(e, d, nz, nu, st) : closed_loop_impl<double>(e, d, nz, nu, st);
 }
 
 // fossen/parameters.py:3-33

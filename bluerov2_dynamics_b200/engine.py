@@ -169,6 +169,19 @@ class LinearizeResult:
     health: Optional[torch.Tensor]   # int64 [2]: vehicles with a non-finite result / near theta = +-pi/2, or None
 
 
+@dataclass
+class ClosedLoopResult:
+    """Closed-loop rollout of N vehicles under affine state feedback (Engine.closed_loop), projected lag coordinates."""
+    z: torch.Tensor                  # [N, NZ] z after the last step
+    z_traj: Optional[torch.Tensor]   # [S, N, NZ] z after steps stride, 2 stride, ..., or None
+    u_traj: Optional[torch.Tensor]   # [S, N, NU] the applied (clamped) input of the step ending at each snapshot, or None
+    cost: Optional[torch.Tensor]     # [N] accumulated stage cost (engine scalar type), or None
+    health: Optional[torch.Tensor]   # int64 [2]: vehicles with a non-finite final z / near theta = +-pi/2, or None
+
+
+_CL_LAYOUTS = ("const_shared", "shared", "const", "tnc")
+
+
 def default_allocation():
     """(alloc [6,8], r [8,3], dir [8,3]) from the reference's thruster geometry formula."""
     a, r, d = np.zeros((6, 8)), np.zeros((8, 3)), np.zeros((8, 3))
@@ -923,6 +936,126 @@ class Engine:
         with torch.cuda.device(self.device):
             L.check(L.lib.brov_linearize(self._h, C.byref(d), self._stream()))
         return LinearizeResult(A=J[..., :nz], B=J[..., nz:], z=z, z_traj=zt, health=hc)
+
+    def _cl_operand(self, v, inner: tuple, layout: str, n: int, what: str):
+        """(tensor, stride_t, stride_n, T or None) of a closed-loop operand with trailing shape `inner`"""
+        t = self.tensor(v)
+        nd = len(inner)
+        if layout == "auto":
+            extra = t.dim() - nd
+            layout = {0: "const_shared", 1: "shared", 2: "tnc"}.get(extra)
+            if layout is None:
+                raise ValueError(f"{what} has {t.dim()} dimensions; expected {nd} to {nd + 2}")
+        if layout not in _CL_LAYOUTS:
+            raise ValueError(f"{what} layout must be auto|" + "|".join(_CL_LAYOUTS))
+        size = int(np.prod(inner))
+        lead = {"const_shared": (), "shared": (None,), "const": (n,), "tnc": (None, n)}[layout]
+        if t.dim() != len(lead) + nd or tuple(t.shape[len(lead):]) != inner or \
+                any(w is not None and t.shape[q] != w for q, w in enumerate(lead)):
+            want = ", ".join(["T" if w is None else str(w) for w in lead] + [str(q) for q in inner])
+            raise ValueError(f"{what} ({layout}) must have shape [{want}], got {tuple(t.shape)}")
+        st, sn = {"const_shared": (0, 0), "shared": (size, 0), "const": (0, size), "tnc": (n * size, size)}[layout]
+        T_ = t.shape[0] if layout in ("shared", "tnc") else None
+        return t, st, sn, T_
+
+    def closed_loop(self, x0, K, z_ref, u_ref, steps: Optional[int] = None, dt: float = 0.02, integrator: str = "rk4",
+                    lag0=None, lag_repr: str = "thruster", k_layout: str = "auto", ref_layout: str = "auto",
+                    u_min=None, u_max=None, stride: int = 0, want_u: bool = False, cost_q=None, cost_r=None,
+                    cost: Optional[torch.Tensor] = None, cost_accumulate: bool = False,
+                    z_out: Optional[torch.Tensor] = None, health: bool = False,
+                    singular_eps: float = 0.0) -> ClosedLoopResult:
+        """Closed-loop rollout of N vehicles with an affine state-feedback law evaluated in the kernel
+        (brov_closed_loop): at every step k, with z_k = [x_k | Z_k] as in `linearize` (NZ = 30 / 12 / 13),
+            dz = z_k - z_ref_k   (Euler-angle models: angles wrapped to (-pi, pi]),
+            u_k = clamp(u_ref_k - K_k dz, u_min, u_max),   z_{k+1} = the rollout's step from z_k under u_k.
+
+        K has rows [NU, NZ] (the K numpy builds from a DARE solution), z_ref [NZ], u_ref [NU].  Each operand has one
+        of four layouts (k_layout / ref_layout; ref_layout applies to z_ref and u_ref):
+          "const_shared" [...]        one value for every vehicle and step
+          "shared"       [T, ...]     time-varying, shared by every vehicle
+          "const"        [N, ...]     constant per vehicle (never chosen by "auto": name it)
+          "tnc"          [T, N, ...]  time-varying per vehicle
+        "auto" picks from the number of dimensions.  T comes from the time-varying operands, which must agree; with
+        none of them give steps=.  lag0 (thruster model): per-thruster [N,24] (lag_repr="thruster") or projected
+        [N,18] (lag_repr="projected"); None = zeros.  The result is always in projected lag coordinates.
+
+        u_min / u_max: scalars or per-channel (default +-1 for thruster8, unbounded for the wrench models).
+        stride > 0 returns z after every stride-th step (z_traj [T//stride, N, NZ]); want_u adds the applied inputs of
+        those steps (u_traj [T//stride, N, NU]).  cost_q [NZ] / cost_r [NU] (diagonal weights) turn on the cost
+        sum_k dz'Q dz + (u_k - u_ref_k)'R (u_k - u_ref_k) per vehicle, written into `cost` if given and added to its
+        values with cost_accumulate (chunked calls add up bit for bit).  The engine's shared coefficients or its
+        per-vehicle table (set_vehicle_physical, N rows) are used."""
+        x0 = self.tensor(x0)
+        self._check_rows(x0, self.nx, "x0")
+        n = x0.shape[0]
+        nz, nu = self.nz, self.nu
+        Kt, kst, ksn, kT = self._cl_operand(K, (nu, nz), k_layout, n, "K")
+        zr, zst, zsn, zT = self._cl_operand(z_ref, (nz,), ref_layout, n, "z_ref")
+        ur, ust, usn, uT = self._cl_operand(u_ref, (nu,), ref_layout, n, "u_ref")
+        Ts = {t for t in (kT, zT, uT) if t is not None}
+        if steps is not None:
+            Ts.add(int(steps))
+        if len(Ts) != 1:
+            raise ValueError("the time-varying operands disagree on T" if Ts else
+                             "no operand is time-varying: give steps=")
+        steps = Ts.pop()
+        if lag_repr not in ("thruster", "projected"):
+            raise ValueError("lag_repr must be 'thruster' or 'projected'")
+        z0 = x0
+        if self.model == "thruster8":
+            if lag0 is None:
+                Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
+            elif lag_repr == "thruster":
+                Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
+            else:
+                Z0 = self.tensor(lag0).reshape(n, 18)
+            z0 = torch.cat([x0, Z0], dim=1).contiguous()
+        lim = 1.0 if self.model == "thruster8" else np.inf
+        lo = np.broadcast_to(np.asarray(-lim if u_min is None else u_min, float), (nu,))
+        hi = np.broadcast_to(np.asarray(lim if u_max is None else u_max, float), (nu,))
+        if z_out is None:
+            z_out = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
+        else:
+            self._check_lag_inout(z_out, n, nz)
+        zt = ut = None
+        if stride:
+            S = steps // int(stride)
+            zt = torch.empty((S, n, nz), device=self.device, dtype=self.tdtype)
+            ut = torch.empty((S, n, nu), device=self.device, dtype=self.tdtype) if want_u else None
+        want_cost = cost is not None or cost_q is not None or cost_r is not None
+        if want_cost:
+            if cost is None:
+                cost = torch.zeros(n, device=self.device, dtype=self.tdtype)
+            self._check_lag_inout(cost, n, 1)
+        hc = torch.zeros(2, device=self.device, dtype=torch.int64) if health else None
+        d = L.ClosedLoopDesc()
+        d.struct_size = C.sizeof(L.ClosedLoopDesc)
+        d.integrator = INTEGRATORS[integrator]
+        d.n, d.steps, d.dt = n, steps, float(dt)
+        d.z0_dev, d.z_out_dev = z0.data_ptr(), z_out.data_ptr()
+        d.K_dev, d.K_stride_t, d.K_stride_n = Kt.data_ptr(), kst, ksn
+        d.z_ref_dev, d.z_ref_stride_t, d.z_ref_stride_n = zr.data_ptr(), zst, zsn
+        d.u_ref_dev, d.u_ref_stride_t, d.u_ref_stride_n = ur.data_ptr(), ust, usn
+        for r in range(nu):
+            d.u_min[r], d.u_max[r] = float(lo[r]), float(hi[r])
+        if cost_q is not None:
+            q = np.broadcast_to(np.asarray(cost_q, float), (nz,))
+            for j in range(nz):
+                d.q[j] = float(q[j])
+        if cost_r is not None:
+            rw = np.broadcast_to(np.asarray(cost_r, float), (nu,))
+            for r in range(nu):
+                d.r[r] = float(rw[r])
+        d.traj_dev = zt.data_ptr() if zt is not None and zt.numel() else None
+        d.u_traj_dev = ut.data_ptr() if ut is not None and ut.numel() else None
+        d.stride = int(stride)
+        d.cost_dev = cost.data_ptr() if want_cost else None
+        d.cost_accumulate = int(bool(cost_accumulate))
+        d.health_dev = hc.data_ptr() if hc is not None else None
+        d.singular_eps = float(singular_eps)
+        with torch.cuda.device(self.device):
+            L.check(L.lib.brov_closed_loop(self._h, C.byref(d), self._stream()))
+        return ClosedLoopResult(z=z_out, z_traj=zt, u_traj=ut, cost=cost if want_cost else None, health=hc)
 
     # ------------------------------------------------------------------ host-buffer API (end-to-end path)
     def rollout_host(self, x0: np.ndarray, U: Optional[np.ndarray] = None, dt: float = 0.02, integrator: str = "rk4",

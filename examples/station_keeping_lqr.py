@@ -6,9 +6,11 @@
    Engine.linearize.
 2. Discrete LQR on the linearisation at the trim (scipy.linalg.solve_discrete_are).
 3. Closed-loop Monte-Carlo: 4096 vehicles start from the trim perturbed by up to +-0.5 m in position, +-0.3 rad in
-   roll / pitch / yaw and +-0.2 m/s (rad/s) in the body rates, and are driven step by step through Engine.step with
-   u = clip(u* - K (z - z*), -1, 1), where z uses the projected lag (Engine.project_lag of the per-thruster state).
-4. Prints the trim residual, the fraction of vehicles that settle and their settling times.
+   roll / pitch / yaw and +-0.2 m/s (rad/s) in the body rates, and run under u = clip(u* - K (z - z*), -1, 1) with the
+   feedback evaluated inside the kernel (Engine.closed_loop, chunks of 100 steps, z after every step for the band).
+4. Robustness: the same LQR on 4096 vehicles whose added masses and linear / quadratic damping are each off by up to
+   +-20 % (a per-vehicle coefficient table, Engine.set_vehicle_physical).
+5. Prints the trim residual, the fraction of vehicles that settle and their settling times.
 
     python examples/station_keeping_lqr.py [--vehicles 4096] [--seconds 30]
 """
@@ -55,6 +57,28 @@ def lag_steady(u, steps=2000):
     return r.lag[0].reshape(8, 3)
 
 
+def settle(e, x, lag24, zs, us, K, steps, chunk=100):
+    """closed loop from (x, per-thruster lag) under u = clip(u* - K (z - z*), -1, 1) in chunks of `chunk` steps;
+    returns (settling times [s] of the vehicles that settle, settled mask)"""
+    n = x.shape[0]
+    inside = torch.zeros((steps, n), dtype=torch.bool, device=e.device)
+    lag, repr_ = lag24, "thruster"
+    zs_t = torch.as_tensor(zs, device=e.device)
+    for k0 in range(0, steps, chunk):
+        m = min(chunk, steps - k0)
+        r = e.closed_loop(x, K, zs, us, steps=m, dt=DT, lag0=lag, lag_repr=repr_, stride=1)
+        x, lag, repr_ = r.z[:, :NX], r.z[:, NX:], "projected"
+        err = (r.z_traj[:, :, :NX] - zs_t[:NX]).abs()
+        err[:, :, 3:6] = torch.remainder(err[:, :, 3:6] + np.pi, 2 * np.pi) - np.pi      # angle error on (-pi, pi]
+        err = err.abs()
+        inside[k0:k0 + m] = (err[..., :3].amax(2) < 0.02) & (err[..., 3:6].amax(2) < 0.02) & (err[..., 6:].amax(2) < 0.02)
+    # settled: inside the band from some step to the end; settling time = first such step
+    stay = torch.flip(torch.cumprod(torch.flip(inside, [0]).to(torch.int32), 0), [0]).bool()
+    settled = stay[-1]
+    first = torch.where(stay.any(0), stay.to(torch.int8).argmax(0), steps)
+    return (first[settled].double() + 1).cpu().numpy() * DT, settled
+
+
 def run(vehicles=4096, seconds=30.0, seed=0, verbose=True):
     e = B.Engine("thruster8", "f64")
     t0 = time.perf_counter()
@@ -75,32 +99,26 @@ def run(vehicles=4096, seconds=30.0, seed=0, verbose=True):
     x[:, 0:3] += rng.uniform(-0.5, 0.5, (n, 3))
     x[:, 3:6] += rng.uniform(-0.3, 0.3, (n, 3))
     x[:, 6:12] += rng.uniform(-0.2, 0.2, (n, 6))
-    dev = e.device
-    xt = torch.as_tensor(x, device=dev)
-    lag = lag_steady(us).reshape(1, 24).repeat(n, 1).contiguous()
-    zs_t = torch.as_tensor(zs, device=dev)
-    us_t = torch.as_tensor(us, device=dev)
-    Kt = torch.as_tensor(K, device=dev)
     steps = int(round(seconds / DT))
-    inside = torch.zeros((steps, n), dtype=torch.bool, device=dev)
-    for k in range(steps):
-        dz = torch.cat([xt, e.project_lag(lag)], dim=1) - zs_t
-        dz[:, 5] = torch.remainder(dz[:, 5] + np.pi, 2 * np.pi) - np.pi       # yaw error on (-pi, pi]
-        u = torch.clamp(us_t - dz @ Kt.T, -1.0, 1.0)
-        xt = e.step(xt, u, lag=lag, dt=DT).xT                                   # lag advanced in place
-        err = torch.cat([xt[:, :3] - zs_t[:3], dz[:, 3:6], xt[:, 6:12]], dim=1).abs()
-        inside[k] = (err[:, :3].amax(1) < 0.02) & (err[:, 3:6].amax(1) < 0.02) & (err[:, 6:].amax(1) < 0.02)
-    # settled: inside the band from some step to the end; settling time = first such step
-    stay = torch.flip(torch.cumprod(torch.flip(inside, [0]).to(torch.int32), 0), [0]).bool()
-    settled = stay[-1]
-    first = torch.where(stay.any(0), stay.to(torch.int8).argmax(0), steps)
-    ts = (first[settled].double() + 1).cpu().numpy() * DT
+    lag = lag_steady(us).reshape(1, 24).repeat(n, 1)
+    ts, settled = settle(e, x, lag, zs, us, K, steps)
+    # robustness: every vehicle's added masses and damping off by up to +-20 %
+    table = np.tile(e.phys, (n, 1))
+    for grp in ("added", "lin", "quad"):
+        idx = B.engine.PARAM_GROUPS[grp]
+        table[:, idx] *= rng.uniform(0.8, 1.2, (n, len(idx)))
+    table = B.with_minv(table)
+    e.set_vehicle_physical(table)
+    ts_pv, settled_pv = settle(e, x, lag, zs, us, K, steps)
+    e.set_vehicle_physical(None)
     wall = time.perf_counter() - t0
     out = dict(trim_residual=resid, newton_iters=iters + 1, newton_residual=float(res), u_trim=us.tolist(),
                closed_loop_spectral_radius=rho, vehicles=n, seconds=seconds,
                settled_fraction=float(settled.float().mean()),
                settling_time_s={"median": float(np.median(ts)), "p95": float(np.percentile(ts, 95)),
                                 "max": float(ts.max())} if ts.size else None,
+               perturbed_settled_fraction=float(settled_pv.float().mean()),
+               perturbed_settling_time_median_s=float(np.median(ts_pv)) if ts_pv.size else None,
                wall_s=wall)
     if verbose:
         print(f"trim at {DEPTH} m depth: {out['newton_iters']} Newton steps, residual |Phi(z*,u*) - z*| = {resid:.3e}")
@@ -111,6 +129,9 @@ def run(vehicles=4096, seconds=30.0, seed=0, verbose=True):
         if ts.size:
             s = out["settling_time_s"]
             print(f"  settling time median {s['median']:.2f} s, p95 {s['p95']:.2f} s, max {s['max']:.2f} s")
+        print(f"same LQR, {n} vehicles with added masses and damping each off by up to +-20 %: "
+              f"{100 * out['perturbed_settled_fraction']:.2f} % settle"
+              + (f", median {out['perturbed_settling_time_median_s']:.2f} s" if ts_pv.size else ""))
         print(f"  wall time {wall:.2f} s")
     return out
 

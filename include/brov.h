@@ -423,6 +423,64 @@ typedef struct brov_linearize_desc {
 } brov_linearize_desc;
 int brov_linearize(brov_engine_t* e, const brov_linearize_desc* d, void* stream);
 
+/* Closed-loop rollouts: an affine state-feedback law evaluated in the kernel at the start of every integrator step —
+ * running an LQR / TVLQR on many vehicles, a robustness Monte-Carlo of a controller over a per-vehicle coefficient
+ * table, scoring a controller without storing trajectories.  For vehicle i and step k = 0 .. steps-1, with
+ * z_k = [x_k | Z_k] as in brov_linearize (NZ = 30 / 12 / 13 and NU = 8 / 6 / 6 for thruster8 / wrench12 / quat13; Z the
+ * allocation-projected lag in [6][3] order):
+ *     dz      = z_k - zr_k        Euler-angle models: dz[3..5] -= 2 pi rint(dz[3..5] / 2 pi); quat13: plain difference
+ *     u_k     = clamp(ur_k - K_k dz, u_min, u_max)   per channel; a NaN stays NaN (compare-select, not fmin / fmax)
+ *     cost   += sum_j q_j dz_j^2 + sum_r r_r (u_k - ur_k)_r^2                       (only with cost_dev)
+ *     z_{k+1} = Phi(z_k, u_k)     the step brov_rollout takes (same integrate_step, projected lag)
+ * The feedback and the cost are evaluated in the engine's scalar type, every sum in a fixed order with fused
+ * multiply-adds, so results are bit-reproducible and independent of the operand layout and of the other vehicles.
+ * Operands (engine scalar type) use the rollout's stride addressing, 64-bit:
+ *     K  [k*K_stride_t + i*K_stride_n + r*NZ + j]        row-major [NU][NZ], the K numpy builds from a DARE solution
+ *     zr [k*z_ref_stride_t + i*z_ref_stride_n + j]
+ *     ur [k*u_ref_stride_t + i*u_ref_stride_n + r]
+ * so each may be constant and shared (both strides 0), time-varying and shared ([steps][...]), constant per vehicle
+ * ([n][...]) or time-varying per vehicle ([steps][n][...]).
+ *   u_min / u_max: per-channel bounds (the first NU used; +-INFINITY for none); q[NZ], r[NU]: diagonal cost weights
+ *   (unused tails ignored);
+ *   z0_dev [n][NZ]; z_out_dev [n][NZ] (required; may alias z0_dev);
+ *   traj_dev [steps / stride][n][NZ] or NULL: z after steps stride, 2 stride, ...;
+ *   u_traj_dev [steps / stride][n][NU] or NULL: the applied (clamped) input of the step that ends at each snapshot;
+ *   cost_dev [n] or NULL: the accumulated cost, added to the incoming values when cost_accumulate (chunked calls add
+ *   up bit for bit), else overwritten;
+ *   health_dev (unsigned long long[2] or NULL, zeroed by the call): vehicles with a non-finite final z / that came
+ *   within singular_eps (0 = 1e-3) of theta = +-pi/2 at the start of some step.
+ * Coefficients: the engine's shared set, or its per-vehicle table (brov_set_vehicle_params, pv_n == n).  RK4 / Euler,
+ * f64 and f32 engines.  Double-integrator engines and the first-order wrench lag return BROV_EUNSUPPORTED.  BROV_EINVAL:
+ * n or steps < 0, dt <= 0, negative strides, NULL K / zr / ur with n * steps > 0, u_min > u_max or a NaN bound, a
+ * trajectory without stride >= 1, a table / n mismatch.  n = 0 is a no-op; steps = 0 copies z0 to z_out (and zeroes
+ * cost_dev unless cost_accumulate). */
+typedef struct brov_closed_loop_desc {
+    uint32_t struct_size;       /* = sizeof(brov_closed_loop_desc) */
+    int32_t integrator;
+    long long n;
+    long long steps;
+    double dt;
+    const void* z0_dev;
+    void* z_out_dev;
+    const void* K_dev;
+    long long K_stride_t, K_stride_n;
+    const void* z_ref_dev;
+    long long z_ref_stride_t, z_ref_stride_n;
+    const void* u_ref_dev;
+    long long u_ref_stride_t, u_ref_stride_n;
+    double u_min[8], u_max[8];
+    double q[30], r[8];
+    void* traj_dev;
+    void* u_traj_dev;
+    long long stride;
+    void* cost_dev;
+    int32_t cost_accumulate;
+    int32_t reserved;
+    void* health_dev;
+    double singular_eps;
+} brov_closed_loop_desc;
+int brov_closed_loop(brov_engine_t* e, const brov_closed_loop_desc* d, void* stream);
+
 /* Reduced 9-state RHS — `bluerov_compute(t, x_, u_)` (fossen/bluerov_torch.py:20-67, constants fossen/parameters.py).
  * x [B][9], u [B][4], out [B][9]. */
 int brov_reduced9_rhs(int dtype, const void* x_dev, const void* u_dev, void* out_dev, long long B, void* stream);

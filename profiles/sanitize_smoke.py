@@ -54,6 +54,12 @@ for dtype in ("f64", "f32"):
                 for integ in ("rk4", "euler"):
                     rl = e.linearize(x0[:101], U[:5, :101], dt=dt, integrator=integ, health=True)
                     assert torch.isfinite(rl.A).all() and int(rl.health[0]) == 0
+            # closed loop: ragged n (partial last warp of the snapshot tiles), per-vehicle time-varying gains, cost
+            nz = e.nz
+            Kc = rng.normal(0, 0.05, (T, 101, nu, nz))
+            rc = e.closed_loop(x0[:101], Kc, np.zeros(nz), np.zeros(nu), dt=dt, stride=2, want_u=True,
+                               cost_q=1.0, cost_r=1.0, health=True, u_min=-1.0, u_max=1.0)
+            assert torch.isfinite(rc.z).all() and int(rc.health[0]) == 0
         e.rhs(x0, U[0])
         e.step(x0, U[0], dt=dt, integrator="euler")
         if model != "thruster8":
