@@ -16,7 +16,8 @@ CPU fallback — importing this package without the built library raises.
 import importlib as _importlib
 
 __all__ = ["Engine", "RolloutResult", "InputGenerator", "BrovError", "default_physical", "derive_params", "default_allocation",
-           "lag_discretize", "with_minv", "coefficient_directions", "parameter_indices", "GradResult", "LinearizeResult", "ClosedLoopResult", "reduced9_rhs",
+           "lag_discretize", "with_minv", "coefficient_directions", "parameter_indices", "GradResult", "LinearizeResult", "ClosedLoopResult", "EkfResult",
+           "reduced9_rhs",
            "fma_peak", "pinned_empty", "install_as_fossen", "LIB_PATH"]
 
 _FROM_LIB = ("BrovError", "LIB_PATH")

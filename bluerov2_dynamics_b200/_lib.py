@@ -100,6 +100,18 @@ class ClosedLoopDesc(C.Structure):
                 ("singular_eps", C.c_double)]
 
 
+class EkfDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
+                ("dt", C.c_double), ("z0_dev", C.c_void_p), ("P0_dev", C.c_void_p), ("u_dev", C.c_void_p),
+                ("u_stride_t", C.c_longlong), ("u_stride_n", C.c_longlong), ("y_dev", C.c_void_p),
+                ("y_stride_t", C.c_longlong), ("y_stride_n", C.c_longlong), ("q_dev", C.c_void_p),
+                ("q_stride_n", C.c_longlong), ("r_dev", C.c_void_p), ("r_stride_n", C.c_longlong),
+                ("z_out_dev", C.c_void_p), ("P_out_dev", C.c_void_p), ("x_traj_dev", C.c_void_p),
+                ("P_traj_dev", C.c_void_p), ("stride", C.c_longlong), ("loglik_dev", C.c_void_p),
+                ("nis_dev", C.c_void_p), ("count_dev", C.c_void_p), ("stats_accumulate", C.c_int32),
+                ("reserved", C.c_int32), ("health_dev", C.c_void_p), ("singular_eps", C.c_double)]
+
+
 class RolloutHostDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
                 ("dt", C.c_double), ("x0_host", C.c_void_p), ("xT_host", C.c_void_p), ("u_host", C.c_void_p),
@@ -163,6 +175,7 @@ _PROTOS = {
     "brov_multistep_se_grad": (C.c_int, [C.c_void_p, C.POINTER(SeGradDesc), C.c_void_p]),
     "brov_linearize": (C.c_int, [C.c_void_p, C.POINTER(LinearizeDesc), C.c_void_p]),
     "brov_closed_loop": (C.c_int, [C.c_void_p, C.POINTER(ClosedLoopDesc), C.c_void_p]),
+    "brov_ekf": (C.c_int, [C.c_void_p, C.POINTER(EkfDesc), C.c_void_p]),
     "brov_reduced9_rhs": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "brov_koopman_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_void_p)]),
     "brov_koopman_destroy": (None, [C.c_void_p]),

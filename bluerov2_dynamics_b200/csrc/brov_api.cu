@@ -1311,6 +1311,90 @@ extern "C" int brov_closed_loop(brov_engine_t* e, const brov_closed_loop_desc* d
     return e->dtype == BROV_F32 ? closed_loop_impl<float>(e, d, nz, nu, st) : closed_loop_impl<double>(e, d, nz, nu, st);
 }
 
+// the noise variances are read back and checked on the host before the launch: q >= 0, r > 0 (a NaN fails both)
+static int check_noise(const void* dev, long long sn, long long n, int nx, bool strict, const char* what, cudaStream_t st) {
+    const size_t cnt = (size_t)(sn ? (n - 1) * sn + nx : nx);
+    std::vector<double> h(cnt);
+    CUDA_TRY(cudaMemcpyAsync(h.data(), dev, cnt * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    for (long long i = 0; i < (sn ? n : 1); ++i)
+        for (int j = 0; j < nx; ++j) {
+            const double v = h[(size_t)(i * sn + j)];
+            if (!(strict ? v > 0.0 : v >= 0.0) || !std::isfinite(v))
+                return fail(BROV_EINVAL, "%s[%lld][%d] = %g must be %s", what, sn ? i : 0LL, j, v,
+                            strict ? "positive and finite" : "non-negative and finite");
+        }
+    return BROV_OK;
+}
+
+extern "C" int brov_ekf(brov_engine_t* e, const brov_ekf_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_ekf_desc)) return fail(BROV_EINVAL, "brov_ekf_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "ekf serves the Fossen models, not double-integrator engines");
+    if (e->model == BROV_WRENCH_QUAT13)
+        return fail(BROV_EUNSUPPORTED, "ekf does not serve quat13: the covariance of a unit quaternion is singular (use wrench12)");
+    if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the filter runs in fp64: create the engine with BROV_F64");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "ekf does not support the first-order wrench lag");
+    if (e->pv) return fail(BROV_EUNSUPPORTED, "ekf uses the shared coefficients: clear the per-vehicle table first");
+    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
+    if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
+    if (d->steps < 0 || d->steps > (1LL << 30)) return fail(BROV_EINVAL, "steps = %lld must be 0 .. 2^30", d->steps);
+    if (!(d->dt > 0.0) || !std::isfinite(d->dt)) return fail(BROV_EINVAL, "dt must be a positive finite number");
+    if (d->u_stride_t < 0 || d->u_stride_n < 0 || d->y_stride_t < 0 || d->y_stride_n < 0 || d->q_stride_n < 0 ||
+        d->r_stride_n < 0)
+        return fail(BROV_EINVAL, "negative operand stride");
+    if ((d->x_traj_dev || d->P_traj_dev) && d->stride < 1) return fail(BROV_EINVAL, "stride must be >= 1 with a trajectory buffer");
+    const bool stats = d->loglik_dev || d->nis_dev || d->count_dev;
+    if (stats && !(d->loglik_dev && d->nis_dev && d->count_dev)) return fail(BROV_EINVAL, "loglik, nis and count go together");
+    if (d->n == 0) return BROV_OK;
+    if (!d->z0_dev || !d->P0_dev || !d->z_out_dev || !d->P_out_dev) return fail(BROV_EINVAL, "z0, P0, z_out and P_out must not be NULL");
+    const int nx = model_nx(e->model), nz = nx + (e->model == BROV_THRUSTER8_LAG3 ? 18 : 0);
+    CUDA_TRY(cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d->steps == 0) {
+        if (d->z_out_dev != d->z0_dev)
+            CUDA_TRY(cudaMemcpyAsync(d->z_out_dev, d->z0_dev, (size_t)d->n * nz * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        if (d->P_out_dev != d->P0_dev)
+            CUDA_TRY(cudaMemcpyAsync(d->P_out_dev, d->P0_dev, (size_t)d->n * nx * nx * sizeof(double), cudaMemcpyDeviceToDevice, st));
+        if (stats && !d->stats_accumulate) {
+            CUDA_TRY(cudaMemsetAsync(d->loglik_dev, 0, (size_t)d->n * sizeof(double), st));
+            CUDA_TRY(cudaMemsetAsync(d->nis_dev, 0, (size_t)d->n * sizeof(double), st));
+            CUDA_TRY(cudaMemsetAsync(d->count_dev, 0, (size_t)d->n * sizeof(long long), st));
+        }
+        if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+        return BROV_OK;
+    }
+    if (!d->u_dev || !d->y_dev || !d->q_dev || !d->r_dev) return fail(BROV_EINVAL, "u, y, q and r must not be NULL");
+    int rc = check_noise(d->q_dev, d->q_stride_n, d->n, nx, false, "q", st);
+    if (rc) return rc;
+    if ((rc = check_noise(d->r_dev, d->r_stride_n, d->n, nx, true, "r", st))) return rc;
+    EkfArgs a;
+    memset(&a, 0, sizeof(a));
+    if ((rc = make_consts<double>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c))) return rc;
+    a.z0 = (const double*)d->z0_dev;
+    a.P0 = (const double*)d->P0_dev;
+    a.U = (const double*)d->u_dev; a.ust = d->u_stride_t; a.usn = d->u_stride_n;
+    a.Y = (const double*)d->y_dev; a.yst = d->y_stride_t; a.ysn = d->y_stride_n;
+    a.q = (const double*)d->q_dev; a.qsn = d->q_stride_n;
+    a.r = (const double*)d->r_dev; a.rsn = d->r_stride_n;
+    a.z_out = (double*)d->z_out_dev;
+    a.P_out = (double*)d->P_out_dev;
+    a.x_traj = (double*)d->x_traj_dev;
+    a.P_traj = (double*)d->P_traj_dev;
+    a.loglik = (double*)d->loglik_dev;
+    a.nis = (double*)d->nis_dev;
+    a.count = (long long*)d->count_dev;
+    a.accumulate = d->stats_accumulate ? 1 : 0;
+    a.health = (unsigned long long*)d->health_dev;
+    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    a.n = d->n;
+    a.steps = (int)d->steps;
+    a.stride = (d->x_traj_dev || d->P_traj_dev) ? (int)std::min<long long>(d->stride, 0x7fffffffLL) : 0x7fffffff;
+    if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+    CUDA_TRY(launch_ekf(e->model, d->integrator, a, st));
+    return BROV_OK;
+}
+
 // fossen/parameters.py:3-33
 template <typename T> static Red9Consts<T> red9_consts() {
     const double m = 11.4, g = 9.82, F_bouy = 1026 * 0.0115 * g;

@@ -231,4 +231,213 @@ cudaError_t launch_linearize(int model, int integ, const LinArgs& a, cudaStream_
     return cudaErrorInvalidValue;
 }
 
+// ekf_kernel   one thread per (filter, state column j), NX threads per filter.  At every step thread j takes the dual
+//              step seeded along e_j (the primal is recomputed identically by every thread of the filter, as in
+//              linearize_kernel) and writes column j of A_k into shared memory.  Thread i then forms row i of A P and
+//              the upper triangle of row i of A P A^T + diag(q), mirrored, so P stays exactly symmetric.  The scalar
+//              updates run over the measured components in order; each writes the Joseph-form P into the other half
+//              of a per-filter ping-pong buffer.  Every thread of a block executes the same barrier sequence: a filter
+//              with nothing measured at component m skips the arithmetic, not the barrier.
+template <int MODEL, int INTEG>
+__global__ void __launch_bounds__(EkfDim<MODEL>::THREADS) ekf_kernel(const __grid_constant__ EkfArgs a) {
+    using D = EkfDim<MODEL>;
+    constexpr int NX = D::NX, NU = D::NU, NZ = D::NZ, V = D::V, NN = NX * NX;
+    constexpr bool THR = MODEL == MODEL_THRUSTER8;
+    constexpr int NL = THR ? 18 : 1;
+    constexpr double TWO_PI = 6.283185307179586, INV_2PI = 0.15915494309189535, LOG_2PI = 1.8378770664093453;
+    __shared__ double sA[V * NN];          // [V][NX][NX]: A_k of the block's filters
+    __shared__ double sP[2 * V * NN];      // [2][V][NX][NX]: P and the temporary, swapped by the updates
+    __shared__ int flags[V];               // bit 0: non-finite result, bit 1: came near theta = +-pi/2
+    const int tid = threadIdx.x;
+    const int fl = tid / NX, j = tid - fl * NX;
+    const long long f = (long long)blockIdx.x * V + fl;
+    const bool act = f < a.n;
+    const int nv = (int)(a.n - (long long)blockIdx.x * V < V ? a.n - (long long)blockIdx.x * V : V);
+    if (tid < V) flags[tid] = 0;
+    double* A = sA + fl * NN;
+    int cur = 0;                           // which half of sP holds this filter's P (the same in all its threads)
+    double x[NX], lag[NL];
+#pragma unroll
+    for (int q = 0; q < NX; ++q) x[q] = act ? a.z0[f * NZ + q] : 0.0;
+#pragma unroll
+    for (int q = 0; q < NL; ++q) lag[q] = (THR && act) ? a.z0[f * NZ + NX + q] : 0.0;
+    if (act) {
+#pragma unroll
+        for (int c = 0; c < NX; ++c) sP[fl * NN + j * NX + c] = a.P0[f * NN + j * NX + c];
+    }
+    const double qj = act ? a.q[f * a.qsn + j] : 0.0;
+    const double* rf = a.r + (act ? f : 0) * a.rsn;
+    double ll = 0.0, nis = 0.0;
+    long long cnt = 0;
+    if (a.loglik && a.accumulate && act) { ll = a.loglik[f]; nis = a.nis[f]; cnt = a.count[f]; }
+    bool sing = false;
+    int countdown = a.stride;
+    long long snap = 0;
+    const double zero6[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    for (int k = 0; k < a.steps; ++k) {
+        // predict: the primal step and column j of A_k
+        if (act) {
+            const double* uk = a.U + (long long)k * a.ust + f * a.usn;
+            double Fw[6];
+            if constexpr (THR) {
+                double F[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(a.c, uk[i]);
+                allocate_wrench<double>(a.c, F, Fw);
+            } else {
+#pragma unroll
+                for (int r = 0; r < NU; ++r) Fw[r] = uk[r];
+            }
+            Dual xd[NX];
+#pragma unroll
+            for (int q = 0; q < NX; ++q) xd[q] = Dual(x[q], q == j ? 1.0 : 0.0);
+            double acth;
+            integrate_step_lin<MODEL, INTEG>(a.c, xd, lag, Fw, zero6, -1, acth);
+            sing |= acth < a.eps;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) {
+                A[q * NX + j] = xd[q].d;
+                x[q] = xd[q].v;
+            }
+            if constexpr (THR) lag_advance<double, true>(a.c, lag, Fw);
+        }
+        __syncthreads();
+        if (act) {   // row j of A P into the free half
+            const double* P = sP + cur * V * NN + fl * NN;
+            double* Tm = sP + (cur ^ 1) * V * NN + fl * NN;
+#pragma unroll
+            for (int c = 0; c < NX; ++c) {
+                double s = 0.0;
+#pragma unroll
+                for (int q = 0; q < NX; ++q) s = fma(A[j * NX + q], P[q * NX + c], s);
+                Tm[j * NX + c] = s;
+            }
+        }
+        __syncthreads();
+        if (act) {   // row j of (A P) A^T + diag(q), upper triangle, mirrored
+            double* P = sP + cur * V * NN + fl * NN;
+            const double* Tm = sP + (cur ^ 1) * V * NN + fl * NN;
+#pragma unroll
+            for (int c = 0; c < NX; ++c) {
+                if (c < j) continue;
+                double s = 0.0;
+#pragma unroll
+                for (int q = 0; q < NX; ++q) s = fma(Tm[j * NX + q], A[c * NX + q], s);
+                if (c == j) s += qj;
+                P[j * NX + c] = s;
+                P[c * NX + j] = s;
+            }
+        }
+        __syncthreads();
+        // update: one scalar measurement per component, in order
+        const double* yk = a.Y + (long long)k * a.yst + f * a.ysn;
+#pragma unroll
+        for (int m = 0; m < NX; ++m) {
+            const double y = act ? yk[m] : 0.0;
+            if (act && finite_(y)) {
+                const double* P = sP + cur * V * NN + fl * NN;
+                double* Pn = sP + (cur ^ 1) * V * NN + fl * NN;
+                const double rm = rf[m];
+                double nu = y - x[m];
+                if (m >= 3 && m < 6) nu = fma(-TWO_PI, rint(nu * INV_2PI), nu);
+                const double pmm = P[m * NX + m];
+                const double s = pmm + rm;
+                const double inv_s = 1.0 / s;   // one division per update: g = P[:, m] (1 / s)
+                double g[NX];
+#pragma unroll
+                for (int c = 0; c < NX; ++c) {
+                    g[c] = P[m * NX + c] * inv_s;
+                    x[c] = fma(g[c], nu, x[c]);
+                }
+                // Joseph form: (I - g e_m^T) P (I - g e_m^T)^T + r g g^T, entry (j, c)
+                const double gj = P[m * NX + j] * inv_s;
+                const double kjm = P[j * NX + m] - gj * pmm;
+#pragma unroll
+                for (int c = 0; c < NX; ++c) {
+                    if (c < j) continue;
+                    const double v = (P[j * NX + c] - gj * P[m * NX + c]) - kjm * g[c] + rm * gj * g[c];
+                    Pn[j * NX + c] = v;
+                    Pn[c * NX + j] = v;
+                }
+                const double e2 = nu * nu * inv_s;
+                ll -= 0.5 * (e2 + log(s) + LOG_2PI);
+                nis += e2;
+                ++cnt;
+                cur ^= 1;
+            }
+            __syncthreads();
+        }
+        if (--countdown == 0) {
+            countdown = a.stride;
+            if (act) {
+                const double* P = sP + cur * V * NN + fl * NN;
+                if (a.x_traj) {
+                    double xj = x[0];   // x[j] without a dynamically indexed (local-memory) array
+#pragma unroll
+                    for (int q = 1; q < NX; ++q) xj = q == j ? x[q] : xj;
+                    a.x_traj[(snap * a.n + f) * NX + j] = xj;
+                }
+                if (a.P_traj) {
+                    double* pt = a.P_traj + ((snap * a.n + f) * NX + j) * NX;
+#pragma unroll
+                    for (int c = 0; c < NX; ++c) pt[c] = P[j * NX + c];
+                }
+            }
+            ++snap;
+        }
+    }
+    bool bad = false;
+    if (act) {
+        const double* P = sP + cur * V * NN + fl * NN;
+#pragma unroll
+        for (int c = 0; c < NX; ++c) {
+            a.P_out[f * NN + j * NX + c] = P[j * NX + c];
+            bad |= !finite_(P[j * NX + c]);
+        }
+        if (j == 0) {
+#pragma unroll
+            for (int q = 0; q < NX; ++q) {
+                a.z_out[f * NZ + q] = x[q];
+                bad |= !finite_(x[q]);
+            }
+            if constexpr (THR) {
+#pragma unroll
+                for (int q = 0; q < NL; ++q) {
+                    a.z_out[f * NZ + NX + q] = lag[q];
+                    bad |= !finite_(lag[q]);
+                }
+            }
+            if (a.loglik) { a.loglik[f] = ll; a.nis[f] = nis; a.count[f] = cnt; }
+        }
+    }
+    if (a.health) {
+        if (act && (bad || sing)) atomicOr(&flags[fl], (bad ? 1 : 0) | (sing && j == 0 ? 2 : 0));
+        __syncthreads();
+        if (tid == 0) {
+            unsigned long long nb = 0, ns = 0;
+            for (int w = 0; w < nv; ++w) { nb += flags[w] & 1; ns += (flags[w] >> 1) & 1; }
+            if (nb) atomicAdd(a.health + 0, nb);
+            if (ns) atomicAdd(a.health + 1, ns);
+        }
+    }
+}
+
+template <int MODEL, int INTEG>
+static cudaError_t ekf_go(const EkfArgs& a, cudaStream_t st) {
+    using D = EkfDim<MODEL>;
+    const long long grid = (a.n + D::V - 1) / D::V;
+    ekf_kernel<MODEL, INTEG><<<(unsigned)grid, D::THREADS, 0, st>>>(a);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_ekf(int model, int integ, const EkfArgs& a, cudaStream_t st) {
+    switch (model) {
+        case MODEL_THRUSTER8:
+            return integ == INTEG_RK4 ? ekf_go<MODEL_THRUSTER8, INTEG_RK4>(a, st) : ekf_go<MODEL_THRUSTER8, INTEG_EULER>(a, st);
+        case MODEL_WRENCH12:
+            return integ == INTEG_RK4 ? ekf_go<MODEL_WRENCH12, INTEG_RK4>(a, st) : ekf_go<MODEL_WRENCH12, INTEG_EULER>(a, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
 }  // namespace brov

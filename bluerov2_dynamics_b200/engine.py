@@ -179,6 +179,19 @@ class ClosedLoopResult:
     health: Optional[torch.Tensor]   # int64 [2]: vehicles with a non-finite final z / near theta = +-pi/2, or None
 
 
+@dataclass
+class EkfResult:
+    """N extended Kalman filters run over one measurement series each (Engine.ekf), projected lag coordinates."""
+    z: torch.Tensor                  # [N, NZ] the estimate z = [x | Z] after the last step
+    P: torch.Tensor                  # [N, NX, NX] its covariance (exactly symmetric)
+    x_traj: Optional[torch.Tensor]   # [S, N, NX] the state estimate after steps stride, 2 stride, ..., or None
+    P_traj: Optional[torch.Tensor]   # [S, N, NX, NX] the covariance at the same steps (want_cov), or None
+    loglik: torch.Tensor             # [N] float64 log-likelihood of the measurements
+    nis: torch.Tensor                # [N] float64 sum of the normalised innovations squared
+    count: torch.Tensor              # [N] int64 number of scalar measurements used
+    health: Optional[torch.Tensor]   # int64 [2]: filters with a non-finite z or P / near theta = +-pi/2, or None
+
+
 _CL_LAYOUTS = ("const_shared", "shared", "const", "tnc")
 
 
@@ -1056,6 +1069,138 @@ class Engine:
         with torch.cuda.device(self.device):
             L.check(L.lib.brov_closed_loop(self._h, C.byref(d), self._stream()))
         return ClosedLoopResult(z=z_out, z_traj=zt, u_traj=ut, cost=cost if want_cost else None, health=hc)
+
+    def ekf(self, x0, P0, U, Y, q, r, dt: float = 0.02, integrator: str = "rk4", lag0=None, lag_repr: str = "thruster",
+            u_layout: str = "auto", y_layout: str = "auto", stride: int = 0, want_cov: bool = False, stats=None,
+            stats_accumulate: bool = False, health: bool = False, singular_eps: float = 0.0) -> EkfResult:
+        """N extended Kalman filters on the engine's model (brov_ekf), each over its own measurement series: at every
+        step k the prediction x- = Phi(z_k, u_k), P- = A_k P_k A_k^T + diag(q) with the exact step Jacobian A_k of
+        `linearize`, then one scalar update per component j with a finite Y[k, j] (NaN = not measured), in order:
+            nu = y_j - x-_j (angles wrapped to one turn), s = P-_jj + r_j, g = P-[:, j] / s,
+            x- += g nu, P- = (I - g e_j') P- (I - g e_j')' + r_j g g'  (Joseph form),
+            loglik -= (nu^2 / s + log s + log 2 pi) / 2, nis += nu^2 / s, count += 1.
+        Y[k] measures the state AFTER the step taken with U[k]: for a recorded series X, U pass x0 = X[0],
+        U = U[:-1], Y = X[1:].  The covariance covers x only (NX = 12); the projected lag is a deterministic filter
+        of the inputs.  A non-finite Y entry (NaN, and also +-inf) is not measured.  q and r are checked on the host
+        before the launch, so the call synchronises the engine's stream.  fp64 engines with shared coefficients,
+        thruster8 and wrench12.
+
+        x0 [N, NX]; lag0 (thruster model): per-thruster [N,24] (lag_repr="thruster") or projected [N,18]
+        (lag_repr="projected"); None = zeros.  P0: [NX, NX] (one matrix for every filter), [N, NX, NX], or the
+        diagonal [NX] / [N, NX] (a 2-D [NX, NX] P0 is always a full matrix).
+        U: "tnc" [T, N, NU] (the default for 3-D), "shared" [T, NU] (the default for 2-D), or "const" [N, NU].
+        Y: "tnc" [T, N, NX] (the default for 3-D) or "shared" [T, NX] (the default for 2-D); T comes from Y.
+        q, r: diagonal process / measurement noise variances, [NX] shared or [N, NX] per filter; q >= 0, r > 0.
+        stride > 0 returns x after every stride-th step (x_traj [T//stride, N, NX]), and with want_cov P at the same
+        steps (P_traj).  stats: (loglik, nis, count) tensors ([N] float64, float64, int64 on the engine's device)
+        to write into; with stats_accumulate the call adds to their values, so that chunked calls (carrying z and P)
+        add up bit for bit."""
+        x0 = self.tensor(x0)
+        self._check_rows(x0, self.nx, "x0")
+        n, nx, nz, nu = x0.shape[0], self.nx, self.nz, self.nu
+        Yt = self.tensor(Y)
+        if y_layout == "auto":
+            y_layout = "tnc" if Yt.dim() == 3 else "shared"
+        if y_layout == "tnc":
+            if Yt.dim() != 3 or Yt.shape[1] != n or Yt.shape[2] != nx:
+                raise ValueError(f"Y must have shape [T, {n}, {nx}], got {tuple(Yt.shape)}")
+            yst, ysn = n * nx, nx
+        elif y_layout == "shared":
+            self._check_rows(Yt, nx, "Y")
+            yst, ysn = nx, 0
+        else:
+            raise ValueError("y_layout must be auto|tnc|shared")
+        steps = Yt.shape[0]
+        Ut = self.tensor(U)
+        if u_layout == "auto":
+            u_layout = "tnc" if Ut.dim() == 3 else "shared"
+        if u_layout == "tnc":
+            if Ut.dim() != 3 or Ut.shape[1] != n or Ut.shape[2] != nu:
+                raise ValueError(f"U must have shape [T, {n}, {nu}], got {tuple(Ut.shape)}")
+            ust, usn = n * nu, nu
+        elif u_layout == "shared":
+            self._check_rows(Ut, nu, "U")
+            ust, usn = nu, 0
+        elif u_layout == "const":
+            if Ut.dim() != 2 or Ut.shape[0] != n or Ut.shape[1] != nu:
+                raise ValueError(f"U must have shape [{n}, {nu}], got {tuple(Ut.shape)}")
+            ust, usn = 0, nu
+        else:
+            raise ValueError("u_layout must be auto|tnc|shared|const")
+        if u_layout != "const" and Ut.shape[0] != steps:
+            raise ValueError(f"U has {Ut.shape[0]} steps and Y {steps}")
+
+        def noise(v, what):
+            t = self.tensor(v)
+            if t.dim() == 1 and t.shape[0] == nx:
+                return t, 0
+            if t.dim() == 2 and tuple(t.shape) == (n, nx):
+                return t, nx
+            raise ValueError(f"{what} must have shape [{nx}] or [{n}, {nx}], got {tuple(t.shape)}")
+        qt, qsn = noise(q, "q")
+        rt, rsn = noise(r, "r")
+        P0t = self.tensor(P0)
+        if P0t.dim() == 2 and tuple(P0t.shape) == (nx, nx):
+            P0t = P0t.expand(n, nx, nx)
+        elif P0t.dim() == 1 and P0t.shape[0] == nx:
+            P0t = torch.diag_embed(P0t.expand(n, nx))
+        elif P0t.dim() == 2 and tuple(P0t.shape) == (n, nx):
+            P0t = torch.diag_embed(P0t)
+        elif P0t.dim() != 3 or tuple(P0t.shape) != (n, nx, nx):
+            raise ValueError(f"P0 must have shape [{nx}, {nx}], [{n}, {nx}, {nx}], [{nx}] or [{n}, {nx}], "
+                             f"got {tuple(P0t.shape)}")
+        P0t = P0t.contiguous()
+        if lag_repr not in ("thruster", "projected"):
+            raise ValueError("lag_repr must be 'thruster' or 'projected'")
+        z0 = x0
+        if self.model == "thruster8":
+            if lag0 is None:
+                Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
+            elif lag_repr == "thruster":
+                Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
+            else:
+                Z0 = self.tensor(lag0).reshape(n, 18)
+            z0 = torch.cat([x0, Z0], dim=1).contiguous()
+        if stats is None:
+            if stats_accumulate:
+                raise ValueError("stats_accumulate needs stats=(loglik, nis, count)")
+            ll = torch.empty(n, device=self.device, dtype=torch.float64)
+            ni = torch.empty(n, device=self.device, dtype=torch.float64)
+            cnt = torch.empty(n, device=self.device, dtype=torch.int64)
+        else:
+            ll, ni, cnt = stats
+            for t, dty, what in ((ll, torch.float64, "loglik"), (ni, torch.float64, "nis"), (cnt, torch.int64, "count")):
+                if (not isinstance(t, torch.Tensor) or t.device != self.device or t.dtype != dty
+                        or not t.is_contiguous() or tuple(t.shape) != (n,)):
+                    raise ValueError(f"stats {what} must be a contiguous {dty} tensor of shape [{n}] on {self.device}")
+        z = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
+        P = torch.empty((n, nx, nx), device=self.device, dtype=self.tdtype)
+        xt = Pt = None
+        if stride:
+            S = steps // int(stride)
+            xt = torch.empty((S, n, nx), device=self.device, dtype=self.tdtype)
+            Pt = torch.empty((S, n, nx, nx), device=self.device, dtype=self.tdtype) if want_cov else None
+        hc = torch.zeros(2, device=self.device, dtype=torch.int64) if health else None
+        d = L.EkfDesc()
+        d.struct_size = C.sizeof(L.EkfDesc)
+        d.integrator = INTEGRATORS[integrator]
+        d.n, d.steps, d.dt = n, steps, float(dt)
+        d.z0_dev, d.P0_dev = z0.data_ptr(), P0t.data_ptr()
+        d.u_dev, d.u_stride_t, d.u_stride_n = Ut.data_ptr(), ust, usn
+        d.y_dev, d.y_stride_t, d.y_stride_n = Yt.data_ptr(), yst, ysn
+        d.q_dev, d.q_stride_n = qt.data_ptr(), qsn
+        d.r_dev, d.r_stride_n = rt.data_ptr(), rsn
+        d.z_out_dev, d.P_out_dev = z.data_ptr(), P.data_ptr()
+        d.x_traj_dev = xt.data_ptr() if xt is not None and xt.numel() else None
+        d.P_traj_dev = Pt.data_ptr() if Pt is not None and Pt.numel() else None
+        d.stride = int(stride)
+        d.loglik_dev, d.nis_dev, d.count_dev = ll.data_ptr(), ni.data_ptr(), cnt.data_ptr()
+        d.stats_accumulate = int(bool(stats_accumulate))
+        d.health_dev = hc.data_ptr() if hc is not None else None
+        d.singular_eps = float(singular_eps)
+        with torch.cuda.device(self.device):
+            L.check(L.lib.brov_ekf(self._h, C.byref(d), self._stream()))
+        return EkfResult(z=z, P=P, x_traj=xt, P_traj=Pt, loglik=ll, nis=ni, count=cnt, health=hc)
 
     # ------------------------------------------------------------------ host-buffer API (end-to-end path)
     def rollout_host(self, x0: np.ndarray, U: Optional[np.ndarray] = None, dt: float = 0.02, integrator: str = "rk4",

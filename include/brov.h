@@ -481,6 +481,75 @@ typedef struct brov_closed_loop_desc {
 } brov_closed_loop_desc;
 int brov_closed_loop(brov_engine_t* e, const brov_closed_loop_desc* d, void* stream);
 
+/* Extended Kalman filters on the Fossen models — state estimation from noisy or partial measurements of the state
+ * components (depth, attitude, gyro, DVL, position fixes, each at its own rate), a Monte-Carlo consistency check over
+ * many noise realisations, one filter per candidate noise setting scored by likelihood, a fleet of vehicles.
+ * For filter i, with z = [x | Z] as in brov_linearize (NX = 12; Z the allocation-projected lag, thruster model only)
+ * and k = 0 .. steps-1:
+ *   predict   x- = Phi_x(x_k, Z_k, u_k),  Z_{k+1} = Phi_Z(Z_k, u_k)   (the step brov_linearize takes)
+ *             P- = A_k P_k A_k^T + diag(q)                          A_k = dx'/dx at (z_k, u_k), NX x NX
+ *   update    for j = 0 .. NX-1 with y_k[j] finite, in that order (a NaN marks a component not measured at this
+ *             step; +-inf is treated the same way, so a sensor that reports inf for a fault is skipped, not applied):
+ *             nu = y_k[j] - x-[j]      (j = 3, 4, 5: wrapped to one turn, nu -= 2 pi rint(nu / 2 pi), as in
+ *                                       brov_closed_loop)
+ *             s = P-[j][j] + r[j];     g = P-[:, j] (1 / s)    (one division; nu^2 / s below likewise)
+ *             x- += g nu;              P- <- (I - g e_j^T) P- (I - g e_j^T)^T + r[j] g g^T      (Joseph form)
+ *             loglik -= (nu^2 / s + log s + log 2 pi) / 2;   nis += nu^2 / s;   count += 1
+ *   x_{k+1} = x-,  P_{k+1} = P-
+ * The measurement model is a selection of state components with diagonal R, so the sequential scalar updates are the
+ * joint Kalman update and loglik is the exact Gaussian log-likelihood of the measured components.  y_k measures the
+ * state AFTER the step taken with u_k.  The covariance covers x only: Z is a deterministic filter of the known inputs.
+ * Only the upper triangle of every P is computed; it is mirrored, so P is exactly symmetric.  Every sum has a fixed
+ * order, so results are bit-reproducible and independent of the operand layout and of the other filters.
+ * Operands use the rollout's stride addressing, 64-bit:
+ *   u [k*u_stride_t + i*u_stride_n + c]   y [k*y_stride_t + i*y_stride_n + j]   (per-filter, shared or constant)
+ *   q [i*q_stride_n + j], r [i*r_stride_n + j]   (q_stride_n / r_stride_n = 0: one set shared by every filter)
+ *   z0_dev [n][NZ]; P0_dev [n][NX][NX]; z_out_dev [n][NZ] and P_out_dev [n][NX][NX] (required; may alias z0 / P0);
+ *   x_traj_dev [steps / stride][n][NX] or NULL: x after steps stride, 2 stride, ...;
+ *   P_traj_dev [steps / stride][n][NX][NX] or NULL: P at the same steps;
+ *   loglik_dev [n], nis_dev [n] (double), count_dev [n] (int64): all three or none; added to the incoming values when
+ *   stats_accumulate (chunked calls add up bit for bit), else overwritten;
+ *   health_dev (unsigned long long[2] or NULL, zeroed by the call): filters with a non-finite final z or P / that came
+ *   within singular_eps (0 = 1e-3) of theta = +-pi/2 at the start of some step.
+ * The engine's shared coefficients, allocation and lag discretisation for dt are used.  fp64 engines, thruster8 and
+ * wrench12, RK4 / Euler.  quat13 (the covariance of a unit quaternion is singular), double-integrator engines, the
+ * first-order wrench lag, f32 engines and an engine with a per-vehicle coefficient table return BROV_EUNSUPPORTED.
+ * BROV_EINVAL: n or steps < 0, dt <= 0, negative strides, q < 0 or r <= 0 (NaN included), NULL required pointers with
+ * n * steps > 0, a trajectory without stride >= 1.  n = 0 is a no-op; steps = 0 copies z0 and P0 to the outputs (and
+ * zeroes the statistics unless stats_accumulate).  Before the launch the call copies q and r to the host to check
+ * them and synchronises `stream` for that copy, so it blocks the calling thread and cannot be captured in a CUDA
+ * graph.  All arrays dev. */
+typedef struct brov_ekf_desc {
+    uint32_t struct_size;       /* = sizeof(brov_ekf_desc) */
+    int32_t integrator;
+    long long n;
+    long long steps;
+    double dt;
+    const void* z0_dev;
+    const void* P0_dev;
+    const void* u_dev;
+    long long u_stride_t, u_stride_n;
+    const void* y_dev;
+    long long y_stride_t, y_stride_n;
+    const void* q_dev;
+    long long q_stride_n;
+    const void* r_dev;
+    long long r_stride_n;
+    void* z_out_dev;
+    void* P_out_dev;
+    void* x_traj_dev;
+    void* P_traj_dev;
+    long long stride;
+    void* loglik_dev;
+    void* nis_dev;
+    void* count_dev;
+    int32_t stats_accumulate;
+    int32_t reserved;
+    void* health_dev;
+    double singular_eps;
+} brov_ekf_desc;
+int brov_ekf(brov_engine_t* e, const brov_ekf_desc* d, void* stream);
+
 /* Reduced 9-state RHS — `bluerov_compute(t, x_, u_)` (fossen/bluerov_torch.py:20-67, constants fossen/parameters.py).
  * x [B][9], u [B][4], out [B][9]. */
 int brov_reduced9_rhs(int dtype, const void* x_dev, const void* u_dev, void* out_dev, long long B, void* stream);

@@ -60,6 +60,15 @@ for dtype in ("f64", "f32"):
             rc = e.closed_loop(x0[:101], Kc, np.zeros(nz), np.zeros(nu), dt=dt, stride=2, want_u=True,
                                cost_q=1.0, cost_r=1.0, health=True, u_min=-1.0, u_max=1.0)
             assert torch.isfinite(rc.z).all() and int(rc.health[0]) == 0
+            if dtype == "f64" and model != "quat13":
+                # extended Kalman filters: partial last block, NaN measurement masks, per-filter q and r, P snapshots
+                Ye = x0[:101] + 0.01 * rng.standard_normal((T, 101, nx))
+                Ye[rng.random(Ye.shape) < 0.5] = np.nan
+                for integ in ("rk4", "euler"):
+                    re_ = e.ekf(x0[:101], np.eye(nx) * 0.01, U[:, :101], Ye, rng.uniform(1e-6, 1e-4, (101, nx)),
+                                rng.uniform(1e-4, 1e-3, (101, nx)), dt=dt, integrator=integ, stride=4, want_cov=True,
+                                health=True)
+                    assert torch.isfinite(re_.P).all() and int(re_.health[0]) == 0
         e.rhs(x0, U[0])
         e.step(x0, U[0], dt=dt, integrator="euler")
         if model != "thruster8":
