@@ -17,6 +17,7 @@ import importlib as _importlib
 
 __all__ = ["Engine", "RolloutResult", "InputGenerator", "BrovError", "default_physical", "derive_params", "default_allocation",
            "lag_discretize", "with_minv", "coefficient_directions", "parameter_indices", "GradResult", "LinearizeResult", "ClosedLoopResult", "EkfResult",
+           "VjpResult",
            "reduced9_rhs",
            "fma_peak", "pinned_empty", "install_as_fossen", "LIB_PATH"]
 

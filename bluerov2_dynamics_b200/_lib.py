@@ -112,6 +112,15 @@ class EkfDesc(C.Structure):
                 ("reserved", C.c_int32), ("health_dev", C.c_void_p), ("singular_eps", C.c_double)]
 
 
+class RolloutVjpDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
+                ("dt", C.c_double), ("z0_dev", C.c_void_p), ("u_dev", C.c_void_p), ("u_stride_t", C.c_longlong),
+                ("u_stride_n", C.c_longlong), ("gtraj_dev", C.c_void_p), ("stride", C.c_longlong),
+                ("gzT_dev", C.c_void_p), ("gz0_dev", C.c_void_p), ("gu_dev", C.c_void_p), ("z_out_dev", C.c_void_p),
+                ("workspace_dev", C.c_void_p), ("workspace_bytes", C.c_size_t), ("health_dev", C.c_void_p),
+                ("singular_eps", C.c_double)]
+
+
 class RolloutHostDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
                 ("dt", C.c_double), ("x0_host", C.c_void_p), ("xT_host", C.c_void_p), ("u_host", C.c_void_p),
@@ -176,6 +185,8 @@ _PROTOS = {
     "brov_linearize": (C.c_int, [C.c_void_p, C.POINTER(LinearizeDesc), C.c_void_p]),
     "brov_closed_loop": (C.c_int, [C.c_void_p, C.POINTER(ClosedLoopDesc), C.c_void_p]),
     "brov_ekf": (C.c_int, [C.c_void_p, C.POINTER(EkfDesc), C.c_void_p]),
+    "brov_rollout_vjp": (C.c_int, [C.c_void_p, C.POINTER(RolloutVjpDesc), C.c_void_p]),
+    "brov_rollout_vjp_workspace_bytes": (C.c_size_t, [C.c_int, C.c_longlong, C.c_longlong]),
     "brov_reduced9_rhs": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "brov_koopman_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_void_p)]),
     "brov_koopman_destroy": (None, [C.c_void_p]),

@@ -19,7 +19,7 @@ CSRC = os.path.join(PKG, "csrc")
 OUT = os.path.join(PKG, "libbrov.so")
 BUILD = os.path.join(PKG, "build")
 SOURCES = ["brov_api.cu", "brov_kernels_f32.cu", "brov_kernels_f64.cu", "brov_koopman.cu", "brov_pinc.cu", "brov_grad.cu",
-           "brov_lin.cu", "brov_cl.cu"]
+           "brov_lin.cu", "brov_cl.cu", "brov_adj.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]
 

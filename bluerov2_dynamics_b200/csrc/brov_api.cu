@@ -16,6 +16,7 @@
 #include "brov_grad.cuh"
 #include "brov_lin.cuh"
 #include "brov_cl.cuh"
+#include "brov_adj.cuh"
 
 using namespace brov;
 
@@ -1392,6 +1393,54 @@ extern "C" int brov_ekf(brov_engine_t* e, const brov_ekf_desc* d, void* stream) 
     a.stride = (d->x_traj_dev || d->P_traj_dev) ? (int)std::min<long long>(d->stride, 0x7fffffffLL) : 0x7fffffff;
     if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
     CUDA_TRY(launch_ekf(e->model, d->integrator, a, st));
+    return BROV_OK;
+}
+
+extern "C" size_t brov_rollout_vjp_workspace_bytes(int model, long long n, long long steps) {
+    if (model != BROV_THRUSTER8_LAG3 && model != BROV_WRENCH_EULER12 && model != BROV_WRENCH_QUAT13) return 0;
+    const int nz = model_nx(model) + (model == BROV_THRUSTER8_LAG3 ? 18 : 0);
+    return adjoint_workspace_bytes(nz, n, steps);
+}
+
+extern "C" int brov_rollout_vjp(brov_engine_t* e, const brov_rollout_vjp_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_rollout_vjp_desc)) return fail(BROV_EINVAL, "brov_rollout_vjp_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "rollout_vjp serves the Fossen models, not double-integrator engines");
+    if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the gradients are computed in fp64: create the engine with BROV_F64");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "rollout_vjp does not support the first-order wrench lag");
+    if (e->pv) return fail(BROV_EUNSUPPORTED, "rollout_vjp uses the shared coefficients: clear the per-vehicle table first");
+    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
+    if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
+    if (d->steps < 1 || d->steps > (1LL << 30)) return fail(BROV_EINVAL, "steps = %lld must be 1 .. 2^30", d->steps);
+    if (!(d->dt > 0.0) || !std::isfinite(d->dt)) return fail(BROV_EINVAL, "dt must be a positive finite number");
+    if (d->u_stride_t < 0 || d->u_stride_n < 0) return fail(BROV_EINVAL, "negative input stride");
+    if (d->gtraj_dev && d->stride < 1) return fail(BROV_EINVAL, "stride must be >= 1 with a trajectory cotangent");
+    if (d->n == 0) return BROV_OK;
+    if (!d->z0_dev || !d->u_dev || !d->gz0_dev || !d->gu_dev) return fail(BROV_EINVAL, "z0, u, gz0 and gu must not be NULL");
+    const size_t need = brov_rollout_vjp_workspace_bytes(e->model, d->n, d->steps);
+    if (!d->workspace_dev || d->workspace_bytes < need) return fail(BROV_EINVAL, "workspace too small: need %zu bytes", need);
+    AdjArgs a;
+    memset(&a, 0, sizeof(a));
+    int rc = make_consts<double>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c);
+    if (rc) return rc;
+    a.z0 = (const double*)d->z0_dev;
+    a.U = (const double*)d->u_dev;
+    a.ust = d->u_stride_t; a.usn = d->u_stride_n;
+    a.gtraj = (const double*)d->gtraj_dev;
+    a.gzT = (const double*)d->gzT_dev;
+    a.gz0 = (double*)d->gz0_dev;
+    a.gU = (double*)d->gu_dev;
+    a.z_out = (double*)d->z_out_dev;
+    a.ws = (double*)d->workspace_dev;
+    a.health = (unsigned long long*)d->health_dev;
+    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    a.n = d->n;
+    a.steps = (int)d->steps;
+    a.stride = d->gtraj_dev ? (int)std::min<long long>(d->stride, 0x7fffffffLL) : 1;
+    CUDA_TRY(cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+    CUDA_TRY(launch_adjoint(e->model, d->integrator, a, st));
     return BROV_OK;
 }
 

@@ -218,6 +218,15 @@ template <typename T> __device__ __forceinline__ T thrust_poly(const Consts<T>& 
     }
 }
 
+// dF/dV of the T200 curve F(V) = V p(V^2): 9 a z^4 + 7 b z^3 + 5 c z^2 + 3 d z + e with z = V^2
+__device__ __forceinline__ double thrust_poly_d(const Consts<double>& c, double V) {
+    const double z = V * V;
+    double p = 9.0 * c.poly[0] * z + 7.0 * c.poly[1];
+    p = p * z + 5.0 * c.poly[2];
+    p = p * z + 3.0 * c.poly[3];
+    return p * z + c.poly[4];
+}
+
 // nu_dot = Minv (tau - C(nu) nu - D(nu_r) nu_r - g); g from (sin th, cos th sin phi, cos th cos phi).
 // Every axis is ONE chain of fused multiply-adds onto tau_i: the Coriolis terms (closed form of C_RB + C_A times nu,
 // fossen/BlueROV2.py:280-325), the restoring terms (:340-355) and the damping term (:327-338) are accumulated with
@@ -248,6 +257,38 @@ __device__ __forceinline__ void nu_dot(const T* __restrict__ nu, const T* __rest
         T d = p[KP_DQ + i] * abs_(nur[i]) + p[KP_DL + i];
         out[i] = p[KP_MINV + i] * (t[i] - d * nur[i]);
     }
+}
+
+// Reverse mode of nu_dot (fp64): g[6] is the cotangent of out.  Returns the cotangents of nu (gnu), of nur (gnur), of
+// the three restoring-term inputs (sth, cs, cc) and of tau (gtau).  Branch taken: d|x| = sign(x) dx, sign(0) = 0.
+template <class P>
+__device__ __forceinline__ void nu_dot_vjp(const double* __restrict__ nu, const double* __restrict__ nur, const P& p,
+                                           const double* __restrict__ g, double* __restrict__ gnu,
+                                           double* __restrict__ gnur, double& gsth, double& gcs, double& gcc,
+                                           double* __restrict__ gtau) {
+    const double u = nu[0], v = nu[1], w = nu[2], pp = nu[3], q = nu[4], r = nu[5];
+    const double a1u = p[KP_A + 0] * u, a2v = p[KP_A + 1] * v, a3w = p[KP_A + 2] * w;
+    const double wmb = p[KP_WMB], xbB = p[KP_XBB + 0], ybB = p[KP_XBB + 1], zbB = p[KP_XBB + 2];
+    double e[6];   // cotangent of t[i] (= of tau[i])
+#pragma unroll
+    for (int i = 0; i < 6; ++i) {
+        e[i] = p[KP_MINV + i] * g[i];
+        gtau[i] = e[i];
+        // d(d_i nur_i) / d nur_i = 2 DQ_i |nur_i| + DL_i
+        const double s = nur[i] > 0.0 ? 1.0 : (nur[i] < 0.0 ? -1.0 : 0.0);
+        const double dd = p[KP_DQ + i] * abs_(nur[i]) + p[KP_DL + i] + p[KP_DQ + i] * s * nur[i];
+        gnur[i] = -e[i] * dd;
+    }
+    const double ga1u = q * e[2] - r * e[1], ga2v = r * e[0] - pp * e[2], ga3w = pp * e[1] - q * e[0];
+    gnu[0] = p[KP_A + 0] * ga1u - p[KP_DA + 1] * w * e[4] - p[KP_DA + 2] * v * e[5];
+    gnu[1] = p[KP_A + 1] * ga2v - p[KP_DA + 0] * w * e[3] - p[KP_DA + 2] * u * e[5];
+    gnu[2] = p[KP_A + 2] * ga3w - p[KP_DA + 0] * v * e[3] - p[KP_DA + 1] * u * e[4];
+    gnu[3] = a3w * e[1] - a2v * e[2] - p[KP_DB + 1] * r * e[4] - p[KP_DB + 2] * q * e[5];
+    gnu[4] = a1u * e[2] - a3w * e[0] - p[KP_DB + 0] * r * e[3] - p[KP_DB + 2] * pp * e[5];
+    gnu[5] = a2v * e[0] - a1u * e[1] - p[KP_DB + 0] * q * e[3] - p[KP_DB + 1] * pp * e[4];
+    gsth = zbB * e[4] - wmb * e[0] - ybB * e[5];
+    gcs = wmb * e[1] + zbB * e[3] - xbB * e[5];
+    gcc = wmb * e[2] - ybB * e[3] + xbB * e[4];
 }
 
 // Euler-angle models: xdot[12] from x[12] and the body wrench tau[6].
@@ -367,6 +408,94 @@ __device__ __forceinline__ void rhs_euler12(const T* __restrict__ x, const Trig<
     nu_dot<T>(nu, nur, tau, sth, cth * sphi, cth * cphi, p, xd + 6);
 }
 
+// Reverse mode of rhs_euler12 (fp64) at (x, tau) with the sines and cosines tr of x[3..5]: g[12] is the cotangent of
+// xd; a[12] receives the cotangent of x and gtau[6] that of tau.  Same convention as the dual instantiation of
+// rhs_euler12: the clamped cos(theta) (|c| < 1e-7) is a constant, otherwise d(1/c) = -dc / c^2.
+template <class P>
+__device__ __forceinline__ void rhs_euler12_vjp(const double* __restrict__ x, const Trig<double>& tr,
+                                                const P& p, bool has_current, const double* __restrict__ g,
+                                                double* __restrict__ a, double* __restrict__ gtau) {
+    const double sphi = tr.sphi, cphi = tr.cphi, sth = tr.sth, cth = tr.cth, spsi = tr.spsi, cpsi = tr.cpsi;
+    const double* nu = x + 6;
+    double nur[6] = {nu[0], nu[1], nu[2], nu[3], nu[4], nu[5]};
+    double cx = 0.0, cy = 0.0, cz = 0.0, x1 = 0.0, y1 = 0.0, z2 = 0.0;
+    if (has_current) {
+        cx = p[KP_CUR + 0]; cy = p[KP_CUR + 1]; cz = p[KP_CUR + 2];
+        x1 = cpsi * cx + spsi * cy;
+        y1 = cpsi * cy - spsi * cx;
+        const double x2 = cth * x1 - sth * cz;
+        z2 = sth * x1 + cth * cz;
+        const double y3 = cphi * y1 + sphi * z2;
+        const double z3 = cphi * z2 - sphi * y1;
+        nur[0] -= x2;
+        nur[1] -= y3;
+        nur[2] -= z3;
+    }
+    double gnu[6], gnur[6], gsth, gcs, gcc;
+    nu_dot_vjp(nu, nur, p, g + 6, gnu, gnur, gsth, gcs, gcc, gtau);
+    double gsphi = cth * gcs, gcphi = cth * gcc, gcth = sphi * gcs + cphi * gcc, gspsi = 0.0, gcpsi = 0.0;
+#pragma unroll
+    for (int i = 0; i < 6; ++i) gnu[i] += gnur[i];
+    if (has_current) {   // nur[0..2] -= (x2, y3, z3)
+        const double gx2 = -gnur[0], gy3 = -gnur[1], gz3 = -gnur[2];
+        const double gy1 = cphi * gy3 - sphi * gz3;
+        const double gz2 = sphi * gy3 + cphi * gz3;
+        gcphi += y1 * gy3 + z2 * gz3;
+        gsphi += z2 * gy3 - y1 * gz3;
+        const double gx1 = cth * gx2 + sth * gz2;
+        gcth += x1 * gx2 + cz * gz2;
+        gsth += x1 * gz2 - cz * gx2;
+        gcpsi += cx * gx1 + cy * gy1;
+        gspsi += cy * gx1 - cx * gy1;
+    }
+    // Euler rates
+    {
+        double ic;
+        const bool clamped = fabs(cth) < 1e-7;
+        if (clamped) {
+            const double ct = (cth > 0.0) ? 1e-7 : ((cth < 0.0) ? -1e-7 : 0.0);
+            ic = (ct == 0.0) ? (double)INFINITY : rcp_nr(ct);
+        } else {
+            ic = rcp_nr(cth);
+        }
+        const double sq = sphi * nu[4] + cphi * nu[5];
+        const double psd = sq * ic;
+        gnu[3] += g[3];
+        gsth += psd * g[3];
+        const double gpsd = g[5] + sth * g[3];
+        const double gsq = ic * gpsd;
+        if (!clamped) gcth -= ic * ic * (sq * gpsd);
+        gsphi += nu[4] * gsq - nu[5] * g[4];
+        gcphi += nu[5] * gsq + nu[4] * g[4];
+        gnu[4] += sphi * gsq + cphi * g[4];
+        gnu[5] += cphi * gsq - sphi * g[4];
+    }
+    // p_dot = Rz(psi) Ry(theta) Rx(phi) nu_1
+    {
+        const double v1 = cphi * nu[1] - sphi * nu[2];
+        const double w1 = sphi * nu[1] + cphi * nu[2];
+        const double u2 = cth * nu[0] + sth * w1;
+        const double gu2 = cpsi * g[0] + spsi * g[1];
+        const double gv1 = cpsi * g[1] - spsi * g[0];
+        gcpsi += u2 * g[0] + v1 * g[1];
+        gspsi += u2 * g[1] - v1 * g[0];
+        const double gw1 = cth * g[2] + sth * gu2;
+        gnu[0] += cth * gu2 - sth * g[2];
+        gcth += w1 * g[2] + nu[0] * gu2;
+        gsth += w1 * gu2 - nu[0] * g[2];
+        gnu[1] += cphi * gv1 + sphi * gw1;
+        gnu[2] += cphi * gw1 - sphi * gv1;
+        gcphi += nu[1] * gv1 + nu[2] * gw1;
+        gsphi += nu[1] * gw1 - nu[2] * gv1;
+    }
+    a[0] = 0.0; a[1] = 0.0; a[2] = 0.0;
+    a[3] = cphi * gsphi - sphi * gcphi;
+    a[4] = cth * gsth - sth * gcth;
+    a[5] = cpsi * gspsi - spsi * gcpsi;
+#pragma unroll
+    for (int i = 0; i < 6; ++i) a[6 + i] = gnu[i];
+}
+
 // Quaternion model: xdot[13] from x[13] = [pos, qw qx qy qz, nu] (fossen/BlueROV2_wrench.py:322-367).
 template <typename T, class P>
 __device__ __forceinline__ void rhs_quat13(const T* __restrict__ x, const T* __restrict__ tau, const P& p,
@@ -398,6 +527,89 @@ __device__ __forceinline__ void rhs_quat13(const T* __restrict__ x, const T* __r
         nur[2] -= R02 * cx + R12 * cy + R22 * cz;
     }
     nu_dot<T>(nu, nur, tau, -R20, R21, R22, p, xd + 7);
+}
+
+// Reverse mode of the normalisation q -> q / |q| at a raw q with |q| >= 1e-12: g[4] (cotangent of the unit
+// quaternion) is replaced by that of the raw one, (g - y (y . g)) / |q| with y = q / |q|.  Below 1e-12 the fallback
+// (1, 0, 0, 0) is a constant: the cotangent is zero.
+__device__ __forceinline__ void quat_normalize_vjp(const double* __restrict__ q, double* __restrict__ g) {
+    const double n = sqrt(q[0] * q[0] + q[1] * q[1] + q[2] * q[2] + q[3] * q[3]);
+    if (n < 1e-12) { g[0] = g[1] = g[2] = g[3] = 0.0; return; }
+    const double in = rcp_nr(n);
+    const double y0 = q[0] * in, y1 = q[1] * in, y2 = q[2] * in, y3 = q[3] * in;
+    const double yg = y0 * g[0] + y1 * g[1] + y2 * g[2] + y3 * g[3];
+    g[0] = (g[0] - y0 * yg) * in;
+    g[1] = (g[1] - y1 * yg) * in;
+    g[2] = (g[2] - y2 * yg) * in;
+    g[3] = (g[3] - y3 * yg) * in;
+}
+
+// Reverse mode of rhs_quat13 (fp64) at (x, tau): g[13] is the cotangent of xd; a[13] receives the cotangent of x and
+// gtau[6] that of tau.  The quaternion is normalised inside the right-hand side, so its cotangent passes through
+// quat_normalize_vjp.
+template <class P>
+__device__ __forceinline__ void rhs_quat13_vjp(const double* __restrict__ x, const P& p, bool has_current,
+                                               const double* __restrict__ g, double* __restrict__ a,
+                                               double* __restrict__ gtau) {
+    double qw = x[3], qx = x[4], qy = x[5], qz = x[6];
+    {
+        const double n = sqrt(qw * qw + qx * qx + qy * qy + qz * qz);
+        if (n < 1e-12) { qw = 1.0; qx = qy = qz = 0.0; }
+        else { const double in = rcp_nr(n); qw *= in; qx *= in; qy *= in; qz *= in; }
+    }
+    const double* nu = x + 7;
+    const double R00 = 1.0 - 2.0 * (qy * qy + qz * qz), R01 = 2.0 * (qx * qy - qz * qw), R02 = 2.0 * (qx * qz + qy * qw);
+    const double R10 = 2.0 * (qx * qy + qz * qw), R11 = 1.0 - 2.0 * (qx * qx + qz * qz), R12 = 2.0 * (qy * qz - qx * qw);
+    const double R20 = 2.0 * (qx * qz - qy * qw), R21 = 2.0 * (qy * qz + qx * qw), R22 = 1.0 - 2.0 * (qx * qx + qy * qy);
+    double nur[6] = {nu[0], nu[1], nu[2], nu[3], nu[4], nu[5]};
+    double cx = 0.0, cy = 0.0, cz = 0.0;
+    if (has_current) {
+        cx = p[KP_CUR + 0]; cy = p[KP_CUR + 1]; cz = p[KP_CUR + 2];
+        nur[0] -= R00 * cx + R10 * cy + R20 * cz;
+        nur[1] -= R01 * cx + R11 * cy + R21 * cz;
+        nur[2] -= R02 * cx + R12 * cy + R22 * cz;
+    }
+    double gnu[6], gnur[6], gsth, gcs, gcc;
+    nu_dot_vjp(nu, nur, p, g + 7, gnu, gnur, gsth, gcs, gcc, gtau);
+    // restoring terms: sth = -R20, cs = R21, cc = R22
+    double gR00 = 0.0, gR01 = 0.0, gR02 = 0.0, gR10 = 0.0, gR11 = 0.0, gR12 = 0.0;
+    double gR20 = -gsth, gR21 = gcs, gR22 = gcc;
+#pragma unroll
+    for (int i = 0; i < 6; ++i) gnu[i] += gnur[i];
+    if (has_current) {
+        gR00 -= cx * gnur[0]; gR10 -= cy * gnur[0]; gR20 -= cz * gnur[0];
+        gR01 -= cx * gnur[1]; gR11 -= cy * gnur[1]; gR21 -= cz * gnur[1];
+        gR02 -= cx * gnur[2]; gR12 -= cy * gnur[2]; gR22 -= cz * gnur[2];
+    }
+    // position rates xd[0..2] = R nu[0..2]
+    gR00 += g[0] * nu[0]; gR01 += g[0] * nu[1]; gR02 += g[0] * nu[2];
+    gR10 += g[1] * nu[0]; gR11 += g[1] * nu[1]; gR12 += g[1] * nu[2];
+    gR20 += g[2] * nu[0]; gR21 += g[2] * nu[1]; gR22 += g[2] * nu[2];
+    gnu[0] += R00 * g[0] + R10 * g[1] + R20 * g[2];
+    gnu[1] += R01 * g[0] + R11 * g[1] + R21 * g[2];
+    gnu[2] += R02 * g[0] + R12 * g[1] + R22 * g[2];
+    // quaternion rates xd[3..6] = 1/2 q (x) [0, w]
+    const double wp = nu[3], wq = nu[4], wr = nu[5];
+    const double h3 = 0.5 * g[3], h4 = 0.5 * g[4], h5 = 0.5 * g[5], h6 = 0.5 * g[6];
+    double gq[4];
+    gq[0] = h4 * wp + h5 * wq + h6 * wr;
+    gq[1] = h6 * wq - h3 * wp - h5 * wr;
+    gq[2] = h4 * wr - h3 * wq - h6 * wp;
+    gq[3] = h5 * wp - h3 * wr - h4 * wq;
+    gnu[3] += qw * h4 + qz * h5 - qx * h3 - qy * h6;
+    gnu[4] += qw * h5 + qx * h6 - qy * h3 - qz * h4;
+    gnu[5] += qw * h6 + qy * h4 - qz * h3 - qx * h5;
+    // rotation matrix entries -> unit quaternion
+    gq[0] += 2.0 * (qz * (gR10 - gR01) + qy * (gR02 - gR20) + qx * (gR21 - gR12));
+    gq[1] += 2.0 * (qy * (gR01 + gR10) + qz * (gR02 + gR20) + qw * (gR21 - gR12)) - 4.0 * qx * (gR11 + gR22);
+    gq[2] += 2.0 * (qx * (gR01 + gR10) + qw * (gR02 - gR20) + qz * (gR12 + gR21)) - 4.0 * qy * (gR00 + gR22);
+    gq[3] += 2.0 * (qw * (gR10 - gR01) + qx * (gR02 + gR20) + qy * (gR12 + gR21)) - 4.0 * qz * (gR00 + gR11);
+    quat_normalize_vjp(x + 3, gq);
+    a[0] = 0.0; a[1] = 0.0; a[2] = 0.0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) a[3 + i] = gq[i];
+#pragma unroll
+    for (int i = 0; i < 6; ++i) a[7 + i] = gnu[i];
 }
 
 template <typename T> __device__ __forceinline__ void quat_renorm(T* q) {

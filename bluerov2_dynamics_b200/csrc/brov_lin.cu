@@ -19,15 +19,6 @@ namespace brov {
 __device__ __forceinline__ Dual operator+(Dual a, double b) { return Dual(a.v + b, a.d); }
 __device__ __forceinline__ Dual operator-(Dual a, double b) { return Dual(a.v - b, a.d); }
 
-// dF/dV of the T200 curve F(V) = V p(V^2): 9 a z^4 + 7 b z^3 + 5 c z^2 + 3 d z + e with z = V^2
-__device__ __forceinline__ double thrust_poly_d(const Consts<double>& c, double V) {
-    const double z = V * V;
-    double p = 9.0 * c.poly[0] * z + 7.0 * c.poly[1];
-    p = p * z + 5.0 * c.poly[2];
-    p = p * z + 3.0 * c.poly[3];
-    return p * z + c.poly[4];
-}
-
 // One integrator step with the state as dual numbers.  The body wrench of sub-step s has the value of Fw (thruster: the
 // allocated static thrust, turned into the lagged wrench here; wrench models: the input) and the tangent g_s * tvec,
 // g_s = lagG[s][lagk] for a lag column and lagH[s] otherwise (thruster), 1 (wrench models).  Same stage structure as

@@ -192,6 +192,16 @@ class EkfResult:
     health: Optional[torch.Tensor]   # int64 [2]: filters with a non-finite z or P / near theta = +-pi/2, or None
 
 
+@dataclass
+class VjpResult:
+    """Reverse-mode gradients of N rollouts (Engine.rollout_vjp) for L = sum_k <c_k, x_k> + <g_T, z_T>."""
+    gx0: torch.Tensor                # [N, NX] dL/dx_0
+    glag0: Optional[torch.Tensor]    # dL/dlag_0 in the representation of lag0 ([N, 24] or [N, 18]), None for wrench models
+    gU: torch.Tensor                 # [T, N, NU] dL/du_k (always per vehicle)
+    z: torch.Tensor                  # [N, NZ] z after the last step (the primal of linearize, projected lag)
+    health: Optional[torch.Tensor]   # int64 [2]: vehicles with a non-finite z or gradient / near theta = +-pi/2, or None
+
+
 _CL_LAYOUTS = ("const_shared", "shared", "const", "tnc")
 
 
@@ -950,6 +960,116 @@ class Engine:
             L.check(L.lib.brov_linearize(self._h, C.byref(d), self._stream()))
         return LinearizeResult(A=J[..., :nz], B=J[..., nz:], z=z, z_traj=zt, health=hc)
 
+    def _inputs(self, U, n: int, u_layout: str):
+        """(tensor, steps, stride_t, stride_n) of a rollout input U in the layouts of `rollout`"""
+        if u_layout == "const":
+            Ut, steps = U
+            Ut = self.tensor(Ut)
+            if Ut.dim() != 2 or Ut.shape[0] != n or Ut.shape[1] != self.nu:
+                raise ValueError(f"U must have shape [{n}, {self.nu}], got {tuple(Ut.shape)}")
+            return Ut, int(steps), 0, self.nu
+        Ut = self.tensor(U)
+        if u_layout == "auto":
+            u_layout = "tnc" if Ut.dim() == 3 else "shared"
+        if u_layout == "tnc":
+            if Ut.dim() != 3 or Ut.shape[1] != n or Ut.shape[2] != self.nu:
+                raise ValueError(f"U must have shape [T, {n}, {self.nu}], got {tuple(Ut.shape)}")
+            return Ut, Ut.shape[0], n * self.nu, self.nu
+        if u_layout == "shared":
+            if Ut.dim() != 2 or Ut.shape[1] != self.nu:
+                raise ValueError(f"U must have shape [T, {self.nu}], got {tuple(Ut.shape)}")
+            return Ut, Ut.shape[0], self.nu, 0
+        raise ValueError("u_layout must be auto|tnc|shared|const")
+
+    def rollout_vjp(self, x0, U, gtraj=None, gzT=None, stride: int = 0, dt: float = 0.02, integrator: str = "rk4",
+                    lag0=None, lag_repr: str = "thruster", u_layout: str = "auto", health: bool = False,
+                    singular_eps: float = 0.0) -> VjpResult:
+        """Reverse-mode gradients of N rollouts (brov_rollout_vjp): for every vehicle, with
+            L = sum_{k = stride, 2 stride, ... <= T} <c_k, x_k> + <g_T, z_T>,
+        returns dL/dz_0 (as gx0 and glag0) and dL/du_k for every step, in one launch and without forming the step
+        Jacobians.  The step is differentiated as `linearize` differentiates it, so the result equals the chain
+        lambda_k = A_k^T lambda_{k+1} + c_k, gu_k = B_k^T lambda_{k+1} over linearize's Jacobians to rounding.
+
+        gtraj [T//stride, N, NX]: the cotangents c_k, in the layout of rollout's traj (None: no trajectory term);
+        gzT [N, NZ]: the terminal cotangent on z_T = [x_T | Z_T] (projected lag for the thruster model; None: zero).
+        U as in `rollout` ([T,N,NU] "tnc", [T,NU] "shared", (U [N,NU], T) "const"); gU is always [T, N, NU].
+        lag0 (thruster model): per-thruster [N,24] with lag_repr="thruster", projected [N,18] with "projected";
+        glag0 comes back in the same representation (per thruster: P^T gZ0 by the chain rule with Z = P L).
+        The call allocates its workspace, T * N * NZ doubles; split longer horizons as include/brov.h describes.
+        fp64 engines with shared coefficients."""
+        x0 = self.tensor(x0)
+        self._check_rows(x0, self.nx, "x0")
+        n = x0.shape[0]
+        Ut, steps, st, sn = self._inputs(U, n, u_layout)
+        if lag_repr not in ("thruster", "projected"):
+            raise ValueError("lag_repr must be 'thruster' or 'projected'")
+        nz = self.nz
+        thr = self.model == "thruster8"
+        z0 = x0
+        if thr:
+            if lag0 is None:
+                Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
+            elif lag_repr == "thruster":
+                Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
+            else:
+                Z0 = self.tensor(lag0).reshape(n, 18)
+            z0 = torch.cat([x0, Z0], dim=1).contiguous()
+        gt = None
+        if gtraj is not None:
+            gt = self.tensor(gtraj)
+            ns = steps // int(stride) if int(stride) >= 1 else None
+            if ns is not None and tuple(gt.shape) != (ns, n, self.nx):
+                raise ValueError(f"gtraj must have shape [{ns}, {n}, {self.nx}], got {tuple(gt.shape)}")
+        gT = None
+        if gzT is not None:
+            gT = self.tensor(gzT)
+            if tuple(gT.shape) != (n, nz):
+                raise ValueError(f"gzT must have shape [{n}, {nz}], got {tuple(gT.shape)}")
+        gz0 = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
+        gU = torch.empty((steps, n, self.nu), device=self.device, dtype=self.tdtype)
+        z = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
+        wsb = int(L.lib.brov_rollout_vjp_workspace_bytes(MODELS[self.model], n, steps))
+        ws = torch.empty((max(wsb, 8) + 7) // 8, device=self.device, dtype=torch.float64)
+        hc = torch.zeros(2, device=self.device, dtype=torch.int64) if health else None
+        d = L.RolloutVjpDesc()
+        d.struct_size = C.sizeof(L.RolloutVjpDesc)
+        d.integrator = INTEGRATORS[integrator]
+        d.n, d.steps, d.dt = n, steps, float(dt)
+        d.z0_dev, d.u_dev = z0.data_ptr(), Ut.data_ptr()
+        d.u_stride_t, d.u_stride_n = st, sn
+        # an empty gtraj (stride > T: no snapshot) is no trajectory term
+        d.gtraj_dev = gt.data_ptr() if (gt is not None and gt.numel()) else None
+        d.stride = int(stride)
+        d.gzT_dev = gT.data_ptr() if gT is not None else None
+        d.gz0_dev, d.gu_dev, d.z_out_dev = gz0.data_ptr(), gU.data_ptr(), z.data_ptr()
+        d.workspace_dev, d.workspace_bytes = ws.data_ptr(), ws.numel() * 8
+        d.health_dev = hc.data_ptr() if hc is not None else None
+        d.singular_eps = float(singular_eps)
+        with torch.cuda.device(self.device):
+            L.check(L.lib.brov_rollout_vjp(self._h, C.byref(d), self._stream()))
+        gx0 = gz0[:, :self.nx]
+        glag0 = None
+        if thr:
+            gZ0 = gz0[:, self.nx:]
+            if lag_repr == "thruster":
+                A = self.tensor(self._alloc)
+                glag0 = torch.einsum("ci,nck->nik", A, gZ0.reshape(n, 6, 3)).reshape(n, 24).contiguous()
+            else:
+                glag0 = gZ0
+        return VjpResult(gx0=gx0, glag0=glag0, gU=gU, z=z, health=hc)
+
+    def rollout_diff(self, x0: torch.Tensor, U: torch.Tensor, lag0: Optional[torch.Tensor] = None, dt: float = 0.02,
+                     integrator: str = "rk4", stride: int = 1, lag_repr: str = "projected"):
+        """Differentiable rollout: (traj [T//stride, N, NX] or None for stride 0, xT [N, NX], lagT [N, 18] or None)
+        as `rollout` returns them, with torch autograd gradients to x0, U [T, N, NU] (per vehicle) and lag0 [N, 18].
+        The forward is `rollout`; the backward is one `rollout_vjp` call.  The lag is exchanged in projected
+        coordinates (lag_repr="projected"), the form whose derivative the adjoint carries."""
+        if lag_repr != "projected":
+            raise ValueError("rollout_diff exchanges the projected lag: lag_repr must be 'projected'")
+        lag_t = lag0 if (lag0 is not None and self.model == "thruster8") else None
+        traj, xT, lagT = _RolloutDiff.apply(self, x0, U, lag_t, float(dt), integrator, int(stride))
+        return (traj if stride else None), xT, (lagT if self.model == "thruster8" else None)
+
     def _cl_operand(self, v, inner: tuple, layout: str, n: int, what: str):
         """(tensor, stride_t, stride_n, T or None) of a closed-loop operand with trailing shape `inner`"""
         t = self.tensor(v)
@@ -1264,6 +1384,47 @@ class Engine:
             d.health_host = health.ctypes.data_as(C.POINTER(C.c_ulonglong))
         L.check(L.lib.brov_rollout_host(self._h, C.byref(d)))
         return xT, lag_out, traj
+
+
+class _RolloutDiff(torch.autograd.Function):
+    """Engine.rollout forward, Engine.rollout_vjp backward (Engine.rollout_diff)."""
+
+    @staticmethod
+    def forward(ctx, eng, x0, U, lag0, dt, integrator, stride):
+        if U.dim() != 3:
+            raise ValueError("rollout_diff takes a per-vehicle U [T, N, NU]")
+        thr = eng.model == "thruster8"
+        r = eng.rollout(x0.detach(), U.detach(), dt=dt, integrator=integrator,
+                        lag0=lag0.detach() if lag0 is not None else None, stride=stride,
+                        lag_repr="projected", want_lag=thr)
+        ctx.eng, ctx.dt, ctx.integrator, ctx.stride = eng, dt, integrator, stride
+        ctx.has_lag = lag0 is not None
+        ctx.save_for_backward(x0, U, *([lag0] if lag0 is not None else []))
+        n = x0.shape[0]
+        traj = r.traj if stride else torch.empty((0, n, eng.nx), device=eng.device, dtype=eng.tdtype)
+        lagT = r.lag if thr else torch.empty((n, 0), device=eng.device, dtype=eng.tdtype)
+        return traj, r.xT, lagT
+
+    @staticmethod
+    def backward(ctx, gtraj, gxT, glagT):
+        eng = ctx.eng
+        saved = ctx.saved_tensors
+        x0, U = saved[0], saved[1]
+        lag0 = saved[2] if ctx.has_lag else None
+        n = x0.shape[0]
+        thr = eng.model == "thruster8"
+        gx = gxT if gxT is not None else torch.zeros((n, eng.nx), device=eng.device, dtype=eng.tdtype)
+        if thr:
+            gl = glagT if glagT is not None else torch.zeros((n, 18), device=eng.device, dtype=eng.tdtype)
+            gzT = torch.cat([gx, gl], dim=1).contiguous()
+        else:
+            gzT = gx.contiguous()
+        gt = gtraj.contiguous() if (gtraj is not None and ctx.stride and gtraj.numel()) else None
+        res = eng.rollout_vjp(x0.detach(), U.detach(), gtraj=gt, gzT=gzT, stride=ctx.stride if gt is not None else 0,
+                              dt=ctx.dt, integrator=ctx.integrator, lag0=lag0.detach() if lag0 is not None else None,
+                              lag_repr="projected", u_layout="tnc")
+        glag = res.glag0 if (thr and ctx.has_lag) else None
+        return None, res.gx0, res.gU, glag, None, None, None
 
 
 def reduced9_rhs(x: torch.Tensor, u: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:

@@ -550,6 +550,58 @@ typedef struct brov_ekf_desc {
 } brov_ekf_desc;
 int brov_ekf(brov_engine_t* e, const brov_ekf_desc* d, void* stream);
 
+/* Reverse-mode (adjoint) gradients of batched rollouts — what gradient-based trajectory optimisation, training a policy
+ * or a learned model through the simulator, and sensitivity studies need.  With z_{k+1} = Phi(z_k, u_k) the step of
+ * brov_linearize (z = [x (NX) | Z (18, thruster model only)], NZ = 30 / 12 / 13, NU = 8 / 6 / 6) and, per vehicle,
+ *     L = sum_{k = stride, 2 stride, ... <= steps} <c_k, x_k> + <g_T, z_steps>
+ * the call returns gz0 = dL/dz_0 and gu[k] = dL/du_k.  c_k comes from gtraj_dev in the layout of brov_rollout's
+ * trajectory, [steps / stride][n][NX] (NULL: no trajectory term); g_T from gzT_dev [n][NZ] (NULL: zero).  The
+ * derivative is that of the step brov_linearize differentiates (full sines and cosines in every stage, branch taken:
+ * d|x| = sign(x) dx, the clamped cos(theta) and the quaternion fallback are constants; the quaternion renormalised
+ * after the step), so gz0 and gu equal the chain lambda_k = A_k^T lambda_{k+1} + c_k, gu_k = B_k^T lambda_{k+1} over
+ * brov_linearize's J to rounding, without forming J.  One thread per vehicle runs the forward pass, storing every z_k
+ * in the workspace, then the reverse sweep; every sum has a fixed order, so results are bit-reproducible and
+ * independent of the input layout and of the other vehicles.
+ *   z0_dev [n][NZ]; u_dev with u_stride_t / u_stride_n as in brov_linearize_desc (per-vehicle, shared or constant);
+ *   gz0_dev [n][NZ] (required; may alias gzT_dev); gu_dev [steps][n][NU] (required);
+ *   z_out_dev [n][NZ] or NULL: z after the last step (the primal of brov_linearize: it agrees with brov_rollout to
+ *   rounding, not bit for bit);
+ *   workspace_dev: at least brov_rollout_vjp_workspace_bytes(model, n, steps) bytes (n * steps * NZ doubles);
+ *   health_dev (unsigned long long[2] or NULL, zeroed by the call): vehicles with a non-finite z, gz0 or gu entry /
+ *   that came within singular_eps (0 = 1e-3) of theta = +-pi/2 at the start of some step.
+ * Chaining (horizons longer than a workspace allows): split at t1, a multiple of stride when gtraj_dev is used.  The
+ * gz0 of the call over [t1, steps], started from z_{t1} = the z_out of a call over [0, t1], is the gzT of the call over
+ * [0, t1] (whose gtraj slice ends with c_{t1}).  The chained gradients equal those of one call bit for bit.
+ * fp64 engines, Fossen models, RK4 / Euler, the engine's shared coefficients, allocation and lag discretisation for dt.
+ * f32 engines, double-integrator engines, the first-order wrench lag and an engine with a per-vehicle coefficient table
+ * return BROV_EUNSUPPORTED.  BROV_EINVAL (before any launch): n < 0, steps < 1, dt <= 0, negative input strides, NULL
+ * required pointers, gtraj_dev with stride < 1, a workspace smaller than needed.  n = 0 is a no-op.  All arrays double,
+ * dev. */
+typedef struct brov_rollout_vjp_desc {
+    uint32_t struct_size;       /* = sizeof(brov_rollout_vjp_desc) */
+    int32_t integrator;
+    long long n;
+    long long steps;
+    double dt;
+    const void* z0_dev;
+    const void* u_dev;
+    long long u_stride_t, u_stride_n;
+    const void* gtraj_dev;
+    long long stride;
+    const void* gzT_dev;
+    void* gz0_dev;
+    void* gu_dev;
+    void* z_out_dev;
+    void* workspace_dev;
+    size_t workspace_bytes;
+    void* health_dev;
+    double singular_eps;
+} brov_rollout_vjp_desc;
+int brov_rollout_vjp(brov_engine_t* e, const brov_rollout_vjp_desc* d, void* stream);
+/* workspace of brov_rollout_vjp: n * steps * NZ * sizeof(double) for the Fossen models (0 for other models or n, steps
+ * <= 0; SIZE_MAX if the size does not fit in size_t) */
+size_t brov_rollout_vjp_workspace_bytes(int model, long long n, long long steps);
+
 /* Reduced 9-state RHS — `bluerov_compute(t, x_, u_)` (fossen/bluerov_torch.py:20-67, constants fossen/parameters.py).
  * x [B][9], u [B][4], out [B][9]. */
 int brov_reduced9_rhs(int dtype, const void* x_dev, const void* u_dev, void* out_dev, long long B, void* stream);
