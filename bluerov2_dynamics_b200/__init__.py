@@ -15,7 +15,7 @@ CPU fallback — importing this package without the built library raises.
 """
 import importlib as _importlib
 
-__all__ = ["Engine", "RolloutResult", "InputGenerator", "BrovError", "default_physical", "derive_params", "default_allocation",
+__all__ = ["Engine", "RolloutResult", "InputGenerator", "BrovError", "default_physical", "derive_params", "derive_params_torch", "default_allocation",
            "lag_discretize", "with_minv", "coefficient_directions", "parameter_indices", "GradResult", "LinearizeResult", "ClosedLoopResult", "EkfResult",
            "VjpResult",
            "reduced9_rhs",

@@ -121,6 +121,10 @@ class RolloutVjpDesc(C.Structure):
                 ("singular_eps", C.c_double)]
 
 
+class RolloutVjpCoefDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("reserved", C.c_int32), ("vjp", RolloutVjpDesc), ("gkp_dev", C.c_void_p)]
+
+
 class RolloutHostDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
                 ("dt", C.c_double), ("x0_host", C.c_void_p), ("xT_host", C.c_void_p), ("u_host", C.c_void_p),
@@ -187,6 +191,7 @@ _PROTOS = {
     "brov_ekf": (C.c_int, [C.c_void_p, C.POINTER(EkfDesc), C.c_void_p]),
     "brov_rollout_vjp": (C.c_int, [C.c_void_p, C.POINTER(RolloutVjpDesc), C.c_void_p]),
     "brov_rollout_vjp_workspace_bytes": (C.c_size_t, [C.c_int, C.c_longlong, C.c_longlong]),
+    "brov_rollout_vjp_coef": (C.c_int, [C.c_void_p, C.POINTER(RolloutVjpCoefDesc), C.c_void_p]),
     "brov_reduced9_rhs": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "brov_koopman_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_void_p)]),
     "brov_koopman_destroy": (None, [C.c_void_p]),

@@ -8,6 +8,10 @@
 //                    forward loop ran (so the map it differentiates is exactly the stored one), stages them in shared
 //                    memory and sweeps the stages in reverse with the hand-written vector-Jacobian products of the
 //                    right-hand sides (rhs_euler12_vjp / rhs_quat13_vjp, brov_device.cuh).
+//   adjoint_coef_kernel  the same sweeps (adjoint_vehicle) that also accumulate dL/dkp of the vehicle's coefficients:
+//                    one lambda^T df/dkp per stage (nu_dot_coef_vjp), added to the thread's column of a shared-memory
+//                    accumulator [ADJ_NKPG][thread]; the coefficients come from the constant bank or, PV, from the
+//                    vehicle's column of the per-vehicle table staged in shared memory.
 //
 // Every sum has a fixed order, so the results are bit-reproducible and independent of the other vehicles.
 #include "brov_adj.cuh"
@@ -15,11 +19,10 @@
 namespace brov {
 
 // right-hand side of sub-step s at the stage state xs, as linearize evaluates it (full sines and cosines)
-template <int MODEL>
-__device__ __forceinline__ void adj_rhs(const Consts<double>& c, int s, const double* __restrict__ xs,
+template <int MODEL, class P>
+__device__ __forceinline__ void adj_rhs(const Consts<double>& c, const P& p, int s, const double* __restrict__ xs,
                                         const double* __restrict__ Z, const double* __restrict__ Fw,
                                         double* __restrict__ out, double& abs_cth) {
-    const ParamsConst<double> p{c.kp};
     const bool cur = c.has_current != 0;
     double tau[6];
     if constexpr (MODEL == MODEL_THRUSTER8) {
@@ -41,8 +44,8 @@ __device__ __forceinline__ void adj_rhs(const Consts<double>& c, int s, const do
 // One primal step x <- Phi_x(x, Z, Fw); the lag is advanced by the caller.  STAGES (the backward loop's recompute): the
 // RK4 stage states xs_1..xs_3 go to sx[((s-1)*NX + i) * ADJ_THREADS] and the quaternion before its renormalisation to
 // qpre; the last stage's right-hand side is evaluated only when the renormalisation needs it.
-template <int MODEL, int INTEG, bool STAGES>
-__device__ __forceinline__ void adj_step(const Consts<double>& c, double* __restrict__ x, const double* __restrict__ Z,
+template <int MODEL, int INTEG, bool STAGES, class P>
+__device__ __forceinline__ void adj_step(const Consts<double>& c, const P& p, double* __restrict__ x, const double* __restrict__ Z,
                                          const double* __restrict__ Fw, double* __restrict__ sx,
                                          double* __restrict__ qpre, double& abs_cth) {
     constexpr int NX = ModelDim<MODEL>::NX;
@@ -51,13 +54,13 @@ __device__ __forceinline__ void adj_step(const Consts<double>& c, double* __rest
     abs_cth = 1.0;
     double k[NX];
     if constexpr (INTEG == INTEG_EULER) {
-        adj_rhs<MODEL>(c, 0, x, Z, Fw, k, abs_cth);
+        adj_rhs<MODEL>(c, p, 0, x, Z, Fw, k, abs_cth);
 #pragma unroll
         for (int i = 0; i < NX; ++i) x[i] += dt * k[i];
     } else {
         double acc[NX], xs[NX];
         const double hdt = 0.5 * dt;
-        adj_rhs<MODEL>(c, 0, x, Z, Fw, k, abs_cth);
+        adj_rhs<MODEL>(c, p, 0, x, Z, Fw, k, abs_cth);
 #pragma unroll
         for (int s = 1; s <= 3; ++s) {
             const double w = (s == 1) ? 1.0 : 2.0;
@@ -71,7 +74,7 @@ __device__ __forceinline__ void adj_step(const Consts<double>& c, double* __rest
             if constexpr (STAGES && !QUAT) {
                 if (s == 3) return;
             }
-            adj_rhs<MODEL>(c, s, xs, Z, Fw, k, abs_cth);
+            adj_rhs<MODEL>(c, p, s, xs, Z, Fw, k, abs_cth);
         }
         const double dt6 = dt * (1.0 / 6.0);
 #pragma unroll
@@ -131,7 +134,7 @@ __global__ void __launch_bounds__(ADJ_THREADS) adjoint_kernel(const __grid_const
                 for (int r = 0; r < 6; ++r) Fw[r] = uk[r];
             }
             double acth;
-            adj_step<MODEL, INTEG, false>(c, x, Z, Fw, nullptr, nullptr, acth);
+            adj_step<MODEL, INTEG, false>(c, p, x, Z, Fw, nullptr, nullptr, acth);
             sing |= acth < a.eps;
             if constexpr (THR) lag_advance<double, true>(c, Z, Fw);
         }
@@ -186,7 +189,7 @@ __global__ void __launch_bounds__(ADJ_THREADS) adjoint_kernel(const __grid_const
 #pragma unroll
                 for (int q = 0; q < NX; ++q) xw[q] = x[q];
                 double acth;
-                adj_step<MODEL, INTEG, true>(c, xw, Z, Fw, sx, qpre, acth);
+                adj_step<MODEL, INTEG, true>(c, p, xw, Z, Fw, sx, qpre, acth);
             }
             if constexpr (QUAT) quat_normalize_vjp(qpre, lam + 3);
             // lag: Z' = lagA Z_c + lagB Fw_c per channel
@@ -324,6 +327,291 @@ cudaError_t launch_adjoint(int model, int integ, const AdjArgs& a, cudaStream_t 
         case MODEL_THRUSTER8: return adjoint_integ<MODEL_THRUSTER8>(integ, a, st);
         case MODEL_WRENCH12: return adjoint_integ<MODEL_WRENCH12>(integ, a, st);
         case MODEL_QUAT13: return adjoint_integ<MODEL_QUAT13>(integ, a, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+// a shared-memory column of the coefficient cotangent: entry j of this thread at base[j * ADJ_THREADS]
+struct CoefAcc {
+    double* base;
+    __device__ __forceinline__ double& operator[](int j) const { return base[j * ADJ_THREADS]; }
+};
+
+// adjoint_kernel plus the coefficient cotangent (brov_rollout_vjp_coef).  The sweeps are adjoint_kernel's; in addition
+// every stage of every step adds lambda^T df/dkp (rhs_*_vjp<true>, nu_dot_coef_vjp) to the thread's column gk of a
+// shared-memory accumulator, in a fixed order, and the column goes to gkp [KP_COUNT][n] at the end.  Dynamic shared
+// memory, one column per thread (conflict-free): [RK4 stage buffer (3 NX) | gk (ADJ_NKPG) | PV: the vehicle's column
+// of the per-vehicle table (KP_COUNT), staged as closed_loop_kernel stages it].  The engine's has_current selects the
+// primal; the reverse always runs the current path (nu - R^T 0 = nu), so gk[KP_CUR ..] exists without a current.
+// (A separate kernel rather than flags on adjoint_kernel: that one's code stays exactly as it was.)
+template <int MODEL, int INTEG, bool PV>
+__global__ void __launch_bounds__(ADJ_THREADS) adjoint_coef_kernel(const __grid_constant__ AdjCoefArgs ca) {
+    constexpr int NX = LinDim<MODEL>::NX, NU = LinDim<MODEL>::NU, NZ = LinDim<MODEL>::NZ;
+    constexpr bool THR = MODEL == MODEL_THRUSTER8;
+    constexpr bool QUAT = ModelDim<MODEL>::QUAT;
+    constexpr int NL = THR ? 18 : 1;
+    extern __shared__ double smem[];
+    const AdjArgs& a = ca.a;
+    const Consts<double>& c = a.c;
+    const int tid = threadIdx.x;
+    double* sx = smem + tid;
+    const long long v = (long long)blockIdx.x * ADJ_THREADS + tid;
+    const long long n = a.n;
+    double* col = smem + adjoint_coef_stage_rows(MODEL, INTEG) * ADJ_THREADS + tid;
+    const CoefAcc gk{col};
+#pragma unroll
+    for (int j = 0; j < ADJ_NKPG; ++j) gk[j] = 0.0;
+    typename std::conditional<PV, ParamsShared<double>, ParamsConst<double>>::type p;
+    if constexpr (PV) {
+        const double* pvt = ca.pv + (v < n ? v : 0);
+#pragma unroll 4
+        for (int j = 0; j < KP_COUNT; ++j) col[(ADJ_NKPG + j) * ADJ_THREADS] = pvt[(long long)j * n];
+        p.base = col + ADJ_NKPG * ADJ_THREADS;
+        p.pitch = ADJ_THREADS;
+    } else {
+        p.kp = c.kp;
+    }
+    bool bad = false, sing = false;
+    if (v < n) {
+        // ---- forward: z_k -> workspace
+        double x[NX], Z[NL];
+#pragma unroll
+        for (int q = 0; q < NX; ++q) x[q] = a.z0[v * NZ + q];
+#pragma unroll
+        for (int q = 0; q < NL; ++q) Z[q] = THR ? a.z0[v * NZ + NX + q] : 0.0;
+        for (int k = 0; k < a.steps; ++k) {
+            double* wk = a.ws + (long long)k * NZ * n + v;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) wk[q * n] = x[q];
+            if constexpr (THR) {
+#pragma unroll
+                for (int q = 0; q < NL; ++q) wk[(NX + q) * n] = Z[q];
+            }
+            const double* uk = a.U + (long long)k * a.ust + v * a.usn;
+            double Fw[6];
+            if constexpr (THR) {
+                double F[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, uk[i]);
+                allocate_wrench<double>(c, F, Fw);
+            } else {
+#pragma unroll
+                for (int r = 0; r < 6; ++r) Fw[r] = uk[r];
+            }
+            double acth;
+            adj_step<MODEL, INTEG, false>(c, p, x, Z, Fw, nullptr, nullptr, acth);
+            sing |= acth < a.eps;
+            if constexpr (THR) lag_advance<double, true>(c, Z, Fw);
+        }
+#pragma unroll
+        for (int q = 0; q < NX; ++q) bad |= !adj_finite(x[q]);
+#pragma unroll
+        for (int q = 0; q < NL; ++q) bad |= THR && !adj_finite(Z[q]);
+        if (a.z_out) {
+#pragma unroll
+            for (int q = 0; q < NX; ++q) a.z_out[v * NZ + q] = x[q];
+            if constexpr (THR) {
+#pragma unroll
+                for (int q = 0; q < NL; ++q) a.z_out[v * NZ + NX + q] = Z[q];
+            }
+        }
+
+        // ---- backward: lam = dL/dx_k, mu = dL/dZ_k
+        double lam[NX], mu[NL];
+#pragma unroll
+        for (int q = 0; q < NX; ++q) lam[q] = a.gzT ? a.gzT[v * NZ + q] : 0.0;
+#pragma unroll
+        for (int q = 0; q < NL; ++q) mu[q] = (THR && a.gzT) ? a.gzT[v * NZ + NX + q] : 0.0;
+        if (a.gtraj && a.steps % a.stride == 0) {
+            const double* gt = a.gtraj + ((long long)(a.steps / a.stride - 1) * n + v) * NX;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) lam[q] += gt[q];
+        }
+        const double dt = c.dt, hdt = 0.5 * dt, dt6 = dt * (1.0 / 6.0), dt3 = 2.0 * dt6;
+        for (int k = a.steps - 1; k >= 0; --k) {
+            const double* wk = a.ws + (long long)k * NZ * n + v;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
+            if constexpr (THR) {
+#pragma unroll
+                for (int q = 0; q < NL; ++q) Z[q] = wk[(NX + q) * n];
+            }
+            const double* uk = a.U + (long long)k * a.ust + v * a.usn;
+            double Fw[6];
+            if constexpr (THR) {
+                double F[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, uk[i]);
+                allocate_wrench<double>(c, F, Fw);
+            } else {
+#pragma unroll
+                for (int r = 0; r < 6; ++r) Fw[r] = uk[r];
+            }
+            // recompute the stage states (and the quaternion before its renormalisation)
+            double qpre[4];
+            if constexpr (INTEG == INTEG_RK4 || QUAT) {
+                double xw[NX];
+#pragma unroll
+                for (int q = 0; q < NX; ++q) xw[q] = x[q];
+                double acth;
+                adj_step<MODEL, INTEG, true>(c, p, xw, Z, Fw, sx, qpre, acth);
+            }
+            if constexpr (QUAT) quat_normalize_vjp(qpre, lam + 3);
+            // lag: Z' = lagA Z_c + lagB Fw_c per channel
+            double muF[6];
+            if constexpr (THR) {
+#pragma unroll
+                for (int ch = 0; ch < 6; ++ch) {
+                    const double m0 = mu[3 * ch], m1 = mu[3 * ch + 1], m2 = mu[3 * ch + 2];
+#pragma unroll
+                    for (int j = 0; j < 3; ++j) mu[3 * ch + j] = c.lagA[0][j] * m0 + c.lagA[1][j] * m1 + c.lagA[2][j] * m2;
+                    muF[ch] = c.lagB[0] * m0 + c.lagB[1] * m1 + c.lagB[2] * m2;
+                }
+            } else {
+#pragma unroll
+                for (int ch = 0; ch < 6; ++ch) muF[ch] = 0.0;
+            }
+            double lamp[NX], kap[NX];
+#pragma unroll
+            for (int q = 0; q < NX; ++q) lamp[q] = lam[q];
+            // stage s at xs with the cotangent kap of its right-hand side: lam += a, the wrench cotangent b into
+            // mu / muF (thruster: tau_s = lagG[s] . Z_c + lagH[s] Fw_c) or muF (wrench models: tau = u)
+            auto stage_vjp = [&](int s, const double* xs, double* ga) {
+                double b[6];
+                double tau[6];
+                if constexpr (THR) {
+                    thruster_tau<double, true>(c, s, Z, Fw, tau);
+                } else {
+#pragma unroll
+                    for (int r = 0; r < 6; ++r) tau[r] = Fw[r];
+                }
+                if constexpr (QUAT) {
+                    rhs_quat13_vjp<true>(xs, p, true, kap, ga, b, tau, gk);
+                } else {
+                    Trig<double> tr;
+                    trig_full<double>(c, xs + 3, tr);
+                    rhs_euler12_vjp<true>(xs, tr, p, true, kap, ga, b, tau, gk);
+                }
+
+#pragma unroll
+                for (int q = 0; q < NX; ++q) lam[q] += ga[q];
+#pragma unroll
+                for (int ch = 0; ch < 6; ++ch) {
+                    if constexpr (THR) {
+#pragma unroll
+                        for (int j = 0; j < 3; ++j) mu[3 * ch + j] += c.lagG[s][j] * b[ch];
+                        muF[ch] += c.lagH[s] * b[ch];
+                    } else {
+                        muF[ch] += b[ch];
+                    }
+                }
+            };
+            double ga[NX];
+            if constexpr (INTEG == INTEG_EULER) {
+#pragma unroll
+                for (int q = 0; q < NX; ++q) kap[q] = dt * lamp[q];
+                stage_vjp(0, x, ga);
+            } else {
+                // x' = x + dt/6 (k0 + 2 k1 + 2 k2 + k3), xs_s = x + h_s k_{s-1}
+#pragma unroll
+                for (int q = 0; q < NX; ++q) kap[q] = dt6 * lamp[q];
+#pragma unroll
+                for (int s = 3; s >= 1; --s) {
+                    double xs[NX];
+#pragma unroll
+                    for (int q = 0; q < NX; ++q) xs[q] = sx[((s - 1) * NX + q) * ADJ_THREADS];
+                    stage_vjp(s, xs, ga);
+                    const double cs = (s == 1) ? dt6 : dt3;
+                    const double hs = (s == 3) ? dt : hdt;
+#pragma unroll
+                    for (int q = 0; q < NX; ++q) kap[q] = fma(hs, ga[q], cs * lamp[q]);
+                }
+                // stage 0 is z_k itself: reloaded rather than held through the sweep (register pressure)
+#pragma unroll
+                for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
+                stage_vjp(0, x, ga);
+            }
+            // input: thruster gu_i = F'(u_i) sum_c alloc[c][i] muF[c] (the allocation's structural zeros skipped, as
+            // in allocate_wrench); wrench models gu = muF
+            double* gu = a.gU + ((long long)k * n + v) * NU;
+            if constexpr (THR) {
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int r = 0; r < 6; ++r) {
+                        const bool nz = (r < 2) ? (i < 4) : (r == 2) ? (i >= 4) : (r == 5) ? (i < 4) : true;
+                        if (nz) s += c.alloc[r][i] * muF[r];
+                    }
+                    const double g = thrust_poly_d(c, uk[i]) * s;
+                    gu[i] = g;
+                    bad |= !adj_finite(g);
+                }
+            } else {
+#pragma unroll
+                for (int i = 0; i < 6; ++i) {
+                    gu[i] = muF[i];
+                    bad |= !adj_finite(muF[i]);
+                }
+            }
+            if (a.gtraj && k > 0 && k % a.stride == 0) {
+                const double* gt = a.gtraj + ((long long)(k / a.stride - 1) * n + v) * NX;
+#pragma unroll
+                for (int q = 0; q < NX; ++q) lam[q] += gt[q];
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < NX; ++q) {
+            a.gz0[v * NZ + q] = lam[q];
+            bad |= !adj_finite(lam[q]);
+        }
+        if constexpr (THR) {
+#pragma unroll
+            for (int q = 0; q < NL; ++q) {
+                a.gz0[v * NZ + NX + q] = mu[q];
+                bad |= !adj_finite(mu[q]);
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < KP_COUNT; ++j) {
+            const double g = j < ADJ_NKPG ? gk[j] : 0.0;
+            ca.gkp[(long long)j * n + v] = g;
+            bad |= !adj_finite(g);
+        }
+    }
+    if (a.health) {
+        const int nb = __syncthreads_count(bad);
+        const int ns = __syncthreads_count(sing);
+        if (tid == 0) {
+            if (nb) atomicAdd(a.health + 0, (unsigned long long)nb);
+            if (ns) atomicAdd(a.health + 1, (unsigned long long)ns);
+        }
+    }
+}
+
+template <int MODEL, int INTEG, bool PV>
+static cudaError_t adjoint_coef_go(const AdjCoefArgs& a, cudaStream_t st) {
+    auto kern = adjoint_coef_kernel<MODEL, INTEG, PV>;
+    const size_t smem = adjoint_coef_smem_bytes(MODEL, INTEG, PV);
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    const long long grid = (a.a.n + ADJ_THREADS - 1) / ADJ_THREADS;
+    kern<<<(unsigned)grid, ADJ_THREADS, smem, st>>>(a);
+    return cudaGetLastError();
+}
+
+template <int MODEL>
+static cudaError_t adjoint_coef_integ(int integ, const AdjCoefArgs& a, cudaStream_t st) {
+    const bool pv = a.pv != nullptr;
+    if (integ == INTEG_RK4) return pv ? adjoint_coef_go<MODEL, INTEG_RK4, true>(a, st) : adjoint_coef_go<MODEL, INTEG_RK4, false>(a, st);
+    return pv ? adjoint_coef_go<MODEL, INTEG_EULER, true>(a, st) : adjoint_coef_go<MODEL, INTEG_EULER, false>(a, st);
+}
+
+cudaError_t launch_adjoint_coef(int model, int integ, const AdjCoefArgs& a, cudaStream_t st) {
+    switch (model) {
+        case MODEL_THRUSTER8: return adjoint_coef_integ<MODEL_THRUSTER8>(integ, a, st);
+        case MODEL_WRENCH12: return adjoint_coef_integ<MODEL_WRENCH12>(integ, a, st);
+        case MODEL_QUAT13: return adjoint_coef_integ<MODEL_QUAT13>(integ, a, st);
     }
     return cudaErrorInvalidValue;
 }

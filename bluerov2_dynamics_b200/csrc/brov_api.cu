@@ -1402,13 +1402,9 @@ extern "C" size_t brov_rollout_vjp_workspace_bytes(int model, long long n, long 
     return adjoint_workspace_bytes(nz, n, steps);
 }
 
-extern "C" int brov_rollout_vjp(brov_engine_t* e, const brov_rollout_vjp_desc* d, void* stream) {
-    if (!e) return fail(BROV_EINVAL, "NULL engine");
-    if (!d || d->struct_size != sizeof(brov_rollout_vjp_desc)) return fail(BROV_EINVAL, "brov_rollout_vjp_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
-    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "rollout_vjp serves the Fossen models, not double-integrator engines");
-    if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the gradients are computed in fp64: create the engine with BROV_F64");
-    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "rollout_vjp does not support the first-order wrench lag");
-    if (e->pv) return fail(BROV_EUNSUPPORTED, "rollout_vjp uses the shared coefficients: clear the per-vehicle table first");
+// the argument checks of brov_rollout_vjp / brov_rollout_vjp_coef in order, then (n > 0) the kernel arguments a and the
+// health counters zeroed on st
+static int rollout_vjp_args(brov_engine_t* e, const brov_rollout_vjp_desc* d, AdjArgs* a, cudaStream_t st) {
     if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
     if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
     if (d->steps < 1 || d->steps > (1LL << 30)) return fail(BROV_EINVAL, "steps = %lld must be 1 .. 2^30", d->steps);
@@ -1419,28 +1415,63 @@ extern "C" int brov_rollout_vjp(brov_engine_t* e, const brov_rollout_vjp_desc* d
     if (!d->z0_dev || !d->u_dev || !d->gz0_dev || !d->gu_dev) return fail(BROV_EINVAL, "z0, u, gz0 and gu must not be NULL");
     const size_t need = brov_rollout_vjp_workspace_bytes(e->model, d->n, d->steps);
     if (!d->workspace_dev || d->workspace_bytes < need) return fail(BROV_EINVAL, "workspace too small: need %zu bytes", need);
-    AdjArgs a;
-    memset(&a, 0, sizeof(a));
-    int rc = make_consts<double>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c);
+    memset(a, 0, sizeof(*a));
+    int rc = make_consts<double>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a->c);
     if (rc) return rc;
-    a.z0 = (const double*)d->z0_dev;
-    a.U = (const double*)d->u_dev;
-    a.ust = d->u_stride_t; a.usn = d->u_stride_n;
-    a.gtraj = (const double*)d->gtraj_dev;
-    a.gzT = (const double*)d->gzT_dev;
-    a.gz0 = (double*)d->gz0_dev;
-    a.gU = (double*)d->gu_dev;
-    a.z_out = (double*)d->z_out_dev;
-    a.ws = (double*)d->workspace_dev;
-    a.health = (unsigned long long*)d->health_dev;
-    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
-    a.n = d->n;
-    a.steps = (int)d->steps;
-    a.stride = d->gtraj_dev ? (int)std::min<long long>(d->stride, 0x7fffffffLL) : 1;
+    a->z0 = (const double*)d->z0_dev;
+    a->U = (const double*)d->u_dev;
+    a->ust = d->u_stride_t; a->usn = d->u_stride_n;
+    a->gtraj = (const double*)d->gtraj_dev;
+    a->gzT = (const double*)d->gzT_dev;
+    a->gz0 = (double*)d->gz0_dev;
+    a->gU = (double*)d->gu_dev;
+    a->z_out = (double*)d->z_out_dev;
+    a->ws = (double*)d->workspace_dev;
+    a->health = (unsigned long long*)d->health_dev;
+    a->eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    a->n = d->n;
+    a->steps = (int)d->steps;
+    a->stride = d->gtraj_dev ? (int)std::min<long long>(d->stride, 0x7fffffffLL) : 1;
     CUDA_TRY(cudaSetDevice(e->device));
-    cudaStream_t st = (cudaStream_t)stream;
     if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+    return BROV_OK;
+}
+
+static int rollout_vjp_common(brov_engine_t* e, const brov_rollout_vjp_desc* d) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_rollout_vjp_desc)) return fail(BROV_EINVAL, "brov_rollout_vjp_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "rollout_vjp serves the Fossen models, not double-integrator engines");
+    if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the gradients are computed in fp64: create the engine with BROV_F64");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "rollout_vjp does not support the first-order wrench lag");
+    return BROV_OK;
+}
+
+extern "C" int brov_rollout_vjp(brov_engine_t* e, const brov_rollout_vjp_desc* d, void* stream) {
+    int rc = rollout_vjp_common(e, d);
+    if (rc) return rc;
+    if (e->pv) return fail(BROV_EUNSUPPORTED, "rollout_vjp uses the shared coefficients: clear the per-vehicle table first");
+    AdjArgs a;
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = rollout_vjp_args(e, d, &a, st);
+    if (rc || d->n == 0) return rc;
     CUDA_TRY(launch_adjoint(e->model, d->integrator, a, st));
+    return BROV_OK;
+}
+
+extern "C" int brov_rollout_vjp_coef(brov_engine_t* e, const brov_rollout_vjp_coef_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_rollout_vjp_coef_desc)) return fail(BROV_EINVAL, "brov_rollout_vjp_coef_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    int rc = rollout_vjp_common(e, &d->vjp);
+    if (rc) return rc;
+    if (e->pv && e->pv_n != d->vjp.n) return fail(BROV_EINVAL, "vehicle table has %lld rows, call has n = %lld", e->pv_n, d->vjp.n);
+    if (d->vjp.n != 0 && !d->gkp_dev) return fail(BROV_EINVAL, "gkp must not be NULL");
+    AdjCoefArgs a;
+    cudaStream_t st = (cudaStream_t)stream;
+    rc = rollout_vjp_args(e, &d->vjp, &a.a, st);
+    if (rc || d->vjp.n == 0) return rc;
+    a.gkp = (double*)d->gkp_dev;
+    a.pv = (const double*)e->pv;
+    CUDA_TRY(launch_adjoint_coef(e->model, d->vjp.integrator, a, st));
     return BROV_OK;
 }
 

@@ -291,6 +291,46 @@ __device__ __forceinline__ void nu_dot_vjp(const double* __restrict__ nu, const 
     gcc = wmb * e[2] - ybB * e[3] + xbB * e[4];
 }
 
+// Coefficient cotangent of nu_dot (fp64) at (nu, nur, tau, sth, cs, cc) with the cotangent g[6] of out: adds
+// d<g, out>/d kp to gk[KP_MINV .. KP_XBB + 2] (the current enters through nur: rhs_euler12_vjp / rhs_quat13_vjp add
+// gk[KP_CUR ..]).  gk is any indexable accumulator of doubles (a shared-memory column in the adjoint kernel).
+template <class P, class G>
+__device__ __forceinline__ void nu_dot_coef_vjp(const double* __restrict__ nu, const double* __restrict__ nur,
+                                                const double* __restrict__ tau, double sth, double cs, double cc,
+                                                const P& p, const double* __restrict__ g, const G& gk) {
+    const double u = nu[0], v = nu[1], w = nu[2], pp = nu[3], q = nu[4], r = nu[5];
+    const double a1u = p[KP_A + 0] * u, a2v = p[KP_A + 1] * v, a3w = p[KP_A + 2] * w;
+    const double wmb = p[KP_WMB], xbB = p[KP_XBB + 0], ybB = p[KP_XBB + 1], zbB = p[KP_XBB + 2];
+    double t[6], e[6];
+    t[0] = tau[0] - a3w * q + a2v * r - wmb * sth;
+    t[1] = tau[1] - a1u * r + a3w * pp + wmb * cs;
+    t[2] = tau[2] - a2v * pp + a1u * q + wmb * cc;
+    t[3] = tau[3] - p[KP_DA + 0] * (v * w) - p[KP_DB + 0] * (q * r) - ybB * cc + zbB * cs;
+    t[4] = tau[4] - p[KP_DA + 1] * (u * w) - p[KP_DB + 1] * (pp * r) + zbB * sth + xbB * cc;
+    t[5] = tau[5] - p[KP_DA + 2] * (u * v) - p[KP_DB + 2] * (pp * q) - xbB * cs - ybB * sth;
+#pragma unroll
+    for (int i = 0; i < 6; ++i) {
+        e[i] = p[KP_MINV + i] * g[i];
+        const double an = abs_(nur[i]);
+        gk[KP_MINV + i] += g[i] * (t[i] - (p[KP_DQ + i] * an + p[KP_DL + i]) * nur[i]);
+        gk[KP_DL + i] -= e[i] * nur[i];
+        gk[KP_DQ + i] -= e[i] * an * nur[i];
+    }
+    gk[KP_A + 0] += u * (q * e[2] - r * e[1]);
+    gk[KP_A + 1] += v * (r * e[0] - pp * e[2]);
+    gk[KP_A + 2] += w * (pp * e[1] - q * e[0]);
+    gk[KP_DA + 0] -= v * w * e[3];
+    gk[KP_DA + 1] -= u * w * e[4];
+    gk[KP_DA + 2] -= u * v * e[5];
+    gk[KP_DB + 0] -= q * r * e[3];
+    gk[KP_DB + 1] -= pp * r * e[4];
+    gk[KP_DB + 2] -= pp * q * e[5];
+    gk[KP_WMB] += cs * e[1] + cc * e[2] - sth * e[0];
+    gk[KP_XBB + 0] += cc * e[4] - cs * e[5];
+    gk[KP_XBB + 1] -= cc * e[3] + sth * e[5];
+    gk[KP_XBB + 2] += cs * e[3] + sth * e[4];
+}
+
 // Euler-angle models: xdot[12] from x[12] and the body wrench tau[6].
 template <typename T> struct Trig { T sphi, cphi, sth, cth, spsi, cpsi; };
 
@@ -411,10 +451,13 @@ __device__ __forceinline__ void rhs_euler12(const T* __restrict__ x, const Trig<
 // Reverse mode of rhs_euler12 (fp64) at (x, tau) with the sines and cosines tr of x[3..5]: g[12] is the cotangent of
 // xd; a[12] receives the cotangent of x and gtau[6] that of tau.  Same convention as the dual instantiation of
 // rhs_euler12: the clamped cos(theta) (|c| < 1e-7) is a constant, otherwise d(1/c) = -dc / c^2.
-template <class P>
+// COEF: also adds the coefficient cotangent to gk (nu_dot_coef_vjp at the wrench tau, and gk[KP_CUR ..] = -R gnur,
+// which needs has_current: with a zero current nu - R^T 0 = nu, so the primal is unchanged).
+template <bool COEF = false, class P, class G = double*>
 __device__ __forceinline__ void rhs_euler12_vjp(const double* __restrict__ x, const Trig<double>& tr,
                                                 const P& p, bool has_current, const double* __restrict__ g,
-                                                double* __restrict__ a, double* __restrict__ gtau) {
+                                                double* __restrict__ a, double* __restrict__ gtau,
+                                                const double* __restrict__ tau = nullptr, const G& gk = G()) {
     const double sphi = tr.sphi, cphi = tr.cphi, sth = tr.sth, cth = tr.cth, spsi = tr.spsi, cpsi = tr.cpsi;
     const double* nu = x + 6;
     double nur[6] = {nu[0], nu[1], nu[2], nu[3], nu[4], nu[5]};
@@ -433,6 +476,7 @@ __device__ __forceinline__ void rhs_euler12_vjp(const double* __restrict__ x, co
     }
     double gnu[6], gnur[6], gsth, gcs, gcc;
     nu_dot_vjp(nu, nur, p, g + 6, gnu, gnur, gsth, gcs, gcc, gtau);
+    if constexpr (COEF) nu_dot_coef_vjp(nu, nur, tau, sth, cth * sphi, cth * cphi, p, g + 6, gk);
     double gsphi = cth * gcs, gcphi = cth * gcc, gcth = sphi * gcs + cphi * gcc, gspsi = 0.0, gcpsi = 0.0;
 #pragma unroll
     for (int i = 0; i < 6; ++i) gnu[i] += gnur[i];
@@ -447,6 +491,11 @@ __device__ __forceinline__ void rhs_euler12_vjp(const double* __restrict__ x, co
         gsth += x1 * gz2 - cz * gx2;
         gcpsi += cx * gx1 + cy * gy1;
         gspsi += cy * gx1 - cx * gy1;
+        if constexpr (COEF) {   // x1, y1 = Rz^T c; (x2, z2) = Ry^T (x1, cz)
+            gk[KP_CUR + 0] += cpsi * gx1 - spsi * gy1;
+            gk[KP_CUR + 1] += spsi * gx1 + cpsi * gy1;
+            gk[KP_CUR + 2] += cth * gz2 - sth * gx2;
+        }
     }
     // Euler rates
     {
@@ -546,11 +595,12 @@ __device__ __forceinline__ void quat_normalize_vjp(const double* __restrict__ q,
 
 // Reverse mode of rhs_quat13 (fp64) at (x, tau): g[13] is the cotangent of xd; a[13] receives the cotangent of x and
 // gtau[6] that of tau.  The quaternion is normalised inside the right-hand side, so its cotangent passes through
-// quat_normalize_vjp.
-template <class P>
+// quat_normalize_vjp.  COEF: as rhs_euler12_vjp.
+template <bool COEF = false, class P, class G = double*>
 __device__ __forceinline__ void rhs_quat13_vjp(const double* __restrict__ x, const P& p, bool has_current,
                                                const double* __restrict__ g, double* __restrict__ a,
-                                               double* __restrict__ gtau) {
+                                               double* __restrict__ gtau, const double* __restrict__ tau = nullptr,
+                                               const G& gk = G()) {
     double qw = x[3], qx = x[4], qy = x[5], qz = x[6];
     {
         const double n = sqrt(qw * qw + qx * qx + qy * qy + qz * qz);
@@ -571,6 +621,7 @@ __device__ __forceinline__ void rhs_quat13_vjp(const double* __restrict__ x, con
     }
     double gnu[6], gnur[6], gsth, gcs, gcc;
     nu_dot_vjp(nu, nur, p, g + 7, gnu, gnur, gsth, gcs, gcc, gtau);
+    if constexpr (COEF) nu_dot_coef_vjp(nu, nur, tau, -R20, R21, R22, p, g + 7, gk);
     // restoring terms: sth = -R20, cs = R21, cc = R22
     double gR00 = 0.0, gR01 = 0.0, gR02 = 0.0, gR10 = 0.0, gR11 = 0.0, gR12 = 0.0;
     double gR20 = -gsth, gR21 = gcs, gR22 = gcc;
@@ -580,6 +631,11 @@ __device__ __forceinline__ void rhs_quat13_vjp(const double* __restrict__ x, con
         gR00 -= cx * gnur[0]; gR10 -= cy * gnur[0]; gR20 -= cz * gnur[0];
         gR01 -= cx * gnur[1]; gR11 -= cy * gnur[1]; gR21 -= cz * gnur[1];
         gR02 -= cx * gnur[2]; gR12 -= cy * gnur[2]; gR22 -= cz * gnur[2];
+        if constexpr (COEF) {   // nur[0..2] -= R^T c
+            gk[KP_CUR + 0] -= R00 * gnur[0] + R01 * gnur[1] + R02 * gnur[2];
+            gk[KP_CUR + 1] -= R10 * gnur[0] + R11 * gnur[1] + R12 * gnur[2];
+            gk[KP_CUR + 2] -= R20 * gnur[0] + R21 * gnur[1] + R22 * gnur[2];
+        }
     }
     // position rates xd[0..2] = R nu[0..2]
     gR00 += g[0] * nu[0]; gR01 += g[0] * nu[1]; gR02 += g[0] * nu[2];

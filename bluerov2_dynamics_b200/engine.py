@@ -9,6 +9,7 @@ vehicles / windows with one kernel launch.  Array conventions follow the referen
 from __future__ import annotations
 
 import ctypes as C
+from contextlib import contextmanager, nullcontext as _nullcontext
 from dataclasses import dataclass
 from typing import Optional, Sequence
 
@@ -58,6 +59,29 @@ def with_minv(phys: np.ndarray) -> np.ndarray:
 
 # kernel coefficient vector layout (include/brov.h, csrc/brov_device.cuh KP_*)
 KP_MINV, KP_A, KP_DA, KP_DB, KP_DL, KP_DQ, KP_WMB, KP_XBB, KP_CUR = 0, 6, 9, 12, 15, 21, 27, 28, 31
+
+
+def derive_params_torch(phys: torch.Tensor, rebuild_minv: bool = True) -> torch.Tensor:
+    """Differentiable torch twin of derive_params(with_minv(phys)) (of derive_params(phys) without rebuild_minv):
+    physical vector(s) [..., NPHYS] -> kernel coefficients [..., NKP], same dtype and device, so that dL/dphys follows
+    from a coefficient gradient (Engine.rollout_diff(kp=...), Engine.rollout_vjp(coef=True)) by autograd.  Its
+    Jacobian is coefficient_directions.  The first-order wrench lag entry (1/T_lag1, 0 without a lag) carries no
+    gradient."""
+    ph = phys
+    m = ph[..., L.PH_M:L.PH_M + 1]
+    a = m - ph[..., L.PH_ADDED:L.PH_ADDED + 3]
+    b = ph[..., L.PH_I:L.PH_I + 3] - ph[..., L.PH_ADDED + 3:L.PH_ADDED + 6]
+    minv = torch.cat([1.0 / a, 1.0 / b], dim=-1) if rebuild_minv else ph[..., L.PH_MINV:L.PH_MINV + 6]
+    a0, a1, a2 = a.unbind(-1)
+    b0, b1, b2 = b.unbind(-1)
+    B = ph[..., L.PH_B:L.PH_B + 1]
+    tl = ph[..., L.PH_TLAG1:L.PH_TLAG1 + 1].detach()
+    ilag = torch.where(tl > 0.0, 1.0 / torch.where(tl > 0.0, tl, torch.ones_like(tl)), torch.zeros_like(tl))
+    return torch.cat([minv, a, torch.stack([a2 - a1, a0 - a2, a1 - a0], dim=-1),
+                      torch.stack([b2 - b1, b0 - b2, b1 - b0], dim=-1),
+                      -ph[..., L.PH_LIN:L.PH_LIN + 6], -ph[..., L.PH_QUAD:L.PH_QUAD + 6],
+                      ph[..., L.PH_W:L.PH_W + 1] - B, ph[..., L.PH_XB:L.PH_XB + 3] * B,
+                      ph[..., L.PH_CURRENT:L.PH_CURRENT + 3], ilag, torch.zeros_like(ilag)], dim=-1)
 
 # names of the physical vector's entries: the reference's attribute names (fossen/BlueROV2.py:81-150); the ocean
 # current is `current_speed` split into its NED components, diag(Minv) is named after the velocity it scales
@@ -200,6 +224,7 @@ class VjpResult:
     gU: torch.Tensor                 # [T, N, NU] dL/du_k (always per vehicle)
     z: torch.Tensor                  # [N, NZ] z after the last step (the primal of linearize, projected lag)
     health: Optional[torch.Tensor]   # int64 [2]: vehicles with a non-finite z or gradient / near theta = +-pi/2, or None
+    gkp: Optional[torch.Tensor] = None   # [N, NKP] dL/dkp of each vehicle's coefficients (coef=True), or None
 
 
 _CL_LAYOUTS = ("const_shared", "shared", "const", "tnc")
@@ -277,6 +302,7 @@ class Engine:
         L.check(L.lib.brov_create(MODELS[model], self._code, self.device_index, C.byref(h)))
         self._h = h
         self._pv = None
+        self._pv_current = False
         self._ws = None
         self._alloc = None if self.is_di else default_allocation()[0]   # last allocation pushed to the library
         self.phys = default_physical(rho)
@@ -311,7 +337,30 @@ class Engine:
         soa = torch.from_numpy(np.ascontiguousarray(kp.T)).to(self.device, self.tdtype).contiguous()  # [NKP, N]
         self._pv = soa
         any_current = bool(np.any(np.asarray(phys_table, float)[..., L.PH_CURRENT:L.PH_CURRENT + 3] != 0.0))
+        self._pv_current = any_current
         L.check(L.lib.brov_set_vehicle_params(self._h, soa.data_ptr(), soa.shape[1], int(any_current)))
+
+    @contextmanager
+    def _coefficients(self, kp: torch.Tensor):
+        """Runs the body with the kernel coefficients kp (float64 [NKP]: shared, [N, NKP]: a per-vehicle table) in
+        place of the engine's own, which are restored afterwards, also when the body raises."""
+        k = kp.detach()
+        try:
+            if k.dim() == 1:
+                L.check(L.lib.brov_set_vehicle_params(self._h, None, 0, 0))
+                L.check(L.lib.brov_set_params(self._h, L.dptr(np.ascontiguousarray(k.cpu().numpy()))))
+            else:
+                soa = k.t().contiguous()
+                cur = bool((k[:, KP_CUR:KP_CUR + 3] != 0).any())
+                L.check(L.lib.brov_set_vehicle_params(self._h, soa.data_ptr(), soa.shape[1], int(cur)))
+            yield
+        finally:
+            self.set_physical(self.phys)
+            if self._pv is None:
+                L.check(L.lib.brov_set_vehicle_params(self._h, None, 0, 0))
+            else:
+                L.check(L.lib.brov_set_vehicle_params(self._h, self._pv.data_ptr(), self._pv.shape[1],
+                                                      int(self._pv_current)))
 
     def set_wrench_lag1(self, enable: bool, T_lag: Optional[float] = None) -> None:
         """First-order wrench lag tau_dot = (tau_cmd - tau)/T_lag (extension; wrench models only)."""
@@ -983,7 +1032,7 @@ class Engine:
 
     def rollout_vjp(self, x0, U, gtraj=None, gzT=None, stride: int = 0, dt: float = 0.02, integrator: str = "rk4",
                     lag0=None, lag_repr: str = "thruster", u_layout: str = "auto", health: bool = False,
-                    singular_eps: float = 0.0) -> VjpResult:
+                    singular_eps: float = 0.0, coef: bool = False) -> VjpResult:
         """Reverse-mode gradients of N rollouts (brov_rollout_vjp): for every vehicle, with
             L = sum_{k = stride, 2 stride, ... <= T} <c_k, x_k> + <g_T, z_T>,
         returns dL/dz_0 (as gx0 and glag0) and dL/du_k for every step, in one launch and without forming the step
@@ -996,7 +1045,10 @@ class Engine:
         lag0 (thruster model): per-thruster [N,24] with lag_repr="thruster", projected [N,18] with "projected";
         glag0 comes back in the same representation (per thruster: P^T gZ0 by the chain rule with Z = P L).
         The call allocates its workspace, T * N * NZ doubles; split longer horizons as include/brov.h describes.
-        fp64 engines with shared coefficients."""
+        fp64 engines with shared coefficients.
+        coef=True (brov_rollout_vjp_coef): also returns gkp [N, NKP], dL/dkp of each vehicle's kernel coefficients
+        (derive_params layout; the lag entries are 0), and accepts a per-vehicle table (set_vehicle_physical) of N
+        rows; with shared coefficients their gradient is gkp.sum(0).  gx0, glag0 and gU are those of coef=False."""
         x0 = self.tensor(x0)
         self._check_rows(x0, self.nx, "x0")
         n = x0.shape[0]
@@ -1045,8 +1097,18 @@ class Engine:
         d.workspace_dev, d.workspace_bytes = ws.data_ptr(), ws.numel() * 8
         d.health_dev = hc.data_ptr() if hc is not None else None
         d.singular_eps = float(singular_eps)
+        gkp = None
         with torch.cuda.device(self.device):
-            L.check(L.lib.brov_rollout_vjp(self._h, C.byref(d), self._stream()))
+            if coef:
+                gkp = torch.empty((L.NKP, n), device=self.device, dtype=torch.float64)
+                dc = L.RolloutVjpCoefDesc()
+                dc.struct_size = C.sizeof(L.RolloutVjpCoefDesc)
+                dc.vjp = d
+                dc.gkp_dev = gkp.data_ptr()
+                L.check(L.lib.brov_rollout_vjp_coef(self._h, C.byref(dc), self._stream()))
+                gkp = gkp.t()
+            else:
+                L.check(L.lib.brov_rollout_vjp(self._h, C.byref(d), self._stream()))
         gx0 = gz0[:, :self.nx]
         glag0 = None
         if thr:
@@ -1056,18 +1118,32 @@ class Engine:
                 glag0 = torch.einsum("ci,nck->nik", A, gZ0.reshape(n, 6, 3)).reshape(n, 24).contiguous()
             else:
                 glag0 = gZ0
-        return VjpResult(gx0=gx0, glag0=glag0, gU=gU, z=z, health=hc)
+        return VjpResult(gx0=gx0, glag0=glag0, gU=gU, z=z, health=hc, gkp=gkp)
 
     def rollout_diff(self, x0: torch.Tensor, U: torch.Tensor, lag0: Optional[torch.Tensor] = None, dt: float = 0.02,
-                     integrator: str = "rk4", stride: int = 1, lag_repr: str = "projected"):
+                     integrator: str = "rk4", stride: int = 1, lag_repr: str = "projected",
+                     kp: Optional[torch.Tensor] = None):
         """Differentiable rollout: (traj [T//stride, N, NX] or None for stride 0, xT [N, NX], lagT [N, 18] or None)
         as `rollout` returns them, with torch autograd gradients to x0, U [T, N, NU] (per vehicle) and lag0 [N, 18].
         The forward is `rollout`; the backward is one `rollout_vjp` call.  The lag is exchanged in projected
-        coordinates (lag_repr="projected"), the form whose derivative the adjoint carries."""
+        coordinates (lag_repr="projected"), the form whose derivative the adjoint carries.
+        kp (float64, [NKP] shared or [N, NKP] per vehicle, e.g. from derive_params_torch): the rollout runs with these
+        kernel coefficients instead of the engine's, and their gradient flows back (rollout_vjp(coef=True), summed
+        over the vehicles for [NKP]).  The engine's own coefficients and table are restored after the forward and
+        the backward, also when either raises."""
         if lag_repr != "projected":
             raise ValueError("rollout_diff exchanges the projected lag: lag_repr must be 'projected'")
+        if kp is not None:
+            n = x0.shape[0]
+            if not isinstance(kp, torch.Tensor) or kp.dtype != torch.float64:
+                raise ValueError("kp must be a float64 tensor")
+            if tuple(kp.shape) not in ((L.NKP,), (n, L.NKP)):
+                raise ValueError(f"kp must have shape [{L.NKP}] or [{n}, {L.NKP}], got {tuple(kp.shape)}")
+            if self.dtype != "f64" or self.is_di:
+                raise ValueError("coefficient gradients need an fp64 engine of a Fossen model")
+            kp = kp.to(self.device)
         lag_t = lag0 if (lag0 is not None and self.model == "thruster8") else None
-        traj, xT, lagT = _RolloutDiff.apply(self, x0, U, lag_t, float(dt), integrator, int(stride))
+        traj, xT, lagT = _RolloutDiff.apply(self, x0, U, lag_t, float(dt), integrator, int(stride), kp)
         return (traj if stride else None), xT, (lagT if self.model == "thruster8" else None)
 
     def _cl_operand(self, v, inner: tuple, layout: str, n: int, what: str):
@@ -1390,15 +1466,17 @@ class _RolloutDiff(torch.autograd.Function):
     """Engine.rollout forward, Engine.rollout_vjp backward (Engine.rollout_diff)."""
 
     @staticmethod
-    def forward(ctx, eng, x0, U, lag0, dt, integrator, stride):
+    def forward(ctx, eng, x0, U, lag0, dt, integrator, stride, kp=None):
         if U.dim() != 3:
             raise ValueError("rollout_diff takes a per-vehicle U [T, N, NU]")
         thr = eng.model == "thruster8"
-        r = eng.rollout(x0.detach(), U.detach(), dt=dt, integrator=integrator,
-                        lag0=lag0.detach() if lag0 is not None else None, stride=stride,
-                        lag_repr="projected", want_lag=thr)
+        with eng._coefficients(kp) if kp is not None else _nullcontext():
+            r = eng.rollout(x0.detach(), U.detach(), dt=dt, integrator=integrator,
+                            lag0=lag0.detach() if lag0 is not None else None, stride=stride,
+                            lag_repr="projected", want_lag=thr)
         ctx.eng, ctx.dt, ctx.integrator, ctx.stride = eng, dt, integrator, stride
         ctx.has_lag = lag0 is not None
+        ctx.kp = kp.detach() if kp is not None else None
         ctx.save_for_backward(x0, U, *([lag0] if lag0 is not None else []))
         n = x0.shape[0]
         traj = r.traj if stride else torch.empty((0, n, eng.nx), device=eng.device, dtype=eng.tdtype)
@@ -1420,11 +1498,17 @@ class _RolloutDiff(torch.autograd.Function):
         else:
             gzT = gx.contiguous()
         gt = gtraj.contiguous() if (gtraj is not None and ctx.stride and gtraj.numel()) else None
-        res = eng.rollout_vjp(x0.detach(), U.detach(), gtraj=gt, gzT=gzT, stride=ctx.stride if gt is not None else 0,
-                              dt=ctx.dt, integrator=ctx.integrator, lag0=lag0.detach() if lag0 is not None else None,
-                              lag_repr="projected", u_layout="tnc")
+        kp = ctx.kp
+        with eng._coefficients(kp) if kp is not None else _nullcontext():
+            res = eng.rollout_vjp(x0.detach(), U.detach(), gtraj=gt, gzT=gzT,
+                                  stride=ctx.stride if gt is not None else 0, dt=ctx.dt, integrator=ctx.integrator,
+                                  lag0=lag0.detach() if lag0 is not None else None, lag_repr="projected",
+                                  u_layout="tnc", coef=kp is not None)
         glag = res.glag0 if (thr and ctx.has_lag) else None
-        return None, res.gx0, res.gU, glag, None, None, None
+        gkp = None
+        if kp is not None:
+            gkp = res.gkp.sum(0) if kp.dim() == 1 else res.gkp
+        return None, res.gx0, res.gU, glag, None, None, None, gkp
 
 
 def reduced9_rhs(x: torch.Tensor, u: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:

@@ -602,6 +602,26 @@ int brov_rollout_vjp(brov_engine_t* e, const brov_rollout_vjp_desc* d, void* str
  * <= 0; SIZE_MAX if the size does not fit in size_t) */
 size_t brov_rollout_vjp_workspace_bytes(int model, long long n, long long steps);
 
+/* brov_rollout_vjp plus the gradient of the same L in the kernel coefficients (the BROV_KP_* vector of
+ * brov_derive_params) of every vehicle: gkp_dev [BROV_NKP][n] (double, required), gkp[j][i] = dL/dkp_j of vehicle i.
+ * Calibration and system identification need it: with phys the physical vector, dL/dphys = gkp^T dkp/dphys (the chain
+ * over brov_derive_params), at the cost of one adjoint sweep whatever the number of parameters.  Every stage adds
+ * lambda^T df/dkp; the entries of the first-order wrench lag and the pad are 0, the current's are computed whether or
+ * not a current is set.  Coefficients: the engine's shared ones, or its per-vehicle table (brov_set_vehicle_params),
+ * which must then have n rows (BROV_EINVAL otherwise).  gkp has the table's layout, so the gradient in shared
+ * coefficients is the sum of gkp over vehicles.  vjp: every field, refusal and the workspace as for
+ * brov_rollout_vjp (vjp.struct_size = sizeof(brov_rollout_vjp_desc)); gx0, gu and z_out are those brov_rollout_vjp
+ * returns.  Vehicles with a non-finite gkp entry count in health_dev[0].  Chaining as for brov_rollout_vjp: gz0 and gu
+ * are those of one call bit for bit; each call writes the gkp of its own steps, and their sum equals the gkp of one call
+ * to rounding. */
+typedef struct brov_rollout_vjp_coef_desc {
+    uint32_t struct_size;          /* = sizeof(brov_rollout_vjp_coef_desc) */
+    int32_t reserved;
+    brov_rollout_vjp_desc vjp;
+    void* gkp_dev;
+} brov_rollout_vjp_coef_desc;
+int brov_rollout_vjp_coef(brov_engine_t* e, const brov_rollout_vjp_coef_desc* d, void* stream);
+
 /* Reduced 9-state RHS — `bluerov_compute(t, x_, u_)` (fossen/bluerov_torch.py:20-67, constants fossen/parameters.py).
  * x [B][9], u [B][4], out [B][9]. */
 int brov_reduced9_rhs(int dtype, const void* x_dev, const void* u_dev, void* out_dev, long long B, void* stream);
