@@ -17,7 +17,7 @@ import importlib as _importlib
 
 __all__ = ["Engine", "RolloutResult", "InputGenerator", "BrovError", "default_physical", "derive_params", "derive_params_torch", "default_allocation",
            "lag_discretize", "with_minv", "coefficient_directions", "parameter_indices", "GradResult", "LinearizeResult", "ClosedLoopResult", "EkfResult",
-           "VjpResult",
+           "VjpResult", "ClosedLoopVjpResult",
            "reduced9_rhs",
            "fma_peak", "pinned_empty", "install_as_fossen", "LIB_PATH"]
 

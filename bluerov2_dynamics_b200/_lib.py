@@ -125,6 +125,19 @@ class RolloutVjpCoefDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("reserved", C.c_int32), ("vjp", RolloutVjpDesc), ("gkp_dev", C.c_void_p)]
 
 
+class ClosedLoopVjpDesc(C.Structure):
+    _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
+                ("dt", C.c_double), ("z0_dev", C.c_void_p), ("K_dev", C.c_void_p), ("K_stride_t", C.c_longlong),
+                ("K_stride_n", C.c_longlong), ("z_ref_dev", C.c_void_p), ("z_ref_stride_t", C.c_longlong),
+                ("z_ref_stride_n", C.c_longlong), ("u_ref_dev", C.c_void_p), ("u_ref_stride_t", C.c_longlong),
+                ("u_ref_stride_n", C.c_longlong), ("u_min", C.c_double * 8), ("u_max", C.c_double * 8),
+                ("q", C.c_double * 30), ("r", C.c_double * 8), ("gtraj_dev", C.c_void_p), ("stride", C.c_longlong),
+                ("gzT_dev", C.c_void_p), ("gcost_dev", C.c_void_p), ("gz0_dev", C.c_void_p), ("gK_dev", C.c_void_p),
+                ("gz_ref_dev", C.c_void_p), ("gu_ref_dev", C.c_void_p), ("z_out_dev", C.c_void_p),
+                ("workspace_dev", C.c_void_p), ("workspace_bytes", C.c_size_t), ("health_dev", C.c_void_p),
+                ("singular_eps", C.c_double)]
+
+
 class RolloutHostDesc(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("integrator", C.c_int32), ("n", C.c_longlong), ("steps", C.c_longlong),
                 ("dt", C.c_double), ("x0_host", C.c_void_p), ("xT_host", C.c_void_p), ("u_host", C.c_void_p),
@@ -192,6 +205,8 @@ _PROTOS = {
     "brov_rollout_vjp": (C.c_int, [C.c_void_p, C.POINTER(RolloutVjpDesc), C.c_void_p]),
     "brov_rollout_vjp_workspace_bytes": (C.c_size_t, [C.c_int, C.c_longlong, C.c_longlong]),
     "brov_rollout_vjp_coef": (C.c_int, [C.c_void_p, C.POINTER(RolloutVjpCoefDesc), C.c_void_p]),
+    "brov_closed_loop_vjp": (C.c_int, [C.c_void_p, C.POINTER(ClosedLoopVjpDesc), C.c_void_p]),
+    "brov_closed_loop_vjp_workspace_bytes": (C.c_size_t, [C.c_int, C.c_longlong, C.c_longlong]),
     "brov_reduced9_rhs": (C.c_int, [C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "brov_koopman_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, _DP, _DP, _DP, C.POINTER(C.c_void_p)]),
     "brov_koopman_destroy": (None, [C.c_void_p]),

@@ -16,6 +16,8 @@
 // Every sum has a fixed order, so the results are bit-reproducible and independent of the other vehicles.
 #include "brov_adj.cuh"
 
+#include <algorithm>
+
 namespace brov {
 
 // right-hand side of sub-step s at the stage state xs, as linearize evaluates it (full sines and cosines)
@@ -612,6 +614,512 @@ cudaError_t launch_adjoint_coef(int model, int integ, const AdjCoefArgs& a, cuda
         case MODEL_THRUSTER8: return adjoint_coef_integ<MODEL_THRUSTER8>(integ, a, st);
         case MODEL_WRENCH12: return adjoint_coef_integ<MODEL_WRENCH12>(integ, a, st);
         case MODEL_QUAT13: return adjoint_coef_integ<MODEL_QUAT13>(integ, a, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+
+// ---------------------------------------------------------------------------------------------------------------
+// closed-loop adjoint (brov_closed_loop_vjp)
+// ---------------------------------------------------------------------------------------------------------------
+
+// dz_j = z_j - zr_j, the Euler angles wrapped to one turn with closed_loop_kernel's arithmetic (derivative 1)
+template <int MODEL>
+__device__ __forceinline__ double cl_dz(double z, double zr, int j) {
+    double d = z - zr;
+    if (!ModelDim<MODEL>::QUAT && j >= 3 && j < 6) d = fma(-6.283185307179586, rint(d * 0.15915494309189535), d);
+    return d;
+}
+
+// u = clamp(ur - K dz, u_min, u_max) with closed_loop_kernel's fixed-order fmas (per j, every channel); m[r]: channel r
+// not clamped (a NaN takes that branch, as the compare-select does)
+template <int MODEL>
+__device__ __forceinline__ void cl_feedback(const ClAdjArgs& a, const double* __restrict__ x, const double* __restrict__ Z,
+                                            const double* Kk, const double* zrk, const double* urk, double* __restrict__ u,
+                                            bool* __restrict__ m) {
+    constexpr int NX = LinDim<MODEL>::NX, NU = LinDim<MODEL>::NU, NZ = LinDim<MODEL>::NZ;
+#pragma unroll
+    for (int r = 0; r < NU; ++r) u[r] = __ldg(urk + r);
+#pragma unroll
+    for (int j = 0; j < NZ; ++j) {
+        const double d = cl_dz<MODEL>(j < NX ? x[j] : Z[j < NX ? 0 : j - NX], __ldg(zrk + j), j);
+#pragma unroll
+        for (int r = 0; r < NU; ++r) u[r] = fma(-Kk[r * NZ + j], d, u[r]);
+    }
+#pragma unroll
+    for (int r = 0; r < NU; ++r) {
+        const bool lo = u[r] < a.u_min[r], hi = u[r] > a.u_max[r];
+        m[r] = !(lo || hi);
+        u[r] = lo ? a.u_min[r] : (hi ? a.u_max[r] : u[r]);
+    }
+}
+
+// The sweep of brov_closed_loop_vjp, a sibling of adjoint_kernel / adjoint_coef_kernel (their code stays as it was).
+// Forward: u_k from the feedback law, the primal step of adjoint_kernel, z_k to the workspace.  Reverse: reload z_k,
+// recompute u_k (never stored) and the stage states, run adjoint_kernel's step VJP (lambda_{k+1} -> A^T lambda,
+// B^T lambda), then the feedback:
+//     gv = m . (B^T lambda + 2 g_c r . (u - ur))          dL/dv_k, m the clamp mask
+//     gdz = -K_k^T gv + 2 g_c q . dz_k                    lambda_k = A^T lambda + gdz + c_k (the lag rows into mu)
+// and stores gv, dL/dur_k = gv - 2 g_c r . (u - ur) and dL/dzr_k = -gdz for the reductions.  Dynamic shared memory:
+// [RK4 stage buffer (3 NX rows) | PV: the vehicle's table column (KP_COUNT rows) | the staged K (k_smem)].
+template <int MODEL, int INTEG, bool PV>
+__global__ void __launch_bounds__(ADJ_THREADS) closed_loop_adjoint_kernel(const __grid_constant__ ClAdjArgs a) {
+    constexpr int NX = LinDim<MODEL>::NX, NU = LinDim<MODEL>::NU, NZ = LinDim<MODEL>::NZ;
+    constexpr bool THR = MODEL == MODEL_THRUSTER8;
+    constexpr bool QUAT = ModelDim<MODEL>::QUAT;
+    constexpr int NL = THR ? 18 : 1;
+    extern __shared__ double smem[];
+    const Consts<double>& c = a.c;
+    const bool cur = c.has_current != 0;
+    const int tid = threadIdx.x;
+    double* sx = smem + tid;
+    const long long v = (long long)blockIdx.x * ADJ_THREADS + tid;
+    const long long n = a.n;
+    const long long vc = v < n ? v : n - 1;   // dead lanes stage the last vehicle's column, never store
+    double* rest = smem + adjoint_coef_stage_rows(MODEL, INTEG) * ADJ_THREADS;
+    typename std::conditional<PV, ParamsShared<double>, ParamsConst<double>>::type p;
+    if constexpr (PV) {
+        const double* pvt = a.pv + vc;
+#pragma unroll 4
+        for (int j = 0; j < KP_COUNT; ++j) rest[j * ADJ_THREADS + tid] = pvt[(long long)j * n];
+        p.base = rest + tid;
+        p.pitch = ADJ_THREADS;
+        rest += KP_COUNT * ADJ_THREADS;
+    } else {
+        p.kp = c.kp;
+    }
+    const double* Kp;
+    if (a.k_smem) {
+        for (int j = tid; j < NU * NZ; j += ADJ_THREADS) rest[j] = a.K[j];
+        Kp = rest;
+    } else {
+        Kp = a.K + vc * a.K_sn;
+    }
+    __syncthreads();
+    bool bad = false, sing = false;
+    if (v < n) {
+        const double* zrp = a.zr + v * a.zr_sn;
+        const double* urp = a.ur + v * a.ur_sn;
+        // ---- forward: z_k -> workspace
+        double x[NX], Z[NL];
+#pragma unroll
+        for (int q = 0; q < NX; ++q) x[q] = a.z0[v * NZ + q];
+#pragma unroll
+        for (int q = 0; q < NL; ++q) Z[q] = THR ? a.z0[v * NZ + NX + q] : 0.0;
+        for (int k = 0; k < a.steps; ++k) {
+            double* wk = a.ws + (long long)k * NZ * n + v;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) wk[q * n] = x[q];
+            if constexpr (THR) {
+#pragma unroll
+                for (int q = 0; q < NL; ++q) wk[(NX + q) * n] = Z[q];
+            }
+            double u[NU];
+            bool m[NU];
+            cl_feedback<MODEL>(a, x, Z, Kp + (long long)k * a.K_st, zrp + (long long)k * a.zr_st,
+                               urp + (long long)k * a.ur_st, u, m);
+            double Fw[6];
+            if constexpr (THR) {
+                double F[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, u[i]);
+                allocate_wrench<double>(c, F, Fw);
+            } else {
+#pragma unroll
+                for (int r = 0; r < 6; ++r) Fw[r] = u[r];
+            }
+            double acth;
+            adj_step<MODEL, INTEG, false>(c, p, x, Z, Fw, nullptr, nullptr, acth);
+            sing |= acth < a.eps;
+            if constexpr (THR) lag_advance<double, true>(c, Z, Fw);
+        }
+#pragma unroll
+        for (int q = 0; q < NX; ++q) bad |= !adj_finite(x[q]);
+#pragma unroll
+        for (int q = 0; q < NL; ++q) bad |= THR && !adj_finite(Z[q]);
+        if (a.z_out) {
+#pragma unroll
+            for (int q = 0; q < NX; ++q) a.z_out[v * NZ + q] = x[q];
+            if constexpr (THR) {
+#pragma unroll
+                for (int q = 0; q < NL; ++q) a.z_out[v * NZ + NX + q] = Z[q];
+            }
+        }
+
+        // ---- backward: lam = dL/dx_k, mu = dL/dZ_k
+        double lam[NX], mu[NL];
+#pragma unroll
+        for (int q = 0; q < NX; ++q) lam[q] = a.gzT ? a.gzT[v * NZ + q] : 0.0;
+#pragma unroll
+        for (int q = 0; q < NL; ++q) mu[q] = (THR && a.gzT) ? a.gzT[v * NZ + NX + q] : 0.0;
+        if (a.gtraj && a.steps % a.stride == 0) {
+            const double* gt = a.gtraj + ((long long)(a.steps / a.stride - 1) * n + v) * NZ;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) lam[q] += gt[q];
+            if constexpr (THR) {
+#pragma unroll
+                for (int q = 0; q < NL; ++q) mu[q] += gt[NX + q];
+            }
+        }
+        const bool cost = a.gcost != nullptr;
+        const double gc2 = cost ? 2.0 * a.gcost[v] : 0.0;
+        const double dt = c.dt, hdt = 0.5 * dt, dt6 = dt * (1.0 / 6.0), dt3 = 2.0 * dt6;
+        for (int k = a.steps - 1; k >= 0; --k) {
+            const double* wk = a.ws + (long long)k * NZ * n + v;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
+            if constexpr (THR) {
+#pragma unroll
+                for (int q = 0; q < NL; ++q) Z[q] = wk[(NX + q) * n];
+            }
+            const double* Kk = Kp + (long long)k * a.K_st;
+            const double* zrk = zrp + (long long)k * a.zr_st;
+            const double* urk = urp + (long long)k * a.ur_st;
+            double u[NU];
+            bool m[NU];
+            cl_feedback<MODEL>(a, x, Z, Kk, zrk, urk, u, m);
+            double Fw[6];
+            if constexpr (THR) {
+                double F[8];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, u[i]);
+                allocate_wrench<double>(c, F, Fw);
+            } else {
+#pragma unroll
+                for (int r = 0; r < 6; ++r) Fw[r] = u[r];
+            }
+            // recompute the stage states (and the quaternion before its renormalisation)
+            double qpre[4];
+            if constexpr (INTEG == INTEG_RK4 || QUAT) {
+                double xw[NX];
+#pragma unroll
+                for (int q = 0; q < NX; ++q) xw[q] = x[q];
+                double acth;
+                adj_step<MODEL, INTEG, true>(c, p, xw, Z, Fw, sx, qpre, acth);
+            }
+            if constexpr (QUAT) quat_normalize_vjp(qpre, lam + 3);
+            // lag: Z' = lagA Z_c + lagB Fw_c per channel
+            double muF[6];
+            if constexpr (THR) {
+#pragma unroll
+                for (int ch = 0; ch < 6; ++ch) {
+                    const double m0 = mu[3 * ch], m1 = mu[3 * ch + 1], m2 = mu[3 * ch + 2];
+#pragma unroll
+                    for (int j = 0; j < 3; ++j) mu[3 * ch + j] = c.lagA[0][j] * m0 + c.lagA[1][j] * m1 + c.lagA[2][j] * m2;
+                    muF[ch] = c.lagB[0] * m0 + c.lagB[1] * m1 + c.lagB[2] * m2;
+                }
+            } else {
+#pragma unroll
+                for (int ch = 0; ch < 6; ++ch) muF[ch] = 0.0;
+            }
+            double lamp[NX], kap[NX];
+#pragma unroll
+            for (int q = 0; q < NX; ++q) lamp[q] = lam[q];
+            // stage s at xs with the cotangent kap of its right-hand side (as adjoint_kernel)
+            auto stage_vjp = [&](int s, const double* xs, double* ga) {
+                double b[6];
+                if constexpr (QUAT) {
+                    rhs_quat13_vjp(xs, p, cur, kap, ga, b);
+                } else {
+                    Trig<double> tr;
+                    trig_full<double>(c, xs + 3, tr);
+                    rhs_euler12_vjp(xs, tr, p, cur, kap, ga, b);
+                }
+#pragma unroll
+                for (int q = 0; q < NX; ++q) lam[q] += ga[q];
+#pragma unroll
+                for (int ch = 0; ch < 6; ++ch) {
+                    if constexpr (THR) {
+#pragma unroll
+                        for (int j = 0; j < 3; ++j) mu[3 * ch + j] += c.lagG[s][j] * b[ch];
+                        muF[ch] += c.lagH[s] * b[ch];
+                    } else {
+                        muF[ch] += b[ch];
+                    }
+                }
+            };
+            double ga[NX];
+            if constexpr (INTEG == INTEG_EULER) {
+#pragma unroll
+                for (int q = 0; q < NX; ++q) kap[q] = dt * lamp[q];
+                stage_vjp(0, x, ga);
+            } else {
+#pragma unroll
+                for (int q = 0; q < NX; ++q) kap[q] = dt6 * lamp[q];
+#pragma unroll
+                for (int s = 3; s >= 1; --s) {
+                    double xs[NX];
+#pragma unroll
+                    for (int q = 0; q < NX; ++q) xs[q] = sx[((s - 1) * NX + q) * ADJ_THREADS];
+                    stage_vjp(s, xs, ga);
+                    const double cs = (s == 1) ? dt6 : dt3;
+                    const double hs = (s == 3) ? dt : hdt;
+#pragma unroll
+                    for (int q = 0; q < NX; ++q) kap[q] = fma(hs, ga[q], cs * lamp[q]);
+                }
+#pragma unroll
+                for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
+                stage_vjp(0, x, ga);
+            }
+            // the feedback: gu = B^T lambda as adjoint_kernel forms it, then gv and dL/dur
+            double gv[NU];
+#pragma unroll
+            for (int i = 0; i < NU; ++i) {
+                double g;
+                if constexpr (THR) {
+                    double s = 0.0;
+#pragma unroll
+                    for (int r = 0; r < 6; ++r) {
+                        const bool nz = (r < 2) ? (i < 4) : (r == 2) ? (i >= 4) : (r == 5) ? (i < 4) : true;
+                        if (nz) s += c.alloc[r][i] * muF[r];
+                    }
+                    g = thrust_poly_d(c, u[i]) * s;
+                } else {
+                    g = muF[i];
+                }
+                const double gc = cost ? gc2 * a.r[i] * (u[i] - __ldg(urk + i)) : 0.0;
+                gv[i] = m[i] ? g + gc : 0.0;
+                const double gur = gv[i] - gc;
+                bad |= !adj_finite(gur);
+                if (a.wgv) a.wgv[((long long)k * NU + i) * n + v] = gv[i];
+                if (a.wgur) a.wgur[((long long)k * NU + i) * n + v] = gur;
+            }
+            // lambda_k = A^T lambda + gdz (+ c_k below); dL/dzr_k = -gdz.  With the gain gradient requested, its entries
+            // -gv_r dz_j are all finite exactly when max_r |gv_r| max_j |dz_j| is (the dz maximum keeps a NaN; a
+            // non-finite gv is counted through dL/dur)
+            const bool gk = a.wgv != nullptr;
+            double dmax = 0.0;
+#pragma unroll
+            for (int j = 0; j < NZ; ++j) {
+                const double zj = j < NX ? x[j] : Z[j < NX ? 0 : j - NX];
+                const double d = (cost || gk) ? cl_dz<MODEL>(zj, __ldg(zrk + j), j) : 0.0;
+                dmax = fabs(d) > dmax || d != d ? fabs(d) : dmax;
+                double g = cost ? gc2 * a.q[j] * d : 0.0;
+#pragma unroll
+                for (int r = 0; r < NU; ++r) g = fma(-Kk[r * NZ + j], gv[r], g);
+                if (j < NX) lam[j] += g; else mu[j < NX ? 0 : j - NX] += g;
+                bad |= !adj_finite(g);
+                if (a.wgzr) a.wgzr[((long long)k * NZ + j) * n + v] = -g;
+            }
+            if (gk) {
+                double gvmax = 0.0;
+#pragma unroll
+                for (int r = 0; r < NU; ++r) gvmax = fabs(gv[r]) > gvmax ? fabs(gv[r]) : gvmax;
+                bad |= !adj_finite(gvmax * dmax);
+            }
+            if (a.gtraj && k > 0 && k % a.stride == 0) {
+                const double* gt = a.gtraj + ((long long)(k / a.stride - 1) * n + v) * NZ;
+#pragma unroll
+                for (int q = 0; q < NX; ++q) lam[q] += gt[q];
+                if constexpr (THR) {
+#pragma unroll
+                    for (int q = 0; q < NL; ++q) mu[q] += gt[NX + q];
+                }
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < NX; ++q) {
+            a.gz0[v * NZ + q] = lam[q];
+            bad |= !adj_finite(lam[q]);
+        }
+        if constexpr (THR) {
+#pragma unroll
+            for (int q = 0; q < NL; ++q) {
+                a.gz0[v * NZ + NX + q] = mu[q];
+                bad |= !adj_finite(mu[q]);
+            }
+        }
+    }
+    if (a.health) {
+        const int nb = __syncthreads_count(bad);
+        const int ns = __syncthreads_count(sing);
+        if (tid == 0) {
+            if (nb) atomicAdd(a.health + 0, (unsigned long long)nb);
+            if (ns) atomicAdd(a.health + 1, (unsigned long long)ns);
+        }
+    }
+}
+
+template <int MODEL, int INTEG, bool PV>
+static cudaError_t closed_loop_adjoint_go(const ClAdjArgs& a, cudaStream_t st) {
+    constexpr int KN = LinDim<MODEL>::NU * LinDim<MODEL>::NZ;
+    auto kern = closed_loop_adjoint_kernel<MODEL, INTEG, PV>;
+    const size_t smem = (size_t)(adjoint_coef_stage_rows(MODEL, INTEG) + (PV ? KP_COUNT : 0)) * ADJ_THREADS * sizeof(double) +
+                        (a.k_smem ? (size_t)KN * sizeof(double) : 0);
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    const long long grid = (a.n + ADJ_THREADS - 1) / ADJ_THREADS;
+    kern<<<(unsigned)grid, ADJ_THREADS, smem, st>>>(a);
+    return cudaGetLastError();
+}
+
+template <int MODEL>
+static cudaError_t closed_loop_adjoint_integ(int integ, const ClAdjArgs& a, cudaStream_t st) {
+    const bool pv = a.pv != nullptr;
+    if (integ == INTEG_RK4)
+        return pv ? closed_loop_adjoint_go<MODEL, INTEG_RK4, true>(a, st) : closed_loop_adjoint_go<MODEL, INTEG_RK4, false>(a, st);
+    return pv ? closed_loop_adjoint_go<MODEL, INTEG_EULER, true>(a, st) : closed_loop_adjoint_go<MODEL, INTEG_EULER, false>(a, st);
+}
+
+cudaError_t launch_closed_loop_adjoint(int model, int integ, const ClAdjArgs& a, cudaStream_t st) {
+    switch (model) {
+        case MODEL_THRUSTER8: return closed_loop_adjoint_integ<MODEL_THRUSTER8>(integ, a, st);
+        case MODEL_WRENCH12: return closed_loop_adjoint_integ<MODEL_WRENCH12>(integ, a, st);
+        case MODEL_QUAT13: return closed_loop_adjoint_integ<MODEL_QUAT13>(integ, a, st);
+    }
+    return cudaErrorInvalidValue;
+}
+
+// ---- the operand gradients: per (step k, vehicle i) Y rows of R values; value r of row y is element elem(y, r)
+struct ClRedArgs {
+    const double* ws;             // z_k [steps][NZ][n]
+    const double* wgv;            // [steps][NU][n]
+    const double* src;            // WHICH 1 / 2: [steps][Y][n]; SCR: the scratch [E][n] (one "step")
+    const double* zr;
+    long long zr_st, zr_sn;
+    double* out;                  // element (k, i, e) at out[k*st + i*sn + e*se]
+    long long st, sn, se;
+    long long n;
+    int steps;
+};
+
+template <int MODEL, int WHICH, bool SCR> struct ClRed {
+    static constexpr int NZ = LinDim<MODEL>::NZ, NU = LinDim<MODEL>::NU;
+    static constexpr int E = WHICH == 0 ? NU * NZ : (WHICH == 1 ? NZ : NU);   // elements of the operand
+    static constexpr int Y = SCR ? E : (WHICH == 2 ? NU : NZ);
+    static constexpr int R = (WHICH == 0 && !SCR) ? NU : 1;
+    static __device__ __forceinline__ long long elem(int y, int r) { return R > 1 ? (long long)r * NZ + y : y; }
+    static __device__ __forceinline__ void load(const ClRedArgs& a, long long k, long long i, int y, double* val) {
+        const long long n = a.n;
+        if constexpr (R > 1) {
+            // dL/dK_k = -gv dz^T
+            const double d = cl_dz<MODEL>(a.ws[(k * NZ + y) * n + i], a.zr[k * a.zr_st + i * a.zr_sn + y], y);
+#pragma unroll
+            for (int r = 0; r < R; ++r) val[r] = -(a.wgv[(k * NU + r) * n + i] * d);
+        } else {
+            val[0] = a.src[(k * Y + y) * n + i];
+        }
+    }
+};
+
+// one thread per (vehicle, row), 32 vehicles x Y rows per block.  TNC: every (step, vehicle) has its own elements, the
+// steps spread over gridDim.y; otherwise the sum over the steps in order k = 0, 1, ... (a per-vehicle operand, or the
+// first stage of a shared constant one)
+template <int MODEL, int WHICH, bool TNC>
+__global__ void __launch_bounds__(1024) cl_red_steps_kernel(const ClRedArgs a) {
+    using S = ClRed<MODEL, WHICH, false>;
+    const long long i = (long long)blockIdx.x * 32 + threadIdx.x;
+    const int y = threadIdx.y;
+    if (i >= a.n) return;
+    double val[S::R];
+    if constexpr (TNC) {
+        for (long long k = blockIdx.y; k < a.steps; k += gridDim.y) {
+            S::load(a, k, i, y, val);
+#pragma unroll
+            for (int r = 0; r < S::R; ++r) a.out[k * a.st + i * a.sn + S::elem(y, r) * a.se] = val[r];
+        }
+    } else {
+        double acc[S::R];
+#pragma unroll
+        for (int r = 0; r < S::R; ++r) acc[r] = 0.0;
+        for (long long k = 0; k < a.steps; ++k) {
+            S::load(a, k, i, y, val);
+#pragma unroll
+            for (int r = 0; r < S::R; ++r) acc[r] += val[r];
+        }
+#pragma unroll
+        for (int r = 0; r < S::R; ++r) a.out[i * a.sn + S::elem(y, r) * a.se] = acc[r];
+    }
+}
+
+// the sum over the vehicles of row (k, y), one block per row: thread t adds vehicles t, t + 256, ... in order, then a
+// fixed shared-memory tree over the threads
+constexpr int CL_RED_THREADS = 256;
+template <int MODEL, int WHICH, bool SCR>
+__global__ void __launch_bounds__(CL_RED_THREADS) cl_red_vehicles_kernel(const ClRedArgs a) {
+    using S = ClRed<MODEL, WHICH, SCR>;
+    __shared__ double red[S::R][CL_RED_THREADS];
+    const int t = threadIdx.x;
+    const long long rows = (long long)a.steps * S::Y;
+    for (long long row = blockIdx.x; row < rows; row += gridDim.x) {
+        const long long k = row / S::Y;
+        const int y = (int)(row % S::Y);
+        double acc[S::R], val[S::R];
+#pragma unroll
+        for (int r = 0; r < S::R; ++r) acc[r] = 0.0;
+        for (long long i = t; i < a.n; i += CL_RED_THREADS) {
+            S::load(a, k, i, y, val);
+#pragma unroll
+            for (int r = 0; r < S::R; ++r) acc[r] += val[r];
+        }
+#pragma unroll
+        for (int r = 0; r < S::R; ++r) red[r][t] = acc[r];
+        __syncthreads();
+        for (int h = CL_RED_THREADS / 2; h > 0; h >>= 1) {
+            if (t < h) {
+#pragma unroll
+                for (int r = 0; r < S::R; ++r) red[r][t] += red[r][t + h];
+            }
+            __syncthreads();
+        }
+        if (t < S::R) a.out[k * a.st + S::elem(y, t) * a.se] = red[t][0];
+        __syncthreads();
+    }
+}
+
+template <int MODEL, int WHICH>
+static cudaError_t cl_reduce(const ClAdjArgs& c, double* out, long long st, long long sn, double* scratch, cudaStream_t s) {
+    using S = ClRed<MODEL, WHICH, false>;
+    ClRedArgs a;
+    a.ws = c.ws;
+    a.wgv = c.wgv;
+    a.src = WHICH == 1 ? c.wgzr : c.wgur;
+    a.zr = c.zr; a.zr_st = c.zr_st; a.zr_sn = c.zr_sn;
+    a.out = out; a.st = st; a.sn = sn; a.se = 1;
+    a.n = c.n;
+    a.steps = c.steps;
+    const dim3 blk(32, S::Y);
+    const unsigned gx = (unsigned)((c.n + 31) / 32);
+    const unsigned vgrid = (unsigned)std::min<long long>((long long)c.steps * S::Y, 1LL << 20);
+    if (st != 0 && sn != 0) {
+        cl_red_steps_kernel<MODEL, WHICH, true><<<dim3(gx, (unsigned)std::min(c.steps, 65535)), blk, 0, s>>>(a);
+    } else if (sn != 0) {
+        cl_red_steps_kernel<MODEL, WHICH, false><<<gx, blk, 0, s>>>(a);
+    } else if (st != 0) {
+        cl_red_vehicles_kernel<MODEL, WHICH, false><<<vgrid, CL_RED_THREADS, 0, s>>>(a);
+    } else {
+        // shared and constant: the per-vehicle sums over the steps into scratch [E][n], then their sum over vehicles
+        ClRedArgs b = a;
+        b.out = scratch; b.st = 0; b.sn = 1; b.se = c.n;
+        cl_red_steps_kernel<MODEL, WHICH, false><<<gx, blk, 0, s>>>(b);
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+        b = a;
+        b.src = scratch;
+        b.steps = 1;
+        cl_red_vehicles_kernel<MODEL, WHICH, true><<<ClRed<MODEL, WHICH, true>::Y, CL_RED_THREADS, 0, s>>>(b);
+    }
+    return cudaGetLastError();
+}
+
+template <int MODEL>
+static cudaError_t cl_reduce_which(int which, const ClAdjArgs& a, double* out, long long st, long long sn, double* scr,
+                                   cudaStream_t s) {
+    switch (which) {
+        case 0: return cl_reduce<MODEL, 0>(a, out, st, sn, scr, s);
+        case 1: return cl_reduce<MODEL, 1>(a, out, st, sn, scr, s);
+        case 2: return cl_reduce<MODEL, 2>(a, out, st, sn, scr, s);
+    }
+    return cudaErrorInvalidValue;
+}
+
+cudaError_t launch_closed_loop_adjoint_reduce(int model, int which, const ClAdjArgs& a, double* out, long long st,
+                                              long long sn, double* scratch, cudaStream_t s) {
+    if (a.n <= 0 || a.steps <= 0) return cudaSuccess;
+    switch (model) {
+        case MODEL_THRUSTER8: return cl_reduce_which<MODEL_THRUSTER8>(which, a, out, st, sn, scratch, s);
+        case MODEL_WRENCH12: return cl_reduce_which<MODEL_WRENCH12>(which, a, out, st, sn, scratch, s);
+        case MODEL_QUAT13: return cl_reduce_which<MODEL_QUAT13>(which, a, out, st, sn, scratch, s);
     }
     return cudaErrorInvalidValue;
 }

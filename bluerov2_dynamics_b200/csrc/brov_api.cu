@@ -1475,6 +1475,100 @@ extern "C" int brov_rollout_vjp_coef(brov_engine_t* e, const brov_rollout_vjp_co
     return BROV_OK;
 }
 
+extern "C" size_t brov_closed_loop_vjp_workspace_bytes(int model, long long n, long long steps) {
+    if (model != BROV_THRUSTER8_LAG3 && model != BROV_WRENCH_EULER12 && model != BROV_WRENCH_QUAT13) return 0;
+    const int nz = model_nx(model) + (model == BROV_THRUSTER8_LAG3 ? 18 : 0);
+    return cl_adjoint_workspace_bytes(nz, model_nu(model), n, steps);
+}
+
+// no two (step, vehicle) pairs of an operand of E elements addressed at k*st + i*sn + e share an element unless a
+// stride is 0 (then the gradient sums them)
+static bool cl_strides_disjoint(long long st, long long sn, long long steps, long long n, long long E) {
+    if (steps <= 1) st = 0;
+    if (n <= 1) sn = 0;
+    if (st == 0 && sn == 0) return true;
+    if (sn == 0) return st >= E;
+    if (st == 0) return sn >= E;
+    return (sn >= E && st / sn >= n) || (st >= E && sn / st >= steps);
+}
+
+extern "C" int brov_closed_loop_vjp(brov_engine_t* e, const brov_closed_loop_vjp_desc* d, void* stream) {
+    if (!e) return fail(BROV_EINVAL, "NULL engine");
+    if (!d || d->struct_size != sizeof(brov_closed_loop_vjp_desc)) return fail(BROV_EINVAL, "brov_closed_loop_vjp_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "closed_loop_vjp serves the Fossen models, not double-integrator engines");
+    if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the gradients are computed in fp64: create the engine with BROV_F64");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "closed_loop_vjp does not support the first-order wrench lag");
+    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
+    if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
+    if (d->steps < 1 || d->steps > (1LL << 30)) return fail(BROV_EINVAL, "steps = %lld must be 1 .. 2^30", d->steps);
+    if (!(d->dt > 0.0) || !std::isfinite(d->dt)) return fail(BROV_EINVAL, "dt must be a positive finite number");
+    if (d->K_stride_t < 0 || d->K_stride_n < 0 || d->z_ref_stride_t < 0 || d->z_ref_stride_n < 0 || d->u_ref_stride_t < 0 ||
+        d->u_ref_stride_n < 0)
+        return fail(BROV_EINVAL, "negative operand stride");
+    const bool thr = e->model == BROV_THRUSTER8_LAG3;
+    const int nz = model_nx(e->model) + (thr ? 18 : 0), nu = model_nu(e->model);
+    for (int r = 0; r < nu; ++r)
+        if (std::isnan(d->u_min[r]) || std::isnan(d->u_max[r]) || d->u_min[r] > d->u_max[r])
+            return fail(BROV_EINVAL, "input bounds of channel %d: u_min = %g, u_max = %g", r, d->u_min[r], d->u_max[r]);
+    if (d->gtraj_dev && d->stride < 1) return fail(BROV_EINVAL, "stride must be >= 1 with a trajectory cotangent");
+    if (e->pv && e->pv_n != d->n) return fail(BROV_EINVAL, "vehicle table has %lld rows, call has n = %lld", e->pv_n, d->n);
+    if (d->n == 0) return BROV_OK;
+    if (!d->z0_dev || !d->gz0_dev) return fail(BROV_EINVAL, "z0 and gz0 must not be NULL");
+    if (!d->K_dev || !d->z_ref_dev || !d->u_ref_dev) return fail(BROV_EINVAL, "K, z_ref and u_ref must not be NULL");
+    struct Op { void* g; long long st, sn; int E; const char* what; } ops[3] = {
+        {d->gK_dev, d->K_stride_t, d->K_stride_n, nu * nz, "K"},
+        {d->gz_ref_dev, d->z_ref_stride_t, d->z_ref_stride_n, nz, "z_ref"},
+        {d->gu_ref_dev, d->u_ref_stride_t, d->u_ref_stride_n, nu, "u_ref"}};
+    // the workspace this request needs: z_k, the cotangents of the requested operands, the scratch of a constant one
+    unsigned long long per = nz, scr = 0;
+    for (int w = 0; w < 3; ++w) {
+        if (!ops[w].g) continue;
+        if (!cl_strides_disjoint(ops[w].st, ops[w].sn, d->steps, d->n, ops[w].E))
+            return fail(BROV_EINVAL, "the gradient of %s needs strides under which distinct (step, vehicle) pairs do not overlap", ops[w].what);
+        per += w == 1 ? nz : nu;
+        if (ops[w].st == 0 && ops[w].sn == 0) scr = std::max<unsigned long long>(scr, ops[w].E);
+    }
+    const size_t need = cl_adjoint_bytes(per, scr, d->n, d->steps);    // checked: SIZE_MAX when it does not fit
+    if (!d->workspace_dev || d->workspace_bytes < need) return fail(BROV_EINVAL, "workspace too small: need %zu bytes", need);
+
+    ClAdjArgs a;
+    memset(&a, 0, sizeof(a));
+    int rc = make_consts<double>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c);
+    if (rc) return rc;
+    a.z0 = (const double*)d->z0_dev;
+    a.K = (const double*)d->K_dev; a.K_st = d->K_stride_t; a.K_sn = d->K_stride_n;
+    a.zr = (const double*)d->z_ref_dev; a.zr_st = d->z_ref_stride_t; a.zr_sn = d->z_ref_stride_n;
+    a.ur = (const double*)d->u_ref_dev; a.ur_st = d->u_ref_stride_t; a.ur_sn = d->u_ref_stride_n;
+    a.k_smem = (a.K_st == 0 && a.K_sn == 0) ? 1 : 0;
+    a.pv = (const double*)e->pv;
+    a.gtraj = (const double*)d->gtraj_dev;
+    a.gzT = (const double*)d->gzT_dev;
+    a.gcost = (const double*)d->gcost_dev;
+    a.gz0 = (double*)d->gz0_dev;
+    a.z_out = (double*)d->z_out_dev;
+    double* w = (double*)d->workspace_dev;
+    const size_t slab = (size_t)d->n * (size_t)d->steps;
+    a.ws = w; w += slab * nz;
+    if (d->gK_dev) { a.wgv = w; w += slab * nu; }
+    if (d->gz_ref_dev) { a.wgzr = w; w += slab * nz; }
+    if (d->gu_ref_dev) { a.wgur = w; w += slab * nu; }
+    double* scratch = w;
+    a.health = (unsigned long long*)d->health_dev;
+    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    for (int r = 0; r < 8; ++r) { a.u_min[r] = d->u_min[r]; a.u_max[r] = d->u_max[r]; a.r[r] = r < nu ? d->r[r] : 0.0; }
+    for (int j = 0; j < CL_MAX_NZ; ++j) a.q[j] = j < nz ? d->q[j] : 0.0;
+    a.n = d->n;
+    a.steps = (int)d->steps;
+    a.stride = d->gtraj_dev ? (int)std::min<long long>(d->stride, 0x7fffffffLL) : 1;
+    CUDA_TRY(cudaSetDevice(e->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d->health_dev) CUDA_TRY(cudaMemsetAsync(d->health_dev, 0, 2 * sizeof(unsigned long long), st));
+    CUDA_TRY(launch_closed_loop_adjoint(e->model, d->integrator, a, st));
+    for (int o = 0; o < 3; ++o)
+        if (ops[o].g) CUDA_TRY(launch_closed_loop_adjoint_reduce(e->model, o, a, (double*)ops[o].g, ops[o].st, ops[o].sn, scratch, st));
+    return BROV_OK;
+}
+
 // fossen/parameters.py:3-33
 template <typename T> static Red9Consts<T> red9_consts() {
     const double m = 11.4, g = 9.82, F_bouy = 1026 * 0.0115 * g;

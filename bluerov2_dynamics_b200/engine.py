@@ -227,6 +227,19 @@ class VjpResult:
     gkp: Optional[torch.Tensor] = None   # [N, NKP] dL/dkp of each vehicle's coefficients (coef=True), or None
 
 
+@dataclass
+class ClosedLoopVjpResult:
+    """Reverse-mode gradients of N closed-loop rollouts (Engine.closed_loop_vjp), each operand gradient in the shape of
+    the operand passed (a layout with a shared dimension gets the sum over it)."""
+    gx0: torch.Tensor                # [N, NX] dL/dx_0
+    glag0: Optional[torch.Tensor]    # dL/dlag_0 in the representation of lag0 ([N, 24] or [N, 18]), None for wrench models
+    gK: Optional[torch.Tensor]       # dL/dK, or None when not wanted
+    gz_ref: Optional[torch.Tensor]   # dL/dz_ref, or None when not wanted
+    gu_ref: Optional[torch.Tensor]   # dL/du_ref, or None when not wanted
+    z: torch.Tensor                  # [N, NZ] z after the last step (the primal of linearize, projected lag)
+    health: Optional[torch.Tensor]   # int64 [2]: vehicles with a non-finite z or gradient / near theta = +-pi/2, or None
+
+
 _CL_LAYOUTS = ("const_shared", "shared", "const", "tnc")
 
 
@@ -1167,33 +1180,8 @@ class Engine:
         T_ = t.shape[0] if layout in ("shared", "tnc") else None
         return t, st, sn, T_
 
-    def closed_loop(self, x0, K, z_ref, u_ref, steps: Optional[int] = None, dt: float = 0.02, integrator: str = "rk4",
-                    lag0=None, lag_repr: str = "thruster", k_layout: str = "auto", ref_layout: str = "auto",
-                    u_min=None, u_max=None, stride: int = 0, want_u: bool = False, cost_q=None, cost_r=None,
-                    cost: Optional[torch.Tensor] = None, cost_accumulate: bool = False,
-                    z_out: Optional[torch.Tensor] = None, health: bool = False,
-                    singular_eps: float = 0.0) -> ClosedLoopResult:
-        """Closed-loop rollout of N vehicles with an affine state-feedback law evaluated in the kernel
-        (brov_closed_loop): at every step k, with z_k = [x_k | Z_k] as in `linearize` (NZ = 30 / 12 / 13),
-            dz = z_k - z_ref_k   (Euler-angle models: angles wrapped to (-pi, pi]),
-            u_k = clamp(u_ref_k - K_k dz, u_min, u_max),   z_{k+1} = the rollout's step from z_k under u_k.
-
-        K has rows [NU, NZ] (the K numpy builds from a DARE solution), z_ref [NZ], u_ref [NU].  Each operand has one
-        of four layouts (k_layout / ref_layout; ref_layout applies to z_ref and u_ref):
-          "const_shared" [...]        one value for every vehicle and step
-          "shared"       [T, ...]     time-varying, shared by every vehicle
-          "const"        [N, ...]     constant per vehicle (never chosen by "auto": name it)
-          "tnc"          [T, N, ...]  time-varying per vehicle
-        "auto" picks from the number of dimensions.  T comes from the time-varying operands, which must agree; with
-        none of them give steps=.  lag0 (thruster model): per-thruster [N,24] (lag_repr="thruster") or projected
-        [N,18] (lag_repr="projected"); None = zeros.  The result is always in projected lag coordinates.
-
-        u_min / u_max: scalars or per-channel (default +-1 for thruster8, unbounded for the wrench models).
-        stride > 0 returns z after every stride-th step (z_traj [T//stride, N, NZ]); want_u adds the applied inputs of
-        those steps (u_traj [T//stride, N, NU]).  cost_q [NZ] / cost_r [NU] (diagonal weights) turn on the cost
-        sum_k dz'Q dz + (u_k - u_ref_k)'R (u_k - u_ref_k) per vehicle, written into `cost` if given and added to its
-        values with cost_accumulate (chunked calls add up bit for bit).  The engine's shared coefficients or its
-        per-vehicle table (set_vehicle_physical, N rows) are used."""
+    def _cl_setup(self, x0, K, z_ref, u_ref, steps, lag0, lag_repr, k_layout, ref_layout, u_min, u_max):
+        """(n, steps, z0, (K, st, sn), (z_ref, st, sn), (u_ref, st, sn), u_min [NU], u_max [NU]) of a closed-loop call"""
         x0 = self.tensor(x0)
         self._check_rows(x0, self.nx, "x0")
         n = x0.shape[0]
@@ -1222,6 +1210,38 @@ class Engine:
         lim = 1.0 if self.model == "thruster8" else np.inf
         lo = np.broadcast_to(np.asarray(-lim if u_min is None else u_min, float), (nu,))
         hi = np.broadcast_to(np.asarray(lim if u_max is None else u_max, float), (nu,))
+        return n, steps, z0, (Kt, kst, ksn), (zr, zst, zsn), (ur, ust, usn), lo, hi
+
+    def closed_loop(self, x0, K, z_ref, u_ref, steps: Optional[int] = None, dt: float = 0.02, integrator: str = "rk4",
+                    lag0=None, lag_repr: str = "thruster", k_layout: str = "auto", ref_layout: str = "auto",
+                    u_min=None, u_max=None, stride: int = 0, want_u: bool = False, cost_q=None, cost_r=None,
+                    cost: Optional[torch.Tensor] = None, cost_accumulate: bool = False,
+                    z_out: Optional[torch.Tensor] = None, health: bool = False,
+                    singular_eps: float = 0.0) -> ClosedLoopResult:
+        """Closed-loop rollout of N vehicles with an affine state-feedback law evaluated in the kernel
+        (brov_closed_loop): at every step k, with z_k = [x_k | Z_k] as in `linearize` (NZ = 30 / 12 / 13),
+            dz = z_k - z_ref_k   (Euler-angle models: angles wrapped to (-pi, pi]),
+            u_k = clamp(u_ref_k - K_k dz, u_min, u_max),   z_{k+1} = the rollout's step from z_k under u_k.
+
+        K has rows [NU, NZ] (the K numpy builds from a DARE solution), z_ref [NZ], u_ref [NU].  Each operand has one
+        of four layouts (k_layout / ref_layout; ref_layout applies to z_ref and u_ref):
+          "const_shared" [...]        one value for every vehicle and step
+          "shared"       [T, ...]     time-varying, shared by every vehicle
+          "const"        [N, ...]     constant per vehicle (never chosen by "auto": name it)
+          "tnc"          [T, N, ...]  time-varying per vehicle
+        "auto" picks from the number of dimensions.  T comes from the time-varying operands, which must agree; with
+        none of them give steps=.  lag0 (thruster model): per-thruster [N,24] (lag_repr="thruster") or projected
+        [N,18] (lag_repr="projected"); None = zeros.  The result is always in projected lag coordinates.
+
+        u_min / u_max: scalars or per-channel (default +-1 for thruster8, unbounded for the wrench models).
+        stride > 0 returns z after every stride-th step (z_traj [T//stride, N, NZ]); want_u adds the applied inputs of
+        those steps (u_traj [T//stride, N, NU]).  cost_q [NZ] / cost_r [NU] (diagonal weights) turn on the cost
+        sum_k dz'Q dz + (u_k - u_ref_k)'R (u_k - u_ref_k) per vehicle, written into `cost` if given and added to its
+        values with cost_accumulate (chunked calls add up bit for bit).  The engine's shared coefficients or its
+        per-vehicle table (set_vehicle_physical, N rows) are used."""
+        n, steps, z0, (Kt, kst, ksn), (zr, zst, zsn), (ur, ust, usn), lo, hi = self._cl_setup(
+            x0, K, z_ref, u_ref, steps, lag0, lag_repr, k_layout, ref_layout, u_min, u_max)
+        nz, nu = self.nz, self.nu
         if z_out is None:
             z_out = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
         else:
@@ -1265,6 +1285,119 @@ class Engine:
         with torch.cuda.device(self.device):
             L.check(L.lib.brov_closed_loop(self._h, C.byref(d), self._stream()))
         return ClosedLoopResult(z=z_out, z_traj=zt, u_traj=ut, cost=cost if want_cost else None, health=hc)
+
+    def closed_loop_vjp(self, x0, K, z_ref, u_ref, gtraj=None, gzT=None, gcost=None, stride: int = 0,
+                        want: Sequence[str] = ("K", "z_ref", "u_ref"), steps: Optional[int] = None, dt: float = 0.02,
+                        integrator: str = "rk4", lag0=None, lag_repr: str = "thruster", k_layout: str = "auto",
+                        ref_layout: str = "auto", u_min=None, u_max=None, cost_q=None, cost_r=None,
+                        health: bool = False, singular_eps: float = 0.0) -> ClosedLoopVjpResult:
+        """Reverse-mode gradients of N closed-loop rollouts (brov_closed_loop_vjp): for every vehicle, with the
+        feedback law, layouts, bounds and cost weights of `closed_loop`,
+            L = sum_{k = stride, 2 stride, ... <= T} <c_k, z_k> + <g_T, z_T> + g_c cost,
+        returns dL/dz_0 (as gx0 and glag0) and, for the operands named in `want`, dL/dK, dL/dz_ref and dL/du_ref in
+        the shape of the operand passed (a shared dimension gets the sum over it).  The feedback is differentiated
+        through: the clamp has derivative 0 on a saturated channel, the angle wrap derivative 1; the step is
+        differentiated as `rollout_vjp` differentiates it.
+
+        gtraj [T//stride, N, NZ]: c_k on the full z, in the layout of closed_loop's z_traj (None: no trajectory term);
+        gzT [N, NZ] (None: zero); gcost: g_c, a scalar or [N] (None: no cost term).  lag0 (thruster model):
+        per-thruster [N,24] with lag_repr="thruster", projected [N,18] with "projected"; glag0 comes back in the same
+        representation.  The call allocates the workspace the request needs (z_k, plus the cotangents of the operands in
+        `want`).  fp64 engines; the engine's shared coefficients or its per-vehicle table (N rows)."""
+        want = tuple(want)
+        bad = set(want) - {"K", "z_ref", "u_ref"}
+        if bad:
+            raise ValueError(f"want names operands among K, z_ref, u_ref, not {sorted(bad)}")
+        n, steps, z0, (Kt, kst, ksn), (zr, zst, zsn), (ur, ust, usn), lo, hi = self._cl_setup(
+            x0, K, z_ref, u_ref, steps, lag0, lag_repr, k_layout, ref_layout, u_min, u_max)
+        nz, nu = self.nz, self.nu
+        gt = None
+        if gtraj is not None:
+            gt = self.tensor(gtraj)
+            ns = steps // int(stride) if int(stride) >= 1 else None
+            if ns is not None and tuple(gt.shape) != (ns, n, nz):
+                raise ValueError(f"gtraj must have shape [{ns}, {n}, {nz}], got {tuple(gt.shape)}")
+        gT = None
+        if gzT is not None:
+            gT = self.tensor(gzT)
+            if tuple(gT.shape) != (n, nz):
+                raise ValueError(f"gzT must have shape [{n}, {nz}], got {tuple(gT.shape)}")
+        gc = None
+        if gcost is not None:
+            gc = torch.as_tensor(gcost, dtype=self.tdtype, device=self.device)
+            gc = (gc.expand(n) if gc.dim() == 0 else gc.reshape(n)).contiguous()
+        gz0 = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
+        z = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
+        outs = {w: torch.empty_like(t) if w in want else None for w, t in (("K", Kt), ("z_ref", zr), ("u_ref", ur))}
+        # the workspace this request needs (include/brov.h): z_k and the requested operands' cotangents per vehicle and
+        # step, plus one scratch row per vehicle for an operand whose strides are both 0
+        per, scr = nz, 0
+        for w, E, st_, sn_ in (("K", nu * nz, kst, ksn), ("z_ref", nz, zst, zsn), ("u_ref", nu, ust, usn)):
+            if w in want:
+                per += nz if w == "z_ref" else nu
+                scr = max(scr, E) if st_ == 0 and sn_ == 0 else scr
+        ws = torch.empty(max(n * (steps * per + scr), 1), device=self.device, dtype=torch.float64)
+        hc = torch.zeros(2, device=self.device, dtype=torch.int64) if health else None
+        d = L.ClosedLoopVjpDesc()
+        d.struct_size = C.sizeof(L.ClosedLoopVjpDesc)
+        d.integrator = INTEGRATORS[integrator]
+        d.n, d.steps, d.dt = n, steps, float(dt)
+        d.z0_dev = z0.data_ptr()
+        d.K_dev, d.K_stride_t, d.K_stride_n = Kt.data_ptr(), kst, ksn
+        d.z_ref_dev, d.z_ref_stride_t, d.z_ref_stride_n = zr.data_ptr(), zst, zsn
+        d.u_ref_dev, d.u_ref_stride_t, d.u_ref_stride_n = ur.data_ptr(), ust, usn
+        for r in range(nu):
+            d.u_min[r], d.u_max[r] = float(lo[r]), float(hi[r])
+        if cost_q is not None:
+            q = np.broadcast_to(np.asarray(cost_q, float), (nz,))
+            for j in range(nz):
+                d.q[j] = float(q[j])
+        if cost_r is not None:
+            rw = np.broadcast_to(np.asarray(cost_r, float), (nu,))
+            for r in range(nu):
+                d.r[r] = float(rw[r])
+        # an empty gtraj (stride > T: no snapshot) is no trajectory term
+        d.gtraj_dev = gt.data_ptr() if (gt is not None and gt.numel()) else None
+        d.stride = int(stride)
+        d.gzT_dev = gT.data_ptr() if gT is not None else None
+        d.gcost_dev = gc.data_ptr() if gc is not None else None
+        d.gz0_dev, d.z_out_dev = gz0.data_ptr(), z.data_ptr()
+        d.gK_dev = outs["K"].data_ptr() if outs["K"] is not None else None
+        d.gz_ref_dev = outs["z_ref"].data_ptr() if outs["z_ref"] is not None else None
+        d.gu_ref_dev = outs["u_ref"].data_ptr() if outs["u_ref"] is not None else None
+        d.workspace_dev, d.workspace_bytes = ws.data_ptr(), ws.numel() * 8
+        d.health_dev = hc.data_ptr() if hc is not None else None
+        d.singular_eps = float(singular_eps)
+        with torch.cuda.device(self.device):
+            L.check(L.lib.brov_closed_loop_vjp(self._h, C.byref(d), self._stream()))
+        gx0 = gz0[:, :self.nx]
+        glag0 = None
+        if self.model == "thruster8":
+            gZ0 = gz0[:, self.nx:]
+            if lag_repr == "thruster":
+                A = self.tensor(self._alloc)
+                glag0 = torch.einsum("ci,nck->nik", A, gZ0.reshape(n, 6, 3)).reshape(n, 24).contiguous()
+            else:
+                glag0 = gZ0
+        return ClosedLoopVjpResult(gx0=gx0, glag0=glag0, gK=outs["K"], gz_ref=outs["z_ref"], gu_ref=outs["u_ref"],
+                                   z=z, health=hc)
+
+    def closed_loop_diff(self, x0: torch.Tensor, K: torch.Tensor, z_ref: torch.Tensor, u_ref: torch.Tensor,
+                         lag0: Optional[torch.Tensor] = None, steps: Optional[int] = None, dt: float = 0.02,
+                         integrator: str = "rk4", stride: int = 0, k_layout: str = "auto", ref_layout: str = "auto",
+                         u_min=None, u_max=None, cost_q=None, cost_r=None):
+        """Differentiable closed-loop rollout: (z_traj [T//stride, N, NZ] or None for stride 0, z [N, NZ], cost [N] or
+        None without cost weights) as `closed_loop` returns them, with torch autograd gradients to x0, lag0 (projected,
+        [N, 18]), K, z_ref and u_ref in any of the four operand layouts.  The forward is `closed_loop`; the backward is
+        one `closed_loop_vjp` call.  The engine's shared coefficients or its per-vehicle table are used."""
+        if self.dtype != "f64" or self.is_di:
+            raise ValueError("closed-loop gradients need an fp64 engine of a Fossen model")
+        lag_t = lag0 if (lag0 is not None and self.model == "thruster8") else None
+        opts = dict(steps=steps, dt=float(dt), integrator=integrator, stride=int(stride), k_layout=k_layout,
+                    ref_layout=ref_layout, u_min=u_min, u_max=u_max, cost_q=cost_q, cost_r=cost_r)
+        zt, z, cost = _ClosedLoopDiff.apply(self, opts, x0, lag_t, K, z_ref, u_ref)
+        want_cost = cost_q is not None or cost_r is not None
+        return (zt if stride else None), z, (cost if want_cost else None)
 
     def ekf(self, x0, P0, U, Y, q, r, dt: float = 0.02, integrator: str = "rk4", lag0=None, lag_repr: str = "thruster",
             u_layout: str = "auto", y_layout: str = "auto", stride: int = 0, want_cov: bool = False, stats=None,
@@ -1509,6 +1642,41 @@ class _RolloutDiff(torch.autograd.Function):
         if kp is not None:
             gkp = res.gkp.sum(0) if kp.dim() == 1 else res.gkp
         return None, res.gx0, res.gU, glag, None, None, None, gkp
+
+
+class _ClosedLoopDiff(torch.autograd.Function):
+    """Engine.closed_loop forward, Engine.closed_loop_vjp backward (Engine.closed_loop_diff)."""
+
+    @staticmethod
+    def forward(ctx, eng, opts, x0, lag0, K, z_ref, u_ref):
+        o = dict(opts)
+        r = eng.closed_loop(x0.detach(), K.detach(), z_ref.detach(), u_ref.detach(),
+                            lag0=lag0.detach() if lag0 is not None else None, lag_repr="projected", **o)
+        ctx.eng, ctx.opts = eng, o
+        ctx.has_lag = lag0 is not None
+        ctx.save_for_backward(x0, K, z_ref, u_ref, *([lag0] if lag0 is not None else []))
+        n = x0.shape[0]
+        zt = r.z_traj if r.z_traj is not None else torch.empty((0, n, eng.nz), device=eng.device, dtype=eng.tdtype)
+        cost = r.cost if r.cost is not None else torch.empty((0,), device=eng.device, dtype=eng.tdtype)
+        return zt, r.z, cost
+
+    @staticmethod
+    def backward(ctx, gzt, gz, gcost):
+        eng, o = ctx.eng, dict(ctx.opts)
+        saved = ctx.saved_tensors
+        x0, K, z_ref, u_ref = saved[:4]
+        lag0 = saved[4] if ctx.has_lag else None
+        stride = o.pop("stride")
+        gt = gzt.contiguous() if (gzt is not None and stride and gzt.numel()) else None
+        gc = gcost.contiguous() if (gcost is not None and gcost.numel()) else None
+        gT = gz.contiguous() if gz is not None else None
+        need = ctx.needs_input_grad
+        want = tuple(w for w, i in (("K", 4), ("z_ref", 5), ("u_ref", 6)) if need[i])
+        res = eng.closed_loop_vjp(x0.detach(), K.detach(), z_ref.detach(), u_ref.detach(), gtraj=gt, gzT=gT, gcost=gc,
+                                  stride=stride if gt is not None else 0, want=want,
+                                  lag0=lag0.detach() if lag0 is not None else None, lag_repr="projected", **o)
+        glag = res.glag0 if ctx.has_lag else None
+        return None, None, res.gx0, glag, res.gK, res.gz_ref, res.gu_ref
 
 
 def reduced9_rhs(x: torch.Tensor, u: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:

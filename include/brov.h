@@ -622,6 +622,76 @@ typedef struct brov_rollout_vjp_coef_desc {
 } brov_rollout_vjp_coef_desc;
 int brov_rollout_vjp_coef(brov_engine_t* e, const brov_rollout_vjp_coef_desc* d, void* stream);
 
+/* Reverse-mode gradients of closed-loop rollouts (brov_closed_loop) — tuning a feedback gain over a fleet of perturbed
+ * vehicles, optimising the feedforward reference of a tracking controller, training a policy with feedback in the
+ * loop.  In the notation of brov_closed_loop, per vehicle and step k:
+ *     dz_k = wrap(z_k - zr_k)     v_k = ur_k - K_k dz_k     u_k = clamp(v_k, u_min, u_max)     z_{k+1} = Phi(z_k, u_k)
+ *     cost = sum_k sum_j q_j dz_kj^2 + sum_r r_r (u_k - ur_k)_r^2
+ *     L    = sum_{k = stride, 2 stride, ... <= steps} <c_k, z_k> + <g_T, z_steps> + g_c cost
+ * the call returns gz0 = dL/dz_0 and, each when its pointer is not NULL, dL/dK, dL/dzr and dL/dur in the layout of the
+ * operand as passed (same strides): an element read by several steps or vehicles (a zero stride) receives the sum of
+ * their contributions, the gradient of an operand of that shape.  Per step and vehicle the cotangents are
+ *     gv = m . (B_k^T lambda_{k+1} + 2 g_c r . (u_k - ur_k))    (m: 0 on a clamped channel, else 1; a NaN is not clamped)
+ *     dL/dK_k = -gv dz_k^T     dL/dzr_k = -gdz     dL/dur_k = gv - 2 g_c r . (u_k - ur_k)
+ *     gdz = -K_k^T gv + 2 g_c q . dz_k                 lambda_k = A_k^T lambda_{k+1} + gdz + c_k
+ * with A, B the step's Jacobians as brov_rollout_vjp differentiates them and d wrap = 1.  The primal is
+ * brov_linearize's step, so z_out agrees with brov_closed_loop to rounding, not bit for bit.  One thread per vehicle
+ * runs the forward pass (z_k to the workspace) and the reverse sweep (u_k recomputed from z_k, never stored); the
+ * operand gradients are then summed by separate kernels in a fixed order, without floating-point atomics.  Results are
+ * bit-reproducible; gz0 and the gradients of per-vehicle layouts do not depend on the other vehicles or on which
+ * layout holds equal values.
+ *   integrator, n, steps, dt, z0_dev, K / z_ref / u_ref with their strides, u_min / u_max, q, r: as brov_closed_loop_desc;
+ *   gtraj_dev [steps / stride][n][NZ] or NULL: c_k on the full z (closed_loop's traj layout); gzT_dev [n][NZ] or NULL;
+ *   gcost_dev [n] or NULL: g_c per vehicle (NULL: no cost term);
+ *   gz0_dev [n][NZ] (required; may alias gzT_dev); gK_dev, gz_ref_dev, gu_ref_dev or NULL; z_out_dev [n][NZ] or NULL;
+ *   workspace_dev: brov_closed_loop_vjp_workspace_bytes(model, n, steps) bytes always suffice; fewer operand
+ *   gradients need less: n * steps doubles times (NZ, + NU with gK, + NZ with gz_ref, + NU with gu_ref), plus n * E
+ *   doubles when an operand of E elements whose gradient is requested has both strides 0;
+ *   health_dev (unsigned long long[2] or NULL, zeroed by the call): vehicles with a non-finite z, gz0 or per-step
+ *   operand-gradient entry (dL/dur_k, dL/dzr_k and, with gK_dev, dL/dK_k = -gv dz_k^T) / that came within singular_eps
+ *   (0 = 1e-3) of theta = +-pi/2 at the start of some step.
+ * Chaining: split at t1 as for brov_rollout_vjp (gtraj, K, z_ref and u_ref sliced at t1 when time-varying).  gz0 and the
+ * time-sliced gradients (shared and per-vehicle time-varying layouts) equal those of one call bit for bit; each call
+ * writes the sums of a constant layout over its own steps, and these add up to the one-call result to rounding.
+ * Coefficients: the engine's shared set, or its per-vehicle table (n rows).  fp64 engines, Fossen models, RK4 / Euler.
+ * f32 engines, double-integrator engines and the first-order wrench lag return BROV_EUNSUPPORTED.  BROV_EINVAL (before
+ * any launch): every input brov_closed_loop refuses, steps < 1, gtraj_dev with stride < 1, NULL gz0, a requested
+ * operand gradient whose strides make distinct (step, vehicle) pairs overlap, a workspace smaller than needed, a
+ * table / n mismatch.  n = 0 is a no-op.  All arrays double, dev. */
+typedef struct brov_closed_loop_vjp_desc {
+    uint32_t struct_size;       /* = sizeof(brov_closed_loop_vjp_desc) */
+    int32_t integrator;
+    long long n;
+    long long steps;
+    double dt;
+    const void* z0_dev;
+    const void* K_dev;
+    long long K_stride_t, K_stride_n;
+    const void* z_ref_dev;
+    long long z_ref_stride_t, z_ref_stride_n;
+    const void* u_ref_dev;
+    long long u_ref_stride_t, u_ref_stride_n;
+    double u_min[8], u_max[8];
+    double q[30], r[8];
+    const void* gtraj_dev;
+    long long stride;
+    const void* gzT_dev;
+    const void* gcost_dev;
+    void* gz0_dev;
+    void* gK_dev;
+    void* gz_ref_dev;
+    void* gu_ref_dev;
+    void* z_out_dev;
+    void* workspace_dev;
+    size_t workspace_bytes;
+    void* health_dev;
+    double singular_eps;
+} brov_closed_loop_vjp_desc;
+int brov_closed_loop_vjp(brov_engine_t* e, const brov_closed_loop_vjp_desc* d, void* stream);
+/* workspace of brov_closed_loop_vjp with every operand gradient requested: n * (steps * (2 NZ + 2 NU) + NU * NZ)
+ * doubles for the Fossen models (0 for other models or n, steps <= 0; SIZE_MAX if the size does not fit in size_t) */
+size_t brov_closed_loop_vjp_workspace_bytes(int model, long long n, long long steps);
+
 /* Reduced 9-state RHS — `bluerov_compute(t, x_, u_)` (fossen/bluerov_torch.py:20-67, constants fossen/parameters.py).
  * x [B][9], u [B][4], out [B][9]. */
 int brov_reduced9_rhs(int dtype, const void* x_dev, const void* u_dev, void* out_dev, long long B, void* stream);
