@@ -1,24 +1,41 @@
 // brov_adj.cu — reverse-mode (adjoint) gradients of batched rollouts: for a loss L = sum_k <c_k, x_k> + <g_T, z_T> the
-// kernel returns dL/dz_0 and dL/du_k of every vehicle, with the step differentiated as brov_linearize differentiates
+// kernels return dL/dz_0 and dL/du_k of every vehicle, with the step differentiated as brov_linearize differentiates
 // it (full sines and cosines in every stage, branch taken, the quaternion renormalised after the step).
 //
-//   adjoint_kernel   one thread per vehicle, two loops in one launch.  The forward loop takes the primal steps from
-//                    z_0 and stores every z_k in the workspace ([steps][NZ][n], coalesced).  The backward loop runs
-//                    k = steps-1 .. 0: it reloads z_k and u_k, recomputes the step's stage states with the code the
-//                    forward loop ran (so the map it differentiates is exactly the stored one), stages them in shared
-//                    memory and sweeps the stages in reverse with the hand-written vector-Jacobian products of the
-//                    right-hand sides (rhs_euler12_vjp / rhs_quat13_vjp, brov_device.cuh).
-//   adjoint_coef_kernel  the same sweeps (adjoint_vehicle) that also accumulate dL/dkp of the vehicle's coefficients:
-//                    one lambda^T df/dkp per stage (nu_dot_coef_vjp), added to the thread's column of a shared-memory
-//                    accumulator [ADJ_NKPG][thread]; the coefficients come from the constant bank or, PV, from the
-//                    vehicle's column of the per-vehicle table staged in shared memory.
+// One thread per vehicle, two loops in one launch.  The forward loop takes the primal steps from z_0 and stores every
+// z_k in the workspace ([steps][NZ][n], coalesced).  The backward loop runs k = steps-1 .. 0: it reloads z_k, forms
+// the step's input again, recomputes the stage states with the code the forward loop ran (so the map it
+// differentiates is exactly the stored one), stages them in shared memory and sweeps the stages in reverse with the
+// hand-written vector-Jacobian products of the right-hand sides (rhs_euler12_vjp / rhs_quat13_vjp, brov_device.cuh).
+// The three kernels are built from the same pieces (adj_fwd_step, adj_step_vjp, adj_gu and the small I/O helpers):
+//
+//   adjoint_kernel              inputs U read from memory; stores dL/du_k.
+//   adjoint_coef_kernel         adjoint_kernel's sweep, which also accumulates dL/dkp of the vehicle's coefficients.
+//   closed_loop_adjoint_kernel  inputs from the in-kernel feedback law, reversed through the feedback after each step.
 //
 // Every sum has a fixed order, so the results are bit-reproducible and independent of the other vehicles.
 #include "brov_adj.cuh"
 
 #include <algorithm>
+#include <type_traits>
 
 namespace brov {
+
+template <int MODEL> struct AdjDim {
+    static constexpr int NX = LinDim<MODEL>::NX, NU = LinDim<MODEL>::NU, NZ = LinDim<MODEL>::NZ;
+    static constexpr bool THR = MODEL == MODEL_THRUSTER8;
+    static constexpr bool QUAT = ModelDim<MODEL>::QUAT;
+    static constexpr int NL = THR ? 18 : 1;   // the thruster lag Z (one unused entry for the wrench models)
+};
+
+// Dynamic shared memory of the sweep kernels, in rows of ADJ_THREADS doubles (one column per thread, conflict-free):
+// the RK4 stage buffer (3 NX rows) first, then `rows` more rows and `bytes` more bytes of the kernel's own
+__host__ __device__ constexpr int adj_stage_rows(int model, int integ) {
+    return integ == INTEG_RK4 ? 3 * (model == MODEL_QUAT13 ? 13 : 12) : 0;
+}
+constexpr size_t adj_smem_bytes(int model, int integ, int rows, size_t bytes) {
+    return (size_t)(adj_stage_rows(model, integ) + rows) * ADJ_THREADS * sizeof(double) + bytes;
+}
 
 // right-hand side of sub-step s at the stage state xs, as linearize evaluates it (full sines and cosines)
 template <int MODEL, class P>
@@ -93,244 +110,323 @@ __device__ __forceinline__ void adj_step(const Consts<double>& c, const P& p, do
 
 __device__ __forceinline__ bool adj_finite(double v) { return fabs(v) <= 1.7976931348623157e308; }
 
-template <int MODEL, int INTEG>
-__global__ void __launch_bounds__(ADJ_THREADS) adjoint_kernel(const __grid_constant__ AdjArgs a) {
-    constexpr int NX = LinDim<MODEL>::NX, NU = LinDim<MODEL>::NU, NZ = LinDim<MODEL>::NZ;
-    constexpr bool THR = MODEL == MODEL_THRUSTER8;
-    constexpr bool QUAT = ModelDim<MODEL>::QUAT;
-    constexpr int NL = THR ? 18 : 1;
-    constexpr int NSTAGE = INTEG == INTEG_RK4 ? 3 * NX * ADJ_THREADS : 1;
-    __shared__ double stage[NSTAGE];      // RK4: [stage 1..3][i][thread], conflict-free
-    const Consts<double>& c = a.c;
-    const ParamsConst<double> p{c.kp};
-    const bool cur = c.has_current != 0;
-    const int tid = threadIdx.x;
-    double* sx = stage + tid;
-    const long long v = (long long)blockIdx.x * ADJ_THREADS + tid;
-    const long long n = a.n;
-    bool bad = false, sing = false;
-    if (v < n) {
-        // ---- forward: z_k -> workspace
-        double x[NX], Z[NL];
-#pragma unroll
-        for (int q = 0; q < NX; ++q) x[q] = a.z0[v * NZ + q];
-#pragma unroll
-        for (int q = 0; q < NL; ++q) Z[q] = THR ? a.z0[v * NZ + NX + q] : 0.0;
-        for (int k = 0; k < a.steps; ++k) {
-            double* wk = a.ws + (long long)k * NZ * n + v;
-#pragma unroll
-            for (int q = 0; q < NX; ++q) wk[q * n] = x[q];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) wk[(NX + q) * n] = Z[q];
-            }
-            const double* uk = a.U + (long long)k * a.ust + v * a.usn;
-            double Fw[6];
-            if constexpr (THR) {
-                double F[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, uk[i]);
-                allocate_wrench<double>(c, F, Fw);
-            } else {
-#pragma unroll
-                for (int r = 0; r < 6; ++r) Fw[r] = uk[r];
-            }
-            double acth;
-            adj_step<MODEL, INTEG, false>(c, p, x, Z, Fw, nullptr, nullptr, acth);
-            sing |= acth < a.eps;
-            if constexpr (THR) lag_advance<double, true>(c, Z, Fw);
-        }
-#pragma unroll
-        for (int q = 0; q < NX; ++q) bad |= !adj_finite(x[q]);
-#pragma unroll
-        for (int q = 0; q < NL; ++q) bad |= THR && !adj_finite(Z[q]);
-        if (a.z_out) {
-#pragma unroll
-            for (int q = 0; q < NX; ++q) a.z_out[v * NZ + q] = x[q];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) a.z_out[v * NZ + NX + q] = Z[q];
-            }
-        }
+// ---- the pieces of the sweeps
 
-        // ---- backward: lam = dL/dx_k, mu = dL/dZ_k
-        double lam[NX], mu[NL];
+// the wrench of the input row u: thruster8 through the thrust curve and the allocation, the wrench models u itself
+template <int MODEL>
+__device__ __forceinline__ void adj_wrench(const Consts<double>& c, const double* u, double* __restrict__ Fw) {
+    if constexpr (MODEL == MODEL_THRUSTER8) {
+        double F[8];
 #pragma unroll
-        for (int q = 0; q < NX; ++q) lam[q] = a.gzT ? a.gzT[v * NZ + q] : 0.0;
+        for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, u[i]);
+        allocate_wrench<double>(c, F, Fw);
+    } else {
 #pragma unroll
-        for (int q = 0; q < NL; ++q) mu[q] = (THR && a.gzT) ? a.gzT[v * NZ + NX + q] : 0.0;
-        if (a.gtraj && a.steps % a.stride == 0) {
-            const double* gt = a.gtraj + ((long long)(a.steps / a.stride - 1) * n + v) * NX;
+        for (int r = 0; r < 6; ++r) Fw[r] = u[r];
+    }
+}
+
+// vehicle v's initial state from z0 [n][NZ]
+template <int MODEL>
+__device__ __forceinline__ void adj_load_z0(const double* z0, long long v, double* x, double* Z) {
+    using D = AdjDim<MODEL>;
 #pragma unroll
-            for (int q = 0; q < NX; ++q) lam[q] += gt[q];
-        }
-        const double dt = c.dt, hdt = 0.5 * dt, dt6 = dt * (1.0 / 6.0), dt3 = 2.0 * dt6;
-        for (int k = a.steps - 1; k >= 0; --k) {
-            const double* wk = a.ws + (long long)k * NZ * n + v;
+    for (int q = 0; q < D::NX; ++q) x[q] = z0[v * D::NZ + q];
 #pragma unroll
-            for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
-            if constexpr (THR) {
+    for (int q = 0; q < D::NL; ++q) Z[q] = D::THR ? z0[v * D::NZ + D::NX + q] : 0.0;
+}
+
+// z_k to / from its slice wk of the workspace (vehicle index fastest)
+template <int MODEL>
+__device__ __forceinline__ void adj_store_z(double* wk, long long n, const double* x, const double* Z) {
+    using D = AdjDim<MODEL>;
 #pragma unroll
-                for (int q = 0; q < NL; ++q) Z[q] = wk[(NX + q) * n];
-            }
-            const double* uk = a.U + (long long)k * a.ust + v * a.usn;
-            double Fw[6];
-            if constexpr (THR) {
-                double F[8];
+    for (int q = 0; q < D::NX; ++q) wk[q * n] = x[q];
+    if constexpr (D::THR) {
 #pragma unroll
-                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, uk[i]);
-                allocate_wrench<double>(c, F, Fw);
-            } else {
+        for (int q = 0; q < D::NL; ++q) wk[(D::NX + q) * n] = Z[q];
+    }
+}
+template <int MODEL>
+__device__ __forceinline__ void adj_load_z(const double* wk, long long n, double* x, double* Z) {
+    using D = AdjDim<MODEL>;
 #pragma unroll
-                for (int r = 0; r < 6; ++r) Fw[r] = uk[r];
-            }
-            // recompute the stage states (and the quaternion before its renormalisation)
-            double qpre[4];
-            if constexpr (INTEG == INTEG_RK4 || QUAT) {
-                double xw[NX];
+    for (int q = 0; q < D::NX; ++q) x[q] = wk[q * n];
+    if constexpr (D::THR) {
 #pragma unroll
-                for (int q = 0; q < NX; ++q) xw[q] = x[q];
-                double acth;
-                adj_step<MODEL, INTEG, true>(c, p, xw, Z, Fw, sx, qpre, acth);
-            }
-            if constexpr (QUAT) quat_normalize_vjp(qpre, lam + 3);
-            // lag: Z' = lagA Z_c + lagB Fw_c per channel
-            double muF[6];
-            if constexpr (THR) {
+        for (int q = 0; q < D::NL; ++q) Z[q] = wk[(D::NX + q) * n];
+    }
+}
+
+// forward step k from the input row u (z_k already stored): the wrench, the primal step, the singularity flag, the lag
+template <int MODEL, int INTEG, class P>
+__device__ __forceinline__ void adj_fwd_step(const Consts<double>& c, const P& p, double* x, double* Z, const double* u,
+                                             double eps, bool& sing) {
+    double Fw[6];
+    adj_wrench<MODEL>(c, u, Fw);
+    double acth;
+    adj_step<MODEL, INTEG, false>(c, p, x, Z, Fw, nullptr, nullptr, acth);
+    sing |= acth < eps;
+    if constexpr (MODEL == MODEL_THRUSTER8) lag_advance<double, true>(c, Z, Fw);
+}
+
+// the end of the forward loop: the finiteness of z_T, and z_T to z_out [n][NZ] when it is wanted
+template <int MODEL>
+__device__ __forceinline__ void adj_fwd_end(const double* x, const double* Z, double* z_out, long long v, bool& bad) {
+    using D = AdjDim<MODEL>;
 #pragma unroll
-                for (int ch = 0; ch < 6; ++ch) {
-                    const double m0 = mu[3 * ch], m1 = mu[3 * ch + 1], m2 = mu[3 * ch + 2];
+    for (int q = 0; q < D::NX; ++q) bad |= !adj_finite(x[q]);
 #pragma unroll
-                    for (int j = 0; j < 3; ++j) mu[3 * ch + j] = c.lagA[0][j] * m0 + c.lagA[1][j] * m1 + c.lagA[2][j] * m2;
-                    muF[ch] = c.lagB[0] * m0 + c.lagB[1] * m1 + c.lagB[2] * m2;
-                }
-            } else {
+    for (int q = 0; q < D::NL; ++q) bad |= D::THR && !adj_finite(Z[q]);
+    if (z_out) {
 #pragma unroll
-                for (int ch = 0; ch < 6; ++ch) muF[ch] = 0.0;
-            }
-            double lamp[NX], kap[NX];
+        for (int q = 0; q < D::NX; ++q) z_out[v * D::NZ + q] = x[q];
+        if constexpr (D::THR) {
 #pragma unroll
-            for (int q = 0; q < NX; ++q) lamp[q] = lam[q];
-            // stage s at xs with the cotangent kap of its right-hand side: lam += a, the wrench cotangent b into
-            // mu / muF (thruster: tau_s = lagG[s] . Z_c + lagH[s] Fw_c) or muF (wrench models: tau = u)
-            auto stage_vjp = [&](int s, const double* xs, double* ga) {
-                double b[6];
-                if constexpr (QUAT) {
-                    rhs_quat13_vjp(xs, p, cur, kap, ga, b);
-                } else {
-                    Trig<double> tr;
-                    trig_full<double>(c, xs + 3, tr);
-                    rhs_euler12_vjp(xs, tr, p, cur, kap, ga, b);
-                }
-#pragma unroll
-                for (int q = 0; q < NX; ++q) lam[q] += ga[q];
-#pragma unroll
-                for (int ch = 0; ch < 6; ++ch) {
-                    if constexpr (THR) {
-#pragma unroll
-                        for (int j = 0; j < 3; ++j) mu[3 * ch + j] += c.lagG[s][j] * b[ch];
-                        muF[ch] += c.lagH[s] * b[ch];
-                    } else {
-                        muF[ch] += b[ch];
-                    }
-                }
-            };
-            double ga[NX];
-            if constexpr (INTEG == INTEG_EULER) {
-#pragma unroll
-                for (int q = 0; q < NX; ++q) kap[q] = dt * lamp[q];
-                stage_vjp(0, x, ga);
-            } else {
-                // x' = x + dt/6 (k0 + 2 k1 + 2 k2 + k3), xs_s = x + h_s k_{s-1}
-#pragma unroll
-                for (int q = 0; q < NX; ++q) kap[q] = dt6 * lamp[q];
-#pragma unroll
-                for (int s = 3; s >= 1; --s) {
-                    double xs[NX];
-#pragma unroll
-                    for (int q = 0; q < NX; ++q) xs[q] = sx[((s - 1) * NX + q) * ADJ_THREADS];
-                    stage_vjp(s, xs, ga);
-                    const double cs = (s == 1) ? dt6 : dt3;
-                    const double hs = (s == 3) ? dt : hdt;
-#pragma unroll
-                    for (int q = 0; q < NX; ++q) kap[q] = fma(hs, ga[q], cs * lamp[q]);
-                }
-                // stage 0 is z_k itself: reloaded rather than held through the sweep (register pressure)
-#pragma unroll
-                for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
-                stage_vjp(0, x, ga);
-            }
-            // input: thruster gu_i = F'(u_i) sum_c alloc[c][i] muF[c] (the allocation's structural zeros skipped, as
-            // in allocate_wrench); wrench models gu = muF
-            double* gu = a.gU + ((long long)k * n + v) * NU;
-            if constexpr (THR) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    double s = 0.0;
-#pragma unroll
-                    for (int r = 0; r < 6; ++r) {
-                        const bool nz = (r < 2) ? (i < 4) : (r == 2) ? (i >= 4) : (r == 5) ? (i < 4) : true;
-                        if (nz) s += c.alloc[r][i] * muF[r];
-                    }
-                    const double g = thrust_poly_d(c, uk[i]) * s;
-                    gu[i] = g;
-                    bad |= !adj_finite(g);
-                }
-            } else {
-#pragma unroll
-                for (int i = 0; i < 6; ++i) {
-                    gu[i] = muF[i];
-                    bad |= !adj_finite(muF[i]);
-                }
-            }
-            if (a.gtraj && k > 0 && k % a.stride == 0) {
-                const double* gt = a.gtraj + ((long long)(k / a.stride - 1) * n + v) * NX;
-#pragma unroll
-                for (int q = 0; q < NX; ++q) lam[q] += gt[q];
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < NX; ++q) {
-            a.gz0[v * NZ + q] = lam[q];
-            bad |= !adj_finite(lam[q]);
-        }
-        if constexpr (THR) {
-#pragma unroll
-            for (int q = 0; q < NL; ++q) {
-                a.gz0[v * NZ + NX + q] = mu[q];
-                bad |= !adj_finite(mu[q]);
-            }
+            for (int q = 0; q < D::NL; ++q) z_out[v * D::NZ + D::NX + q] = Z[q];
         }
     }
-    if (a.health) {
+}
+
+// lam = dL/dx_T, mu = dL/dZ_T from gzT [n][NZ] (zero without it)
+template <int MODEL>
+__device__ __forceinline__ void adj_load_gzT(const double* gzT, long long v, double* lam, double* mu) {
+    using D = AdjDim<MODEL>;
+#pragma unroll
+    for (int q = 0; q < D::NX; ++q) lam[q] = gzT ? gzT[v * D::NZ + q] : 0.0;
+#pragma unroll
+    for (int q = 0; q < D::NL; ++q) mu[q] = (D::THR && gzT) ? gzT[v * D::NZ + D::NX + q] : 0.0;
+}
+
+// adds snapshot j of the trajectory cotangent gtraj [snapshots][n][NW]: NW = NX covers x (the rollout's snapshots),
+// NW = NZ also the lag (the closed loop's)
+template <int MODEL, int NW>
+__device__ __forceinline__ void adj_add_gtraj(const double* gtraj, long long j, long long n, long long v, double* lam,
+                                              double* mu) {
+    using D = AdjDim<MODEL>;
+    const double* gt = gtraj + (j * n + v) * NW;
+#pragma unroll
+    for (int q = 0; q < D::NX; ++q) lam[q] += gt[q];
+    if constexpr (D::THR && NW == D::NZ) {
+#pragma unroll
+        for (int q = 0; q < D::NL; ++q) mu[q] += gt[D::NX + q];
+    }
+}
+
+// the step sizes of the reverse sweep, formed once before the loop
+struct AdjDt {
+    double dt, hdt, dt6, dt3;
+};
+
+// One reverse step: (lam, mu) = dL/d(x, Z)_{k+1} -> dL/d(x, Z)_k, and muF = dL/dFw_k.  x, Z: z_k (x is z_k again on
+// return); Fw: the step's wrench; wk: z_k in the workspace.  It recomputes the stage states into sx, reverses the
+// quaternion renormalisation and the lag (Z' = lagA Z_c + lagB Fw_c per channel), then sweeps the stages.  COEF: every
+// stage also adds lambda^T df/dkp to the accumulator gk, with the current path always taken (nu - R^T 0 = nu), so
+// gk[KP_CUR ..] exists without a current.  cur: the engine's has_current, read once at the top of the kernel (read
+// here, it changes which products of rhs_quat13_vjp's rotation matrix the compiler fuses into fmas).
+template <int MODEL, int INTEG, bool COEF, class P, class G = double*>
+__device__ __forceinline__ void adj_step_vjp(const Consts<double>& c, const P& p, bool cur, const AdjDt& h, double* x,
+                                             const double* Z, const double* Fw, const double* wk, long long n, double* sx,
+                                             double* lam, double* mu, double* muF, const G& gk = G()) {
+    using D = AdjDim<MODEL>;
+    constexpr int NX = D::NX;
+    constexpr bool THR = D::THR, QUAT = D::QUAT;
+    // recompute the stage states (and the quaternion before its renormalisation)
+    double qpre[4];
+    if constexpr (INTEG == INTEG_RK4 || QUAT) {
+        double xw[NX];
+#pragma unroll
+        for (int q = 0; q < NX; ++q) xw[q] = x[q];
+        double acth;
+        adj_step<MODEL, INTEG, true>(c, p, xw, Z, Fw, sx, qpre, acth);
+    }
+    if constexpr (QUAT) quat_normalize_vjp(qpre, lam + 3);
+    if constexpr (THR) {
+#pragma unroll
+        for (int ch = 0; ch < 6; ++ch) {
+            const double m0 = mu[3 * ch], m1 = mu[3 * ch + 1], m2 = mu[3 * ch + 2];
+#pragma unroll
+            for (int j = 0; j < 3; ++j) mu[3 * ch + j] = c.lagA[0][j] * m0 + c.lagA[1][j] * m1 + c.lagA[2][j] * m2;
+            muF[ch] = c.lagB[0] * m0 + c.lagB[1] * m1 + c.lagB[2] * m2;
+        }
+    } else {
+#pragma unroll
+        for (int ch = 0; ch < 6; ++ch) muF[ch] = 0.0;
+    }
+    double lamp[NX], kap[NX];
+#pragma unroll
+    for (int q = 0; q < NX; ++q) lamp[q] = lam[q];
+    // stage s at xs with the cotangent kap of its right-hand side: lam += a, the wrench cotangent b into
+    // mu / muF (thruster: tau_s = lagG[s] . Z_c + lagH[s] Fw_c) or muF (wrench models: tau = u)
+    auto stage_vjp = [&](int s, const double* xs, double* ga) {
+        double b[6];
+        if constexpr (COEF) {
+            double tau[6];
+            if constexpr (THR) {
+                thruster_tau<double, true>(c, s, Z, Fw, tau);
+            } else {
+#pragma unroll
+                for (int r = 0; r < 6; ++r) tau[r] = Fw[r];
+            }
+            if constexpr (QUAT) {
+                rhs_quat13_vjp<true>(xs, p, true, kap, ga, b, tau, gk);
+            } else {
+                Trig<double> tr;
+                trig_full<double>(c, xs + 3, tr);
+                rhs_euler12_vjp<true>(xs, tr, p, true, kap, ga, b, tau, gk);
+            }
+        } else {
+            if constexpr (QUAT) {
+                rhs_quat13_vjp(xs, p, cur, kap, ga, b);
+            } else {
+                Trig<double> tr;
+                trig_full<double>(c, xs + 3, tr);
+                rhs_euler12_vjp(xs, tr, p, cur, kap, ga, b);
+            }
+        }
+#pragma unroll
+        for (int q = 0; q < NX; ++q) lam[q] += ga[q];
+#pragma unroll
+        for (int ch = 0; ch < 6; ++ch) {
+            if constexpr (THR) {
+#pragma unroll
+                for (int j = 0; j < 3; ++j) mu[3 * ch + j] += c.lagG[s][j] * b[ch];
+                muF[ch] += c.lagH[s] * b[ch];
+            } else {
+                muF[ch] += b[ch];
+            }
+        }
+    };
+    double ga[NX];
+    if constexpr (INTEG == INTEG_EULER) {
+#pragma unroll
+        for (int q = 0; q < NX; ++q) kap[q] = h.dt * lamp[q];
+        stage_vjp(0, x, ga);
+    } else {
+        // x' = x + dt/6 (k0 + 2 k1 + 2 k2 + k3), xs_s = x + h_s k_{s-1}
+#pragma unroll
+        for (int q = 0; q < NX; ++q) kap[q] = h.dt6 * lamp[q];
+#pragma unroll
+        for (int s = 3; s >= 1; --s) {
+            double xs[NX];
+#pragma unroll
+            for (int q = 0; q < NX; ++q) xs[q] = sx[((s - 1) * NX + q) * ADJ_THREADS];
+            stage_vjp(s, xs, ga);
+            const double cs = (s == 1) ? h.dt6 : h.dt3;
+            const double hs = (s == 3) ? h.dt : h.hdt;
+#pragma unroll
+            for (int q = 0; q < NX; ++q) kap[q] = fma(hs, ga[q], cs * lamp[q]);
+        }
+        // stage 0 is z_k itself: reloaded rather than held through the sweep (register pressure)
+#pragma unroll
+        for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
+        stage_vjp(0, x, ga);
+    }
+}
+
+// dL/du_i from the wrench cotangent muF: thruster gu_i = F'(u_i) sum_c alloc[c][i] muF[c] (the allocation's
+// structural zeros skipped, as in allocate_wrench); wrench models gu = muF
+template <int MODEL>
+__device__ __forceinline__ double adj_gu(const Consts<double>& c, const double* muF, const double* u, int i) {
+    if constexpr (MODEL == MODEL_THRUSTER8) {
+        double s = 0.0;
+#pragma unroll
+        for (int r = 0; r < 6; ++r) {
+            const bool nz = (r < 2) ? (i < 4) : (r == 2) ? (i >= 4) : (r == 5) ? (i < 4) : true;
+            if (nz) s += c.alloc[r][i] * muF[r];
+        }
+        return thrust_poly_d(c, u[i]) * s;
+    } else {
+        return muF[i];
+    }
+}
+
+// (lam, mu) = dL/dz_0 to gz0 [n][NZ], with their finiteness
+template <int MODEL>
+__device__ __forceinline__ void adj_store_gz0(double* gz0, long long v, const double* lam, const double* mu, bool& bad) {
+    using D = AdjDim<MODEL>;
+#pragma unroll
+    for (int q = 0; q < D::NX; ++q) {
+        gz0[v * D::NZ + q] = lam[q];
+        bad |= !adj_finite(lam[q]);
+    }
+    if constexpr (D::THR) {
+#pragma unroll
+        for (int q = 0; q < D::NL; ++q) {
+            gz0[v * D::NZ + D::NX + q] = mu[q];
+            bad |= !adj_finite(mu[q]);
+        }
+    }
+}
+
+// the block's counts of vehicles with a non-finite result (health[0]) and with a near-singular Euler step (health[1])
+__device__ __forceinline__ void adj_health(unsigned long long* health, bool bad, bool sing) {
+    if (health) {
         const int nb = __syncthreads_count(bad);
         const int ns = __syncthreads_count(sing);
-        if (tid == 0) {
-            if (nb) atomicAdd(a.health + 0, (unsigned long long)nb);
-            if (ns) atomicAdd(a.health + 1, (unsigned long long)ns);
+        if (threadIdx.x == 0) {
+            if (nb) atomicAdd(health + 0, (unsigned long long)nb);
+            if (ns) atomicAdd(health + 1, (unsigned long long)ns);
         }
     }
 }
 
-template <int MODEL, int INTEG>
-static cudaError_t adjoint_go(const AdjArgs& a, cudaStream_t st) {
-    const long long grid = (a.n + ADJ_THREADS - 1) / ADJ_THREADS;
-    adjoint_kernel<MODEL, INTEG><<<(unsigned)grid, ADJ_THREADS, 0, st>>>(a);
-    return cudaGetLastError();
-}
+// ---- the rollout sweeps (brov_rollout_vjp, brov_rollout_vjp_coef)
 
-template <int MODEL>
-static cudaError_t adjoint_integ(int integ, const AdjArgs& a, cudaStream_t st) {
-    return integ == INTEG_RK4 ? adjoint_go<MODEL, INTEG_RK4>(a, st) : adjoint_go<MODEL, INTEG_EULER>(a, st);
-}
-
-cudaError_t launch_adjoint(int model, int integ, const AdjArgs& a, cudaStream_t st) {
-    switch (model) {
-        case MODEL_THRUSTER8: return adjoint_integ<MODEL_THRUSTER8>(integ, a, st);
-        case MODEL_WRENCH12: return adjoint_integ<MODEL_WRENCH12>(integ, a, st);
-        case MODEL_QUAT13: return adjoint_integ<MODEL_QUAT13>(integ, a, st);
+// vehicle v's sweep of an open-loop rollout: z_T to z_out, dL/du_k to gU, dL/dz_0 to gz0; COEF: lambda^T df/dkp of
+// every stage into gk
+template <int MODEL, int INTEG, bool COEF, class P, class G = double*>
+__device__ __forceinline__ void adj_rollout_sweep(const AdjArgs& a, const P& p, bool cur, double* sx, long long v,
+                                                  bool& bad, bool& sing, const G& gk = G()) {
+    using D = AdjDim<MODEL>;
+    constexpr int NX = D::NX, NU = D::NU, NZ = D::NZ, NL = D::NL;
+    const Consts<double>& c = a.c;
+    const long long n = a.n;
+    // ---- forward: z_k -> workspace
+    double x[NX], Z[NL];
+    adj_load_z0<MODEL>(a.z0, v, x, Z);
+    for (int k = 0; k < a.steps; ++k) {
+        adj_store_z<MODEL>(a.ws + (long long)k * NZ * n + v, n, x, Z);
+        adj_fwd_step<MODEL, INTEG>(c, p, x, Z, a.U + (long long)k * a.ust + v * a.usn, a.eps, sing);
     }
-    return cudaErrorInvalidValue;
+    adj_fwd_end<MODEL>(x, Z, a.z_out, v, bad);
+
+    // ---- backward: lam = dL/dx_k, mu = dL/dZ_k
+    double lam[NX], mu[NL];
+    adj_load_gzT<MODEL>(a.gzT, v, lam, mu);
+    if (a.gtraj && a.steps % a.stride == 0) adj_add_gtraj<MODEL, NX>(a.gtraj, a.steps / a.stride - 1, n, v, lam, mu);
+    const double dt = c.dt, dt6 = dt * (1.0 / 6.0);
+    const AdjDt h{dt, 0.5 * dt, dt6, 2.0 * dt6};
+    for (int k = a.steps - 1; k >= 0; --k) {
+        const double* wk = a.ws + (long long)k * NZ * n + v;
+        adj_load_z<MODEL>(wk, n, x, Z);
+        const double* uk = a.U + (long long)k * a.ust + v * a.usn;
+        double Fw[6], muF[6];
+        adj_wrench<MODEL>(c, uk, Fw);
+        adj_step_vjp<MODEL, INTEG, COEF>(c, p, cur, h, x, Z, Fw, wk, n, sx, lam, mu, muF, gk);
+        double* gu = a.gU + ((long long)k * n + v) * NU;
+#pragma unroll
+        for (int i = 0; i < NU; ++i) {
+            const double g = adj_gu<MODEL>(c, muF, uk, i);
+            gu[i] = g;
+            bad |= !adj_finite(g);
+        }
+        if (a.gtraj && k > 0 && k % a.stride == 0) adj_add_gtraj<MODEL, NX>(a.gtraj, k / a.stride - 1, n, v, lam, mu);
+    }
+    adj_store_gz0<MODEL>(a.gz0, v, lam, mu, bad);
+}
+
+template <int MODEL, int INTEG>
+__global__ void __launch_bounds__(ADJ_THREADS) adjoint_kernel(const __grid_constant__ AdjArgs a) {
+    constexpr int NSTAGE = INTEG == INTEG_RK4 ? 3 * LinDim<MODEL>::NX * ADJ_THREADS : 1;
+    __shared__ double stage[NSTAGE];      // RK4: [stage 1..3][i][thread], conflict-free
+    const ParamsConst<double> p{a.c.kp};
+    const bool cur = a.c.has_current != 0;
+    const int tid = threadIdx.x;
+    const long long v = (long long)blockIdx.x * ADJ_THREADS + tid;
+    bool bad = false, sing = false;
+    if (v < a.n) adj_rollout_sweep<MODEL, INTEG, false>(a, p, cur, stage + tid, v, bad, sing);
+    adj_health(a.health, bad, sing);
 }
 
 // a shared-memory column of the coefficient cotangent: entry j of this thread at base[j * ADJ_THREADS]
@@ -339,27 +435,19 @@ struct CoefAcc {
     __device__ __forceinline__ double& operator[](int j) const { return base[j * ADJ_THREADS]; }
 };
 
-// adjoint_kernel plus the coefficient cotangent (brov_rollout_vjp_coef).  The sweeps are adjoint_kernel's; in addition
-// every stage of every step adds lambda^T df/dkp (rhs_*_vjp<true>, nu_dot_coef_vjp) to the thread's column gk of a
-// shared-memory accumulator, in a fixed order, and the column goes to gkp [KP_COUNT][n] at the end.  Dynamic shared
-// memory, one column per thread (conflict-free): [RK4 stage buffer (3 NX) | gk (ADJ_NKPG) | PV: the vehicle's column
-// of the per-vehicle table (KP_COUNT), staged as closed_loop_kernel stages it].  The engine's has_current selects the
-// primal; the reverse always runs the current path (nu - R^T 0 = nu), so gk[KP_CUR ..] exists without a current.
-// (A separate kernel rather than flags on adjoint_kernel: that one's code stays exactly as it was.)
+// adjoint_kernel's sweep with the coefficient cotangent (brov_rollout_vjp_coef): the thread's column gk of a
+// shared-memory accumulator receives lambda^T df/dkp of every stage (rhs_*_vjp<true>, nu_dot_coef_vjp) in a fixed
+// order and goes to gkp [KP_COUNT][n] at the end.  Dynamic shared memory, one column per thread (conflict-free):
+// [RK4 stage buffer (3 NX) | gk (ADJ_NKPG) | PV: the vehicle's column of the per-vehicle table (KP_COUNT), staged as
+// closed_loop_kernel stages it].
 template <int MODEL, int INTEG, bool PV>
 __global__ void __launch_bounds__(ADJ_THREADS) adjoint_coef_kernel(const __grid_constant__ AdjCoefArgs ca) {
-    constexpr int NX = LinDim<MODEL>::NX, NU = LinDim<MODEL>::NU, NZ = LinDim<MODEL>::NZ;
-    constexpr bool THR = MODEL == MODEL_THRUSTER8;
-    constexpr bool QUAT = ModelDim<MODEL>::QUAT;
-    constexpr int NL = THR ? 18 : 1;
     extern __shared__ double smem[];
     const AdjArgs& a = ca.a;
-    const Consts<double>& c = a.c;
     const int tid = threadIdx.x;
-    double* sx = smem + tid;
     const long long v = (long long)blockIdx.x * ADJ_THREADS + tid;
     const long long n = a.n;
-    double* col = smem + adjoint_coef_stage_rows(MODEL, INTEG) * ADJ_THREADS + tid;
+    double* col = smem + adj_stage_rows(MODEL, INTEG) * ADJ_THREADS + tid;
     const CoefAcc gk{col};
 #pragma unroll
     for (int j = 0; j < ADJ_NKPG; ++j) gk[j] = 0.0;
@@ -371,209 +459,11 @@ __global__ void __launch_bounds__(ADJ_THREADS) adjoint_coef_kernel(const __grid_
         p.base = col + ADJ_NKPG * ADJ_THREADS;
         p.pitch = ADJ_THREADS;
     } else {
-        p.kp = c.kp;
+        p.kp = a.c.kp;
     }
     bool bad = false, sing = false;
     if (v < n) {
-        // ---- forward: z_k -> workspace
-        double x[NX], Z[NL];
-#pragma unroll
-        for (int q = 0; q < NX; ++q) x[q] = a.z0[v * NZ + q];
-#pragma unroll
-        for (int q = 0; q < NL; ++q) Z[q] = THR ? a.z0[v * NZ + NX + q] : 0.0;
-        for (int k = 0; k < a.steps; ++k) {
-            double* wk = a.ws + (long long)k * NZ * n + v;
-#pragma unroll
-            for (int q = 0; q < NX; ++q) wk[q * n] = x[q];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) wk[(NX + q) * n] = Z[q];
-            }
-            const double* uk = a.U + (long long)k * a.ust + v * a.usn;
-            double Fw[6];
-            if constexpr (THR) {
-                double F[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, uk[i]);
-                allocate_wrench<double>(c, F, Fw);
-            } else {
-#pragma unroll
-                for (int r = 0; r < 6; ++r) Fw[r] = uk[r];
-            }
-            double acth;
-            adj_step<MODEL, INTEG, false>(c, p, x, Z, Fw, nullptr, nullptr, acth);
-            sing |= acth < a.eps;
-            if constexpr (THR) lag_advance<double, true>(c, Z, Fw);
-        }
-#pragma unroll
-        for (int q = 0; q < NX; ++q) bad |= !adj_finite(x[q]);
-#pragma unroll
-        for (int q = 0; q < NL; ++q) bad |= THR && !adj_finite(Z[q]);
-        if (a.z_out) {
-#pragma unroll
-            for (int q = 0; q < NX; ++q) a.z_out[v * NZ + q] = x[q];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) a.z_out[v * NZ + NX + q] = Z[q];
-            }
-        }
-
-        // ---- backward: lam = dL/dx_k, mu = dL/dZ_k
-        double lam[NX], mu[NL];
-#pragma unroll
-        for (int q = 0; q < NX; ++q) lam[q] = a.gzT ? a.gzT[v * NZ + q] : 0.0;
-#pragma unroll
-        for (int q = 0; q < NL; ++q) mu[q] = (THR && a.gzT) ? a.gzT[v * NZ + NX + q] : 0.0;
-        if (a.gtraj && a.steps % a.stride == 0) {
-            const double* gt = a.gtraj + ((long long)(a.steps / a.stride - 1) * n + v) * NX;
-#pragma unroll
-            for (int q = 0; q < NX; ++q) lam[q] += gt[q];
-        }
-        const double dt = c.dt, hdt = 0.5 * dt, dt6 = dt * (1.0 / 6.0), dt3 = 2.0 * dt6;
-        for (int k = a.steps - 1; k >= 0; --k) {
-            const double* wk = a.ws + (long long)k * NZ * n + v;
-#pragma unroll
-            for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) Z[q] = wk[(NX + q) * n];
-            }
-            const double* uk = a.U + (long long)k * a.ust + v * a.usn;
-            double Fw[6];
-            if constexpr (THR) {
-                double F[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, uk[i]);
-                allocate_wrench<double>(c, F, Fw);
-            } else {
-#pragma unroll
-                for (int r = 0; r < 6; ++r) Fw[r] = uk[r];
-            }
-            // recompute the stage states (and the quaternion before its renormalisation)
-            double qpre[4];
-            if constexpr (INTEG == INTEG_RK4 || QUAT) {
-                double xw[NX];
-#pragma unroll
-                for (int q = 0; q < NX; ++q) xw[q] = x[q];
-                double acth;
-                adj_step<MODEL, INTEG, true>(c, p, xw, Z, Fw, sx, qpre, acth);
-            }
-            if constexpr (QUAT) quat_normalize_vjp(qpre, lam + 3);
-            // lag: Z' = lagA Z_c + lagB Fw_c per channel
-            double muF[6];
-            if constexpr (THR) {
-#pragma unroll
-                for (int ch = 0; ch < 6; ++ch) {
-                    const double m0 = mu[3 * ch], m1 = mu[3 * ch + 1], m2 = mu[3 * ch + 2];
-#pragma unroll
-                    for (int j = 0; j < 3; ++j) mu[3 * ch + j] = c.lagA[0][j] * m0 + c.lagA[1][j] * m1 + c.lagA[2][j] * m2;
-                    muF[ch] = c.lagB[0] * m0 + c.lagB[1] * m1 + c.lagB[2] * m2;
-                }
-            } else {
-#pragma unroll
-                for (int ch = 0; ch < 6; ++ch) muF[ch] = 0.0;
-            }
-            double lamp[NX], kap[NX];
-#pragma unroll
-            for (int q = 0; q < NX; ++q) lamp[q] = lam[q];
-            // stage s at xs with the cotangent kap of its right-hand side: lam += a, the wrench cotangent b into
-            // mu / muF (thruster: tau_s = lagG[s] . Z_c + lagH[s] Fw_c) or muF (wrench models: tau = u)
-            auto stage_vjp = [&](int s, const double* xs, double* ga) {
-                double b[6];
-                double tau[6];
-                if constexpr (THR) {
-                    thruster_tau<double, true>(c, s, Z, Fw, tau);
-                } else {
-#pragma unroll
-                    for (int r = 0; r < 6; ++r) tau[r] = Fw[r];
-                }
-                if constexpr (QUAT) {
-                    rhs_quat13_vjp<true>(xs, p, true, kap, ga, b, tau, gk);
-                } else {
-                    Trig<double> tr;
-                    trig_full<double>(c, xs + 3, tr);
-                    rhs_euler12_vjp<true>(xs, tr, p, true, kap, ga, b, tau, gk);
-                }
-
-#pragma unroll
-                for (int q = 0; q < NX; ++q) lam[q] += ga[q];
-#pragma unroll
-                for (int ch = 0; ch < 6; ++ch) {
-                    if constexpr (THR) {
-#pragma unroll
-                        for (int j = 0; j < 3; ++j) mu[3 * ch + j] += c.lagG[s][j] * b[ch];
-                        muF[ch] += c.lagH[s] * b[ch];
-                    } else {
-                        muF[ch] += b[ch];
-                    }
-                }
-            };
-            double ga[NX];
-            if constexpr (INTEG == INTEG_EULER) {
-#pragma unroll
-                for (int q = 0; q < NX; ++q) kap[q] = dt * lamp[q];
-                stage_vjp(0, x, ga);
-            } else {
-                // x' = x + dt/6 (k0 + 2 k1 + 2 k2 + k3), xs_s = x + h_s k_{s-1}
-#pragma unroll
-                for (int q = 0; q < NX; ++q) kap[q] = dt6 * lamp[q];
-#pragma unroll
-                for (int s = 3; s >= 1; --s) {
-                    double xs[NX];
-#pragma unroll
-                    for (int q = 0; q < NX; ++q) xs[q] = sx[((s - 1) * NX + q) * ADJ_THREADS];
-                    stage_vjp(s, xs, ga);
-                    const double cs = (s == 1) ? dt6 : dt3;
-                    const double hs = (s == 3) ? dt : hdt;
-#pragma unroll
-                    for (int q = 0; q < NX; ++q) kap[q] = fma(hs, ga[q], cs * lamp[q]);
-                }
-                // stage 0 is z_k itself: reloaded rather than held through the sweep (register pressure)
-#pragma unroll
-                for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
-                stage_vjp(0, x, ga);
-            }
-            // input: thruster gu_i = F'(u_i) sum_c alloc[c][i] muF[c] (the allocation's structural zeros skipped, as
-            // in allocate_wrench); wrench models gu = muF
-            double* gu = a.gU + ((long long)k * n + v) * NU;
-            if constexpr (THR) {
-#pragma unroll
-                for (int i = 0; i < 8; ++i) {
-                    double s = 0.0;
-#pragma unroll
-                    for (int r = 0; r < 6; ++r) {
-                        const bool nz = (r < 2) ? (i < 4) : (r == 2) ? (i >= 4) : (r == 5) ? (i < 4) : true;
-                        if (nz) s += c.alloc[r][i] * muF[r];
-                    }
-                    const double g = thrust_poly_d(c, uk[i]) * s;
-                    gu[i] = g;
-                    bad |= !adj_finite(g);
-                }
-            } else {
-#pragma unroll
-                for (int i = 0; i < 6; ++i) {
-                    gu[i] = muF[i];
-                    bad |= !adj_finite(muF[i]);
-                }
-            }
-            if (a.gtraj && k > 0 && k % a.stride == 0) {
-                const double* gt = a.gtraj + ((long long)(k / a.stride - 1) * n + v) * NX;
-#pragma unroll
-                for (int q = 0; q < NX; ++q) lam[q] += gt[q];
-            }
-        }
-#pragma unroll
-        for (int q = 0; q < NX; ++q) {
-            a.gz0[v * NZ + q] = lam[q];
-            bad |= !adj_finite(lam[q]);
-        }
-        if constexpr (THR) {
-#pragma unroll
-            for (int q = 0; q < NL; ++q) {
-                a.gz0[v * NZ + NX + q] = mu[q];
-                bad |= !adj_finite(mu[q]);
-            }
-        }
+        adj_rollout_sweep<MODEL, INTEG, true>(a, p, true, smem + tid, v, bad, sing, gk);
 #pragma unroll
         for (int j = 0; j < KP_COUNT; ++j) {
             const double g = j < ADJ_NKPG ? gk[j] : 0.0;
@@ -581,41 +471,7 @@ __global__ void __launch_bounds__(ADJ_THREADS) adjoint_coef_kernel(const __grid_
             bad |= !adj_finite(g);
         }
     }
-    if (a.health) {
-        const int nb = __syncthreads_count(bad);
-        const int ns = __syncthreads_count(sing);
-        if (tid == 0) {
-            if (nb) atomicAdd(a.health + 0, (unsigned long long)nb);
-            if (ns) atomicAdd(a.health + 1, (unsigned long long)ns);
-        }
-    }
-}
-
-template <int MODEL, int INTEG, bool PV>
-static cudaError_t adjoint_coef_go(const AdjCoefArgs& a, cudaStream_t st) {
-    auto kern = adjoint_coef_kernel<MODEL, INTEG, PV>;
-    const size_t smem = adjoint_coef_smem_bytes(MODEL, INTEG, PV);
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    const long long grid = (a.a.n + ADJ_THREADS - 1) / ADJ_THREADS;
-    kern<<<(unsigned)grid, ADJ_THREADS, smem, st>>>(a);
-    return cudaGetLastError();
-}
-
-template <int MODEL>
-static cudaError_t adjoint_coef_integ(int integ, const AdjCoefArgs& a, cudaStream_t st) {
-    const bool pv = a.pv != nullptr;
-    if (integ == INTEG_RK4) return pv ? adjoint_coef_go<MODEL, INTEG_RK4, true>(a, st) : adjoint_coef_go<MODEL, INTEG_RK4, false>(a, st);
-    return pv ? adjoint_coef_go<MODEL, INTEG_EULER, true>(a, st) : adjoint_coef_go<MODEL, INTEG_EULER, false>(a, st);
-}
-
-cudaError_t launch_adjoint_coef(int model, int integ, const AdjCoefArgs& a, cudaStream_t st) {
-    switch (model) {
-        case MODEL_THRUSTER8: return adjoint_coef_integ<MODEL_THRUSTER8>(integ, a, st);
-        case MODEL_WRENCH12: return adjoint_coef_integ<MODEL_WRENCH12>(integ, a, st);
-        case MODEL_QUAT13: return adjoint_coef_integ<MODEL_QUAT13>(integ, a, st);
-    }
-    return cudaErrorInvalidValue;
+    adj_health(a.health, bad, sing);
 }
 
 
@@ -654,20 +510,17 @@ __device__ __forceinline__ void cl_feedback(const ClAdjArgs& a, const double* __
     }
 }
 
-// The sweep of brov_closed_loop_vjp, a sibling of adjoint_kernel / adjoint_coef_kernel (their code stays as it was).
-// Forward: u_k from the feedback law, the primal step of adjoint_kernel, z_k to the workspace.  Reverse: reload z_k,
-// recompute u_k (never stored) and the stage states, run adjoint_kernel's step VJP (lambda_{k+1} -> A^T lambda,
-// B^T lambda), then the feedback:
+// The sweep of brov_closed_loop_vjp: the rollout sweep's pieces with u_k from the feedback law.  Forward: z_k to the
+// workspace, u_k, the primal step.  Reverse: reload z_k, recompute u_k (never stored), the step VJP (lambda_{k+1} ->
+// A^T lambda, B^T lambda = adj_gu), then the feedback:
 //     gv = m . (B^T lambda + 2 g_c r . (u - ur))          dL/dv_k, m the clamp mask
 //     gdz = -K_k^T gv + 2 g_c q . dz_k                    lambda_k = A^T lambda + gdz + c_k (the lag rows into mu)
 // and stores gv, dL/dur_k = gv - 2 g_c r . (u - ur) and dL/dzr_k = -gdz for the reductions.  Dynamic shared memory:
 // [RK4 stage buffer (3 NX rows) | PV: the vehicle's table column (KP_COUNT rows) | the staged K (k_smem)].
 template <int MODEL, int INTEG, bool PV>
 __global__ void __launch_bounds__(ADJ_THREADS) closed_loop_adjoint_kernel(const __grid_constant__ ClAdjArgs a) {
-    constexpr int NX = LinDim<MODEL>::NX, NU = LinDim<MODEL>::NU, NZ = LinDim<MODEL>::NZ;
-    constexpr bool THR = MODEL == MODEL_THRUSTER8;
-    constexpr bool QUAT = ModelDim<MODEL>::QUAT;
-    constexpr int NL = THR ? 18 : 1;
+    using D = AdjDim<MODEL>;
+    constexpr int NX = D::NX, NU = D::NU, NZ = D::NZ, NL = D::NL;
     extern __shared__ double smem[];
     const Consts<double>& c = a.c;
     const bool cur = c.has_current != 0;
@@ -676,7 +529,7 @@ __global__ void __launch_bounds__(ADJ_THREADS) closed_loop_adjoint_kernel(const 
     const long long v = (long long)blockIdx.x * ADJ_THREADS + tid;
     const long long n = a.n;
     const long long vc = v < n ? v : n - 1;   // dead lanes stage the last vehicle's column, never store
-    double* rest = smem + adjoint_coef_stage_rows(MODEL, INTEG) * ADJ_THREADS;
+    double* rest = smem + adj_stage_rows(MODEL, INTEG) * ADJ_THREADS;
     typename std::conditional<PV, ParamsShared<double>, ParamsConst<double>>::type p;
     if constexpr (PV) {
         const double* pvt = a.pv + vc;
@@ -702,181 +555,42 @@ __global__ void __launch_bounds__(ADJ_THREADS) closed_loop_adjoint_kernel(const 
         const double* urp = a.ur + v * a.ur_sn;
         // ---- forward: z_k -> workspace
         double x[NX], Z[NL];
-#pragma unroll
-        for (int q = 0; q < NX; ++q) x[q] = a.z0[v * NZ + q];
-#pragma unroll
-        for (int q = 0; q < NL; ++q) Z[q] = THR ? a.z0[v * NZ + NX + q] : 0.0;
+        adj_load_z0<MODEL>(a.z0, v, x, Z);
         for (int k = 0; k < a.steps; ++k) {
-            double* wk = a.ws + (long long)k * NZ * n + v;
-#pragma unroll
-            for (int q = 0; q < NX; ++q) wk[q * n] = x[q];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) wk[(NX + q) * n] = Z[q];
-            }
+            adj_store_z<MODEL>(a.ws + (long long)k * NZ * n + v, n, x, Z);
             double u[NU];
             bool m[NU];
             cl_feedback<MODEL>(a, x, Z, Kp + (long long)k * a.K_st, zrp + (long long)k * a.zr_st,
                                urp + (long long)k * a.ur_st, u, m);
-            double Fw[6];
-            if constexpr (THR) {
-                double F[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, u[i]);
-                allocate_wrench<double>(c, F, Fw);
-            } else {
-#pragma unroll
-                for (int r = 0; r < 6; ++r) Fw[r] = u[r];
-            }
-            double acth;
-            adj_step<MODEL, INTEG, false>(c, p, x, Z, Fw, nullptr, nullptr, acth);
-            sing |= acth < a.eps;
-            if constexpr (THR) lag_advance<double, true>(c, Z, Fw);
+            adj_fwd_step<MODEL, INTEG>(c, p, x, Z, u, a.eps, sing);
         }
-#pragma unroll
-        for (int q = 0; q < NX; ++q) bad |= !adj_finite(x[q]);
-#pragma unroll
-        for (int q = 0; q < NL; ++q) bad |= THR && !adj_finite(Z[q]);
-        if (a.z_out) {
-#pragma unroll
-            for (int q = 0; q < NX; ++q) a.z_out[v * NZ + q] = x[q];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) a.z_out[v * NZ + NX + q] = Z[q];
-            }
-        }
+        adj_fwd_end<MODEL>(x, Z, a.z_out, v, bad);
 
         // ---- backward: lam = dL/dx_k, mu = dL/dZ_k
         double lam[NX], mu[NL];
-#pragma unroll
-        for (int q = 0; q < NX; ++q) lam[q] = a.gzT ? a.gzT[v * NZ + q] : 0.0;
-#pragma unroll
-        for (int q = 0; q < NL; ++q) mu[q] = (THR && a.gzT) ? a.gzT[v * NZ + NX + q] : 0.0;
-        if (a.gtraj && a.steps % a.stride == 0) {
-            const double* gt = a.gtraj + ((long long)(a.steps / a.stride - 1) * n + v) * NZ;
-#pragma unroll
-            for (int q = 0; q < NX; ++q) lam[q] += gt[q];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) mu[q] += gt[NX + q];
-            }
-        }
+        adj_load_gzT<MODEL>(a.gzT, v, lam, mu);
+        if (a.gtraj && a.steps % a.stride == 0) adj_add_gtraj<MODEL, NZ>(a.gtraj, a.steps / a.stride - 1, n, v, lam, mu);
         const bool cost = a.gcost != nullptr;
         const double gc2 = cost ? 2.0 * a.gcost[v] : 0.0;
-        const double dt = c.dt, hdt = 0.5 * dt, dt6 = dt * (1.0 / 6.0), dt3 = 2.0 * dt6;
+        const double dt = c.dt, dt6 = dt * (1.0 / 6.0);
+        const AdjDt h{dt, 0.5 * dt, dt6, 2.0 * dt6};
         for (int k = a.steps - 1; k >= 0; --k) {
             const double* wk = a.ws + (long long)k * NZ * n + v;
-#pragma unroll
-            for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
-            if constexpr (THR) {
-#pragma unroll
-                for (int q = 0; q < NL; ++q) Z[q] = wk[(NX + q) * n];
-            }
+            adj_load_z<MODEL>(wk, n, x, Z);
             const double* Kk = Kp + (long long)k * a.K_st;
             const double* zrk = zrp + (long long)k * a.zr_st;
             const double* urk = urp + (long long)k * a.ur_st;
             double u[NU];
             bool m[NU];
             cl_feedback<MODEL>(a, x, Z, Kk, zrk, urk, u, m);
-            double Fw[6];
-            if constexpr (THR) {
-                double F[8];
-#pragma unroll
-                for (int i = 0; i < 8; ++i) F[i] = thrust_poly<double>(c, u[i]);
-                allocate_wrench<double>(c, F, Fw);
-            } else {
-#pragma unroll
-                for (int r = 0; r < 6; ++r) Fw[r] = u[r];
-            }
-            // recompute the stage states (and the quaternion before its renormalisation)
-            double qpre[4];
-            if constexpr (INTEG == INTEG_RK4 || QUAT) {
-                double xw[NX];
-#pragma unroll
-                for (int q = 0; q < NX; ++q) xw[q] = x[q];
-                double acth;
-                adj_step<MODEL, INTEG, true>(c, p, xw, Z, Fw, sx, qpre, acth);
-            }
-            if constexpr (QUAT) quat_normalize_vjp(qpre, lam + 3);
-            // lag: Z' = lagA Z_c + lagB Fw_c per channel
-            double muF[6];
-            if constexpr (THR) {
-#pragma unroll
-                for (int ch = 0; ch < 6; ++ch) {
-                    const double m0 = mu[3 * ch], m1 = mu[3 * ch + 1], m2 = mu[3 * ch + 2];
-#pragma unroll
-                    for (int j = 0; j < 3; ++j) mu[3 * ch + j] = c.lagA[0][j] * m0 + c.lagA[1][j] * m1 + c.lagA[2][j] * m2;
-                    muF[ch] = c.lagB[0] * m0 + c.lagB[1] * m1 + c.lagB[2] * m2;
-                }
-            } else {
-#pragma unroll
-                for (int ch = 0; ch < 6; ++ch) muF[ch] = 0.0;
-            }
-            double lamp[NX], kap[NX];
-#pragma unroll
-            for (int q = 0; q < NX; ++q) lamp[q] = lam[q];
-            // stage s at xs with the cotangent kap of its right-hand side (as adjoint_kernel)
-            auto stage_vjp = [&](int s, const double* xs, double* ga) {
-                double b[6];
-                if constexpr (QUAT) {
-                    rhs_quat13_vjp(xs, p, cur, kap, ga, b);
-                } else {
-                    Trig<double> tr;
-                    trig_full<double>(c, xs + 3, tr);
-                    rhs_euler12_vjp(xs, tr, p, cur, kap, ga, b);
-                }
-#pragma unroll
-                for (int q = 0; q < NX; ++q) lam[q] += ga[q];
-#pragma unroll
-                for (int ch = 0; ch < 6; ++ch) {
-                    if constexpr (THR) {
-#pragma unroll
-                        for (int j = 0; j < 3; ++j) mu[3 * ch + j] += c.lagG[s][j] * b[ch];
-                        muF[ch] += c.lagH[s] * b[ch];
-                    } else {
-                        muF[ch] += b[ch];
-                    }
-                }
-            };
-            double ga[NX];
-            if constexpr (INTEG == INTEG_EULER) {
-#pragma unroll
-                for (int q = 0; q < NX; ++q) kap[q] = dt * lamp[q];
-                stage_vjp(0, x, ga);
-            } else {
-#pragma unroll
-                for (int q = 0; q < NX; ++q) kap[q] = dt6 * lamp[q];
-#pragma unroll
-                for (int s = 3; s >= 1; --s) {
-                    double xs[NX];
-#pragma unroll
-                    for (int q = 0; q < NX; ++q) xs[q] = sx[((s - 1) * NX + q) * ADJ_THREADS];
-                    stage_vjp(s, xs, ga);
-                    const double cs = (s == 1) ? dt6 : dt3;
-                    const double hs = (s == 3) ? dt : hdt;
-#pragma unroll
-                    for (int q = 0; q < NX; ++q) kap[q] = fma(hs, ga[q], cs * lamp[q]);
-                }
-#pragma unroll
-                for (int q = 0; q < NX; ++q) x[q] = wk[q * n];
-                stage_vjp(0, x, ga);
-            }
-            // the feedback: gu = B^T lambda as adjoint_kernel forms it, then gv and dL/dur
+            double Fw[6], muF[6];
+            adj_wrench<MODEL>(c, u, Fw);
+            adj_step_vjp<MODEL, INTEG, false>(c, p, cur, h, x, Z, Fw, wk, n, sx, lam, mu, muF);
+            // the feedback: gv and dL/dur from gu = B^T lambda
             double gv[NU];
 #pragma unroll
             for (int i = 0; i < NU; ++i) {
-                double g;
-                if constexpr (THR) {
-                    double s = 0.0;
-#pragma unroll
-                    for (int r = 0; r < 6; ++r) {
-                        const bool nz = (r < 2) ? (i < 4) : (r == 2) ? (i >= 4) : (r == 5) ? (i < 4) : true;
-                        if (nz) s += c.alloc[r][i] * muF[r];
-                    }
-                    g = thrust_poly_d(c, u[i]) * s;
-                } else {
-                    g = muF[i];
-                }
+                const double g = adj_gu<MODEL>(c, muF, u, i);
                 const double gc = cost ? gc2 * a.r[i] * (u[i] - __ldg(urk + i)) : 0.0;
                 gv[i] = m[i] ? g + gc : 0.0;
                 const double gur = gv[i] - gc;
@@ -907,67 +621,66 @@ __global__ void __launch_bounds__(ADJ_THREADS) closed_loop_adjoint_kernel(const 
                 for (int r = 0; r < NU; ++r) gvmax = fabs(gv[r]) > gvmax ? fabs(gv[r]) : gvmax;
                 bad |= !adj_finite(gvmax * dmax);
             }
-            if (a.gtraj && k > 0 && k % a.stride == 0) {
-                const double* gt = a.gtraj + ((long long)(k / a.stride - 1) * n + v) * NZ;
-#pragma unroll
-                for (int q = 0; q < NX; ++q) lam[q] += gt[q];
-                if constexpr (THR) {
-#pragma unroll
-                    for (int q = 0; q < NL; ++q) mu[q] += gt[NX + q];
-                }
-            }
+            if (a.gtraj && k > 0 && k % a.stride == 0) adj_add_gtraj<MODEL, NZ>(a.gtraj, k / a.stride - 1, n, v, lam, mu);
         }
-#pragma unroll
-        for (int q = 0; q < NX; ++q) {
-            a.gz0[v * NZ + q] = lam[q];
-            bad |= !adj_finite(lam[q]);
-        }
-        if constexpr (THR) {
-#pragma unroll
-            for (int q = 0; q < NL; ++q) {
-                a.gz0[v * NZ + NX + q] = mu[q];
-                bad |= !adj_finite(mu[q]);
-            }
-        }
+        adj_store_gz0<MODEL>(a.gz0, v, lam, mu, bad);
     }
-    if (a.health) {
-        const int nb = __syncthreads_count(bad);
-        const int ns = __syncthreads_count(sing);
-        if (tid == 0) {
-            if (nb) atomicAdd(a.health + 0, (unsigned long long)nb);
-            if (ns) atomicAdd(a.health + 1, (unsigned long long)ns);
-        }
-    }
+    adj_health(a.health, bad, sing);
 }
 
-template <int MODEL, int INTEG, bool PV>
-static cudaError_t closed_loop_adjoint_go(const ClAdjArgs& a, cudaStream_t st) {
-    constexpr int KN = LinDim<MODEL>::NU * LinDim<MODEL>::NZ;
-    auto kern = closed_loop_adjoint_kernel<MODEL, INTEG, PV>;
-    const size_t smem = (size_t)(adjoint_coef_stage_rows(MODEL, INTEG) + (PV ? KP_COUNT : 0)) * ADJ_THREADS * sizeof(double) +
-                        (a.k_smem ? (size_t)KN * sizeof(double) : 0);
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    const long long grid = (a.n + ADJ_THREADS - 1) / ADJ_THREADS;
+// ---- the launches: one model x integrator (x PV) ladder
+
+template <int V> using AdjInt = std::integral_constant<int, V>;
+template <bool V> using AdjBool = std::integral_constant<bool, V>;
+
+// go(model, integ, pv) with compile-time tags; PV only where pv is set
+template <class Go>
+static cudaError_t adj_dispatch(int model, int integ, bool pv, Go go) {
+    auto by_integ = [&](auto m) -> cudaError_t {
+        if (integ == INTEG_RK4) return pv ? go(m, AdjInt<INTEG_RK4>(), AdjBool<true>()) : go(m, AdjInt<INTEG_RK4>(), AdjBool<false>());
+        return pv ? go(m, AdjInt<INTEG_EULER>(), AdjBool<true>()) : go(m, AdjInt<INTEG_EULER>(), AdjBool<false>());
+    };
+    switch (model) {
+        case MODEL_THRUSTER8: return by_integ(AdjInt<MODEL_THRUSTER8>());
+        case MODEL_WRENCH12: return by_integ(AdjInt<MODEL_WRENCH12>());
+        case MODEL_QUAT13: return by_integ(AdjInt<MODEL_QUAT13>());
+    }
+    return cudaErrorInvalidValue;
+}
+
+// one thread per vehicle in blocks of ADJ_THREADS, with smem bytes of dynamic shared memory
+template <class Args>
+static cudaError_t adj_launch(void (*kern)(Args), size_t smem, long long n, const Args& a, cudaStream_t st) {
+    if (smem) {
+        const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    const long long grid = (n + ADJ_THREADS - 1) / ADJ_THREADS;
     kern<<<(unsigned)grid, ADJ_THREADS, smem, st>>>(a);
     return cudaGetLastError();
 }
 
-template <int MODEL>
-static cudaError_t closed_loop_adjoint_integ(int integ, const ClAdjArgs& a, cudaStream_t st) {
-    const bool pv = a.pv != nullptr;
-    if (integ == INTEG_RK4)
-        return pv ? closed_loop_adjoint_go<MODEL, INTEG_RK4, true>(a, st) : closed_loop_adjoint_go<MODEL, INTEG_RK4, false>(a, st);
-    return pv ? closed_loop_adjoint_go<MODEL, INTEG_EULER, true>(a, st) : closed_loop_adjoint_go<MODEL, INTEG_EULER, false>(a, st);
+cudaError_t launch_adjoint(int model, int integ, const AdjArgs& a, cudaStream_t st) {
+    return adj_dispatch(model, integ, false, [&](auto m, auto i, auto) {
+        return adj_launch(adjoint_kernel<decltype(m)::value, decltype(i)::value>, 0, a.n, a, st);
+    });
+}
+
+cudaError_t launch_adjoint_coef(int model, int integ, const AdjCoefArgs& a, cudaStream_t st) {
+    return adj_dispatch(model, integ, a.pv != nullptr, [&](auto m, auto i, auto pv) {
+        constexpr int M = decltype(m)::value, I = decltype(i)::value;
+        constexpr bool PV = decltype(pv)::value;
+        return adj_launch(adjoint_coef_kernel<M, I, PV>, adj_smem_bytes(M, I, ADJ_NKPG + (PV ? KP_COUNT : 0), 0), a.a.n, a, st);
+    });
 }
 
 cudaError_t launch_closed_loop_adjoint(int model, int integ, const ClAdjArgs& a, cudaStream_t st) {
-    switch (model) {
-        case MODEL_THRUSTER8: return closed_loop_adjoint_integ<MODEL_THRUSTER8>(integ, a, st);
-        case MODEL_WRENCH12: return closed_loop_adjoint_integ<MODEL_WRENCH12>(integ, a, st);
-        case MODEL_QUAT13: return closed_loop_adjoint_integ<MODEL_QUAT13>(integ, a, st);
-    }
-    return cudaErrorInvalidValue;
+    return adj_dispatch(model, integ, a.pv != nullptr, [&](auto m, auto i, auto pv) {
+        constexpr int M = decltype(m)::value, I = decltype(i)::value;
+        constexpr bool PV = decltype(pv)::value;
+        const size_t k_bytes = a.k_smem ? (size_t)LinDim<M>::NU * LinDim<M>::NZ * sizeof(double) : 0;
+        return adj_launch(closed_loop_adjoint_kernel<M, I, PV>, adj_smem_bytes(M, I, PV ? KP_COUNT : 0, k_bytes), a.n, a, st);
+    });
 }
 
 // ---- the operand gradients: per (step k, vehicle i) Y rows of R values; value r of row y is element elem(y, r)

@@ -45,15 +45,6 @@ struct AdjCoefArgs {
     const double* pv;             // the per-vehicle table [KP_COUNT][n], or nullptr: the shared a.c.kp
 };
 
-// rows of ADJ_THREADS doubles in the dynamic shared memory of adjoint_coef_kernel: the RK4 stage buffer (3 NX), the
-// coefficient cotangent (ADJ_NKPG) and, PV, the staged vehicle table (KP_COUNT)
-__host__ __device__ constexpr int adjoint_coef_stage_rows(int model, int integ) {
-    return integ == INTEG_RK4 ? 3 * (model == MODEL_QUAT13 ? 13 : 12) : 0;
-}
-constexpr size_t adjoint_coef_smem_bytes(int model, int integ, bool pv) {
-    return (size_t)(adjoint_coef_stage_rows(model, integ) + ADJ_NKPG + (pv ? KP_COUNT : 0)) * ADJ_THREADS * sizeof(double);
-}
-
 // adjoint_kernel plus the coefficient cotangent (brov_rollout_vjp_coef): same models, integrators and a as launch_adjoint
 cudaError_t launch_adjoint_coef(int model, int integ, const AdjCoefArgs& a, cudaStream_t st);
 

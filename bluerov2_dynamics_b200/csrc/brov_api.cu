@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstring>
 #include <new>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/brov.h"
@@ -107,6 +108,8 @@ static const double LAG_CC[3] = {0.0, 5.992, 3.317};                            
 
 static int model_nx(int m) { return (m == BROV_WRENCH_QUAT13 || m == BROV_DI_QUAT13_U6) ? 13 : 12; }
 static int model_nu(int m) { return (m == BROV_THRUSTER8_LAG3 || m == BROV_DI_EULER12_U8) ? 8 : 6; }
+// the state z of the linearize, EKF, closed-loop and adjoint calls: x and, thruster8, the 18 projected lag states
+static int model_nz(int m) { return model_nx(m) + (m == BROV_THRUSTER8_LAG3 ? 18 : 0); }
 static bool model_is_di(int m) { return m >= BROV_DI_EULER12_U8 && m <= BROV_DI_QUAT13_U6; }
 static int model_nlag(const brov_engine* e) {
     return e->model == BROV_THRUSTER8_LAG3 ? 24 : (e->use_lag1 ? 6 : 0);
@@ -1241,31 +1244,65 @@ extern "C" int brov_linearize(brov_engine_t* e, const brov_linearize_desc* d, vo
     return BROV_OK;
 }
 
+// The checks brov_closed_loop and brov_closed_loop_vjp share, in this order: integrator, n, steps (min_steps ..
+// 2^30), dt, operand strides, input bounds, the stride of a trajectory buffer or cotangent (`traj`, named traj_what),
+// the rows of the vehicle table and, when n > 0, the state pointers (z0 and `out`, named in out_what) and the
+// operands.  A caller with nothing left to do for n = 0 returns after it.
+template <class Desc>
+static int cl_check(const brov_engine* e, const Desc* d, long long min_steps, bool traj, const char* traj_what,
+                    const void* out, const char* out_what) {
+    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
+    if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
+    if (d->steps < min_steps || d->steps > (1LL << 30))
+        return fail(BROV_EINVAL, "steps = %lld must be %lld .. 2^30", d->steps, min_steps);
+    if (!(d->dt > 0.0) || !std::isfinite(d->dt)) return fail(BROV_EINVAL, "dt must be a positive finite number");
+    if (d->K_stride_t < 0 || d->K_stride_n < 0 || d->z_ref_stride_t < 0 || d->z_ref_stride_n < 0 || d->u_ref_stride_t < 0 ||
+        d->u_ref_stride_n < 0)
+        return fail(BROV_EINVAL, "negative operand stride");
+    for (int r = 0; r < model_nu(e->model); ++r)
+        if (std::isnan(d->u_min[r]) || std::isnan(d->u_max[r]) || d->u_min[r] > d->u_max[r])
+            return fail(BROV_EINVAL, "input bounds of channel %d: u_min = %g, u_max = %g", r, d->u_min[r], d->u_max[r]);
+    if (traj && d->stride < 1) return fail(BROV_EINVAL, "stride must be >= 1 with a %s", traj_what);
+    if (e->pv && e->pv_n != d->n) return fail(BROV_EINVAL, "vehicle table has %lld rows, call has n = %lld", e->pv_n, d->n);
+    if (d->n == 0) return BROV_OK;
+    if (!d->z0_dev || !out) return fail(BROV_EINVAL, "z0 and %s must not be NULL", out_what);
+    if (d->steps > 0 && (!d->K_dev || !d->z_ref_dev || !d->u_ref_dev)) return fail(BROV_EINVAL, "K, z_ref and u_ref must not be NULL");
+    return BROV_OK;
+}
+
+// the operand fields of ClArgs<T> / ClAdjArgs from a closed-loop descriptor: K, z_ref and u_ref with their strides,
+// the shared-memory K, the vehicle table, the bounds, the cost weights (zero past nu / NZ) and eps
+template <class Args, class Desc>
+static void cl_operands(const brov_engine* e, const Desc* d, Args* a) {
+    using T = typename std::remove_const<typename std::remove_pointer<decltype(a->K)>::type>::type;
+    const int nz = model_nz(e->model), nu = model_nu(e->model);
+    a->K = (const T*)d->K_dev; a->K_st = d->K_stride_t; a->K_sn = d->K_stride_n;
+    a->zr = (const T*)d->z_ref_dev; a->zr_st = d->z_ref_stride_t; a->zr_sn = d->z_ref_stride_n;
+    a->ur = (const T*)d->u_ref_dev; a->ur_st = d->u_ref_stride_t; a->ur_sn = d->u_ref_stride_n;
+    a->k_smem = (a->K_st == 0 && a->K_sn == 0) ? 1 : 0;
+    a->pv = (const T*)e->pv;
+    a->eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
+    for (int r = 0; r < 8; ++r) { a->u_min[r] = (T)d->u_min[r]; a->u_max[r] = (T)d->u_max[r]; a->r[r] = r < nu ? (T)d->r[r] : T(0); }
+    for (int j = 0; j < CL_MAX_NZ; ++j) a->q[j] = j < nz ? (T)d->q[j] : T(0);
+}
+
 template <typename T>
 static int closed_loop_impl(brov_engine* e, const brov_closed_loop_desc* d, int nz, int nu, cudaStream_t st) {
     ClArgs<T> a;
     memset(&a, 0, sizeof(a));
     int rc = make_consts<T>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c);
     if (rc) return rc;
+    cl_operands(e, d, &a);
     a.z0 = (const T*)d->z0_dev;
     a.z_out = (T*)d->z_out_dev;
-    a.K = (const T*)d->K_dev; a.K_st = d->K_stride_t; a.K_sn = d->K_stride_n;
-    a.zr = (const T*)d->z_ref_dev; a.zr_st = d->z_ref_stride_t; a.zr_sn = d->z_ref_stride_n;
-    a.ur = (const T*)d->u_ref_dev; a.ur_st = d->u_ref_stride_t; a.ur_sn = d->u_ref_stride_n;
-    a.k_smem = (a.K_st == 0 && a.K_sn == 0) ? 1 : 0;
-    if (a.k_smem) a.K_st = 0;
-    a.pv = (const T*)e->pv;
     a.traj = (T*)d->traj_dev;
     a.u_traj = (T*)d->u_traj_dev;
     a.cost = (T*)d->cost_dev;
     a.cost_accumulate = d->cost_accumulate ? 1 : 0;
     a.health = (unsigned long long*)d->health_dev;
-    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
-    for (int r = 0; r < 8; ++r) { a.u_min[r] = (T)d->u_min[r]; a.u_max[r] = (T)d->u_max[r]; a.r[r] = r < nu ? (T)d->r[r] : T(0); }
-    for (int j = 0; j < CL_MAX_NZ; ++j) a.q[j] = j < nz ? (T)d->q[j] : T(0);
     a.n = d->n;
     a.steps = (int)d->steps;
-    a.stride = (d->traj_dev || d->u_traj_dev) ? (int)d->stride : 0x7fffffff;
+    a.stride = (d->traj_dev || d->u_traj_dev) ? (int)std::min<long long>(d->stride, 0x7fffffffLL) : 0x7fffffff;
     a.traj_vec = d->traj_dev && aligned(d->traj_dev, 16) && ((size_t)d->n * nz * sizeof(T)) % 16 == 0;
     a.u_traj_vec = d->u_traj_dev && aligned(d->u_traj_dev, 16) && ((size_t)d->n * nu * sizeof(T)) % 16 == 0;
     // Threads per block: 128 once that still gives every SM a block, else 64 or 32 — one thread per vehicle leaves
@@ -1282,23 +1319,9 @@ extern "C" int brov_closed_loop(brov_engine_t* e, const brov_closed_loop_desc* d
     if (!d || d->struct_size != sizeof(brov_closed_loop_desc)) return fail(BROV_EINVAL, "brov_closed_loop_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
     if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "closed_loop serves the Fossen models, not double-integrator engines");
     if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "closed_loop does not support the first-order wrench lag");
-    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
-    if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
-    if (d->steps < 0 || d->steps > (1LL << 30)) return fail(BROV_EINVAL, "steps = %lld must be 0 .. 2^30", d->steps);
-    if (!(d->dt > 0.0) || !std::isfinite(d->dt)) return fail(BROV_EINVAL, "dt must be a positive finite number");
-    if (d->K_stride_t < 0 || d->K_stride_n < 0 || d->z_ref_stride_t < 0 || d->z_ref_stride_n < 0 || d->u_ref_stride_t < 0 ||
-        d->u_ref_stride_n < 0)
-        return fail(BROV_EINVAL, "negative operand stride");
-    const bool thr = e->model == BROV_THRUSTER8_LAG3;
-    const int nz = model_nx(e->model) + (thr ? 18 : 0), nu = model_nu(e->model);
-    for (int r = 0; r < nu; ++r)
-        if (std::isnan(d->u_min[r]) || std::isnan(d->u_max[r]) || d->u_min[r] > d->u_max[r])
-            return fail(BROV_EINVAL, "input bounds of channel %d: u_min = %g, u_max = %g", r, d->u_min[r], d->u_max[r]);
-    if ((d->traj_dev || d->u_traj_dev) && d->stride < 1) return fail(BROV_EINVAL, "stride must be >= 1 with a trajectory buffer");
-    if (e->pv && e->pv_n != d->n) return fail(BROV_EINVAL, "vehicle table has %lld rows, call has n = %lld", e->pv_n, d->n);
-    if (d->n == 0) return BROV_OK;
-    if (!d->z0_dev || !d->z_out_dev) return fail(BROV_EINVAL, "z0 and z_out must not be NULL");
-    if (d->steps > 0 && (!d->K_dev || !d->z_ref_dev || !d->u_ref_dev)) return fail(BROV_EINVAL, "K, z_ref and u_ref must not be NULL");
+    int rc = cl_check(e, d, 0, d->traj_dev || d->u_traj_dev, "trajectory buffer", d->z_out_dev, "z_out");
+    if (rc || d->n == 0) return rc;
+    const int nz = model_nz(e->model), nu = model_nu(e->model);
     CUDA_TRY(cudaSetDevice(e->device));
     cudaStream_t st = (cudaStream_t)stream;
     if (d->steps == 0) {
@@ -1349,7 +1372,7 @@ extern "C" int brov_ekf(brov_engine_t* e, const brov_ekf_desc* d, void* stream) 
     if (stats && !(d->loglik_dev && d->nis_dev && d->count_dev)) return fail(BROV_EINVAL, "loglik, nis and count go together");
     if (d->n == 0) return BROV_OK;
     if (!d->z0_dev || !d->P0_dev || !d->z_out_dev || !d->P_out_dev) return fail(BROV_EINVAL, "z0, P0, z_out and P_out must not be NULL");
-    const int nx = model_nx(e->model), nz = nx + (e->model == BROV_THRUSTER8_LAG3 ? 18 : 0);
+    const int nx = model_nx(e->model), nz = model_nz(e->model);
     CUDA_TRY(cudaSetDevice(e->device));
     cudaStream_t st = (cudaStream_t)stream;
     if (d->steps == 0) {
@@ -1398,8 +1421,7 @@ extern "C" int brov_ekf(brov_engine_t* e, const brov_ekf_desc* d, void* stream) 
 
 extern "C" size_t brov_rollout_vjp_workspace_bytes(int model, long long n, long long steps) {
     if (model != BROV_THRUSTER8_LAG3 && model != BROV_WRENCH_EULER12 && model != BROV_WRENCH_QUAT13) return 0;
-    const int nz = model_nx(model) + (model == BROV_THRUSTER8_LAG3 ? 18 : 0);
-    return adjoint_workspace_bytes(nz, n, steps);
+    return adjoint_workspace_bytes(model_nz(model), n, steps);
 }
 
 // the argument checks of brov_rollout_vjp / brov_rollout_vjp_coef in order, then (n > 0) the kernel arguments a and the
@@ -1437,17 +1459,21 @@ static int rollout_vjp_args(brov_engine_t* e, const brov_rollout_vjp_desc* d, Ad
     return BROV_OK;
 }
 
-static int rollout_vjp_common(brov_engine_t* e, const brov_rollout_vjp_desc* d) {
+// The refusals every fp64 gradient call starts with, in this order: no engine, a descriptor of the wrong size
+// (bad_desc names it; nullptr when the sizes match), a double-integrator engine, an f32 engine, the first-order wrench
+// lag.  `what` names the call in the messages.
+static int grad_prologue(const brov_engine_t* e, const char* bad_desc, const char* what) {
     if (!e) return fail(BROV_EINVAL, "NULL engine");
-    if (!d || d->struct_size != sizeof(brov_rollout_vjp_desc)) return fail(BROV_EINVAL, "brov_rollout_vjp_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
-    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "rollout_vjp serves the Fossen models, not double-integrator engines");
+    if (bad_desc) return fail(BROV_EINVAL, "%s size mismatch (ABI %d)", bad_desc, BROV_ABI_VERSION);
+    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "%s serves the Fossen models, not double-integrator engines", what);
     if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the gradients are computed in fp64: create the engine with BROV_F64");
-    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "rollout_vjp does not support the first-order wrench lag");
+    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "%s does not support the first-order wrench lag", what);
     return BROV_OK;
 }
 
 extern "C" int brov_rollout_vjp(brov_engine_t* e, const brov_rollout_vjp_desc* d, void* stream) {
-    int rc = rollout_vjp_common(e, d);
+    int rc = grad_prologue(e, !d || d->struct_size != sizeof(brov_rollout_vjp_desc) ? "brov_rollout_vjp_desc" : nullptr,
+                           "rollout_vjp");
     if (rc) return rc;
     if (e->pv) return fail(BROV_EUNSUPPORTED, "rollout_vjp uses the shared coefficients: clear the per-vehicle table first");
     AdjArgs a;
@@ -1459,9 +1485,9 @@ extern "C" int brov_rollout_vjp(brov_engine_t* e, const brov_rollout_vjp_desc* d
 }
 
 extern "C" int brov_rollout_vjp_coef(brov_engine_t* e, const brov_rollout_vjp_coef_desc* d, void* stream) {
-    if (!e) return fail(BROV_EINVAL, "NULL engine");
-    if (!d || d->struct_size != sizeof(brov_rollout_vjp_coef_desc)) return fail(BROV_EINVAL, "brov_rollout_vjp_coef_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
-    int rc = rollout_vjp_common(e, &d->vjp);
+    const char* bad_desc = !d || d->struct_size != sizeof(brov_rollout_vjp_coef_desc) ? "brov_rollout_vjp_coef_desc"
+                           : d->vjp.struct_size != sizeof(brov_rollout_vjp_desc) ? "brov_rollout_vjp_desc" : nullptr;
+    int rc = grad_prologue(e, bad_desc, "rollout_vjp");
     if (rc) return rc;
     if (e->pv && e->pv_n != d->vjp.n) return fail(BROV_EINVAL, "vehicle table has %lld rows, call has n = %lld", e->pv_n, d->vjp.n);
     if (d->vjp.n != 0 && !d->gkp_dev) return fail(BROV_EINVAL, "gkp must not be NULL");
@@ -1477,8 +1503,7 @@ extern "C" int brov_rollout_vjp_coef(brov_engine_t* e, const brov_rollout_vjp_co
 
 extern "C" size_t brov_closed_loop_vjp_workspace_bytes(int model, long long n, long long steps) {
     if (model != BROV_THRUSTER8_LAG3 && model != BROV_WRENCH_EULER12 && model != BROV_WRENCH_QUAT13) return 0;
-    const int nz = model_nx(model) + (model == BROV_THRUSTER8_LAG3 ? 18 : 0);
-    return cl_adjoint_workspace_bytes(nz, model_nu(model), n, steps);
+    return cl_adjoint_workspace_bytes(model_nz(model), model_nu(model), n, steps);
 }
 
 // no two (step, vehicle) pairs of an operand of E elements addressed at k*st + i*sn + e share an element unless a
@@ -1493,28 +1518,12 @@ static bool cl_strides_disjoint(long long st, long long sn, long long steps, lon
 }
 
 extern "C" int brov_closed_loop_vjp(brov_engine_t* e, const brov_closed_loop_vjp_desc* d, void* stream) {
-    if (!e) return fail(BROV_EINVAL, "NULL engine");
-    if (!d || d->struct_size != sizeof(brov_closed_loop_vjp_desc)) return fail(BROV_EINVAL, "brov_closed_loop_vjp_desc size mismatch (ABI %d)", BROV_ABI_VERSION);
-    if (model_is_di(e->model)) return fail(BROV_EUNSUPPORTED, "closed_loop_vjp serves the Fossen models, not double-integrator engines");
-    if (e->dtype != BROV_F64) return fail(BROV_EUNSUPPORTED, "the gradients are computed in fp64: create the engine with BROV_F64");
-    if (e->use_lag1) return fail(BROV_EUNSUPPORTED, "closed_loop_vjp does not support the first-order wrench lag");
-    if (d->integrator != BROV_RK4 && d->integrator != BROV_EULER) return fail(BROV_EINVAL, "unknown integrator %d", d->integrator);
-    if (d->n < 0 || d->n > 0x7fffffffLL) return fail(BROV_EINVAL, "n = %lld out of range", d->n);
-    if (d->steps < 1 || d->steps > (1LL << 30)) return fail(BROV_EINVAL, "steps = %lld must be 1 .. 2^30", d->steps);
-    if (!(d->dt > 0.0) || !std::isfinite(d->dt)) return fail(BROV_EINVAL, "dt must be a positive finite number");
-    if (d->K_stride_t < 0 || d->K_stride_n < 0 || d->z_ref_stride_t < 0 || d->z_ref_stride_n < 0 || d->u_ref_stride_t < 0 ||
-        d->u_ref_stride_n < 0)
-        return fail(BROV_EINVAL, "negative operand stride");
-    const bool thr = e->model == BROV_THRUSTER8_LAG3;
-    const int nz = model_nx(e->model) + (thr ? 18 : 0), nu = model_nu(e->model);
-    for (int r = 0; r < nu; ++r)
-        if (std::isnan(d->u_min[r]) || std::isnan(d->u_max[r]) || d->u_min[r] > d->u_max[r])
-            return fail(BROV_EINVAL, "input bounds of channel %d: u_min = %g, u_max = %g", r, d->u_min[r], d->u_max[r]);
-    if (d->gtraj_dev && d->stride < 1) return fail(BROV_EINVAL, "stride must be >= 1 with a trajectory cotangent");
-    if (e->pv && e->pv_n != d->n) return fail(BROV_EINVAL, "vehicle table has %lld rows, call has n = %lld", e->pv_n, d->n);
-    if (d->n == 0) return BROV_OK;
-    if (!d->z0_dev || !d->gz0_dev) return fail(BROV_EINVAL, "z0 and gz0 must not be NULL");
-    if (!d->K_dev || !d->z_ref_dev || !d->u_ref_dev) return fail(BROV_EINVAL, "K, z_ref and u_ref must not be NULL");
+    int rc = grad_prologue(e, !d || d->struct_size != sizeof(brov_closed_loop_vjp_desc) ? "brov_closed_loop_vjp_desc" : nullptr,
+                           "closed_loop_vjp");
+    if (rc) return rc;
+    rc = cl_check(e, d, 1, d->gtraj_dev != nullptr, "trajectory cotangent", d->gz0_dev, "gz0");
+    if (rc || d->n == 0) return rc;
+    const int nz = model_nz(e->model), nu = model_nu(e->model);
     struct Op { void* g; long long st, sn; int E; const char* what; } ops[3] = {
         {d->gK_dev, d->K_stride_t, d->K_stride_n, nu * nz, "K"},
         {d->gz_ref_dev, d->z_ref_stride_t, d->z_ref_stride_n, nz, "z_ref"},
@@ -1533,14 +1542,9 @@ extern "C" int brov_closed_loop_vjp(brov_engine_t* e, const brov_closed_loop_vjp
 
     ClAdjArgs a;
     memset(&a, 0, sizeof(a));
-    int rc = make_consts<double>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c);
-    if (rc) return rc;
+    if ((rc = make_consts<double>(e, d->dt, d->integrator == BROV_RK4 ? 4 : 1, &a.c))) return rc;
+    cl_operands(e, d, &a);
     a.z0 = (const double*)d->z0_dev;
-    a.K = (const double*)d->K_dev; a.K_st = d->K_stride_t; a.K_sn = d->K_stride_n;
-    a.zr = (const double*)d->z_ref_dev; a.zr_st = d->z_ref_stride_t; a.zr_sn = d->z_ref_stride_n;
-    a.ur = (const double*)d->u_ref_dev; a.ur_st = d->u_ref_stride_t; a.ur_sn = d->u_ref_stride_n;
-    a.k_smem = (a.K_st == 0 && a.K_sn == 0) ? 1 : 0;
-    a.pv = (const double*)e->pv;
     a.gtraj = (const double*)d->gtraj_dev;
     a.gzT = (const double*)d->gzT_dev;
     a.gcost = (const double*)d->gcost_dev;
@@ -1554,9 +1558,6 @@ extern "C" int brov_closed_loop_vjp(brov_engine_t* e, const brov_closed_loop_vjp
     if (d->gu_ref_dev) { a.wgur = w; w += slab * nu; }
     double* scratch = w;
     a.health = (unsigned long long*)d->health_dev;
-    a.eps = d->singular_eps > 0.0 ? d->singular_eps : 1e-3;
-    for (int r = 0; r < 8; ++r) { a.u_min[r] = d->u_min[r]; a.u_max[r] = d->u_max[r]; a.r[r] = r < nu ? d->r[r] : 0.0; }
-    for (int j = 0; j < CL_MAX_NZ; ++j) a.q[j] = j < nz ? d->q[j] : 0.0;
     a.n = d->n;
     a.steps = (int)d->steps;
     a.stride = d->gtraj_dev ? (int)std::min<long long>(d->stride, 0x7fffffffLL) : 1;

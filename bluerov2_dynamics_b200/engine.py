@@ -984,18 +984,8 @@ class Engine:
                 steps, st, sn = Ut.shape[0], self.nu, 0
             else:
                 raise ValueError("u_layout must be auto|tnc|shared|const")
-        if lag_repr not in ("thruster", "projected"):
-            raise ValueError("lag_repr must be 'thruster' or 'projected'")
+        z0 = self._z0(x0, lag0, lag_repr, n)
         nz, nc = self.nz, self.nz + self.nu
-        z0 = x0
-        if self.model == "thruster8":
-            if lag0 is None:
-                Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
-            elif lag_repr == "thruster":
-                Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
-            else:
-                Z0 = self.tensor(lag0).reshape(n, 18)
-            z0 = torch.cat([x0, Z0], dim=1).contiguous()
         shape = (steps, n, nz, nc)
         if jac_out is not None:
             if (not isinstance(jac_out, torch.Tensor) or jac_out.device != self.device or jac_out.dtype != torch.float64
@@ -1021,6 +1011,59 @@ class Engine:
         with torch.cuda.device(self.device):
             L.check(L.lib.brov_linearize(self._h, C.byref(d), self._stream()))
         return LinearizeResult(A=J[..., :nz], B=J[..., nz:], z=z, z_traj=zt, health=hc)
+
+    def _z0(self, x0, lag0, lag_repr: str, n: int):
+        """z_0 = [x0 | Z0] of the linearize / adjoint / closed-loop / EKF calls: the thruster model's lag0 per thruster
+        [N,24] (lag_repr="thruster", projected here) or projected [N,18] ("projected"), None = zeros; x0 otherwise"""
+        if lag_repr not in ("thruster", "projected"):
+            raise ValueError("lag_repr must be 'thruster' or 'projected'")
+        if self.model != "thruster8":
+            return x0
+        if lag0 is None:
+            Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
+        elif lag_repr == "thruster":
+            Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
+        else:
+            Z0 = self.tensor(lag0).reshape(n, 18)
+        return torch.cat([x0, Z0], dim=1).contiguous()
+
+    def _glag0(self, gz0, lag_repr: str, n: int):
+        """the lag part of dL/dz_0 in the representation lag0 came in: per thruster P^T gZ0 (Z = P L), or gZ0 itself;
+        None for the wrench models"""
+        if self.model != "thruster8":
+            return None
+        gZ0 = gz0[:, self.nx:]
+        if lag_repr == "thruster":
+            A = self.tensor(self._alloc)
+            return torch.einsum("ci,nck->nik", A, gZ0.reshape(n, 6, 3)).reshape(n, 24).contiguous()
+        return gZ0
+
+    def _cotangents(self, gtraj, gzT, steps: int, stride: int, n: int, width: int):
+        """the trajectory cotangent gtraj [T//stride, N, width] and the terminal one gzT [N, NZ] as tensors (or None),
+        their shapes checked"""
+        gt = None
+        if gtraj is not None:
+            gt = self.tensor(gtraj)
+            ns = steps // int(stride) if int(stride) >= 1 else None
+            if ns is not None and tuple(gt.shape) != (ns, n, width):
+                raise ValueError(f"gtraj must have shape [{ns}, {n}, {width}], got {tuple(gt.shape)}")
+        gT = None
+        if gzT is not None:
+            gT = self.tensor(gzT)
+            if tuple(gT.shape) != (n, self.nz):
+                raise ValueError(f"gzT must have shape [{n}, {self.nz}], got {tuple(gT.shape)}")
+        return gt, gT
+
+    def _cost_weights(self, d, cost_q, cost_r):
+        """the closed-loop cost weights cost_q [NZ] / cost_r [NU] (scalars broadcast; None leaves them zero) into d.q / d.r"""
+        if cost_q is not None:
+            q = np.broadcast_to(np.asarray(cost_q, float), (self.nz,))
+            for j in range(self.nz):
+                d.q[j] = float(q[j])
+        if cost_r is not None:
+            rw = np.broadcast_to(np.asarray(cost_r, float), (self.nu,))
+            for r in range(self.nu):
+                d.r[r] = float(rw[r])
 
     def _inputs(self, U, n: int, u_layout: str):
         """(tensor, steps, stride_t, stride_n) of a rollout input U in the layouts of `rollout`"""
@@ -1066,30 +1109,9 @@ class Engine:
         self._check_rows(x0, self.nx, "x0")
         n = x0.shape[0]
         Ut, steps, st, sn = self._inputs(U, n, u_layout)
-        if lag_repr not in ("thruster", "projected"):
-            raise ValueError("lag_repr must be 'thruster' or 'projected'")
+        z0 = self._z0(x0, lag0, lag_repr, n)
         nz = self.nz
-        thr = self.model == "thruster8"
-        z0 = x0
-        if thr:
-            if lag0 is None:
-                Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
-            elif lag_repr == "thruster":
-                Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
-            else:
-                Z0 = self.tensor(lag0).reshape(n, 18)
-            z0 = torch.cat([x0, Z0], dim=1).contiguous()
-        gt = None
-        if gtraj is not None:
-            gt = self.tensor(gtraj)
-            ns = steps // int(stride) if int(stride) >= 1 else None
-            if ns is not None and tuple(gt.shape) != (ns, n, self.nx):
-                raise ValueError(f"gtraj must have shape [{ns}, {n}, {self.nx}], got {tuple(gt.shape)}")
-        gT = None
-        if gzT is not None:
-            gT = self.tensor(gzT)
-            if tuple(gT.shape) != (n, nz):
-                raise ValueError(f"gzT must have shape [{n}, {nz}], got {tuple(gT.shape)}")
+        gt, gT = self._cotangents(gtraj, gzT, steps, stride, n, self.nx)
         gz0 = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
         gU = torch.empty((steps, n, self.nu), device=self.device, dtype=self.tdtype)
         z = torch.empty((n, nz), device=self.device, dtype=self.tdtype)
@@ -1122,16 +1144,7 @@ class Engine:
                 gkp = gkp.t()
             else:
                 L.check(L.lib.brov_rollout_vjp(self._h, C.byref(d), self._stream()))
-        gx0 = gz0[:, :self.nx]
-        glag0 = None
-        if thr:
-            gZ0 = gz0[:, self.nx:]
-            if lag_repr == "thruster":
-                A = self.tensor(self._alloc)
-                glag0 = torch.einsum("ci,nck->nik", A, gZ0.reshape(n, 6, 3)).reshape(n, 24).contiguous()
-            else:
-                glag0 = gZ0
-        return VjpResult(gx0=gx0, glag0=glag0, gU=gU, z=z, health=hc, gkp=gkp)
+        return VjpResult(gx0=gz0[:, :self.nx], glag0=self._glag0(gz0, lag_repr, n), gU=gU, z=z, health=hc, gkp=gkp)
 
     def rollout_diff(self, x0: torch.Tensor, U: torch.Tensor, lag0: Optional[torch.Tensor] = None, dt: float = 0.02,
                      integrator: str = "rk4", stride: int = 1, lag_repr: str = "projected",
@@ -1196,17 +1209,7 @@ class Engine:
             raise ValueError("the time-varying operands disagree on T" if Ts else
                              "no operand is time-varying: give steps=")
         steps = Ts.pop()
-        if lag_repr not in ("thruster", "projected"):
-            raise ValueError("lag_repr must be 'thruster' or 'projected'")
-        z0 = x0
-        if self.model == "thruster8":
-            if lag0 is None:
-                Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
-            elif lag_repr == "thruster":
-                Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
-            else:
-                Z0 = self.tensor(lag0).reshape(n, 18)
-            z0 = torch.cat([x0, Z0], dim=1).contiguous()
+        z0 = self._z0(x0, lag0, lag_repr, n)
         lim = 1.0 if self.model == "thruster8" else np.inf
         lo = np.broadcast_to(np.asarray(-lim if u_min is None else u_min, float), (nu,))
         hi = np.broadcast_to(np.asarray(lim if u_max is None else u_max, float), (nu,))
@@ -1267,14 +1270,7 @@ class Engine:
         d.u_ref_dev, d.u_ref_stride_t, d.u_ref_stride_n = ur.data_ptr(), ust, usn
         for r in range(nu):
             d.u_min[r], d.u_max[r] = float(lo[r]), float(hi[r])
-        if cost_q is not None:
-            q = np.broadcast_to(np.asarray(cost_q, float), (nz,))
-            for j in range(nz):
-                d.q[j] = float(q[j])
-        if cost_r is not None:
-            rw = np.broadcast_to(np.asarray(cost_r, float), (nu,))
-            for r in range(nu):
-                d.r[r] = float(rw[r])
+        self._cost_weights(d, cost_q, cost_r)
         d.traj_dev = zt.data_ptr() if zt is not None and zt.numel() else None
         d.u_traj_dev = ut.data_ptr() if ut is not None and ut.numel() else None
         d.stride = int(stride)
@@ -1311,17 +1307,7 @@ class Engine:
         n, steps, z0, (Kt, kst, ksn), (zr, zst, zsn), (ur, ust, usn), lo, hi = self._cl_setup(
             x0, K, z_ref, u_ref, steps, lag0, lag_repr, k_layout, ref_layout, u_min, u_max)
         nz, nu = self.nz, self.nu
-        gt = None
-        if gtraj is not None:
-            gt = self.tensor(gtraj)
-            ns = steps // int(stride) if int(stride) >= 1 else None
-            if ns is not None and tuple(gt.shape) != (ns, n, nz):
-                raise ValueError(f"gtraj must have shape [{ns}, {n}, {nz}], got {tuple(gt.shape)}")
-        gT = None
-        if gzT is not None:
-            gT = self.tensor(gzT)
-            if tuple(gT.shape) != (n, nz):
-                raise ValueError(f"gzT must have shape [{n}, {nz}], got {tuple(gT.shape)}")
+        gt, gT = self._cotangents(gtraj, gzT, steps, stride, n, nz)
         gc = None
         if gcost is not None:
             gc = torch.as_tensor(gcost, dtype=self.tdtype, device=self.device)
@@ -1348,14 +1334,7 @@ class Engine:
         d.u_ref_dev, d.u_ref_stride_t, d.u_ref_stride_n = ur.data_ptr(), ust, usn
         for r in range(nu):
             d.u_min[r], d.u_max[r] = float(lo[r]), float(hi[r])
-        if cost_q is not None:
-            q = np.broadcast_to(np.asarray(cost_q, float), (nz,))
-            for j in range(nz):
-                d.q[j] = float(q[j])
-        if cost_r is not None:
-            rw = np.broadcast_to(np.asarray(cost_r, float), (nu,))
-            for r in range(nu):
-                d.r[r] = float(rw[r])
+        self._cost_weights(d, cost_q, cost_r)
         # an empty gtraj (stride > T: no snapshot) is no trajectory term
         d.gtraj_dev = gt.data_ptr() if (gt is not None and gt.numel()) else None
         d.stride = int(stride)
@@ -1370,16 +1349,7 @@ class Engine:
         d.singular_eps = float(singular_eps)
         with torch.cuda.device(self.device):
             L.check(L.lib.brov_closed_loop_vjp(self._h, C.byref(d), self._stream()))
-        gx0 = gz0[:, :self.nx]
-        glag0 = None
-        if self.model == "thruster8":
-            gZ0 = gz0[:, self.nx:]
-            if lag_repr == "thruster":
-                A = self.tensor(self._alloc)
-                glag0 = torch.einsum("ci,nck->nik", A, gZ0.reshape(n, 6, 3)).reshape(n, 24).contiguous()
-            else:
-                glag0 = gZ0
-        return ClosedLoopVjpResult(gx0=gx0, glag0=glag0, gK=outs["K"], gz_ref=outs["z_ref"], gu_ref=outs["u_ref"],
+        return ClosedLoopVjpResult(gx0=gz0[:, :self.nx], glag0=self._glag0(gz0, lag_repr, n), gK=outs["K"], gz_ref=outs["z_ref"], gu_ref=outs["u_ref"],
                                    z=z, health=hc)
 
     def closed_loop_diff(self, x0: torch.Tensor, K: torch.Tensor, z_ref: torch.Tensor, u_ref: torch.Tensor,
@@ -1479,17 +1449,7 @@ class Engine:
             raise ValueError(f"P0 must have shape [{nx}, {nx}], [{n}, {nx}, {nx}], [{nx}] or [{n}, {nx}], "
                              f"got {tuple(P0t.shape)}")
         P0t = P0t.contiguous()
-        if lag_repr not in ("thruster", "projected"):
-            raise ValueError("lag_repr must be 'thruster' or 'projected'")
-        z0 = x0
-        if self.model == "thruster8":
-            if lag0 is None:
-                Z0 = torch.zeros((n, 18), device=self.device, dtype=self.tdtype)
-            elif lag_repr == "thruster":
-                Z0 = self.project_lag(self.tensor(lag0).reshape(n, 24))
-            else:
-                Z0 = self.tensor(lag0).reshape(n, 18)
-            z0 = torch.cat([x0, Z0], dim=1).contiguous()
+        z0 = self._z0(x0, lag0, lag_repr, n)
         if stats is None:
             if stats_accumulate:
                 raise ValueError("stats_accumulate needs stats=(loglik, nis, count)")

@@ -399,6 +399,30 @@ def test_unsupported_and_invalid_calls(B, L):
         e.closed_loop(x, K[:, :12], zs, us, steps=5)
 
 
+def test_stride_beyond_int_range_takes_no_snapshot(B, L):
+    # a 64-bit stride past INT_MAX is a snapshot interval longer than any call: 3 steps take none, and the trajectory
+    # buffer (sized here for 3 snapshots) stays as it was
+    zs, us, K, *_ = _lqr("thruster8", "rk4", False)
+    e = B.Engine("thruster8", "f64")
+    n, steps = 4, 3
+    z = e.tensor(np.tile(zs, (n, 1)))
+    zo = torch.empty_like(z)
+    Kt, zr, ur = e.tensor(K), e.tensor(zs), e.tensor(us)
+    traj = torch.full((steps, n, e.nz), float("nan"), device="cuda", dtype=torch.float64)
+    d = L.ClosedLoopDesc()
+    d.struct_size = C.sizeof(L.ClosedLoopDesc)
+    d.n, d.steps, d.dt = n, steps, DT
+    d.z0_dev, d.z_out_dev = z.data_ptr(), zo.data_ptr()
+    d.K_dev, d.z_ref_dev, d.u_ref_dev = Kt.data_ptr(), zr.data_ptr(), ur.data_ptr()
+    for r in range(8):
+        d.u_min[r], d.u_max[r] = -1.0, 1.0
+    d.traj_dev, d.stride = traj.data_ptr(), 2 ** 32 + 1
+    assert L.lib.brov_closed_loop(e._h, C.byref(d), None) == 0
+    torch.cuda.synchronize()
+    assert torch.isnan(traj).all()
+    assert torch.isfinite(zo).all()
+
+
 def test_full_size_per_vehicle_gains_above_2_31_elements(B):
     e = _engine(B, "thruster8")
     zs, us, K, *_ = _lqr("thruster8", "rk4", False)
